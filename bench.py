@@ -30,6 +30,9 @@ Rank 0 prints ONE JSON line:
                persistent process pool over all host cores, median of passes; also a call-by-call parity check
 
 `--impl reference` times only that CPU path (rank 0 alone when launched under torchrun).
+
+`--dump-outputs DIR` writes the call records of the last timed step (rank 0) as DIR/<field>.npy, so that two builds
+can be compared output for output: the cohort is seeded, so the same arguments give the same inputs.
 """
 import argparse
 import hashlib
@@ -37,6 +40,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -44,6 +48,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the source tree may be read-only: nothing is written there
 
 METRIC = "loci genotyped/sec"
 UNIT = "loci/s"
@@ -73,7 +78,13 @@ def parse_args():
     p.add_argument("--impl", default="tredsw", choices=("tredsw", "reference"))
     p.add_argument("--cpu-sample", type=int, default=0, help="samples in the CPU baseline sample (0 = auto)")
     p.add_argument("--no-cpu-baseline", action="store_true")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the call records of the last "
+                   "timed step of rank 0 as DIR/<field>.npy (float64; ci is n x 4) and DIR/problem.npy (cohort index "
+                   "sample x loci + locus of every row); above 64 MB in all, a fixed seeded sample of the rows")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    return args
 
 
 def distinct_loci(repo):
@@ -233,17 +244,31 @@ def _write_bam(job):
     return path
 
 
-def make_bams(nsamples, workers):
-    """Synthetic whole-sample BAMs of the first `nsamples` cohort samples (written once per box under /tmp)."""
+def make_bams(nsamples, workers, d):
+    """Synthetic whole-sample BAMs of the first `nsamples` cohort samples, written into the directory `d`."""
     import multiprocessing as mp
-    d = os.path.join("/tmp", "tredsw_bench_bams")
-    os.makedirs(d, exist_ok=True)
     jobs = [(os.path.join(d, "s{:04d}.bam".format(s)), s) for s in range(nsamples)]
-    todo = [j for j in jobs if not (os.path.exists(j[0]) and os.path.exists(j[0] + ".bai"))]
-    if todo:
-        with mp.get_context("fork").Pool(processes=max(1, min(workers, len(todo)))) as pool:
-            pool.map(_write_bam, todo, chunksize=1)
+    with mp.get_context("fork").Pool(processes=max(1, min(workers, len(jobs)))) as pool:
+        pool.map(_write_bam, jobs, chunksize=1)
     return [j[0] for j in jobs]
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(d, calls, problem):
+    """--dump-outputs: one float64 .npy per CALL_DTYPE field plus problem.npy.  When the rows exceed DUMP_BYTES, the
+    same seeded sample of rows (kept in order) is written on every run."""
+    cols = {name: calls[name] for name in calls.dtype.names}
+    cols["problem"] = problem
+    row_bytes = 8 * sum(int(np.prod(c.shape[1:])) for c in cols.values())
+    limit = (DUMP_BYTES - 1024 * len(cols)) // row_bytes            # (1 KB per file for the .npy header)
+    rows = np.arange(len(calls))
+    if len(rows) > limit:
+        rows = np.sort(np.random.default_rng(0).choice(len(rows), limit, replace=False))
+    os.makedirs(d, exist_ok=True)
+    for name, c in cols.items():
+        np.save(os.path.join(d, name + ".npy"), np.ascontiguousarray(c[rows], dtype=np.float64))
 
 
 def _ref_run_bam(job):
@@ -509,10 +534,11 @@ def _main(args):
     workers = max(1, min(16, (os.cpu_count() or 1) // max(1, min(world, 8))))
     arrays = build_batches(chunks, workers)
     t_gen = time.perf_counter() - t_gen
-    bams = []
+    bams, bam_dir = [], None
     if rank == 0 and world == 1 and args.from_bam > 0:
         t_b = time.perf_counter()
-        bams = make_bams(args.from_bam, workers)
+        bam_dir = tempfile.TemporaryDirectory(prefix="tredsw_bench_bams-")
+        bams = make_bams(args.from_bam, workers, bam_dir.name)
         t_bams = time.perf_counter() - t_b
     # the CPU baseline's process pool is forked here, before CUDA / NCCL exist in this process (rank 0, N = 1 only)
     ref_pool, ref_pool_error = None, "not requested"
@@ -666,6 +692,9 @@ def _main(args):
     assert local_calls.tobytes() == calls_dev.tobytes(), "device-resident and host paths disagree"
     if rank == 0:
         assert gathered is not None and int(seen.sum()) == sum(timed_counts)
+        if args.dump_outputs:
+            n = timed[-1].nproblems
+            dump_outputs(args.dump_outputs, calls_dev[len(calls_dev) - n:], timed_idx[len(timed_idx) - n:])
 
     # ---- reduce over ranks: timings MAX, unit counters SUM (no data-path collective anywhere) --------
     nprob_timed = sum(b.nproblems for b in timed)
@@ -844,6 +873,7 @@ def _main(args):
                 line["from_bam"] = fb
             except Exception as e:
                 line["from_bam"] = {"error": repr(e)}
+            bam_dir.cleanup()
         if ref_pool is not None:
             ref_pool.close()
         emit(line)

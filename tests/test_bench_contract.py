@@ -42,6 +42,30 @@ def test_own_arm_line(name):
         assert s["bound"] == "hbm" and s["points"] == 32032000 and 0 < s["frac"] < 1
 
 
+def test_dump_outputs_layout_and_seeded_sample(tmp_path, monkeypatch):
+    """--dump-outputs: one float64 .npy per call field + problem.npy; above the size limit the same sorted sample of
+    rows on every run, within the limit."""
+    import numpy as np
+    import bench
+    from tredparse_b200 import cohort
+    calls = np.zeros(1000, cohort.CALL_DTYPE)
+    calls["allele1"], calls["pp"] = np.arange(1000), np.linspace(0, 1, 1000)
+    calls["ci"] = np.arange(4000).reshape(1000, 4)
+    bench.dump_outputs(str(tmp_path / "all"), calls, np.arange(1000) * 30 + 7)
+    names = sorted(p.name for p in (tmp_path / "all").iterdir())
+    assert names == sorted(n + ".npy" for n in cohort.CALL_DTYPE.names + ("problem",))
+    got = {n[:-4]: np.load(str(tmp_path / "all" / n)) for n in names}
+    assert all(a.dtype == np.float64 for a in got.values()) and got["ci"].shape == (1000, 4)
+    assert np.array_equal(got["pp"], calls["pp"]) and np.array_equal(got["problem"], np.arange(1000) * 30 + 7)
+    monkeypatch.setattr(bench, "DUMP_BYTES", 12 * 1024 + 100 * 15 * 8)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), calls, np.arange(1000))
+    a, b = (np.load(str(tmp_path / d / "problem.npy")) for d in ("a", "b"))
+    assert len(a) == 100 and np.array_equal(a, b) and np.all(np.diff(a) > 0)
+    assert np.array_equal(np.load(str(tmp_path / "a" / "allele1.npy")), a)
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= bench.DUMP_BYTES
+
+
 def test_reference_arm_line():
     d = _line("r1_bench_reference.json")
     assert d["impl"] == "reference" and BASE - {"gpu_launches"} <= set(d)

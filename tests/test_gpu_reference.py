@@ -1,6 +1,6 @@
 """The CUDA path against golden vectors produced by the REFERENCE ITSELF (tests/golden/ref_*.json — outputs of
-the reference's own BamParser / IntegratedCaller / tred.run, see tests/golden/make_ref_fixtures.py), and the
-reference's own ctypes Aligner bound to libtredsw.so.  Needs a GPU: run with -m gpu."""
+the reference's own BamParser / IntegratedCaller / tred.run, see tests/golden/make_ref_fixtures.py).  Needs a GPU:
+run with -m gpu."""
 import gzip
 import json
 import os
@@ -30,64 +30,6 @@ def close(a, b, rtol=RTOL, path=""):
         assert abs(a - b) <= rtol * max(abs(a), abs(b)) + 1e-15, (path, a, b)
     else:
         assert a == b, (path, a, b)
-
-
-# ---------------------------------------------------------------------------------------------------------
-# INTEGRATION level 0: the reference's unmodified ssw_wrap.Aligner on the GPU library
-# ---------------------------------------------------------------------------------------------------------
-def _reference_aligner_module():
-    from oracle import refshim
-    from tredparse_b200 import build
-    if not (refshim.available() or refshim.cached("ssw")):
-        pytest.skip("neither /root/reference nor oracle/_ref/refpy is present")
-    return refshim.load(libssw=build.OUT, modules=["ssw"]).ssw
-
-
-@pytest.mark.parametrize("sample,tredname", CASES)
-def test_reference_Aligner_bound_to_libtredsw_reproduces_every_reference_pair(sample, tredname):
-    """ssw_wrap.py (the reference's ctypes binding, src/ssw_wrap.py:54-256) loads libtredsw.so as its libssw.so and
-    aligns the 6,800 + 17,700 (read, template) pairs of the fixtures exactly as BamParser does
-    (bam_parser.py:91-99,133-135); results equal those of the reference's own ssw.c."""
-    ssw = _reference_aligner_module()
-    assert ssw.Aligner.libssw._name.endswith("libssw.so") and os.path.realpath(ssw.Aligner.libssw._name).endswith("libtredsw.so")
-    z = np.load(os.path.join(GOLDEN, "sw_pairs_{}_{}.npz".format(sample, tredname)))
-    reads, templates, pairs = [str(x) for x in z["reads"]], [str(x) for x in z["templates"]], z["pairs"]
-    n = 0
-    for ti, target in enumerate(templates):
-        al = ssw.Aligner(ref_seq=target, match=1, mismatch=5, gap_open=7, gap_extend=2, report_secondary=False)
-        for qi, seq in enumerate(reads):
-            min_len = min(len(seq), len(target)) // 2
-            min_score = max(min_len, 30)
-            r = al.align(seq, min_score=min_score, min_len=min_len)
-            score, rb, re, qb, qe = (int(x) for x in pairs[qi, ti, :5])
-            keep = score >= min_score and (qe - qb + 1) >= min_len
-            if not keep:
-                assert r is None, (qi, ti)
-            else:
-                assert r is not None and (r.score, r.ref_begin, r.ref_end, r.query_begin, r.query_end) == \
-                    (score, rb, re, qb, qe), (qi, ti)
-            n += 1
-    assert n == len(reads) * len(templates)
-
-
-def test_reference_Aligner_cigar_on_libtredsw():
-    ssw = _reference_aligner_module()
-    z = np.load(os.path.join(GOLDEN, "sw_pairs_t001_HD.npz"))
-    reads, templates, pairs = [str(x) for x in z["reads"]], [str(x) for x in z["templates"]], z["pairs"]
-    cigar, clen = z["cigar"], z["cigar_len"]
-    for ti in (3, 40, 41, 98):
-        al = ssw.Aligner(ref_seq=templates[ti], match=1, mismatch=5, gap_open=7, gap_extend=2,
-                         report_secondary=True, report_cigar=True)
-        for qi in range(0, len(reads), 5):
-            r = al.align(reads[qi], min_score=0, min_len=0)
-            if pairs[qi, ti, 0] == 0:
-                continue
-            assert (r.score, r.ref_begin, r.ref_end, r.query_begin, r.query_end) == tuple(int(x) for x in pairs[qi, ti, :5])
-            # PyAlignRes keeps the raw CIGAR words and decodes them with the library's cigar_int_to_len /
-            # cigar_int_to_op (ssw_wrap.py:274-280,313-319); c_char comes back as bytes under Python 3
-            got = [(int(l), op.decode() if isinstance(op, bytes) else op) for l, op in r.iter_cigar]
-            want = [(int(w) >> 4, "MID"[int(w) & 15]) for w in cigar[qi, ti, :clen[qi, ti]]]
-            assert got == want, (qi, ti)
 
 
 # ---------------------------------------------------------------------------------------------------------
@@ -225,19 +167,28 @@ def test_run_chunk_equals_run_sample_by_sample():
 
 def test_tred_run_on_a_synthetic_sample_bam_equals_the_reference(tmp_path):
     """A simulated whole-sample BAM (reads placed around several loci, expansions included): the product's
-    tred.run (native ingest -> fused device pipeline) against the reference's own tred.run on the same file."""
+    tred.run (native ingest -> fused device pipeline) against the stored calls of the CPU oracle on the same file
+    (golden/oracle_sample_bam.json; the oracle is held to the reference's own outputs by test_reference_pinned.py)
+    and, where the reference package can be loaded, against the reference's own tred.run."""
     from oracle import refdrive
-    if not refdrive.usable():
-        pytest.skip("the reference package is not loadable here (oracle/_ref/ not built)")
-    from tredparse_b200 import tred as T, simulate, bamio
+    from tredparse_b200 import tred as T
     from tredparse_b200.meta import TREDsRepo
+    g = golden_module("make_oracle_bam_fixture")
+    with open(os.path.join(GOLDEN, "oracle_sample_bam.json")) as fp:
+        gold = json.load(fp)
     repo = TREDsRepo()
-    names = ["HD", "DM1", "FXS", "FRDA", "SCA10", "ULD", "OPMD", "AR"]
-    sam = bamio.AlignmentFile(os.path.join(GOLDEN, "t001.mini.bam"))
-    refs = list(zip(sam.references, sam.lengths))
+    names = gold["names"]
     path = str(tmp_path / "s.bam")
-    truth = simulate.write_sample_bam(path, repo, names, refs, 3, flank=2000)
-    mine = T.run(("s", path, repo, names, 300, False, False, True, True, "INFO"))["tredCalls"]
-    theirs = refdrive.run_bam(("s", path, names))
-    close(json.loads(json.dumps(mine)), json.loads(json.dumps(theirs, default=float)))
+    truth = g.write_sample(path, repo)
+    assert g.records_sha1(path) == gold["records_sha1"], "the simulator no longer writes the fixture's reads"
+    assert json.loads(json.dumps(truth)) == gold["truth"]
+    mine = json.loads(json.dumps(T.run(("s", path, repo, names, 300, False, False, True, True, "INFO"))["tredCalls"]))
+    for k, v in gold["presteps"].items():
+        close(mine[k], v, path=k)
+    for n in names:
+        for k, v in gold["calls"][n].items():
+            close(mine[n + "." + k], v, path=n + "." + k)
     assert any(mine[n + ".1"] > 0 for n in names)
+    if refdrive.usable():
+        theirs = refdrive.run_bam(("s", path, names))
+        close(mine, json.loads(json.dumps(theirs, default=float)))

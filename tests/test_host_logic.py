@@ -43,22 +43,20 @@ def test_model_tables():
     assert 0 < noise.predict([3, 20, .68, 1.0]) < 1
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/tredparse/data"), reason="reference tree not mounted")
 def test_tables_equal_the_reference_files(repo):
-    import pandas as pd
-    df = pd.read_csv("/root/reference/tredparse/data/TREDs.meta.csv", index_col=0)
-    assert sorted(df.index) == sorted(repo.names)
+    """The columns of the reference's TREDs.meta.csv and its step / stutter models, stored in golden/ref_tables.json."""
+    with open(os.path.join(GOLDEN, "ref_tables.json")) as fp:
+        ref = json.load(fp)
+    assert sorted(ref["catalogue"]) == sorted(repo.names)
     for n in repo.names:
-        row = df.loc[n]
+        row = ref["catalogue"][n]
         assert repo[n].repeat == row["repeat"] and repo[n].prefix == row["prefix"] and repo[n].suffix == row["suffix"]
-        assert "{}:{}-{}".format(repo[n].chr, repo[n].repeat_start, repo[n].repeat_end) == row["repeat_location"]
-    from oracle import likelihood_oracle as lko
-    ref_step = lko.load_step_model("/root/reference/tredparse/data/illumina_v3.pcrfree.stepmodel")
-    ref_w = lko.load_noise_model("/root/reference/tredparse/data/illumina_v3.pcrfree.stuttermodel")
+        assert "{}:{}-{}".format(repo[n].chr, repo[n].repeat_start, repo[n].repeat_end) == \
+            "{}:{}-{}".format(row["chr"], row["repeat_start"], row["repeat_end"])
     ours = models.StepModel().step_size_by_period
-    for p in ref_step:
-        assert np.array_equal(np.asarray(ours[p]), ref_step[p])
-    assert list(models.NoiseModel().weights) == ref_w
+    for p, v in ref["step_size_by_period"].items():
+        assert np.array_equal(np.asarray(ours[int(p)]), np.array(v))
+    assert list(models.NoiseModel().weights) == ref["stutter_weights"]
 
 
 # ---- BAM / BAI -----------------------------------------------------------------------------------------

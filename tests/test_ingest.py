@@ -1,6 +1,6 @@
 """Native BAM ingest (csrc/ingest.cpp, host code) against the Python host path that mirrors the reference —
 BamParser.select_reads (bam_parser.py:194-243), PEextractor (:316-369), BamDepth.region_depth (:404-411) —
-on the committed mini BAMs and, where the reference tree is mounted, on its full test BAMs.  No GPU needed."""
+on the committed mini BAMs.  No GPU needed."""
 import logging
 import os
 
@@ -15,8 +15,6 @@ from tredparse_b200.utils import InputParams
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
 CASES = [("t001", "HD"), ("t002", "DM1")]
 BAMS = [(s, t, os.path.join(GOLDEN, s + ".mini.bam")) for s, t in CASES]
-BAMS += [(s + "_full", t, "/root/reference/tests/{}.bam".format(s)) for s, t in CASES
-         if os.path.exists("/root/reference/tests/{}.bam".format(s))]
 
 
 @pytest.fixture(scope="module")

@@ -108,13 +108,6 @@ def test_emulated_pipeline_equals_host_reader_on_the_fixtures(repo):
     assert _check_batch(None, paths, repo, ["HD", "DM1", "SCA17"], readlen=101) > 50
 
 
-def test_emulated_pipeline_on_the_reference_bams(repo):
-    ref = [p for p in ("/root/reference/tests/t001.bam", "/root/reference/tests/t002.bam") if os.path.exists(p)]
-    if not ref:
-        pytest.skip("reference tree not mounted")
-    assert _check_batch(None, ref, repo, repo.names) > 200
-
-
 def test_emulated_pipeline_on_a_synthetic_whole_sample_bam(repo, tmp_path):
     """~30x at every catalogue locus: thousands of pair candidates per problem (pairing tables, ordered compaction)."""
     names = ["HD", "DM1", "FXS", "SCA10"]

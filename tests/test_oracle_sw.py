@@ -50,24 +50,6 @@ def test_oracle_matches_reference_synthetic_pairs_and_cigars():
         assert c is not None and np.array_equal(c, g)
 
 
-@pytest.mark.skipif(not sw.ref_available(), reason="oracle/_ref/libssw_ref.so not built (needs /root/reference)")
-def test_oracle_matches_live_reference_random():
-    rng = np.random.default_rng(7)
-    q = ["".join(rng.choice(list("ACGTN"), p=[.24, .24, .24, .24, .04], size=int(rng.integers(5, 260))))
-         for _ in range(400)]
-    t = ["".join(rng.choice(list("ACGTN"), p=[.24, .24, .24, .24, .04], size=int(rng.integers(5, 300))))
-         for _ in range(400)]
-    # plant real similarity in half of them
-    for i in range(0, 400, 2):
-        L = min(len(q[i]), len(t[i])) // 2
-        t[i] = t[i][:5] + q[i][:L] + t[i][5:]
-    idx = np.arange(400, dtype=np.int32)
-    a = sw.oracle_align_pairs(q, t, idx, idx)
-    b = sw.ref_align_pairs(q, t, idx, idx)
-    ok = b[:, 0] > 0
-    assert np.array_equal(a[ok], b[ok])
-
-
 @pytest.mark.parametrize("sample,tred", CASES)
 def test_classification_c_vs_python_and_golden_best(sample, tred):
     d, reads, T, qidx, tidx = _pairs("sw_pairs_{}_{}.npz".format(sample, tred))
