@@ -124,9 +124,10 @@ def _expected_best(read, db, P, mu, **score_kw):
 
 
 def test_family_kernel_fast_and_generic_paths_vs_oracle_across_loci():
-    """Simulated reads at loci of every catalogue period (3,4,5,6,12), with N in the motif, 150 and
-    250 bp.  Default scoring goes through the packed fast path; match=2 makes scores exceed the 8-bit
-    boundary column (2*150 >= 256) and forces the generic scalar phase 1.  Both must equal the oracle."""
+    """Simulated reads at loci of every catalogue period (3,4,5,6,12), with N in the motif, 101, 150,
+    250 and 300 bp.  Default scoring goes through the packed fast path while every read of the call is
+    shorter than 256 bp; a 300 bp read, or match=2 (scores exceed the 8-bit boundary column: 2*150 >= 256),
+    forces the generic scalar phase 1 for the whole call.  Every variant must equal the oracle."""
     from tredparse_b200 import ssw
     from tredparse_b200.meta import TREDsRepo
     from oracle import evidence_oracle as evo
@@ -136,7 +137,7 @@ def test_family_kernel_fast_and_generic_paths_vs_oracle_across_loci():
     fams, reads, rfam, dbs = [], [], [], []
     for name in ("HD", "DM2", "SCA10", "SCA36", "ULD", "OPMD", "FXS", "FRDA"):
         t = repo[name]
-        for readlen in (150, 250):
+        for readlen in (101, 150, 250, 300):
             P = len(t.repeat)
             mu = -(-readlen // P)
             fams.append(ssw.make_family(t.prefix, t.repeat, t.suffix, mu))
@@ -159,18 +160,21 @@ def test_family_kernel_fast_and_generic_paths_vs_oracle_across_loci():
                 dbs.append((db, P, mu))
     fams = np.concatenate(fams)
     rfam = np.array(rfam, dtype=np.int32)
+    short = [r for r in range(len(reads)) if len(reads[r]) < 256]        # a call of these runs the packed kernel
     for kw_gpu, kw_or in ((dict(), dict()),
                           (dict(match=2, mismatch=10, gap_open=14, gap_extend=4), dict(match=2, mismatch=10, go=14, ge=4))):
-        out = ssw.classify_reads(reads, rfam, fams, **kw_gpu)
-        ntag = 0
-        for r, (db, P, mu) in enumerate(dbs):
-            e = _expected_best(reads[r], db, P, mu, **kw_or)
-            if e is None:
-                assert out[r, 0] == 0, r
-            else:
-                ntag += 1
-                assert (out[r, 2], out[r, 1], out[r, 0]) == (e[0], e[1], TAGC[e[2]]), (r, e, out[r])
-        assert ntag > len(reads) // 3
+        exp = [_expected_best(reads[r], db, P, mu, **kw_or) for r, (db, P, mu) in enumerate(dbs)]
+        for sel in (list(range(len(reads))), short):
+            out = ssw.classify_reads([reads[r] for r in sel], rfam[sel], fams, **kw_gpu)
+            ntag = 0
+            for k, r in enumerate(sel):
+                e = exp[r]
+                if e is None:
+                    assert out[k, 0] == 0, r
+                else:
+                    ntag += 1
+                    assert (out[k, 2], out[k, 1], out[k, 0]) == (e[0], e[1], TAGC[e[2]]), (r, e, out[k])
+            assert ntag > len(sel) // 3
 
 
 def test_prefilter_is_exact_on_borderline_reads():

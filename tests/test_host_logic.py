@@ -114,6 +114,36 @@ def test_simulation_is_seeded_and_shaped(repo):
     assert long_.nreads > a.nreads                                            # in-repeat reads are kept
 
 
+def test_sample_bam_with_reads_longer_than_the_shortest_fragment(repo, tmp_path):
+    """Fragments are drawn from [200, 999] bp.  For longer reads, a fragment shorter than the read has no full-length
+    proper pair, so write_sample_bam drops it: every record is `<L>M` on the reference and read 2 never starts before
+    read 1 (a short fragment used to give read 2 a negative haplotype index, which numpy wraps silently, or an
+    IndexError).  The 150 bp sample the tred.run fixture is made of keeps its records."""
+    from conftest import golden_module
+    g = golden_module("make_oracle_bam_fixture")
+    with open(os.path.join(GOLDEN, "oracle_sample_bam.json")) as fp:
+        gold = json.load(fp)
+    path = str(tmp_path / "s150.bam")
+    g.write_sample(path, repo)
+    assert g.records_sha1(path) == gold["records_sha1"]
+    sam = bamio.AlignmentFile(os.path.join(GOLDEN, "t001.mini.bam"))
+    refs = list(zip(sam.references, sam.lengths))
+    sam.close()
+    for L in (230, 251, 300):
+        path = str(tmp_path / "s{}.bam".format(L))
+        truth = simulate.write_sample_bam(path, repo, g.NAMES, refs, g.SAMPLE, readlen=L, flank=g.FLANK)
+        assert sorted(truth) == sorted(g.NAMES)
+        pairs = {}
+        for r in bamio.AlignmentFile(path).fetch():
+            assert len(r.query_sequence) == L and r.cigartuples == [(0, L)] and r.reference_start >= 0
+            pairs.setdefault(r.query_name, {})[1 if r.flag & 0x40 else 2] = r
+        assert len(pairs) > 1000
+        for name, p in pairs.items():
+            assert sorted(p) == [1, 2], name
+            assert p[2].reference_start >= p[1].reference_start, name
+            assert (p[1].next_reference_start, p[2].next_reference_start) == (p[2].reference_start, p[1].reference_start)
+
+
 def test_cohort_packing_offsets(repo):
     probs = simulate.simulate_cohort(repo, ["HD", "DM1", "FRDA", "HD"], 2, readlen=150)
     batch = cohort.CohortBatch(probs)

@@ -60,12 +60,12 @@ def _check_batch(ctx, paths, repo, names, alts=True, readlen=150):
             h.close()
 
 
-def _write_sample(path, repo, names, sample, seed):
+def _write_sample(path, repo, names, sample, seed, readlen=150):
     from tredparse_b200 import simulate, bamio
     sam = bamio.AlignmentFile(os.path.join(GOLDEN, "t001.mini.bam"))
     refs = list(zip(sam.references, sam.lengths))
     sam.close()
-    simulate.write_sample_bam(path, repo, names, refs, sample, 150, seed)
+    simulate.write_sample_bam(path, repo, names, refs, sample, readlen, seed)
 
 
 def _raw_deflate(data, level, strategy=zlib.Z_DEFAULT_STRATEGY):
@@ -109,11 +109,13 @@ def test_emulated_pipeline_equals_host_reader_on_the_fixtures(repo):
 
 
 def test_emulated_pipeline_on_a_synthetic_whole_sample_bam(repo, tmp_path):
-    """~30x at every catalogue locus: thousands of pair candidates per problem (pairing tables, ordered compaction)."""
+    """~30x at every catalogue locus: thousands of pair candidates per problem (pairing tables, ordered compaction);
+    150 and 251 bp reads (the read window and the selection rules depend on the read length)."""
     names = ["HD", "DM1", "FXS", "SCA10"]
-    path = str(tmp_path / "s.bam")
-    _write_sample(path, repo, names, 3, 11)
-    assert _check_batch(None, [path], repo, names) > 200
+    for readlen in (150, 251):
+        path = str(tmp_path / "s{}.bam".format(readlen))
+        _write_sample(path, repo, names, 3, 11, readlen)
+        assert _check_batch(None, [path], repo, names, readlen=readlen) > 200
 
 
 def test_corrupt_input_is_reported_per_problem_not_as_evidence(repo, tmp_path):

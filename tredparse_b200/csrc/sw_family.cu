@@ -827,10 +827,20 @@ int launch_classify(tredsw_ctx *ctx, const ClassifyParams &p, int nctas, size_t 
     return TREDSW_OK;
 }
 
+// static shared memory of the classify kernels (score tables, LUT, family): the 48 KB a block gets without opting in
+// bounds static + dynamic bytes together
+int classify_static_smem(size_t *out) {
+    cudaFuncAttributes fa{}, ga{};
+    CUDA_TRY(cudaFuncGetAttributes(&fa, classify_kernel<true>));
+    CUDA_TRY(cudaFuncGetAttributes(&ga, classify_kernel<false>));
+    *out = std::max(fa.sharedSizeBytes, ga.sharedSizeBytes);
+    return TREDSW_OK;
+}
+
 // resident CTAs per SM of the persistent kernels (registers / shared memory), times the SM count
-int persistent_ctas(tredsw_ctx *ctx, size_t smem, bool need_fast, bool need_generic, int *out) {
+int persistent_ctas(tredsw_ctx *ctx, size_t smem, size_t static_smem, bool need_fast, bool need_generic, int *out) {
     int a = 0, b = 0;
-    if (smem > 48 * 1024) {
+    if (smem + static_smem > 48 * 1024) {
         CUDA_TRY(cudaFuncSetAttribute(classify_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         CUDA_TRY(cudaFuncSetAttribute(classify_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     }
@@ -884,7 +894,13 @@ int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_
     const int max_rows = max_m > 0 ? max_m : 1;
     const size_t rows_alloc = (size_t)max_rows + 2;
     const size_t smem = rows_alloc * 32 * 4 + rows_alloc * 32 + 64;
-    if (smem > ctx->smem_optin) { tredsw_set_error("reads too long for shared memory (%zu B)", smem); return TREDSW_ERR_UNSUPPORTED; }
+    size_t static_smem = 0;
+    int rc;
+    if ((rc = classify_static_smem(&static_smem))) return rc;
+    if (smem + static_smem > ctx->smem_optin) {
+        tredsw_set_error("reads too long for shared memory (%zu B)", smem + static_smem);
+        return TREDSW_ERR_UNSUPPORTED;
+    }
     ClassifyParams p{};
     p.rbuf = d_rbuf; p.roff = d_roff; p.families = d_families; p.out = d_out;
     int32_t *w = d_work;
@@ -898,8 +914,8 @@ int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_
     p.match = max_match > 0 ? max_match : 1;
     p.stats = d_stats;
     const int nitems_bound = nreads / 32 + nfamilies + 1;
-    int rc, nctas = 0;
-    if ((rc = persistent_ctas(ctx, smem, need_fast, need_generic, &nctas))) return rc;
+    int nctas = 0;
+    if ((rc = persistent_ctas(ctx, smem, static_smem, need_fast, need_generic, &nctas))) return rc;
     if (nctas > nitems_bound) nctas = nitems_bound;
     // per-CTA scratch: scores [2*max_u][32] u16, potentials [rows][32] u32, then the two work counters
     const size_t score_bytes = (size_t)nctas * 2 * max_u * 32 * sizeof(uint16_t);

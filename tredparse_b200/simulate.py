@@ -195,7 +195,10 @@ def locus_records(tred, tid, alleles, readlen=150, cov_per_hap=15.0, error=0.005
     """Paired reads of one locus as ``bamio.AlignedSegment`` records placed on the reference: haplotype coordinates are
     mapped onto the locus (flanks one to one, the repeat clamped to the reference's copy number), every read gets a
     ``<readlen>M`` CIGAR and proper-pair flags — what an aligner reports for reads around a repeat whose length
-    differs from the reference.  Same haplotypes, fragments and errors as ``simulate_problem`` with the same seed."""
+    differs from the reference.  Haplotypes, fragment lengths and errors follow the model of ``simulate_problem``
+    (not its random stream).  A fragment shorter than the read is dropped: an aligner would not report it as a
+    full-length ``<readlen>M`` proper pair.  Fragments are at least FRAG_MIN long, so for ``readlen <= FRAG_MIN``
+    nothing is dropped and the records do not depend on this rule."""
     from .bamio import AlignedSegment
     rng = np.random.default_rng(seed)
     prefix, suffix, motif = encode(tred.prefix), encode(tred.suffix), encode(tred.repeat)
@@ -218,6 +221,8 @@ def locus_records(tred, tid, alleles, readlen=150, cov_per_hap=15.0, error=0.005
         frag = _fragment_lengths(rng, nfrag)
         start = rng.integers(0, L - frag + 1)
         end = start + frag
+        full = np.nonzero(frag >= readlen)[0]             # then 0 <= start <= end - readlen and end <= L
+        start, end = start[full], end[full]
 
         def to_ref(x):        # haplotype coordinate -> 0-based reference coordinate
             x = np.asarray(x)
@@ -234,8 +239,8 @@ def locus_records(tred, tid, alleles, readlen=150, cov_per_hap=15.0, error=0.005
         for block in (r1, r2):
             err = rng.random(block.shape) < error
             block[err] = rng.integers(0, 4, int(err.sum()))
-        for k in range(nfrag):
-            name = "{}h{}f{}".format(tag, hap_idx, k)
+        for k, fk in enumerate(full):
+            name = "{}h{}f{}".format(tag, hap_idx, fk)
             tl = int(e2[k] - p1[k])
             recs.append(AlignedSegment(name, 0x1 | 0x2 | 0x20 | 0x40, tid, int(p1[k]), 60, [(0, readlen)], tid, int(p2[k]),
                                        tl, "".join(lut[r1[k]])))
