@@ -5,7 +5,7 @@
 
 // Smith-Waterman + classification of every read against its family (sw_family.cu).
 // h_families: host copy (shape decisions); d_* : device buffers.  d_work needs
-// (4*nfamilies + 2 + nreads) int32.  d_stats: 4 x u64 or NULL (must be zeroed by the caller).
+// (12*nfamilies + 2 + nreads) int32: counts, offsets and cursors per (family, strand class), the read order.  d_stats: 4 x u64 or NULL (must be zeroed by the caller).
 int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_t *d_roff, int nreads,
                              const int32_t *d_read_family, const tredsw_family *d_families,
                              const tredsw_family *h_families, int nfamilies, int max_read_len,

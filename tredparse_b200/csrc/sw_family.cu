@@ -11,9 +11,11 @@
 //
 // Mapping of the DP (classify_kernel): one warp = 32 surviving reads of the same family, one thread = one
 // read; persistent single-warp CTAs pull such items from a counter.  Every lane walks the same template
-// columns at the same time, so template bases are warp-uniform; query bases are per lane.
+// columns at the same time, so template bases are warp-uniform; query bases are per lane.  Reads that the
+// pre-filter shows to have candidates on one strand only run two per thread (64 per warp), see phase 1.
 //
-// Phase 1 (scores of all 2*max_units templates), all packed int16x2 = forward template | reverse complement:
+// Phase 1 (scores of all 2*max_units templates), all packed int16x2 = forward template | reverse complement
+// of one read, or read a | read b on one strand:
 //   * the templates of a family are nested — prefix + repeat*u is a prefix of prefix + repeat*(u+1) — so
 //     the main DP (prefix + repeat*max_units) runs once, in 12-column strips held in registers (previous-
 //     row H and running F per column), two query rows in flight; the H/E column between strips lives in
@@ -40,6 +42,10 @@ namespace {
 
 constexpr int FAM_W2 = 16;         // strip width of the scalar phase-2 sweeps
 constexpr int FLANK = 18;          // flank length of the fast path (all catalogue loci)
+// Strand class of a read that reaches the DP, from the q-gram pre-filter: templates of both strands may score
+// >= 30, or only forward / only reverse-complement ones.  Only families of the packed kernel get the single-strand
+// classes; two single-strand reads share a lane there (read a | read b as s16x2 halves).
+constexpr int CLASS_BOTH = 0, CLASS_FWD = 1, CLASS_RC = 2, NCLASS = 3;
 
 struct FamilySmem {
     int8_t prefix[32], suffix[32], repeat[32];
@@ -48,13 +54,13 @@ struct FamilySmem {
 
 struct ClassifyParams {
     const int8_t *rbuf; const int64_t *roff;
-    const int32_t *order;          // read indices grouped by family
-    const int32_t *fam_start;      // [nfam+1] offsets into order
-    const int32_t *chunk_start;    // [nfam+1] offsets into the item (warp-chunk) list, families in fam_perm order
-    const int32_t *fam_perm;       // [nfam] families sorted by period: CTAs that run at the same time mostly
+    const int32_t *order;          // read indices grouped by (family, strand class): group f * NCLASS + class
+    const int32_t *grp_start;      // [ngroups+1] offsets into order
+    const int32_t *chunk_start;    // [ngroups+1] offsets into the item (warp-chunk) list, groups in grp_perm order
+    const int32_t *grp_perm;       // [ngroups] groups sorted by period: CTAs that run at the same time mostly
                                    // share one instantiation of the strip loops (instruction cache)
     const tredsw_family *families;
-    int nfamilies;
+    int ngroups;
     int go, ge;
     int max_rows;
     int allow_fast;                // scores fit the 8-bit boundary column (max_read_len * match < 256)
@@ -118,13 +124,28 @@ __device__ void phase1_generic(const FamilySmem &F, const SwLut *lut, const uint
 }
 
 // ---------------------------------------------------------------------------------------------------
-// Phase 1, fast: nested strips, forward + reverse-complement packed as s16x2.
+// Phase 1, fast: nested strips, two half-strands packed as s16x2.
 // Requires Lp == Ls == FLANK and scores < 256 (8-bit boundary column).
-// Boundary word per row and lane: H_fwd | H_rc << 8 | E_fwd << 16 | E_rc << 24.
+// An item's lanes hold either one read with the forward template in the low half and the reverse
+// complement in the high half ("both" class), or two reads a | b on the same strand (the pre-filter
+// proved the other strand of each has no candidate): the half-strands (sa, sb) are warp-uniform.
+// The query side of a row is the PAIR CODE qa * 6 + qb of the two halves' base codes (qa == qb for
+// "both" items); the score tables have one row per pair code.
+// Boundary word per row and lane: H_a | H_b << 8 | E_a << 16 | E_b << 24.
 // ---------------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t sel2(int tf, int tr) {   // PRMT selector: sign-extended bytes -> s16x2
-    return (uint32_t)tf | ((uint32_t)(8 | tf) << 4) | ((uint32_t)tr << 8) | ((uint32_t)(8 | tr) << 12);
+__device__ __forceinline__ uint32_t sel2(int ta, int tb) {   // PRMT selector: sign-extended bytes -> s16x2
+    return (uint32_t)ta | ((uint32_t)(8 | ta) << 4) | ((uint32_t)tb << 8) | ((uint32_t)(8 | tb) << 12);
 }
+constexpr int NPAIR = 36;                         // pair codes (6 query codes per half)
+constexpr int PAIR_GHOST = SW_CODE_GHOST * 7;     // pair code of a row past the end of both halves
+// own base code of half h (0: a, 1: b) of a pair code; for "both" items (code 7q) either decode gives q
+__device__ __forceinline__ int pair_half(int code, int h) { return h ? code % 6 : code / 6; }
+
+// template bases on strand s (1 = reverse complement: prefix' = rc(suffix), repeat' = rc(repeat), suffix' = rc(prefix))
+__device__ __forceinline__ int comp_code(int c) { return c < 4 ? 3 - c : c; }
+__device__ __forceinline__ int pre_base(const FamilySmem &F, int s, int c) { return s ? comp_code(F.suffix[FLANK - 1 - c]) : F.prefix[c]; }
+__device__ __forceinline__ int rep_base(const FamilySmem &F, int s, int c) { return s ? comp_code(F.repeat[F.P - 1 - c]) : F.repeat[c]; }
+__device__ __forceinline__ int suf_base(const FamilySmem &F, int s, int c) { return s ? comp_code(F.prefix[FLANK - 1 - c]) : F.suffix[c]; }
 
 // One DP cell for both strands (packed s16x2), all operands in registers.  Four integer-pipe instructions:
 //     E~ = E + go, F~ = F + go (gap states stored biased by the opening cost, never clamped: E~ >= H >= 0)
@@ -145,9 +166,10 @@ __device__ __forceinline__ uint32_t sel2(int tf, int tr) {   // PRMT selector: s
         Fv[C] = __viaddmax_s16x2(Fv[C], mge2, HOUT);                                          \
     }
 
-constexpr int STAB_PAD = 36;       // words per query-code row of the score table: >= the widest strip, a multiple of 4
-                                   // (16-byte rows for LDS.128) and == 4 mod 32 so that the rows of different bases
-                                   // start in different bank groups (conflict-free vector loads)
+constexpr int STAB_PAD = 20;       // words per query-code row of the score table: >= the widest strip (FLANK), a
+                                   // multiple of 4 (16-byte rows for LDS.128) and an odd number of 16-byte groups, so
+                                   // that 8 consecutive rows start in all 8 bank groups (vector loads of lanes on
+                                   // different rows conflict as little as the row count allows)
 
 // Columns per main strip: K whole repeat units, about 12 columns.  Measured on B200 (period 3): 30 columns
 // 9.29 ms, 24: 9.06, 18: 8.94, 12: 8.66 per 11,520-problem step — the fully unrolled two-row loop body must
@@ -162,8 +184,8 @@ __host__ __device__ constexpr int instance_period(int P) { return P == 6 ? 3 : P
 // One pass over all query rows of a strip of NC template columns made of K = NC / PER units of PER
 // columns (previous-row H and running F of every strip column in registers).  Two rows are in flight per
 // iteration, skewed by one column (row j at column s, row j+1 at column s-1): two independent dependency
-// chains for the scheduler.  Substitution scores of both strands come from a per-strip table in shared
-// memory indexed by the query base (row, per lane) and the strip column (uniform): vector LDS on the
+// chains for the scheduler.  Substitution scores of both halves come from a per-strip table in shared
+// memory indexed by the pair code (row, per lane) and the strip column (uniform): vector LDS on the
 // otherwise idle LSU pipe instead of one PRMT per cell on the saturated integer pipe.
 //
 //   seg[u]  running maximum of H over the columns of unit u (all rows)
@@ -172,7 +194,7 @@ __host__ __device__ constexpr int instance_period(int P) { return P == 6 ? 3 : P
 //               mu[u] = max(mu[u], H(j-1, last) + A[j], E(j, last -> next) + B[j])
 //           — 2 add-max per row and unit instead of a forked DP over the suffix columns.
 //   bin     (HAS_IN) boundary column entering the strip, bout (HAS_OUT) the one leaving it: H | E~ << 16 as
-//           bytes per strand, one word per row and lane in this CTA's global scratch (L1/L2 resident,
+//           bytes per half, one word per row and lane in this CTA's global scratch (L1/L2 resident,
 //           requested one iteration ahead); every strip keeps its own slot, phase 2 restarts from them
 //   pot     suffix potentials of this warp's reads in global scratch, one word per row and lane
 template <int NC, int PER, bool HAS_IN, bool HAS_OUT, bool HOOK>
@@ -189,7 +211,7 @@ __device__ __forceinline__ void strip_pass(const uint32_t *stab, const uint8_t *
 #pragma unroll
     for (int u = 0; u < K; ++u) pend[u] = 0;
     uint32_t hin_prev = 0;
-    auto code_at = [&](int j) { return j < m ? (int)codes[j * 32 + lane] : SW_CODE_GHOST; };
+    auto code_at = [&](int j) { return j < m ? (int)codes[j * 32 + lane] : PAIR_GHOST; };
     auto row_of = [&](int code) { return reinterpret_cast<const uint4 *>(stab + code * STAB_PAD); };
     // software pipeline: shared-memory operands of row j are requested one iteration ahead, the global ones
     // (boundary column, potentials: L2 latency) two iterations ahead
@@ -264,7 +286,7 @@ __device__ __forceinline__ void strip_pass(const uint32_t *stab, const uint8_t *
 }
 
 // Suffix potentials: the DP of the read against the template's SUFFIX block, run backwards (rows from the
-// last query base up, columns from the last suffix base to the first), both strands packed.
+// last query base up, columns from the last suffix base to the first), both halves packed.
 //   G(j,c)  = best score of a path that STARTS with the aligned pair (j, c) and ends anywhere
 //   GH(j,c) = best score still to gain after the pair (j, c) (>= 0: the path may stop there)
 //   GE(j,c) = best score still to gain for a path that is in a template-axis gap at (j, c)
@@ -274,7 +296,7 @@ __device__ __forceinline__ void strip_pass(const uint32_t *stab, const uint8_t *
 // function of the H/E column entering the block plus the paths that start inside the block, so
 //     max H over the suffix block of template u = max(fresh, max_j H_u(j-1,last)+A[j], max_j E_u(j)+B[j])
 // with A[j] = G(j,0), B[j] = GE(j,0) and fresh = max G — none of which depends on u.
-// pot[j] = A_fwd | A_rc << 8 | (B_fwd - go) << 16 | (B_rc - go) << 24 (signed bytes; 0x80 = -128 on ghost rows).
+// pot[j] = A_a | A_b << 8 | (B_a - go) << 16 | (B_b - go) << 24 (signed bytes; 0x80 = -128 on ghost rows).
 template <int NC>
 __device__ __forceinline__ void suffix_pass(const uint32_t *stab, const uint8_t *codes, int lane, int m, int rows2,
                                             uint32_t *pot, uint32_t &fresh, uint32_t mgo2, uint32_t mge2) {
@@ -284,7 +306,7 @@ __device__ __forceinline__ void suffix_pass(const uint32_t *stab, const uint8_t 
 #pragma unroll
     for (int c = 0; c < NC; ++c) { Grow[c] = 0; Fv[c] = 0; }
     // r = reversed row index; table columns are stored reversed as well (column 0 = last suffix base)
-    auto code_at = [&](int r) { const int j = rows2 - 1 - r; return (j >= 0 && j < m) ? (int)codes[j * 32 + lane] : SW_CODE_GHOST; };
+    auto code_at = [&](int r) { const int j = rows2 - 1 - r; return (j >= 0 && j < m) ? (int)codes[j * 32 + lane] : PAIR_GHOST; };
     auto row_of = [&](int code) { return reinterpret_cast<const uint4 *>(stab + code * STAB_PAD); };
     uint32_t f0 = 0, f1 = 0;
 #define SUFFIX_CELL(GD, E, S, C, GOUT)                                                        \
@@ -320,25 +342,35 @@ __device__ __forceinline__ void suffix_pass(const uint32_t *stab, const uint8_t 
     fresh = __vimax3_s16x2(f0, f1, 0u);
 }
 
-// score table of one strip: stab[q][c] = s16x2( score(q, fwd column c), score(q, rc column c) ), q = 0..5
+// score table of one strip: stab[qa * 6 + qb][c] = s16x2( score(qa, half-a column c), score(qb, half-b column c) )
+// (NROWS == NPAIR, rows by pair code), or stab[q][c] = s16x2( score(q, a column c), score(q, b column c) ) (NROWS == 6)
+template <int NROWS>
 __device__ __forceinline__ void build_stab(uint32_t *stab, const SwLut *lut, int lane, int ncols,
                                            const uint32_t *colsel /* smem, per column PRMT selector */,
                                            uint32_t bias2 = 0u /* added to both halves (PACKED_CELL: go) */) {
-    for (int i = lane; i < 6 * STAB_PAD; i += 32) {
+    static_assert(NROWS == NPAIR || NROWS == 6, "rows by pair code or by single code");
+    for (int i = lane; i < NROWS * STAB_PAD; i += 32) {
         const int q = i / STAB_PAD, c = i % STAB_PAD;
-        stab[i] = (c < ncols) ? __vadd2(sw_prmt(lut->w0[q], lut->w1[q], colsel[c]), bias2) : 0u;
+        const int qa = NROWS == NPAIR ? q / 6 : q, qb = NROWS == NPAIR ? q % 6 : q;
+        uint32_t v = 0u;
+        if (c < ncols) {
+            const uint32_t lo = sw_prmt(lut->w0[qa], lut->w1[qa], colsel[c]), hi = sw_prmt(lut->w0[qb], lut->w1[qb], colsel[c]);
+            v = __vadd2(sw_prmt(lo, hi, 0x7610), bias2);
+        }
+        stab[i] = v;
     }
 }
 
 // Phase-2 strip: the same packed DP over one strip, but recording WHERE the maxima are.
 //   colkey[c] = max over rows of (H << 8 | 255 - row), per strand half (unsigned compare): the column
 //               maximum and the smallest row attaining it — what ssw.c's end_ref / end_read need.
+//   row_code  row of `stab` for query row j of this lane (ghost row past the end)
 //   bin       this lane's boundary column entering the strip (lane offset folded in, 32-word row stride)
 //   bout      (CAPTURE) the H/E column leaving unit `kstar` of the strip = the column entering the
 //             suffix block of this lane's winning template
 // Control flow is uniform across the warp; only addresses and the captured unit differ per lane.
-template <int NC, int PER, bool CAPTURE>
-__device__ __forceinline__ void strip_locate(const uint32_t *stab, const uint8_t *codes, int lane, int m, int rows2,
+template <int NC, int PER, bool CAPTURE, class RowCode>
+__device__ __forceinline__ void strip_locate(const uint32_t *stab, RowCode row_code, int rows2,
                                              const uint32_t *bin, uint32_t *bout, int kstar,
                                              uint32_t (&colkey)[NC], uint32_t mgo2, uint32_t mge2, uint32_t one) {
     constexpr int NG = (NC + 3) / 4;
@@ -346,7 +378,6 @@ __device__ __forceinline__ void strip_locate(const uint32_t *stab, const uint8_t
 #pragma unroll
     for (int c = 0; c < NC; ++c) { Hrow[c] = 0; Fv[c] = 0; colkey[c] = 0; }
     uint32_t hin_prev = 0;
-    auto code_at = [&](int j) { return j < m ? (int)codes[j * 32 + lane] : SW_CODE_GHOST; };
     auto row_of = [&](int code) { return reinterpret_cast<const uint4 *>(stab + code * STAB_PAD); };
     uint32_t bA = bin[0], bB = bin[32];
     // capture without branches: unit k's leaving H / E~ are ANDed with an all-ones mask only for k == kstar
@@ -360,7 +391,7 @@ __device__ __forceinline__ void strip_locate(const uint32_t *stab, const uint8_t
         uint32_t eA = sw_prmt(bA, 0, 0x4342), eB = sw_prmt(bB, 0, 0x4342);
         const int jn = min(j + 2, rows2 - 2);
         bA = bin[jn * 32]; bB = bin[(jn + 1) * 32];
-        const uint4 *rowA = row_of(code_at(j)), *rowB = row_of(code_at(j + 1));
+        const uint4 *rowA = row_of(row_code(j)), *rowB = row_of(row_code(j + 1));
         uint32_t sA[NG * 4], sB[NG * 4];
 #pragma unroll
         for (int g = 0; g < NG; ++g) {
@@ -392,8 +423,9 @@ __device__ __forceinline__ void strip_locate(const uint32_t *stab, const uint8_t
     }
 }
 
-// Exact end coordinates (ssw.c's end_ref, end_read) of every lane's current candidate (units u, strand,
-// score cs), warp-uniform.  end_ref is the first template column whose maximum equals cs.  Phase 1 kept the
+// Exact end coordinates (ssw.c's end_ref, end_read) of every lane's current candidate (units u, score cs) in
+// half `half` of the lane (the candidate's strand in a "both" item, the read in a pair item), warp-uniform.  Only
+// that half of the packed pass is read: its rows are the read's own, whatever the other half holds.  end_ref is the first template column whose maximum equals cs.  Phase 1 kept the
 // running maximum of the main columns after every unit (runs[]): if some unit u_main <= u is the first whose
 // running maximum equals cs, the column lies in that unit's own columns (never in the first FLANK columns:
 // cs >= 30 > FLANK * match) — recompute the main strip holding it from its stored entering boundary and read
@@ -403,18 +435,17 @@ template <int P>
 __device__ __noinline__ void locate_packed(const FamilySmem &F, const SwLut *lut, uint32_t *stab, uint32_t *stab2,
                                            uint32_t *colsel, bool &suffix_table_ready, const uint8_t *codes, int lane,
                                            int m, int m_warp, uint32_t *bnd, const uint32_t *gbnd, int R, int go, int ge,
-                                           uint32_t one, int G, int cs, int u, int u_main, int strand, int *end_ref,
-                                           int *end_read, unsigned long long &cells) {
+                                           uint32_t one, int G, int cs, int u, int u_main, int half, int sa, int sb,
+                                           int *end_ref, int *end_read, unsigned long long &cells) {
     constexpr int K = strip_units(P);
     constexpr int NC = P * K;
     const uint32_t mgo2 = (uint32_t)((-go) & 0xffff) | ((uint32_t)((-go) & 0xffff) << 16);
     const uint32_t mge2 = (uint32_t)((-ge) & 0xffff) | ((uint32_t)((-ge) & 0xffff) << 16);
     const uint32_t go2 = (uint32_t)go * 0x00010001u;
     const int rows2 = (m_warp + 1) & ~1;
-    auto comp = [](int c) { return c < 4 ? 3 - c : c; };
     const int su = G * (u_main > 0 ? u_main : u) - 1;        // last sub-unit of the unit of interest (idle lanes: u = 1)
     const int tstar = su / K, kstar = su % K;                // (K is a multiple of G: units do not straddle strips)
-    const int sh = strand ? 16 : 0;
+    const int sh = half ? 16 : 0;
     int found_col = -1, found_row = 0;
     {
         // main strip tstar (the repeat table of phase 1 stays in shared memory).  Every lane restarts from its
@@ -425,8 +456,10 @@ __device__ __noinline__ void locate_packed(const FamilySmem &F, const SwLut *lut
             for (int j = 0; j < rows2; ++j) bnd[j * 32 + lane] = src[j * 32];
         }
         uint32_t colkey[NC];
-        strip_locate<NC, P, true>(stab, codes, lane, m, rows2, bnd + lane, bnd + lane,
-                                  u_main > 0 ? -1 : kstar, colkey, mgo2, mge2, one);
+        // (pair-code rows: the main table of phase 1 is still in shared memory)
+        auto pair_row = [&](int j) { return j < m ? (int)codes[j * 32 + lane] : PAIR_GHOST; };
+        strip_locate<NC, P, true>(stab, pair_row, rows2, bnd + lane, bnd + lane, u_main > 0 ? -1 : kstar, colkey,
+                                  mgo2, mge2, one);
         if (u_main > 0) {
 #pragma unroll
             for (int c = NC - 1; c >= 0; --c) {
@@ -440,14 +473,16 @@ __device__ __noinline__ void locate_packed(const FamilySmem &F, const SwLut *lut
     if (__any_sync(0xffffffffu, u_main <= 0 && cs < 0x7fff)) {
         // suffix block of every lane's own template, entered through the captured boundary
         if (!suffix_table_ready) {
-            if (lane < FLANK) colsel[lane] = sel2(F.suffix[lane], comp(F.prefix[FLANK - 1 - lane]));
+            if (lane < FLANK) colsel[lane] = sel2(suf_base(F, sa, lane), suf_base(F, sb, lane));
             __syncwarp();
-            build_stab(stab2, lut, lane, FLANK, colsel, go2);
+            build_stab<6>(stab2, lut, lane, FLANK, colsel, go2);
             __syncwarp();
             suffix_table_ready = true;
         }
         uint32_t colkey[FLANK];
-        strip_locate<FLANK, FLANK, false>(stab2, codes, lane, m, rows2, bnd + lane, nullptr, 0, colkey, mgo2, mge2, one);
+        // (rows by this half's own code: a 6-row table suffices, as only this half is read)
+        auto own_row = [&](int j) { return j < m ? pair_half(codes[j * 32 + lane], half) : SW_CODE_GHOST; };
+        strip_locate<FLANK, FLANK, false>(stab2, own_row, rows2, bnd + lane, nullptr, 0, colkey, mgo2, mge2, one);
         if (u_main <= 0) {
 #pragma unroll
             for (int c = FLANK - 1; c >= 0; --c) {
@@ -465,7 +500,7 @@ template <int P>
 __device__ __noinline__ void phase1_packed(const FamilySmem &F, const SwLut *lut, uint32_t *stab, uint32_t *colsel,
                                            const uint8_t *codes, int lane, int m, int m_warp, uint32_t *pot,
                                            uint32_t *gbnd, int R, uint8_t *scores, uint8_t *runs, int go, int ge,
-                                           uint32_t one, int G, unsigned long long &cells) {
+                                           uint32_t one, int G, int sa, int sb, unsigned long long &cells) {
     constexpr int K = strip_units(P);
     constexpr int NC = P * K;
     static_assert(NC <= STAB_PAD && FLANK <= STAB_PAD, "strip wider than the score table");
@@ -473,22 +508,20 @@ __device__ __noinline__ void phase1_packed(const FamilySmem &F, const SwLut *lut
     const uint32_t mge2 = (uint32_t)((-ge) & 0xffff) | ((uint32_t)((-ge) & 0xffff) << 16);
     const uint32_t go2 = (uint32_t)go * 0x00010001u;
     const int rows2 = (m_warp + 1) & ~1;
-    // rc family: prefix' = rc(suffix), repeat' = rc(repeat), suffix' = rc(prefix)
-    auto comp = [](int c) { return c < 4 ? 3 - c : c; };
     // ---- suffix potentials (table columns reversed: column c' = suffix base FLANK-1-c') ---------------
-    if (lane < FLANK) colsel[lane] = sel2(F.suffix[FLANK - 1 - lane], comp(F.prefix[lane]));
+    if (lane < FLANK) colsel[lane] = sel2(suf_base(F, sa, FLANK - 1 - lane), suf_base(F, sb, FLANK - 1 - lane));
     __syncwarp();
-    build_stab(stab, lut, lane, FLANK, colsel);
+    build_stab<NPAIR>(stab, lut, lane, FLANK, colsel);
     __syncwarp();
     uint32_t fresh = 0;
     suffix_pass<FLANK>(stab, codes, lane, m, rows2, pot, fresh, mgo2, mge2);
     __syncwarp();
     // ---- strip 0: the FLANK prefix columns -----------------------------------------------------------
-    if (lane < FLANK) colsel[lane] = sel2(F.prefix[lane], comp(F.suffix[FLANK - 1 - lane]));
+    if (lane < FLANK) colsel[lane] = sel2(pre_base(F, sa, lane), pre_base(F, sb, lane));
     __syncwarp();
-    build_stab(stab, lut, lane, FLANK, colsel, go2);
+    build_stab<NPAIR>(stab, lut, lane, FLANK, colsel, go2);
     __syncwarp();
-    uint32_t run;                   // running maximum over the main columns so far, per strand
+    uint32_t run;                   // running maximum over the main columns so far, per half
     {
         uint32_t seg0[1] = {0u}, mu0[1] = {0u};
         strip_pass<FLANK, FLANK, false, true, false>(stab, codes, lane, m, rows2, nullptr, gbnd, pot, seg0, mu0, mgo2, mge2, one);
@@ -496,9 +529,9 @@ __device__ __noinline__ void phase1_packed(const FamilySmem &F, const SwLut *lut
     }
     __syncwarp();
     // ---- main strips: K repeat units each; the suffix of every template is folded in by the potentials --
-    for (int c = lane; c < NC; c += 32) colsel[c] = sel2(F.repeat[c % F.P], comp(F.repeat[F.P - 1 - c % F.P]));
+    for (int c = lane; c < NC; c += 32) colsel[c] = sel2(rep_base(F, sa, c % F.P), rep_base(F, sb, c % F.P));
     __syncwarp();
-    build_stab(stab, lut, lane, NC, colsel, go2);
+    build_stab<NPAIR>(stab, lut, lane, NC, colsel, go2);
     __syncwarp();
     int nstrips = 0;
     for (int u0 = 0; u0 < F.U * G; u0 += K, ++nstrips) {        // u0, u: sub-units of P columns
@@ -515,6 +548,7 @@ __device__ __noinline__ void phase1_packed(const FamilySmem &F, const SwLut *lut
             if (su % G == 0 && su <= F.U * G) {
                 const int ur = su / G - 1;                          // 0-based real unit
                 const uint32_t best = __vimax3_s16x2(run, mu[u], fresh);
+                // slot 2 * ur + h: half h of the lane (strand h of a "both" item's read, read h of a pair item)
                 scores[(2 * ur + 0) * 32 + lane] = (uint8_t)(best & 0xffu);
                 scores[(2 * ur + 1) * 32 + lane] = (uint8_t)((best >> 16) & 0xffu);
                 runs[(2 * ur + 0) * 32 + lane] = (uint8_t)(run & 0xffu);      // running maximum of the main columns
@@ -528,14 +562,17 @@ __device__ __noinline__ void phase1_packed(const FamilySmem &F, const SwLut *lut
 // ---------------------------------------------------------------------------------------------------
 // FAST = true : every family with 18-bp flanks, period <= 12 and scores < 256 (packed phase 1, u8 scores)
 // FAST = false: everything else (scalar phase 1, u16 scores)
-// Persistent: one warp per CTA, CTAs pull items (32 reads of one family) from a counter; both kernels
-// walk the same item list and skip the items of the other class.
+// Persistent: one warp per CTA, CTAs pull items (32 reads of one family, or 64 single-strand reads of one family
+// and strand, two per lane) from a counter; both kernels walk the same item list and skip the items of the other
+// kernel.
 template <bool FAST>
 __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ SwLut lut;
     __shared__ FamilySmem F;
-    __shared__ __align__(16) uint32_t stab[6 * STAB_PAD], stab2[6 * STAB_PAD];
+    // stab: rows by pair code (phase 1, and the main strips of phase 2); stab2: rows by one half's own code (the
+    // suffix block of phase 2, which reads one half at a time)
+    __shared__ __align__(16) uint32_t stab[NPAIR * STAB_PAD], stab2[6 * STAB_PAD];
     __shared__ uint32_t colsel[STAB_PAD];
     // (shared memory: the reads as codes [rows][32], the score table and ONE boundary column [rows][32] for
     //  phase 2, whose scalar sweeps walk it with dependent load -> compute -> store chains that must not pay
@@ -557,7 +594,7 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
     uint32_t *gbnd = p.gbnd_buf + (size_t)blockIdx.x * (p.nslots + 1) * R * 32;    // [nslots + 1][R][32]
     const uint32_t one = p.one;
     sw_build_lut(&lut, c_fmat25, lane, 32);
-    const int nitems = p.chunk_start[p.nfamilies];
+    const int nitems = p.chunk_start[p.ngroups];
     unsigned long long alg = 0, cells1 = 0, cells2 = 0;
     unsigned nal = 0;
 
@@ -567,13 +604,13 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
         if (lane == 0) item = atomicAdd(p.counter + (FAST ? 1 : 0), 1);
         item = __shfl_sync(0xffffffffu, item, 0);
         if (item >= nitems) break;
-        // item -> family (binary search over chunk_start)
-        int lo = 0, hi = p.nfamilies;
+        // item -> (family, strand class) group (binary search over chunk_start)
+        int lo = 0, hi = p.ngroups;
         while (hi - lo > 1) {
             int mid = (lo + hi) >> 1;
             if (p.chunk_start[mid] <= item) lo = mid; else hi = mid;
         }
-        const int f = p.fam_perm[lo];
+        const int grp = p.grp_perm[lo], f = grp / NCLASS, cls = grp % NCLASS;
         {
             const tredsw_family &g = p.families[f];
             F.prefix[lane] = g.prefix[lane]; F.suffix[lane] = g.suffix[lane]; F.repeat[lane] = g.repeat[lane];
@@ -583,130 +620,154 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
         const bool fast_shape = p.allow_fast && (F.Lp == FLANK && F.Ls == FLANK && F.P >= 1 && F.P <= 12);
         if (fast_shape != FAST) continue;
 
-        const int idx = p.fam_start[f] + 32 * (item - p.chunk_start[lo]) + lane;
-        const bool valid = idx < p.fam_start[f + 1];
-        const int r = valid ? p.order[idx] : -1;
-        int m = 0;
-        const int8_t *q = nullptr;
-        if (valid) { q = p.rbuf + p.roff[r]; m = (int)(p.roff[r + 1] - p.roff[r]); }
-        bool too_long = m > p.max_rows;
-        if (too_long) m = 0;
-        if (m > 0) for_each_base(q, m, [&](int j, int c) { codes[j * 32 + lane] = (uint8_t)((c < 0 || c > 4) ? 4 : c); });
-        const int m_warp = __reduce_max_sync(0xffffffffu, m);
+        // The lane's reads: one read of a "both" item, or reads 2*lane and 2*lane+1 of a pair item's 64 (read h in
+        // half h; a missing partner is a ghost of length 0).  Half-strands (sa, sb) of the item: (fwd, rc) for
+        // "both", (fwd, fwd) or (rc, rc) for a pair item.
+        const bool pair = FAST && cls != CLASS_BOTH;
+        const int sa = cls == CLASS_RC ? 1 : 0, sb = cls == CLASS_FWD ? 0 : 1;
+        const int idx0 = p.grp_start[grp] + (pair ? 64 * (item - p.chunk_start[lo]) + 2 * lane : 32 * (item - p.chunk_start[lo]) + lane);
+        int r0 = -1, r1 = -1, m0 = 0, m1 = 0;
+        const bool valid0 = idx0 < p.grp_start[grp + 1], valid1 = pair && idx0 + 1 < p.grp_start[grp + 1];
+        if (valid0) { r0 = p.order[idx0]; m0 = (int)(p.roff[r0 + 1] - p.roff[r0]); }
+        if (valid1) { r1 = p.order[idx0 + 1]; m1 = (int)(p.roff[r1 + 1] - p.roff[r1]); }
+        const bool too_long0 = m0 > p.max_rows, too_long1 = m1 > p.max_rows;
+        if (too_long0) m0 = 0;
+        if (too_long1) m1 = 0;
+        auto clampc = [](int c) { return (c < 0 || c > 4) ? 4 : c; };
+        // codes: plain base codes in the generic kernel, pair codes qa * 6 + qb (ghost past each read's end) in the
+        // packed one — 7q for a "both" item, whose halves share the read
+        const int m_lane = max(m0, m1);
+        if (!pair) {
+            if (m0 > 0) for_each_base(p.rbuf + p.roff[r0], m0, [&](int j, int c) { codes[j * 32 + lane] = (uint8_t)((FAST ? 7 : 1) * clampc(c)); });
+        } else {
+            if (m0 > 0) for_each_base(p.rbuf + p.roff[r0], m0, [&](int j, int c) { codes[j * 32 + lane] = (uint8_t)(6 * clampc(c) + SW_CODE_GHOST); });
+            for (int j = m0; j < m_lane; ++j) codes[j * 32 + lane] = (uint8_t)PAIR_GHOST;
+            if (m1 > 0) for_each_base(p.rbuf + p.roff[r1], m1, [&](int j, int c) { codes[j * 32 + lane] += (uint8_t)(clampc(c) - SW_CODE_GHOST); });
+        }
+        const int m_warp = __reduce_max_sync(0xffffffffu, m_lane);
         __syncwarp();
 
         if constexpr (!FAST) {
-            phase1_generic(F, &lut, codes, lane, m, m_warp, bnd, scores, p.go, p.ge, cells1);
+            phase1_generic(F, &lut, codes, lane, m0, m_warp, bnd, scores, p.go, p.ge, cells1);
         } else {
             switch (instance_period(F.P)) {
-#define PCASE(PP) case PP: phase1_packed<PP>(F, &lut, stab, colsel, codes, lane, m, m_warp, pot, gbnd, R, scores, runs, p.go, p.ge, one, F.P / PP, cells1); break;
+#define PCASE(PP) case PP: phase1_packed<PP>(F, &lut, stab, colsel, codes, lane, m_lane, m_warp, pot, gbnd, R, scores, runs, p.go, p.ge, one, F.P / PP, sa, sb, cells1); break;
                 PCASE(1) PCASE(2) PCASE(3) PCASE(4) PCASE(5) PCASE(7) PCASE(8) PCASE(9) PCASE(10) PCASE(11) PCASE(12)
 #undef PCASE
             }
         }
         __syncwarp();
 
-        // ---- Phase 2: walk candidates in arg-max order until one yields a tag --------------------------
-        int tag = TREDSW_TAG_NONE, best_u = 0, best_score = -1, rb = -1, re = -1, qb = -1, qe = -1, best_rank = -1;
-        const bool active = valid && m > 0;
-        // next candidate after (last_score, last_rank) in the reference's arg-max order
-        auto pick = [&](int last_score, int last_rank, int &cs, int &cr) {
-            cs = -1; cr = -1;
-            if (!active) return;
-            for (int rank = 0; rank < 2 * F.U; ++rank) {
-                const int sc = scores[rank * 32 + lane];
-                const int n = F.Lp + F.Ls + F.P * (rank / 2 + 1);
-                const int min_len = min(m, n) / 2;
-                if (sc < max(min_len, 30)) continue;
-                if (sc > last_score || (sc == last_score && rank <= last_rank)) continue;   // already tried
-                if (sc > cs) { cs = sc; cr = rank; }
-            }
-        };
-        int cs, cr;
-        pick(0x7fffffff, -1, cs, cr);
-        // Rounds: every lane that still has a candidate evaluates it — end coordinates from one warp-uniform
-        // packed pass (locate_packed), begin coordinates and the tag per lane — until all lanes are settled.
-        // Almost every read settles in the first round.
-        const int max_units_eff = F.clip ? (m + F.P - 1) / F.P : F.U;
-        auto rc_f = [&](int j) { return (int)codes[j * 32 + lane]; };
+        // ---- Phase 2, once per read of the lane: walk candidates in arg-max order until one yields a tag ----------
         bool suffix_table_ready = false;
-        while (__any_sync(0xffffffffu, cr >= 0)) {
-            const bool pending = cr >= 0;
-            const int u = pending ? cr / 2 + 1 : 1, s = pending ? (cr & 1) : 0;
-            int fast_end_ref = -1, fast_end_read = 0;
-            if constexpr (FAST) {
-                if (FLANK * p.match < 30) {
-                    int u_main = 0;                      // first unit whose running main maximum equals cs
-                    if (pending) for (int k = 1; k <= u; ++k) if ((int)runs[(2 * (k - 1) + s) * 32 + lane] == cs) { u_main = k; break; }
-                    switch (instance_period(F.P)) {
-#define PCASE(PP) case PP: locate_packed<PP>(F, &lut, stab, stab2, colsel, suffix_table_ready, codes, lane, m, m_warp, bnd, gbnd, R, p.go, p.ge, one, F.P / PP, pending ? cs : 0x7fff, u, u_main, s, &fast_end_ref, &fast_end_read, cells1); break;
-                        PCASE(1) PCASE(2) PCASE(3) PCASE(4) PCASE(5) PCASE(7) PCASE(8) PCASE(9) PCASE(10) PCASE(11) PCASE(12)
+        for (int h = 0; h < (pair ? 2 : 1); ++h) {
+            const bool valid = h ? valid1 : valid0, too_long = h ? too_long1 : too_long0;
+            const int r = h ? r1 : r0, m = h ? m1 : m0;
+            const int own_strand = h ? sb : sa;        // (pair items: the strand of this read's templates)
+            int tag = TREDSW_TAG_NONE, best_u = 0, best_score = -1, rb = -1, re = -1, qb = -1, qe = -1, best_rank = -1;
+            const bool active = valid && m > 0;
+            // next candidate after (last_score, last_rank) in the reference's arg-max order.  Score slot of rank
+            // 2(u-1) + s: the rank itself in a "both" item; in a pair item only the read's own strand was computed,
+            // in half h — every template of the other strand scores below 30 (q-gram bound) and is never a candidate
+            auto pick = [&](int last_score, int last_rank, int &cs, int &cr) {
+                cs = -1; cr = -1;
+                if (!active) return;
+                for (int rank = 0; rank < 2 * F.U; ++rank) {
+                    if (pair && (rank & 1) != own_strand) continue;
+                    const int sc = scores[(pair ? (rank & ~1) | h : rank) * 32 + lane];
+                    const int n = F.Lp + F.Ls + F.P * (rank / 2 + 1);
+                    const int min_len = min(m, n) / 2;
+                    if (sc < max(min_len, 30)) continue;
+                    if (sc > last_score || (sc == last_score && rank <= last_rank)) continue;   // already tried
+                    if (sc > cs) { cs = sc; cr = rank; }
+                }
+            };
+            int cs, cr;
+            pick(0x7fffffff, -1, cs, cr);
+            // Rounds: every lane that still has a candidate evaluates it — end coordinates from one warp-uniform
+            // packed pass (locate_packed), begin coordinates and the tag per lane — until all lanes are settled.
+            // Almost every read settles in the first round.
+            const int max_units_eff = F.clip ? (m + F.P - 1) / F.P : F.U;
+            auto own_code = [&](int j) { return FAST ? pair_half(codes[j * 32 + lane], h) : (int)codes[j * 32 + lane]; };
+            while (__any_sync(0xffffffffu, cr >= 0)) {
+                const bool pending = cr >= 0;
+                const int u = pending ? cr / 2 + 1 : 1, s = pending ? (cr & 1) : 0;
+                const int half = pair ? h : s;
+                int fast_end_ref = -1, fast_end_read = 0;
+                if constexpr (FAST) {
+                    if (FLANK * p.match < 30) {
+                        int u_main = 0;                      // first unit whose running main maximum equals cs
+                        if (pending) for (int k = 1; k <= u; ++k) if ((int)runs[(2 * (k - 1) + half) * 32 + lane] == cs) { u_main = k; break; }
+                        switch (instance_period(F.P)) {
+#define PCASE(PP) case PP: locate_packed<PP>(F, &lut, stab, stab2, colsel, suffix_table_ready, codes, lane, m, m_warp, bnd, gbnd, R, p.go, p.ge, one, F.P / PP, pending ? cs : 0x7fff, u, u_main, half, sa, sb, &fast_end_ref, &fast_end_read, cells2); break;
+                            PCASE(1) PCASE(2) PCASE(3) PCASE(4) PCASE(5) PCASE(7) PCASE(8) PCASE(9) PCASE(10) PCASE(11) PCASE(12)
 #undef PCASE
-                    }
-                    if (!pending) fast_end_ref = -1;
-                }
-            }
-            if (pending) {
-                const int n = F.Lp + F.Ls + F.P * u;
-                auto cc_f = [&](int i) { return fam_code(F, u, s, n, i); };
-                int end_ref = fast_end_ref, end_read = fast_end_read;
-                if (end_ref < 0) {
-                    // (generic kernel, or a scoring scheme outside the packed pass's preconditions)
-                    // Exact banding (sw_sweep.cuh): a path ending with score cs drifts at most `drift` diagonals
-                    // from the diagonal it starts on.  Forward: it starts at some (i0, j0) with i0 <= n - need,
-                    // j0 <= m - need, where need = ceil(cs / match) aligned pairs are indispensable.
-                    const int drift = sw_max_drift(cs, m, n, p.match, p.go, p.ge);
-                    const int need = (cs + p.match - 1) / p.match;
-                    sw_sweep<FAM_W2, 1, false>(m, m, n, rc_f, cc_f, &lut, bnd + lane, 32, p.go, p.ge, cs, &end_ref, &end_read,
-                                               nullptr, -(m - need) - drift, (n - need) + drift, &cells2);
-                }
-                bool settled = false;
-                if (end_ref >= 0) {      // (always: the score was produced by this very template)
-                    // Reverse: only a path leaving the corner (end_ref, end_read) can reach cs (Appendix A); it
-                    // lives in the (end_read+1) x (end_ref+1) rectangle, which bounds its aligned pairs and
-                    // therefore how far it can drift from the corner's diagonal.
-                    const int rdrift = sw_max_drift(cs, end_read + 1, end_ref + 1, p.match, p.go, p.ge);
-                    int ci = -1, rj = 0;
-                    if (rdrift == 0) {   // no gap affordable: walk the diagonal
-                        const int lim = min(end_read, end_ref) + 1;
-                        int h = 0;
-                        for (int k = 0; k < lim; ++k) {
-                            const int qc = codes[(end_read - k) * 32 + lane];
-                            const int sc = (int)sw_prmt(lut.w0[qc], lut.w1[qc], sw_sel32(fam_code(F, u, s, n, end_ref - k)));
-                            h = max(0, h + sc);
-                            if (h == cs) { ci = rj = k; break; }
                         }
-                        cells2 += (unsigned long long)lim;
-                    }
-                    if (ci < 0) {
-                        auto rc_r = [&](int j) { return (int)codes[(end_read - j) * 32 + lane]; };
-                        auto cc_r = [&](int i) { return fam_code(F, u, s, n, end_ref - i); };
-                        sw_sweep<FAM_W2, 1, false>(end_read + 1, end_read + 1, end_ref + 1, rc_r, cc_r, &lut, bnd + lane, 32,
-                                                   p.go, p.ge, cs, &ci, &rj, nullptr, -rdrift, rdrift, &cells2);
-                    }
-                    const int c_rb = end_ref - ci, c_qb = end_read - rj;
-                    const int t = sw_classify(cs, c_rb, end_ref, c_qb, end_read, m, n, u, F.P, max_units_eff);
-                    if (t != TREDSW_TAG_NONE) {
-                        tag = t; best_u = u; best_score = cs; rb = c_rb; re = end_ref; qb = c_qb; qe = end_read;
-                        best_rank = cr;
-                        settled = true;
+                        if (!pending) fast_end_ref = -1;
                     }
                 }
-                if (settled) cr = -1;
-                else { const int ls = cs, lr = cr; pick(ls, lr, cs, cr); }
+                if (pending) {
+                    const int n = F.Lp + F.Ls + F.P * u;
+                    auto cc_f = [&](int i) { return fam_code(F, u, s, n, i); };
+                    int end_ref = fast_end_ref, end_read = fast_end_read;
+                    if (end_ref < 0) {
+                        // (generic kernel, or a scoring scheme outside the packed pass's preconditions)
+                        // Exact banding (sw_sweep.cuh): a path ending with score cs drifts at most `drift` diagonals
+                        // from the diagonal it starts on.  Forward: it starts at some (i0, j0) with i0 <= n - need,
+                        // j0 <= m - need, where need = ceil(cs / match) aligned pairs are indispensable.
+                        const int drift = sw_max_drift(cs, m, n, p.match, p.go, p.ge);
+                        const int need = (cs + p.match - 1) / p.match;
+                        sw_sweep<FAM_W2, 1, false>(m, m, n, own_code, cc_f, &lut, bnd + lane, 32, p.go, p.ge, cs, &end_ref, &end_read,
+                                                   nullptr, -(m - need) - drift, (n - need) + drift, &cells2);
+                    }
+                    bool settled = false;
+                    if (end_ref >= 0) {      // (always: the score was produced by this very template)
+                        // Reverse: only a path leaving the corner (end_ref, end_read) can reach cs (Appendix A); it
+                        // lives in the (end_read+1) x (end_ref+1) rectangle, which bounds its aligned pairs and
+                        // therefore how far it can drift from the corner's diagonal.
+                        const int rdrift = sw_max_drift(cs, end_read + 1, end_ref + 1, p.match, p.go, p.ge);
+                        int ci = -1, rj = 0;
+                        if (rdrift == 0) {   // no gap affordable: walk the diagonal
+                            const int lim = min(end_read, end_ref) + 1;
+                            int hs = 0;
+                            for (int k = 0; k < lim; ++k) {
+                                const int qc = own_code(end_read - k);
+                                const int sc = (int)sw_prmt(lut.w0[qc], lut.w1[qc], sw_sel32(fam_code(F, u, s, n, end_ref - k)));
+                                hs = max(0, hs + sc);
+                                if (hs == cs) { ci = rj = k; break; }
+                            }
+                            cells2 += (unsigned long long)lim;
+                        }
+                        if (ci < 0) {
+                            auto rc_r = [&](int j) { return own_code(end_read - j); };
+                            auto cc_r = [&](int i) { return fam_code(F, u, s, n, end_ref - i); };
+                            sw_sweep<FAM_W2, 1, false>(end_read + 1, end_read + 1, end_ref + 1, rc_r, cc_r, &lut, bnd + lane, 32,
+                                                       p.go, p.ge, cs, &ci, &rj, nullptr, -rdrift, rdrift, &cells2);
+                        }
+                        const int c_rb = end_ref - ci, c_qb = end_read - rj;
+                        const int t = sw_classify(cs, c_rb, end_ref, c_qb, end_read, m, n, u, F.P, max_units_eff);
+                        if (t != TREDSW_TAG_NONE) {
+                            tag = t; best_u = u; best_score = cs; rb = c_rb; re = end_ref; qb = c_qb; qe = end_read;
+                            best_rank = cr;
+                            settled = true;
+                        }
+                    }
+                    if (settled) cr = -1;
+                    else { const int ls = cs, lr = cr; pick(ls, lr, cs, cr); }
+                }
+                __syncwarp();
             }
-            __syncwarp();
-        }
-        if (valid) {
-            int32_t *o = p.out + (int64_t)r * 8;
-            o[0] = too_long ? -1 : tag; o[1] = best_u; o[2] = best_score; o[3] = rb; o[4] = re; o[5] = qb; o[6] = qe;
-            o[7] = best_rank;
-        }
-        if (p.stats && valid && m > 0) {
-            unsigned long long sum_n = 0;
-            for (int u = 1; u <= F.U; ++u) sum_n += 2ull * (unsigned long long)(F.Lp + F.Ls + F.P * u);
-            alg += (unsigned long long)m * sum_n;
-            nal += (unsigned)(2 * F.U);
+            if (valid) {
+                int32_t *o = p.out + (int64_t)r * 8;
+                o[0] = too_long ? -1 : tag; o[1] = best_u; o[2] = best_score; o[3] = rb; o[4] = re; o[5] = qb; o[6] = qe;
+                o[7] = best_rank;
+            }
+            if (p.stats && active) {
+                unsigned long long sum_n = 0;
+                for (int u = 1; u <= F.U; ++u) sum_n += 2ull * (unsigned long long)(F.Lp + F.Ls + F.P * u);
+                alg += (unsigned long long)m * sum_n;
+                nal += (unsigned)(2 * F.U);
+            }
         }
     }
     if (p.stats) {
@@ -733,18 +794,26 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
 // (Z = aligned N bases, which score 0), and a run of length r shares r - q + 1 q-grams with the template:
 //     shared q-grams >= 30 + X (b - (q-1)) + g (go - (q-1)) - (q-1)(Z + 1) >= 30 - (q-1)(Z + 1)
 // for q - 1 <= min(b, go).  So a read with fewer than 30 - (q-1)(#N + 1) positions whose q-gram occurs in
-// ANY template of the family (per strand) has no candidate at all: it is given the "no tag" record here
+// ANY template of the family (on either strand) has no candidate at all: it is given the "no tag" record here
 // and never reaches the Smith-Waterman kernel.  Exact — no alignment is lost (parity tests cover it).
-struct QgramInfo { int q; int min_score; };       // q == 0: filter off for this family (N in the templates)
+// The same bound per strand gives the read's strand class: when only one strand reaches the threshold, no
+// template of the other strand can score min_score, so that strand can never be a candidate (pick() skips scores
+// below max(min_len, 30)) and the packed kernel computes the read on one strand only, two reads per lane.
+struct QgramInfo {
+    int q;                         // 0: filter off for this family (N in the templates)
+    int min_score;
+    int pair;                      // single-strand classes allowed (packed-kernel family, pairing not switched off)
+};
 constexpr int QTAB_WORDS = 256;                   // 4096 six-mers x 2 bits (forward / reverse-complement templates)
 
+// eff_group[r] = f * NCLASS + strand class, -2 when the read has no candidate, -1 when it has no family
 __global__ void prefilter_kernel(const int8_t *rbuf, const int64_t *roff, int nreads, const int32_t *read_family,
                                  int nfam, const tredsw_family *families, const uint32_t *qtab, const QgramInfo *qinfo,
-                                 int b_minus, int32_t *eff_family, unsigned long long *stats) {
+                                 int b_minus, int32_t *eff_group, unsigned long long *stats) {
     const int r = blockIdx.x * blockDim.x + threadIdx.x;
     unsigned long long alg = 0; unsigned nal = 0;
     if (r < nreads) {
-        int f = read_family[r];
+        int f = read_family[r], cls = CLASS_BOTH;
         if (f < 0 || f >= nfam) f = -1;
         if (f >= 0 && qinfo[f].q > 0) {
             const int q = qinfo[f].q;
@@ -770,9 +839,11 @@ __global__ void prefilter_kernel(const int8_t *rbuf, const int64_t *roff, int nr
                     alg = (unsigned long long)m * sum_n; nal = 2u * (unsigned)g.max_units;
                 }
                 f = -2;
+            } else if (qinfo[f].pair && (hf < thr || hr < thr)) {
+                cls = hf >= thr ? CLASS_FWD : CLASS_RC;
             }
         }
-        eff_family[r] = f;
+        eff_group[r] = f >= 0 ? f * NCLASS + cls : f;
     }
     if (stats) {
         for (int d = 16; d > 0; d >>= 1) { alg += __shfl_down_sync(0xffffffffu, alg, d); nal += __shfl_down_sync(0xffffffffu, nal, d); }
@@ -782,30 +853,34 @@ __global__ void prefilter_kernel(const int8_t *rbuf, const int64_t *roff, int nr
 
 // (reads arrive grouped by problem, so the lanes of a warp mostly share one family: the atomics are
 //  aggregated per warp and distinct family — one atomic instead of up to 32 on the same counter)
-__global__ void fam_count_kernel(const int32_t *read_family, int nreads, int nfam, int32_t *count) {
+__global__ void fam_count_kernel(const int32_t *read_group, int nreads, int ngroups, int32_t *count) {
     const int r = blockIdx.x * blockDim.x + threadIdx.x;
-    int f = r < nreads ? read_family[r] : -1;
-    if (f >= nfam) f = -1;
+    int f = r < nreads ? read_group[r] : -1;
+    if (f >= ngroups) f = -1;
     const unsigned peers = __match_any_sync(0xffffffffu, f);
     if (f >= 0 && (threadIdx.x & 31) == __ffs(peers) - 1) atomicAdd(&count[f], __popc(peers));
 }
-// single block: exclusive scans -> fam_start, chunk_start; cursor := fam_start
-__global__ void fam_scan_kernel(const int32_t *count, int nfam, const int32_t *perm, int32_t *fam_start,
+// single block: exclusive scans -> grp_start, chunk_start; cursor := grp_start.  An item holds 32 reads of a
+// "both" group, 64 of a single-strand group (two per lane).
+__global__ void fam_scan_kernel(const int32_t *count, int ngroups, const int32_t *perm, int32_t *grp_start,
                                 int32_t *chunk_start, int32_t *cursor) {
     if (threadIdx.x == 0 && blockIdx.x == 0) {
         int a = 0, b = 0;
-        for (int f = 0; f < nfam; ++f) { fam_start[f] = a; cursor[f] = a; a += count[f]; }
-        fam_start[nfam] = a;
-        for (int i = 0; i < nfam; ++i) { chunk_start[i] = b; b += (count[perm[i]] + 31) / 32; }
-        chunk_start[nfam] = b;
+        for (int g = 0; g < ngroups; ++g) { grp_start[g] = a; cursor[g] = a; a += count[g]; }
+        grp_start[ngroups] = a;
+        for (int i = 0; i < ngroups; ++i) {
+            const int per = perm[i] % NCLASS == CLASS_BOTH ? 32 : 64;
+            chunk_start[i] = b; b += (count[perm[i]] + per - 1) / per;
+        }
+        chunk_start[ngroups] = b;
     }
 }
-__global__ void fam_scatter_kernel(const int32_t *read_family, int nreads, int nfam, int32_t *cursor,
+__global__ void fam_scatter_kernel(const int32_t *read_group, int nreads, int ngroups, int32_t *cursor,
                                    int32_t *order, int32_t *out) {
     const int r = blockIdx.x * blockDim.x + threadIdx.x;
     const int lane = threadIdx.x & 31;
-    int f = r < nreads ? read_family[r] : -1;
-    if (f >= nfam) f = -1;
+    int f = r < nreads ? read_group[r] : -1;
+    if (f >= ngroups) f = -1;
     const unsigned peers = __match_any_sync(0xffffffffu, f);
     const int leader = __ffs(peers) - 1;
     int base = 0;
@@ -903,17 +978,18 @@ int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_
     }
     ClassifyParams p{};
     p.rbuf = d_rbuf; p.roff = d_roff; p.families = d_families; p.out = d_out;
+    const int ngroups = NCLASS * nfamilies;
     int32_t *w = d_work;
-    int32_t *d_count = w, *d_fam_start = w + nfamilies, *d_chunk_start = d_fam_start + nfamilies + 1,
-            *d_cursor = d_chunk_start + nfamilies + 1, *d_order = d_cursor + nfamilies;
-    CUDA_TRY(cudaMemsetAsync(d_count, 0, nfamilies * sizeof(int32_t), ctx->stream));
+    int32_t *d_count = w, *d_grp_start = w + ngroups, *d_chunk_start = d_grp_start + ngroups + 1,
+            *d_cursor = d_chunk_start + ngroups + 1, *d_order = d_cursor + ngroups;
+    CUDA_TRY(cudaMemsetAsync(d_count, 0, ngroups * sizeof(int32_t), ctx->stream));
     const int tb = 256, nb = (nreads + tb - 1) / tb;
-    p.order = d_order; p.fam_start = d_fam_start; p.chunk_start = d_chunk_start;
-    p.nfamilies = nfamilies; p.go = gap_open; p.ge = gap_extend; p.max_rows = max_rows;
+    p.order = d_order; p.grp_start = d_grp_start; p.chunk_start = d_chunk_start;
+    p.ngroups = ngroups; p.go = gap_open; p.ge = gap_extend; p.max_rows = max_rows;
     p.allow_fast = allow_fast ? 1 : 0;
     p.match = max_match > 0 ? max_match : 1;
     p.stats = d_stats;
-    const int nitems_bound = nreads / 32 + nfamilies + 1;
+    const int nitems_bound = nreads / 32 + ngroups + 1;
     int nctas = 0;
     if ((rc = persistent_ctas(ctx, smem, static_smem, need_fast, need_generic, &nctas))) return rc;
     if (nctas > nitems_bound) nctas = nitems_bound;
@@ -921,7 +997,7 @@ int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_
     const size_t score_bytes = (size_t)nctas * 2 * max_u * 32 * sizeof(uint16_t);
     const size_t pot_bytes = (size_t)nctas * rows_alloc * 32 * sizeof(uint32_t);
     const size_t gbnd_bytes = pot_bytes * (nslots + 1);
-    const size_t perm_bytes = (((size_t)nfamilies * sizeof(int32_t)) + 15) & ~(size_t)15;
+    const size_t perm_bytes = (((size_t)ngroups * sizeof(int32_t)) + 15) & ~(size_t)15;
     const size_t qtab_bytes = (size_t)nfamilies * QTAB_WORDS * sizeof(uint32_t);
     const size_t qinfo_bytes = (((size_t)nfamilies * sizeof(QgramInfo)) + 15) & ~(size_t)15;
     const size_t eff_bytes = (((size_t)nreads * sizeof(int32_t)) + 15) & ~(size_t)15;
@@ -937,17 +1013,19 @@ int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_
     {   // Item order: families grouped by loop instantiation (measured: mixing instantiations on an SM costs far
         // more than any order could gain — they compete for the instruction cache), the groups with the fewest
         // families first: their items run cold code and are the slowest, so they must not form the tail of the
-        // launch; the big uniform group (period 3 for the catalogue) finishes it with short, even items.
-        std::vector<int32_t> perm(nfamilies);
+        // launch; the big uniform group (period 3 for the catalogue) finishes it with short, even items.  The strand
+        // classes of a family stay together, in class order, inside its instantiation's run.
+        std::vector<int32_t> perm(ngroups);
         int group_size[33] = {0};
-        for (int f = 0; f < nfamilies; ++f) { perm[f] = f; ++group_size[instance_period(h_families[f].period)]; }
+        for (int f = 0; f < nfamilies; ++f) ++group_size[instance_period(h_families[f].period)];
+        for (int g = 0; g < ngroups; ++g) perm[g] = g;
         std::stable_sort(perm.begin(), perm.end(), [&](int a, int b) {
-            const int pa = instance_period(h_families[a].period), pb = instance_period(h_families[b].period);
+            const int pa = instance_period(h_families[a / NCLASS].period), pb = instance_period(h_families[b / NCLASS].period);
             if (group_size[pa] != group_size[pb]) return group_size[pa] < group_size[pb];
             return pa < pb; });
         h_perm.swap(perm);
     }
-    p.fam_perm = d_perm;
+    p.grp_perm = d_perm;
     // q-gram pre-filter tables: per family 4096 x 2 bits (q-grams of all forward / all reverse-complement templates)
     uint32_t *d_qtab = reinterpret_cast<uint32_t *>(reinterpret_cast<unsigned char *>(d_perm) + perm_bytes);
     QgramInfo *d_qinfo = reinterpret_cast<QgramInfo *>(reinterpret_cast<unsigned char *>(d_qtab) + qtab_bytes);
@@ -968,6 +1046,8 @@ int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_
         if (q > gap_open + 1) q = gap_open + 1;
         static const bool env_off = getenv("TREDSW_NO_PREFILTER") != nullptr;
         const bool usable = n_ok && diag_ok && q >= 4 && !env_off;
+        // (read on every call, so that one process can compare both modes)
+        const bool pairing = getenv("TREDSW_NO_STRAND_PAIRING") == nullptr;
         std::vector<uint32_t> tab((size_t)nfamilies * QTAB_WORDS, 0u);
         std::vector<QgramInfo> info(nfamilies);
         std::vector<int8_t> t;
@@ -979,6 +1059,7 @@ int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_
             // q-gram with N's is expanded to the concrete q-grams it is compatible with.
             info[f].q = usable ? q : 0;
             info[f].min_score = 30;                         // bam_parser.py:134: min_score = max(min_len, 30)
+            info[f].pair = pairing && allow_fast && g.prefix_len == FLANK && g.suffix_len == FLANK && g.period <= 12;
             if (!info[f].q) continue;
             bool too_many_n = false;
             // every q-gram of a template with u >= u0 units already occurs in the template with u0 units
@@ -1023,7 +1104,7 @@ int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_
         // perm | qtab | qinfo through the page-locked table staging (see stage_small): no pageable copy sits
         // between the input transfer and the kernels of a call
         const void *srcs[4] = {h_perm.data(), tab.data(), info.data(), mat25};
-        const size_t sizes[4] = {(size_t)nfamilies * sizeof(int32_t), qtab_bytes, (size_t)nfamilies * sizeof(QgramInfo), 25};
+        const size_t sizes[4] = {(size_t)ngroups * sizeof(int32_t), qtab_bytes, (size_t)nfamilies * sizeof(QgramInfo), 25};
         size_t offs[4];
         if ((rc = stage_small(ctx, ctx->h_tab, srcs, sizes, 4, offs))) return rc;
         const unsigned char *ht = ctx->h_tab.as<unsigned char>();
@@ -1035,9 +1116,9 @@ int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_
     ctx->mark(0);
     prefilter_kernel<<<nb, tb, 0, ctx->stream>>>(d_rbuf, d_roff, nreads, d_read_family, nfamilies, d_families, d_qtab,
                                                  d_qinfo, b_minus, d_eff, d_stats);
-    fam_count_kernel<<<nb, tb, 0, ctx->stream>>>(d_eff, nreads, nfamilies, d_count);
-    fam_scan_kernel<<<1, 32, 0, ctx->stream>>>(d_count, nfamilies, d_perm, d_fam_start, d_chunk_start, d_cursor);
-    fam_scatter_kernel<<<nb, tb, 0, ctx->stream>>>(d_eff, nreads, nfamilies, d_cursor, d_order, p.out);
+    fam_count_kernel<<<nb, tb, 0, ctx->stream>>>(d_eff, nreads, ngroups, d_count);
+    fam_scan_kernel<<<1, 32, 0, ctx->stream>>>(d_count, ngroups, d_perm, d_grp_start, d_chunk_start, d_cursor);
+    fam_scatter_kernel<<<nb, tb, 0, ctx->stream>>>(d_eff, nreads, ngroups, d_cursor, d_order, p.out);
     CUDA_TRY(cudaGetLastError());
     ctx->launches += 4;
     CUDA_TRY(cudaMemsetAsync(p.counter, 0, 2 * sizeof(int32_t), ctx->stream));
@@ -1074,7 +1155,7 @@ extern "C" int tredsw_classify_reads(tredsw_ctx *ctx, const int8_t *rbuf, const 
     if ((rc = stage_in(ctx, ctx->d_rfam, read_family, (size_t)nreads, flags, &d_rfam))) return rc;
     if ((rc = stage_in(ctx, ctx->d_fam, families, (size_t)nfamilies, flags, &d_fam))) return rc;
     if ((rc = ctx->d_out.ensure((size_t)nreads * 8 * sizeof(int32_t)))) return rc;
-    if ((rc = ctx->d_work.ensure(((size_t)4 * nfamilies + 2 + nreads) * sizeof(int32_t)))) return rc;
+    if ((rc = ctx->d_work.ensure(((size_t)4 * NCLASS * nfamilies + 2 + nreads) * sizeof(int32_t)))) return rc;
     if ((rc = ctx->d_stats.ensure(4 * sizeof(unsigned long long)))) return rc;
     CUDA_TRY(cudaMemsetAsync(ctx->d_stats.p, 0, 4 * sizeof(unsigned long long), ctx->stream));
     if ((rc = tredsw_internal_classify(ctx, d_rbuf, d_roff, nreads, d_rfam, d_fam, families, nfamilies, max_m, mat25,
