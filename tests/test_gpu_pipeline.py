@@ -94,6 +94,34 @@ def test_all_catalogue_loci_on_both_fixtures():
                 assert calls[name + ".PP"] == -1 and calls[name + ".CI"] == "" and calls[name + ".label"] == "missing"
 
 
+def test_unindexed_bams_equal_the_indexed_run_and_the_oracle(tmp_path):
+    """BAMs without a .bai: the Python reader builds the evidence records and the same fused call genotypes them.
+    The calls equal those of the indexed files (floats at the bar of test_runBam_equals_batched_run) and the CPU
+    oracle's at 1e-9.  Every catalogue locus without the alt regions (each alt region is a scan of the whole
+    unindexed file), and the locus with reads with them."""
+    import shutil
+    from tredparse_b200 import tred as T, bamio
+    from tredparse_b200.meta import TREDsRepo
+    from oracle import genotype_oracle, evidence_oracle as evo
+    repo = TREDsRepo()
+    step, w = _models()
+    for sample, hit in CASES:
+        bam = os.path.join(GOLDEN, sample + ".mini.bam")
+        copy = str(tmp_path / (sample + ".noindex.bam"))
+        shutil.copy(bam, copy)
+        sam = bamio.AlignmentFile(bam)
+        for names, alts in ((list(repo.names), False), ([hit], True)):
+            indexed, unindexed = [T.run((sample, path, repo, names, 300, False, False, alts, True, "INFO"))["tredCalls"]
+                                  for path in (bam, copy)]
+            _close(unindexed, indexed, 1e-12)
+            assert unindexed[hit + ".1"] > 0
+            for name in names:
+                exp = genotype_oracle.genotype_locus(sam, repo[name], evo.read_length(sam), step, w, alts=alts)[0]
+                for k, v in exp.items():
+                    _close(unindexed[name + "." + k], v)
+        sam.close()
+
+
 def test_cli_main_writes_reference_layout_json(tmp_path):
     from tredparse_b200 import tred as T
     csv = tmp_path / "samples.csv"
@@ -114,7 +142,7 @@ def test_cli_main_writes_reference_layout_json(tmp_path):
 
 def test_cohort_pipeline_from_native_ingest_equals_run():
     """BAM -> native one-pass ingest (csrc/ingest.cpp) -> all-device cohort pipeline == tred.run's calls
-    (which go BamParser / IntegratedCaller API -> per-stage kernels), and the README's 15|41."""
+    (GPU ingest -> fused call on its device buffers), and the README's 15|41."""
     from tredparse_b200 import tred as T, cohort, ingest
     from tredparse_b200.meta import TREDsRepo
     repo = TREDsRepo()

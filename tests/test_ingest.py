@@ -7,7 +7,7 @@ import os
 import numpy as np
 import pytest
 
-from tredparse_b200 import bamio, ingest, ssw
+from tredparse_b200 import bamio, bam_parser, ingest, ssw
 from tredparse_b200.bam_parser import BamParser, PEextractor, BamDepth
 from tredparse_b200.meta import TREDsRepo
 from tredparse_b200.utils import InputParams
@@ -15,6 +15,7 @@ from tredparse_b200.utils import InputParams
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
 CASES = [("t001", "HD"), ("t002", "DM1")]
 BAMS = [(s, t, os.path.join(GOLDEN, s + ".mini.bam")) for s, t in CASES]
+EMPTY = ("t001", "DM1", os.path.join(GOLDEN, "t001.mini.bam"))      # chr19: no reads in the chr4 mini BAM
 
 
 @pytest.fixture(scope="module")
@@ -35,21 +36,34 @@ def _python_path(bam, tredname, repo, alts):
     return bp, reads, pe, depth
 
 
-@pytest.mark.parametrize("sample,tredname,bam", BAMS, ids=[b[0] for b in BAMS])
+@pytest.mark.parametrize("sample,tredname,bam", BAMS + [EMPTY], ids=[b[0] for b in BAMS] + ["t001-DM1"])
 @pytest.mark.parametrize("alts", [False, True])
 def test_extract_locus_equals_python_host_path(sample, tredname, bam, alts, repo):
     bp, reads, pe, depth = _python_path(bam, tredname, repo, alts)
     with ingest.BamIngest(bam) as ing:
         ev = ing.extract_locus(repo[tredname], 150, alts=bp.alt if alts else (), want_names=True)
-    assert ev.nreads == len(reads) > 50
+    empty = (sample, tredname, bam) == EMPTY
+    assert ev.nreads == len(reads) and (empty or len(reads) > 50)
     assert ev.names == [r.query_name for r in reads]
     assert ev.read_strings() == ["".join(c if c in "ACGT" else "N" for c in r.query_sequence.upper()) for r in reads]
-    assert np.array_equal(ev.reads, np.concatenate([ssw.encode(r.query_sequence) for r in reads]))
-    assert list(ev.global_lens) == list(pe.global_lens) and len(pe.global_lens) > 1000
-    assert list(ev.target_lens) == list(pe.target_lens) and len(pe.target_lens) >= 5
+    assert np.array_equal(ev.reads, np.concatenate([ssw.encode(r.query_sequence) for r in reads] or [np.zeros(0, np.int8)]))
+    assert list(ev.global_lens) == list(pe.global_lens) and (empty or len(pe.global_lens) > 1000)
+    assert list(ev.target_lens) == list(pe.target_lens) and (empty or len(pe.target_lens) >= 5)
     assert ev.depth == depth
     if not alts:
         assert ev.n_unmapped == sum(1 for r in reads if r.is_unmapped)
+    # the same record built from the Python reader (BAMs without a usable index, contigs the native reader lacks)
+    _assert_same_record(bam_parser.extract_locus(bam, repo, tredname, 150, alts, False, logging.getLogger()), ev)
+
+
+def _assert_same_record(a, b):
+    """two ingest.LocusEvidence field for field, array dtypes included"""
+    for f in ingest.LocusEvidence.__slots__:
+        x, y = getattr(a, f), getattr(b, f)
+        if isinstance(y, np.ndarray):
+            assert isinstance(x, np.ndarray) and x.dtype == y.dtype and np.array_equal(x, y), f
+        else:
+            assert type(x) is type(y) and x == y, f
 
 
 def test_missing_locus_and_errors(repo):
@@ -161,15 +175,15 @@ def _evidence_equal(a, b):
 
 
 @pytest.mark.parametrize("sample,tredname,bam", BAMS, ids=[b[0] for b in BAMS])
-def test_threaded_ingest_equals_serial(sample, tredname, bam, repo):
+def test_threaded_ingest_records_equal_serial(sample, tredname, bam, repo):
     from tredparse_b200 import tred as tredmod
     log = logging.getLogger()
     names = list(repo.names)
-    ev1, d1 = tredmod.ingest_loci(bam, repo, names, 150, True, False, log, threads=1)
-    ev4, d4 = tredmod.ingest_loci(bam, repo, names, 150, True, False, log, threads=4)
-    assert d1 == d4 and set(ev1) == set(ev4) and tredname in ev1
+    ev1 = tredmod.ingest_loci(bam, repo, names, 150, True, False, log, threads=1)
+    ev4 = tredmod.ingest_loci(bam, repo, names, 150, True, False, log, threads=4)
+    assert set(ev1) == set(ev4) == set(names)
     assert all(_evidence_equal(ev1[k], ev4[k]) for k in ev1)
-    assert ev1[tredname].nreads > 50 and d1[tredname] > 5
+    assert ev1[tredname].nreads > 50 and ev1[tredname].depth > 5
     # clones are independent handles that share the index
     with ingest.BamIngest(bam) as ing:
         c = ing.clone()
@@ -205,6 +219,69 @@ def test_run_wiring_without_the_gpu(monkeypatch, repo):
     assert dm1[4].nreads == 0 and dm1[3] == 0.0                          # chr19: nothing in the chr4 mini BAM
     assert seen["kw"]["maxinsert"] == 300 and seen["kw"]["fullsearch"] is False
     assert seen["kw"]["clip"] is False and seen["kw"]["repeatpairs"] is True
+
+
+def _unindexed_copy(tmp_path, sample):
+    import shutil
+    path = str(tmp_path / (sample + ".noindex.bam"))
+    shutil.copy(os.path.join(GOLDEN, sample + ".mini.bam"), path)
+    return path
+
+
+def test_unindexed_bam_gets_the_native_evidence_records(monkeypatch, tmp_path, repo):
+    """A BAM without a .bai: the native reader cannot open it, the Python reader builds every locus' record, and the
+    records equal the native reader's on the indexed file — one genotyping batch, whichever reader served a locus."""
+    from tredparse_b200 import tred as tredmod
+    monkeypatch.setattr(tredmod, "GPU_INGEST", False)
+    bam = os.path.join(GOLDEN, "t001.mini.bam")
+    copy = _unindexed_copy(tmp_path, "t001")
+    with pytest.raises(IOError):
+        ingest.BamIngest(copy)
+    # every catalogue locus without the alt regions (each alt region is a scan of the whole unindexed file), and HD
+    # with them
+    for names, alts in ((list(repo.names), False), (["HD"], True)):
+        args, out, items, where, device_batch = tredmod.prepare_chunk(
+            [("t001", copy, repo, names, 300, False, False, alts, True, "INFO")])
+        assert device_batch is None and where == [(0, t) for t in names]
+        gender = "Female" if len(names) > 1 else "Unknown"              # (gender only with an X-linked locus)
+        assert out[0]["tredCalls"]["inferredGender"] == gender and out[0]["tredCalls"]["readLen"] == 150
+        native = tredmod.ingest_loci(bam, repo, names, 150, alts, False, logging.getLogger())
+        for t, (tred, readlen, g, depth, ev) in zip(names, items):
+            assert tred is repo[t] and readlen == 150 and g == gender and depth == ev.depth
+            _assert_same_record(ev, native[t])
+        assert items[names.index("HD")][4].nreads > 50
+
+
+def test_a_failing_genotyping_call_fails_its_chunk(monkeypatch, repo):
+    """No second route: when the fused call raises, run_chunk raises and run_chunks(isolate=True) reports the chunk's
+    samples as errors; the BAM is not read again."""
+    from tredparse_b200 import tred as tredmod
+    monkeypatch.setattr(tredmod, "GPU_INGEST", False)
+    reads, calls = [], []
+    ingest_loci = tredmod.ingest_loci
+
+    def counted_ingest_loci(bam, *a, **k):
+        reads.append(os.path.basename(bam))
+        return ingest_loci(bam, *a, **k)
+
+    def failing_genotype_evidence(items, **kw):
+        calls.append(len(items))
+        if len(calls) == 1:
+            raise RuntimeError("fused call failed")
+        return [{"1": 5} for _ in items]
+    monkeypatch.setattr(tredmod, "ingest_loci", counted_ingest_loci)
+    monkeypatch.setattr(tredmod, "genotype_evidence", failing_genotype_evidence)
+    tasks = [(s, os.path.join(GOLDEN, s + ".mini.bam"), repo, [t], 300, False, False, True, True, "INFO")
+             for s, t in CASES]
+    got = list(tredmod.run_chunks(tasks, chunk=1, isolate=True))
+    assert [r["samplekey"] for r in got] == ["t001", "t002"]
+    assert got[0]["tredCalls"] == {} and "fused call failed" in got[0]["error"]
+    assert "error" not in got[1] and got[1]["tredCalls"]["DM1.1"] == 5
+    assert reads == ["t001.mini.bam", "t002.mini.bam"] and calls == [1, 1]
+    del reads[:], calls[:]
+    with pytest.raises(RuntimeError, match="fused call failed"):
+        tredmod.run_chunk(tasks[:1])
+    assert reads == ["t001.mini.bam"] and calls == [1]
 
 
 # ---- corrupt input must not take the process down ---------------------------------------------------------------

@@ -91,7 +91,7 @@ def main():
         tredmod.ingest_loci(a.bam, repo, names, 150, True, False, log, threads=th)
         t0 = time.perf_counter()
         for _ in range(a.reps):
-            ev, _ = tredmod.ingest_loci(a.bam, repo, names, 150, True, False, log, threads=th)
+            ev = tredmod.ingest_loci(a.bam, repo, names, 150, True, False, log, threads=th)
         dt = (time.perf_counter() - t0) / a.reps
         print("sample of {} loci, {} thread(s): {:8.2f} ms  ({:.0f} loci/s, {} reads)".format(
             len(names), th, dt * 1e3, len(names) / dt, sum(e.nreads for e in ev.values())))

@@ -4,7 +4,8 @@ Evidence extraction from a BAM — host side of the hot path.
 Keeps the reference's ``tredparse/bam_parser.py`` interface: ``BamParser(inputParams).parse()`` with
 ``counts / details / rept / ploidy / READLEN / depth / repeatSize`` (:35-287), ``BamParserResults``
 (:290-313), ``PEextractor`` (:316-369), ``BamReadLen`` (:372-391), ``BamDepth`` (:394-429),
-``read_alignment`` (:432-436), ``rc`` (:448-450).
+``read_alignment`` (:432-436), ``rc`` (:448-450).  ``extract_locus`` packs what ``select_reads``,
+``PEextractor`` and ``BamDepth`` read for one locus into the ``ingest.LocusEvidence`` the native reader produces.
 
 What runs where:
   host   BAM window fetches (own BGZF/BAI reader instead of pysam), read selection rules
@@ -145,6 +146,7 @@ class BamParser:
                         self.logger.debug("Fetch failed for region {}:{}-{} ({})".format(c, s, e, ex))
                         continue
         self.logger.debug("A total of {} unmapped reads in {}:{}-{}".format(n_unmapped, chr, start, end))
+        self.n_unmapped = n_unmapped
         return selected
 
     def absorb(self, names, seqs, results):
@@ -349,3 +351,32 @@ class BamDepth:
                 ing.close()
         self.logger.debug("Y depths (first {} regions): {}".format(N, np.array(depths)))
         return float(np.median(depths))
+
+
+def extract_locus(bam, repo, tredName, readlen, alts, clip, logger):
+    """``ingest.BamIngest.extract_locus(..., want_names=True)`` made of this module's readers, for a BAM the native
+    reader cannot serve (no usable index, contig unknown to it): the reads ``BamParser.select_reads`` keeps,
+    ``PEextractor``'s pair lengths and ``BamDepth.region_depth`` of the +-SPAN window.  A depth lookup that raises
+    gives depth 30, like the reference (tred.py:236-240); a failure to read the reads propagates.
+    :return: ingest.LocusEvidence"""
+    from .ingest import LocusEvidence
+    from .utils import InputParams
+    bp = BamParser(InputParams(bam=bam, READLEN=readlen, repo=repo, tredName=tredName, clip=clip, alts=alts))
+    sam = read_alignment(bam)
+    try:
+        reads = bp.select_reads(sam)
+    finally:
+        sam.close()
+    pe = PEextractor(bp)
+    ev = LocusEvidence()
+    ev.reads, ev.roff = ssw.flatten([r.query_sequence for r in reads])
+    ev.names = [r.query_name for r in reads]
+    ev.global_lens = np.array(pe.global_lens, dtype=np.int32)
+    ev.target_lens = np.array(pe.target_lens, dtype=np.int32)
+    ev.n_unmapped = bp.n_unmapped
+    try:
+        ev.depth = BamDepth(bam, repo.ref, logger).region_depth(bp.chr, max(0, bp.startRepeat - SPAN), bp.endRepeat + SPAN)
+    except Exception as e:
+        logger.error("Exception on `{}` {} ({}). Set depth={}".format(bam, tredName, e, 30))
+        ev.depth = 30
+    return ev

@@ -7,8 +7,14 @@ Keeps the reference's ``tredparse/tred.py`` surface: ``set_argparse`` (:64-103),
 (:296-313), ``to_vcf`` (:316-374), ``main`` (:451-539) and the JSON layout (SURVEY.md Appendix C).
 
 Differences that are the point of this build:
-  * ``run`` batches *all loci of a sample* into one Smith-Waterman launch and one likelihood-grid launch
-    instead of looping ``runBam`` per locus (``runBam`` is still there and gives identical results);
+  * every (sample, locus) gets one evidence record (``ingest.LocusEvidence``: reads, names, pair lengths, depth),
+    from the GPU ingest, the native host reader or — for a BAM without a usable index or a contig the native
+    reader does not know — the Python reader (``bam_parser.extract_locus``); a locus whose window cannot be read
+    gets no record and no call;
+  * ``run`` / ``run_chunk`` genotype *all loci of a chunk of samples* in one fused device call
+    (``genotype_evidence``) instead of looping ``runBam`` per locus (``runBam`` is still there and gives identical
+    results).  If that call fails, the chunk fails: ``run_chunks(..., isolate=True)`` turns that into error records
+    for its samples;
   * samples are sharded over GPUs (``--gpus``), one worker process per GPU, instead of over CPU cores
     with ``multiprocessing.Pool`` (tred.py:528-532).  No collective: workers return their dicts.
 S3 / ``@HLI-id`` inputs are out of scope (SURVEY.md §2 row 5).
@@ -26,12 +32,10 @@ from datetime import datetime as dt, timedelta
 
 import numpy as np
 
-from . import __version__, ssw
-from .utils import DefaultHelpParser, InputParams, mkdir
-from .bam_parser import BamDepth, BamReadLen, BamParser, BamParserResults, PEextractor, SPAN, \
-    FLANKMATCH, read_alignment
-from .models import IntegratedCaller, GridBatch, MIN_SPANNING_PAIRS, pe_kde, mean_std, histogram, \
-    calc_label
+from . import __version__
+from .utils import DefaultHelpParser, mkdir
+from .bam_parser import BamDepth, BamReadLen, BamParser, BamParserResults, extract_locus, read_alignment
+from .models import IntegratedCaller, mean_std, histogram
 from .meta import TREDsRepo
 
 logging.basicConfig()
@@ -128,105 +132,24 @@ def runBam(inputParams):
     return BamParserResults(inputParams, bp, integratedCaller)
 
 
-class _Caller:
-    """Result holder with IntegratedCaller's result attributes (batched path)."""
+def alt_regions(tred, ref, alts, clip):
+    """The mis-mapping regions whose reads are added to a locus (bam_parser.py:215-243): none without alts or with
+    clipped reads; contig names without the 'chr' prefix on a '_nochr' reference."""
+    if not alts or clip:
+        return []
+    return [(c[3:] if "nochr" in ref else c, s, e) for (c, s, e) in tred.alt]
 
 
-class _IngestPE:
-    """PEextractor's attributes filled from a native one-pass extraction (ingest.LocusEvidence)."""
-
-    def __init__(self, bp, ev):
-        self.ref = bp.referenceLen
-        self.global_lens = [int(x) for x in ev.global_lens]
-        self.target_lens = [int(x) for x in ev.target_lens]
-        self.MINPE = bp.endRepeat - bp.startRepeat + 2 * FLANKMATCH + 2
-
-
-def locus_evidence(ing, ip_or_bp, tred, readlen, alts, clip, ref):
+def locus_evidence(ing, tred, readlen, alts, clip, ref):
     """One native pass over the BAM for one locus (reads + names + pair distances + depth)."""
-    alt = []
-    if alts and not clip:
-        for (c, s, e) in tred.alt:
-            alt.append((c[3:] if "nochr" in ref else c, s, e))
-    return ing.extract_locus(tred, readlen, alts=alt, want_names=True)
-
-
-def run_batched(ips, evidence=None):
-    """All loci of one sample: one SW launch + one KDE launch + one grid launch.
-    :param ips: list of InputParams (same BAM).  :param evidence: {tredName: ingest.LocusEvidence} from the
-    native one-pass BAM ingest (optional; without it the Python BAM reader makes the reference's passes).
-    :return: list of BamParserResults (None on failure)."""
-    evidence = evidence or {}
-    parsers, all_seqs, all_names, rfam, fams, spans = [], [], [], [], [], []
-    for ip in ips:
-        bp = BamParser(ip)
-        ev = evidence.get(ip.tredName)
-        if ev is not None:
-            seqs, names = ev.read_strings(), ev.names
-        else:
-            sam = read_alignment(bp.bam)
-            reads = bp.select_reads(sam)
-            sam.close()
-            seqs, names = [r.query_sequence for r in reads], [r.query_name for r in reads]
-        fams.append(bp._buildDB())
-        spans.append((len(all_seqs), len(all_seqs) + len(seqs)))
-        all_seqs += seqs
-        all_names += names
-        rfam += [len(fams) - 1] * len(seqs)
-        parsers.append(bp)
-    if all_seqs:
-        out = ssw.classify_reads(all_seqs, np.array(rfam, dtype=np.int32), np.concatenate(fams))
-    else:
-        out = np.zeros((0, 8), dtype=np.int32)
-    pes, need_kde = [], []
-    for bp, (a, b) in zip(parsers, spans):
-        bp.sw_results = out[a:b]
-        bp.absorb(all_names[a:b], all_seqs[a:b], out[a:b])
-        ev = evidence.get(bp.inputParams.tredName)
-        pe = _IngestPE(bp, ev) if ev is not None else PEextractor(bp)
-        pes.append(pe)
-        if len(pe.global_lens) >= 100 and len(pe.target_lens) >= MIN_SPANNING_PAIRS:
-            need_kde.append(len(pes) - 1)
-    pdfs = {}
-    if need_kde:
-        k = pe_kde([pes[i].global_lens for i in need_kde])
-        pdfs = {i: k[j] for j, i in enumerate(need_kde)}
-    batch = GridBatch()
-    idx = []
-    for i, (ip, bp, pe) in enumerate(zip(ips, parsers, pes)):
-        period = bp.repeatSize
-        obs_spanning = dict((k * period, v) for k, v in bp.counts["FULL"].items())
-        obs_partial = dict((k * period, v) for k, v in bp.counts["PREF"].items())
-        idx.append(batch.add(bp.tred, period, bp.READLEN, obs_spanning, obs_partial, bp.rept, bp.ploidy,
-                             bp.depth, pdfs.get(i), pe.target_lens, pe.ref, pe.MINPE,
-                             maxinsert=ip.kwargs["maxinsert"], fullsearch=ip.kwargs["fullsearch"]))
-    batch.run()
-    results = []
-    for ip, bp, pe, gi in zip(ips, parsers, pes, idx):
-        c = _Caller()
-        c.PEDP, c.PEG, c.PET = len(pe.target_lens), mean_std(pe.global_lens), mean_std(pe.target_lens)
-        c.P_PEG, c.P_PET = histogram(pe.global_lens), histogram(pe.target_lens)
-        period = bp.repeatSize
-        if gi < 0:
-            alleles, PP, CIs = (-1, -1), -1, None
-            c.P_h1 = c.P_h2 = c.P_h1h2 = ""
-        else:
-            s = batch.summarize(gi)
-            alleles, PP, CIs = s["alleles"], s["PP"], s["CIs"]
-            c.P_h1, c.P_h2, c.P_h1h2 = s["P_h1"], s["P_h2"], s["P_h1h2"]
-        c.alleles = sorted(x // period for x in alleles)
-        c.label = calc_label(bp.tred, c.alleles)
-        c.CI = "{}-{}|{}-{}".format(*CIs) if CIs else ""
-        c.PP = PP
-        results.append(BamParserResults(ip, bp, c))
-    return results
+    return ing.extract_locus(tred, readlen, alts=alt_regions(tred, ref, alts, clip), want_names=True)
 
 
 TAGNAME = {1: "FULL", 2: "PREF", 3: "POST", 4: "REPT"}
 
 
 def genotype_evidence(items, maxinsert=300, fullsearch=False, clip=False, repeatpairs=True, ctx=None, device_batch=None):
-    """The fused device path for loci whose evidence came from the native ingest: ONE ``tredsw_genotype_batch_ex``
+    """The fused device path, whichever reader produced the evidence: ONE ``tredsw_genotype_batch_ex``
     call (Smith-Waterman + classification -> tallies -> candidate ranges -> KDE -> likelihood grid -> call / CI / PP
     / label -> sparse posteriors) over any number of (sample, locus) problems, then the reference's per-locus
     result fields (tred.py:251-275) assembled from what comes back.
@@ -239,7 +162,6 @@ def genotype_evidence(items, maxinsert=300, fullsearch=False, clip=False, repeat
     if not items:
         return []
     ploidy_of = lambda tred, gender: 1 if (gender == "Male" and tred.is_xlinked) else tred.ploidy
-    out = None
     if device_batch is not None:
         keys, fam_of = {}, []
         for tred, readlen, gender, depth, ev in items:
@@ -254,7 +176,7 @@ def genotype_evidence(items, maxinsert=300, fullsearch=False, clip=False, repeat
             names=None if (repeatpairs or clip) else [it[4].names for it in items],
             maxinsert=maxinsert, fullsearch=fullsearch, clip=clip, repeatpairs=repeatpairs)
         out = batch.run_ingest(ctx or _lib.default_context(), want_reads=True, want_hist=True, want_post=True)
-    if out is None:
+    else:
         problems = []
         for tred, readlen, gender, depth, ev in items:
             pr = Problem()
@@ -301,38 +223,30 @@ INGEST_THREADS = int(os.environ.get("TREDSW_INGEST_THREADS", "0")) or min(8, os.
 
 
 def ingest_loci(bam, repo, tredNames, READLEN, alts, clip, logger, threads=None, want_names=True):
-    """Evidence and depth of every requested locus of one BAM.
+    """Evidence of every requested locus of one BAM.
     Native ingest (csrc/ingest.cpp): one indexed pass per locus yields reads, pair distances AND depth; the loci
     are dealt to `threads` host threads, each with its own clone of the BAM handle (own file descriptor, shared
-    index; ctypes releases the GIL during the pass).  The Python BAM reader (three passes per locus, like the
-    reference's pysam calls, tred.py:225-243) is the fallback for the depth when a BAM has no usable index or the
-    contig is missing; a locus whose extraction fails gets depth 30 like the reference (tred.py:236-240).
-    :return: ({tredName: ingest.LocusEvidence}, {tredName: depth})"""
+    index; ctypes releases the GIL during the pass).  When the BAM has no usable index or the native reader does not
+    know the contig, ``bam_parser.extract_locus`` builds the same record with the Python BAM reader (three passes per
+    locus, like the reference's pysam calls, tred.py:225-243).  A locus whose window cannot be read (truncated /
+    corrupt BAM) gets no record and so no call: the reference's `except Exception: continue` (tred.py:245-249).
+    :return: {tredName: ingest.LocusEvidence}"""
     ing = None
     try:
         from .ingest import BamIngest
         ing = BamIngest(bam_path(bam))
     except Exception as e:
         logger.debug("native BAM ingest unavailable for `{}` ({}); using the Python reader".format(bam, e))
-    evidence, depths = {}, {}
 
     def one(handle, tred):
         xtred = repo[tred]
-        native = handle is not None and handle.tid(xtred.chr) >= 0
         try:
-            if native:
-                ev = locus_evidence(handle, None, xtred, READLEN, alts, clip, repo.ref)
-                return tred, ev, ev.depth
-            bd = BamDepth(bam, repo.ref, logger)
-            return tred, None, bd.region_depth(xtred.chr, max(0, xtred.repeat_start - SPAN), xtred.repeat_end + SPAN)
+            if handle is not None and handle.tid(xtred.chr) >= 0:
+                return tred, locus_evidence(handle, xtred, READLEN, alts, clip, repo.ref)
+            return tred, extract_locus(bam, repo, tred, READLEN, alts, clip, logger)
         except Exception as e:
-            if native:
-                # the window could not be read (truncated / corrupt BAM): no evidence, no call — the reference's
-                # `except Exception: continue` (tred.py:245-249); reading it again with another reader is pointless
-                logger.error("Exception on `{}` {} ({})".format(bam, tred, e))
-                return tred, None, FAILED
-            logger.error("Exception on `{}` {} ({}). Set depth={}".format(bam, tred, e, 30))
-            return tred, None, 30
+            logger.error("Exception on `{}` {} ({})".format(bam, tred, e))
+            return tred, None
 
     threads = max(1, min(threads or INGEST_THREADS, len(tredNames)))
     if ing is None or threads == 1:
@@ -351,12 +265,12 @@ def ingest_loci(bam, repo, tredNames, READLEN, alts, clip, logger, threads=None,
                 h.close()
     if ing is not None:
         ing.close()
-    for tred, ev, depth in done:
+    evidence = {}
+    for tred, ev in done:
         if ev is not None:
             evidence[tred] = ev
-        depths[tred] = depth
-        logger.debug("Inferred depth at locus {}: {}".format(tred, depth))
-    return evidence, depths
+            logger.debug("Inferred depth at locus {}: {}".format(tred, ev.depth))
+    return evidence
 
 
 GPU_INGEST = os.environ.get("TREDSW_GPU_INGEST", "1") != "0"
@@ -371,9 +285,8 @@ def ingest_chunk_gpu(samples, ctx=None, keep_batch=None):
     :param keep_batch: a list; when every problem of the batch is good, (IngestBatch, [(key, tredName)]) is appended
                        and the batch stays open (the evidence objects are views into it): the caller genotypes from
                        its device buffers and closes it
-    :return: {key: ({tredName: LocusEvidence}, {tredName: depth})} — loci the device path could not serve (contig
-             missing, a block the decoder refused, corrupt records) are left out: the caller reads them with the
-             host reader."""
+    :return: {key: {tredName: LocusEvidence}} — loci the device path could not serve (contig missing, a block the
+             decoder refused, corrupt records) are left out: the caller reads them with the host reader."""
     from . import _lib
     from .ingest import IngestBatch, locus_query
     handles, qs, so, keep, key = [], [], [], [], []
@@ -385,10 +298,7 @@ def ingest_chunk_gpu(samples, ctx=None, keep_batch=None):
             handles.append(h)
             for t in wanted:
                 xtred = repo[t]
-                alt = ()
-                if alts and not clip:
-                    alt = [(c[3:] if "nochr" in repo.ref else c, s, e) for (c, s, e) in xtred.alt] if "nochr" in repo.ref else xtred.alt
-                q = locus_query(h, xtred, READLEN, alts=alt)
+                q = locus_query(h, xtred, READLEN, alts=alt_regions(xtred, repo.ref, alts, clip))
                 if q is None:
                     continue
                 qs.append(q[0]); keep.append(q[1]); so.append(len(handles) - 1); key.append((k, t))
@@ -403,9 +313,7 @@ def ingest_chunk_gpu(samples, ctx=None, keep_batch=None):
                 if b.status[i]:
                     logger.debug("GPU ingest handed {} / {} back (status {})".format(k, t, int(b.status[i])))
                     continue
-                ev = b.evidence(i, copy=not hold)
-                e, d = got.setdefault(k, ({}, {}))
-                e[t], d[t] = ev, ev.depth
+                got.setdefault(k, {})[t] = b.evidence(i, copy=not hold)
             if hold:
                 # every problem is good: the caller may genotype straight from the batch's device buffers
                 keep_batch.append((b, key))
@@ -438,19 +346,6 @@ def presteps(bam, repo, tredNames, logger, ing=None):
         pass
     logger.debug("Read length: {}bp".format(READLEN))
     return {"inferredGender": gender, "depthY": ydepth, "readLen": READLEN}
-
-
-FAILED = object()        # depth marker of a locus whose BAM window could not be read (corrupt / truncated file)
-
-
-def result_fields(tpResult, depth):
-    """BamParserResults -> the per-locus entries of tredCalls (tred.py:251-275), without the '<T>.' prefix."""
-    a = tpResult.alleles
-    return {"1": a[0], "2": a[1], "FR": counter_s(tpResult.counts["FULL"]), "PR": counter_s(tpResult.counts["PREF"]),
-            "RR": counter_s(tpResult.counts["REPT"]), "DP": depth, "FDP": tpResult.FDP, "PDP": tpResult.PDP,
-            "RDP": tpResult.RDP, "PEDP": tpResult.PEDP, "PEG": tpResult.PEG, "PET": tpResult.PET, "CI": tpResult.CI,
-            "PP": tpResult.PP, "label": tpResult.label, "details": tpResult.details, "P_h1": tpResult.P_h1,
-            "P_h2": tpResult.P_h2, "P_h1h2": tpResult.P_h1h2, "P_PEG": tpResult.P_PEG, "P_PET": tpResult.P_PET}
 
 
 def run(arg):
@@ -511,16 +406,13 @@ def prepare_chunk(args, only=None, ctx=None):
         samplekey, bam, repo, tredNames, maxinsert, fullsearch, clip, alts, repeatpairs, log = args[si]
         gender, READLEN = out[si]["tredCalls"]["inferredGender"], out[si]["tredCalls"]["readLen"]
         wanted = wanted_of[si]
-        evidence, depths = got.get(si, ({}, {}))
-        rest = [t for t in wanted if t not in depths]
+        evidence = got.get(si, {})
+        rest = [t for t in wanted if t not in evidence]
         if rest:
-            ev2, d2 = ingest_loci(bam, repo, rest, READLEN, alts, clip, logger, want_names=True)
-            evidence.update(ev2)
-            depths.update(d2)
-        out[si].update(_depths=depths, _gender=gender, _readlen=READLEN)
+            evidence.update(ingest_loci(bam, repo, rest, READLEN, alts, clip, logger, want_names=True))
         for t in wanted:
             if t in evidence:
-                items.append((repo[t], READLEN, gender, depths[t], evidence[t]))
+                items.append((repo[t], READLEN, gender, evidence[t].depth, evidence[t]))
                 where.append((si, t))
     # the fused call can run on the ingest's device buffers when the items are exactly the problems of the batch
     device_batch = None
@@ -548,52 +440,20 @@ def finish_chunk(state, ctx=None):
     args, out, items, where, device_batch = state
     if not args:
         return []
-    _, _, repo, _, maxinsert, fullsearch, clip, alts, repeatpairs, log = args[0]
-    # loci whose evidence came from the ingest: the fused device pipeline, all of them in one call — on the ingest's
-    # own device buffers when the whole chunk came from the GPU ingest, else from a batch assembled on the host
+    _, _, _, _, maxinsert, fullsearch, clip, _, repeatpairs, _ = args[0]
+    # all the loci in one call: on the ingest's own device buffers when the whole chunk came from the GPU ingest,
+    # else from a batch assembled on the host
     try:
-        res = None
-        if device_batch is not None:
-            try:
-                res = genotype_evidence(items, maxinsert=maxinsert, fullsearch=fullsearch, clip=clip,
-                                        repeatpairs=repeatpairs, ctx=ctx, device_batch=device_batch)
-            except Exception as e:
-                logger.error("Device hand-off failed ({}); assembling the batch on the host".format(e))
-        if res is None:
-            res = genotype_evidence(items, maxinsert=maxinsert, fullsearch=fullsearch, clip=clip, repeatpairs=repeatpairs, ctx=ctx)
-        for (si, t), r in zip(where, res):
-            out[si]["_fields"][t] = r
-    except Exception as e:
-        logger.error("Fused run failed ({}); falling back to the per-stage path".format(e))
+        res = genotype_evidence(items, maxinsert=maxinsert, fullsearch=fullsearch, clip=clip, repeatpairs=repeatpairs,
+                                ctx=ctx, device_batch=device_batch)
     finally:
         if device_batch is not None:
             device_batch.close()
-    for o, arg in zip(out, args):
-        samplekey, bam, repo, tredNames, maxinsert, fullsearch, clip, alts, repeatpairs, log = arg
-        fields, depths = o.pop("_fields"), o.pop("_depths", {})
-        wanted, gender, READLEN = o.pop("_names"), o.pop("_gender", "Unknown"), o.pop("_readlen", 150)
-        # the rest (no usable index, contig missing, ...): Python BAM reader + per-stage kernels
-        rest = [t for t in wanted if t not in fields and t in depths and depths[t] is not FAILED]
-        if rest:
-            ips = [InputParams(bam=bam, READLEN=READLEN, tredName=tred, repo=repo, maxinsert=maxinsert,
-                               fullsearch=fullsearch, gender=gender, depth=depths[tred], clip=clip, alts=alts,
-                               repeatpairs=repeatpairs, log=log) for tred in rest]
-            try:
-                results = run_batched(ips, {})
-            except Exception as e:
-                # keep the reference's per-locus isolation (tred.py:245-249): retry one locus at a time
-                logger.error("Batched run failed on `{}` ({}); falling back to per-locus calls".format(bam, e))
-                results = []
-                for ip in ips:
-                    try:
-                        results.append(runBam(ip))
-                    except Exception as e2:
-                        logger.error("Exception on `{}` {} ({})".format(bam, ip.tredName, e2))
-                        results.append(None)
-            for tred, r in zip(rest, results):
-                if r is not None:
-                    fields[tred] = result_fields(r, depths[tred])
-        for tred in wanted:
+    for (si, t), r in zip(where, res):
+        out[si]["_fields"][t] = r
+    for o in out:
+        fields = o.pop("_fields")
+        for tred in o.pop("_names"):
             for k, v in fields.get(tred, {}).items():
                 o["tredCalls"][tred + "." + k] = v
     return out
