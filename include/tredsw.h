@@ -422,8 +422,9 @@ typedef struct {
     const tredsw_locus_summary *summaries;   /* per problem: counts and depth as tredsw_bam_extract_locus reports them */
     const tredsw_problem_span *spans;
     const int32_t *status;      /* per problem: 0 ok; 1 its sample could not be staged (I/O, index, BGZF framing), 2 a block
-                                   failed to inflate or its CRC-32 differs, 3 corrupt records — no evidence is reported for
-                                   such a problem: read it with tredsw_bam_extract_locus (which has zlib behind it) */
+                                   failed to inflate or its CRC-32 differs, 3 corrupt records, 4 (scan only) the file is not
+                                   sorted by coordinate — no evidence is reported for such a problem: read it with
+                                   tredsw_bam_extract_locus (which has zlib behind it) or the Python reader */
     int64_t n_blocks, n_records, comp_bytes, inflated_bytes;
     double ms_host_stage, ms_total;   /* host time: compressed bytes staged; whole call */
     double ms_marks[4];         /* host time at the four synchronisation points: blocks inflated + records counted,
@@ -443,6 +444,35 @@ void tredsw_ingest_batch_free(tredsw_ingest_batch *batch);
 int tredsw_ingest_batch_emulate(tredsw_bam *const *bams, const int32_t *sample_of, const tredsw_locus_query *queries,
                                 int32_t nqueries, uint32_t flags, tredsw_ingest_batch **out);
 int tredsw_inflate_raw_device_code(const uint8_t *in, int64_t in_len, uint8_t *out, int64_t out_len);
+
+/* BAMs without an index.  tredsw_bam_open_unindexed reads the header and leaves the BGZF stream open without looking
+ * for an index: tredsw_bam_tid, tredsw_bam_header_signature, tredsw_bam_read_length and tredsw_bam_clone work on the
+ * handle; tredsw_bam_extract_locus, tredsw_bam_region_depth and tredsw_ingest_batch_run refuse it with
+ * TREDSW_ERR_UNSUPPORTED.  NULL + tredsw_last_error() on failure. */
+tredsw_bam *tredsw_bam_open_unindexed(const char *bam_path);
+/* One sample in ONE streaming pass over the whole file (csrc/bgzf_gpu.cu, run_scan): the host reads the file after
+ * the header slab by slab (slab_bytes compressed bytes a step, 0 = 128 MiB; at least 64 KiB), the device inflates
+ * every block, finds the record boundaries without an index (a candidate per block, verified by chaining from the
+ * known first record), keeps the records that overlap a fetch of `queries` (locus windows and alt regions) and sums
+ * the depth of `depth_regions` (n_depth x (tid, start, end); depth_out[d] = what tredsw_bam_region_depth returns for
+ * region d, NaN when the scan failed).  The result is an ordinary batch (tredsw_ingest_batch_view / _free), with the
+ * same evidence as tredsw_ingest_batch_run on an indexed copy, problem by problem.  Its status is per scan: every
+ * problem gets 1 (I/O, BGZF framing), 2 (a block failed to inflate), 3 (corrupt or truncated records) or 4 (the file is
+ * not sorted by coordinate: tid non-decreasing with -1 last, pos non-decreasing within a tid). */
+int tredsw_ingest_scan_run(tredsw_ctx *ctx, tredsw_bam *bam, const tredsw_locus_query *queries, int32_t nqueries,
+                           const int32_t *depth_regions, int32_t n_depth, double *depth_out, int64_t slab_bytes,
+                           uint32_t flags, tredsw_ingest_batch **out);
+/* TEST INFRASTRUCTURE: the same with every kernel body run serially on the host.  The package never calls it. */
+int tredsw_ingest_scan_emulate(tredsw_bam *bam, const tredsw_locus_query *queries, int32_t nqueries,
+                               const int32_t *depth_regions, int32_t n_depth, double *depth_out, int64_t slab_bytes,
+                               uint32_t flags, tredsw_ingest_batch **out);
+/* Statistics of a scan (zeros for a batch of tredsw_ingest_batch_run), TREDSW_SCAN_NSTATS values: [0] slabs, [1] BGZF
+ * blocks, [2] records scanned, [3] blocks whose candidate record start was wrong and that were walked again, [4]
+ * compressed bytes, [5] inflated bytes, [6] host time reading and framing the slabs (us, summed over slabs; the read of
+ * slab k + 1 overlaps the device work on slab k), [7] time of the device work on the slabs (us, summed), [8] whole call
+ * (us), [9] status of the scan (the per-problem code above; 0 ok). */
+#define TREDSW_SCAN_NSTATS 10
+int tredsw_ingest_scan_stats(const tredsw_ingest_batch *batch, int64_t *stats);
 
 #ifdef __cplusplus
 }

@@ -35,6 +35,8 @@ EXPORTS = [
     # BAM ingest on the GPU (batched); *_emulate / *_device_code run the device code on the host for the CPU tests
     "tredsw_ingest_batch_run", "tredsw_ingest_batch_view", "tredsw_ingest_batch_free", "tredsw_ingest_batch_emulate",
     "tredsw_inflate_raw_device_code",
+    # BAMs without an index: one streaming pass per sample
+    "tredsw_bam_open_unindexed", "tredsw_ingest_scan_run", "tredsw_ingest_scan_emulate", "tredsw_ingest_scan_stats",
 ]
 
 

@@ -321,20 +321,26 @@ class BamDepth:
     # rows of the chrY table that "still have mapped reads" in females and are skipped (bam_parser.py:417-418)
     Y_SKIP_ROWS = (1, 4, 6, 7, 10, 11, 13, 16, 18, 19)
 
-    def get_Y_depth(self, N=5):
-        """Median depth over the first N usable unique chrY regions (bam_parser.py:413-429).  Raises when the
-        BAM has no such contig — the caller then keeps gender 'Unknown' like the reference (tred.py:203-211)."""
-        build = self.ref.split("_")[0]
+    @classmethod
+    def y_regions(cls, ref, N=5):
+        """The first N usable unique chrY regions of the reference build: [(contig, start, end)]"""
+        build = ref.split("_")[0]
         regions = []
         with open(datafile("chrY.tsv")) as fp:
             next(fp)
             for line in fp:
                 b, row, c, start, end, _gc = line.split()
-                if b != build or int(row) in self.Y_SKIP_ROWS:
+                if b != build or int(row) in cls.Y_SKIP_ROWS:
                     continue
                 regions.append((c, int(start), int(end)))
                 if len(regions) >= N:
                     break
+        return regions
+
+    def get_Y_depth(self, N=5):
+        """Median depth over the first N usable unique chrY regions (bam_parser.py:413-429).  Raises when the
+        BAM has no such contig — the caller then keeps gender 'Unknown' like the reference (tred.py:203-211)."""
+        regions = self.y_regions(self.ref, N)
         depths = []
         ing, own = self.ing, False
         if ing is None:

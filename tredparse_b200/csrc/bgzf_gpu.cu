@@ -18,6 +18,10 @@
 //   pair_*                pairing by query name through per-problem open-addressing tables (two smallest record
 //                         indices per name = the reference's "first two records"), distances into pe_lens.
 //
+// A BAM without an index is read by a second front end, run_scan (tredsw_ingest_scan_run): one streaming pass per
+// sample, slab by slab, that finds the record boundaries on the device and hands the records of every fetch to the
+// same selection / compaction / pairing steps (select_and_pair) — see the scan_* bodies of ingest_device.cuh.
+//
 // The per-thread bodies live in ingest_device.cuh as __host__ __device__ functions; the pipeline below is written
 // once against a small backend (allocate / copy / for_each / scan) with a CUDA implementation and a serial host
 // implementation.  The host one is TEST INFRASTRUCTURE (tredsw_ingest_batch_emulate): it lets the CPU suite compare
@@ -30,6 +34,7 @@
 #include <sys/stat.h>
 
 #include <algorithm>
+#include <cmath>
 #include <map>
 #include <memory>
 #include <string>
@@ -43,6 +48,8 @@
 namespace tredsw_gi {       // kernel name tags (they show up in profiler listings: for_each_kernel<tredsw_gi::SelectTag, ...>)
 struct WalkCountTag; struct WalkFillTag; struct SelectTag; struct SummaryTag; struct CompactTag; struct EmitTag;
 struct PairInsertTag; struct PairSecondTag; struct PairEvalTag; struct PairCountTag; struct PairScatterTag;
+// the scan of an unindexed BAM
+struct ScanCandidateTag; struct ScanRepairTag; struct ScanCountTag; struct ScanFillTag; struct ScanMatchTag; struct ScanKeepTag;
 }
 using namespace tredsw_gi;
 
@@ -227,6 +234,7 @@ struct CudaBackend {
     }
     void upload(void *dst, const void *src, size_t bytes) { if (bytes && dst) fail(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, stream), "cudaMemcpyAsync(H2D)"); }
     void download(void *dst, const void *src, size_t bytes) { if (bytes && dst) fail(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, stream), "cudaMemcpyAsync(D2H)"); }
+    void copy(void *dst, const void *src, size_t bytes) { if (bytes && dst) fail(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, stream), "cudaMemcpyAsync(D2D)"); }
     void fill(void *dst, int byte, size_t bytes) { if (bytes && dst) fail(cudaMemsetAsync(dst, byte, bytes, stream), "cudaMemsetAsync"); }
     void sync() { fail(cudaStreamSynchronize(stream), "cudaStreamSynchronize"); }
     template <class Tag, class F> void for_each(int64_t n, F f) {
@@ -301,6 +309,7 @@ struct HostBackend {                                   // serial emulation of th
     void release_intermediates() { for (void *p : mem) free(p); mem.clear(); }
     void upload(void *dst, const void *src, size_t bytes) { if (bytes && dst) memcpy(dst, src, bytes); }
     void download(void *dst, const void *src, size_t bytes) { if (bytes && dst) memcpy(dst, src, bytes); }
+    void copy(void *dst, const void *src, size_t bytes) { if (bytes && dst) memcpy(dst, src, bytes); }
     void fill(void *dst, int byte, size_t bytes) { if (bytes && dst) memset(dst, byte, bytes); }
     void sync() {}
     template <class Tag, class F> void for_each(int64_t n, F f) { for (int64_t i = 0; i < n && !rc; ++i) f(i); }
@@ -358,11 +367,48 @@ struct tredsw_ingest_batch {
     double ms_host_stage = 0, ms_total = 0, ms_marks[4] = {0, 0, 0, 0};
     long long n_blocks = 0, n_records = 0;
     long long comp_bytes = 0, inflated_bytes = 0;
+    int64_t scan_stats[TREDSW_SCAN_NSTATS] = {0};   // tredsw_ingest_scan_stats
 };
 
 namespace {
 
 double now_ms() { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6; }
+
+// The BGZF framing of the block at h, `avail` bytes of which are at hand: 1 parsed, 0 the block is not all there,
+// -1 not a valid block (*why says what is wrong or missing).
+struct BgzfFrame { int xlen, bsize /* bytes of the whole block */, clen; uint32_t crc, isize; };
+int parse_bgzf_block(const uint8_t *h, int64_t avail, BgzfFrame *f, const char **why) {
+    if (avail < 18) { *why = "truncated BGZF block header"; return 0; }
+    if (h[0] != 31 || h[1] != 139 || !(h[3] & 4)) { *why = "not a BGZF block"; return -1; }
+    f->xlen = h[10] | (h[11] << 8);
+    if (12 + f->xlen > avail) { *why = "truncated BGZF block header"; return 0; }
+    int bsize = -1;
+    for (int off = 0; off + 4 <= f->xlen;) {
+        const int slen = h[12 + off + 2] | (h[12 + off + 3] << 8);
+        if (h[12 + off] == 66 && h[12 + off + 1] == 67 && off + 6 <= f->xlen) bsize = h[12 + off + 4] | (h[12 + off + 5] << 8);
+        off += 4 + slen;
+    }
+    if (bsize < 0) { *why = "BGZF block without a BC field"; return -1; }
+    f->clen = bsize - f->xlen - 19;
+    if (f->clen < 0) { *why = "bad BGZF block size"; return -1; }
+    f->bsize = bsize + 1;
+    if (f->bsize > avail) { *why = "truncated BGZF block"; return 0; }
+    memcpy(&f->crc, h + f->bsize - 8, 4); memcpy(&f->isize, h + f->bsize - 4, 4);
+    if (f->isize > 65536) { *why = "BGZF block larger than 64 KiB"; return -1; }
+    return 1;
+}
+
+// the windows of one locus (extract_locus_impl)
+ProblemParams problem_params(const tredsw_locus_query &q) {
+    ProblemParams pp;
+    const int64_t start = q.repeat_start, end = q.repeat_end;
+    pp.tid = q.tid; pp.span = q.span;
+    pp.win_s = std::max<int64_t>(0, start - q.pad); pp.win_e = end + q.pad;
+    pp.read_s = std::max<int64_t>(0, start - q.readlen); pp.read_e = end + q.readlen;
+    pp.pe_s = std::max<int64_t>(start - q.pe_window, 0); pp.pe_e = end + q.pe_window;
+    pp.tstart = start - q.flankmatch; pp.tend = end + q.flankmatch;
+    return pp;
+}
 
 // One sample: the fetches of its problems (the locus window, then the alt regions), their BAI chunks, and the merged
 // ranges of BGZF blocks behind them (every block is read and inflated once per sample).
@@ -382,6 +428,12 @@ struct SamplePlan {
 // ---------------------------------------------------------------------------------------------------------------
 // pipeline
 // ---------------------------------------------------------------------------------------------------------------
+template <class B>
+int select_and_pair(B &be, tredsw_ingest_batch *out, const uint8_t *d_rbytes, const Fetch *d_fetches, const int64_t *d_rpos,
+                    const int32_t *d_rfetch, const uint32_t *d_fbase, int64_t nrec, const std::vector<int32_t> &fetch_first,
+                    const std::vector<ProblemParams> &params, const ProblemParams *d_params, ProblemCounts *d_counts,
+                    bool want_names, double t_begin);
+
 template <class B>
 int run_pipeline(B &be, tredsw_ingest_batch *out, tredsw_bam *const *bams, const int32_t *sample_of,
                         const tredsw_locus_query *queries, int32_t nq, uint32_t flags) {
@@ -403,6 +455,7 @@ int run_pipeline(B &be, tredsw_ingest_batch *out, tredsw_bam *const *bams, const
         SamplePlan &sp = plans[sample_of[i]];
         sp.bam = bams[sample_of[i]];
         if (!sp.bam) { tredsw_set_error("null BAM handle for sample %d", sample_of[i]); return TREDSW_ERR_ARG; }
+        if (!sp.bam->has_index) { tredsw_set_error("%s has no index: scan it (tredsw_ingest_scan_run)", sp.bam->path.c_str()); return TREDSW_ERR_UNSUPPORTED; }
         sp.problems.push_back(i);
     }
     std::vector<ProblemParams> params(nq);
@@ -425,12 +478,7 @@ int run_pipeline(B &be, tredsw_ingest_batch *out, tredsw_bam *const *bams, const
             const tredsw_locus_query &q = queries[p];
             ProblemParams &pp = params[p];
             if (q.tid < 0 || q.tid >= (int)sp.bam->names.size()) { out->status[p] = 1; continue; }
-            const int64_t start = q.repeat_start, end = q.repeat_end;
-            pp.tid = q.tid; pp.span = q.span;
-            pp.win_s = std::max<int64_t>(0, start - q.pad); pp.win_e = end + q.pad;
-            pp.read_s = std::max<int64_t>(0, start - q.readlen); pp.read_e = end + q.readlen;
-            pp.pe_s = std::max<int64_t>(start - q.pe_window, 0); pp.pe_e = end + q.pe_window;
-            pp.tstart = start - q.flankmatch; pp.tend = end + q.flankmatch;
+            pp = problem_params(q);
             auto add_fetch = [&](int kind, int tid, int64_t fs, int64_t fe) {
                 SamplePlan::PFetch f;
                 f.problem = p; f.kind = kind; f.tid = tid; f.start = fs < 0 ? 0 : fs; f.end = fe;
@@ -498,32 +546,16 @@ int run_pipeline(B &be, tredsw_ingest_batch *out, tredsw_bam *const *bams, const
             const size_t first_block = lb.size();
             int64_t o = 0;
             while (sp.ranges[r].first + o <= sp.ranges[r].second) {
-                if (o + 18 > got) { if (o == got && got < sp.range_bytes[r]) { ok = false; why = "short read"; } else if (o < got) { ok = false; why = "truncated BGZF block header"; } break; }
-                const uint8_t *h = dst + o;
-                if (h[0] != 31 || h[1] != 139 || !(h[3] & 4)) { ok = false; why = "not a BGZF block"; break; }
-                const int xlen = h[10] | (h[11] << 8);
-                if (o + 12 + xlen > got) { ok = false; why = "truncated BGZF block header"; break; }
-                int bsize = -1;
-                for (int off = 0; off + 4 <= xlen;) {
-                    const int slen = h[12 + off + 2] | (h[12 + off + 3] << 8);
-                    if (h[12 + off] == 66 && h[12 + off + 1] == 67 && off + 6 <= xlen) bsize = h[12 + off + 4] | (h[12 + off + 5] << 8);
-                    off += 4 + slen;
-                }
-                if (bsize < 0) { ok = false; why = "BGZF block without a BC field"; break; }
-                const int clen = bsize - xlen - 19;
-                if (clen < 0) { ok = false; why = "bad BGZF block size"; break; }
-                if (o + bsize + 1 > got) { ok = false; why = "truncated BGZF block"; break; }
-                const uint8_t *tail = dst + o + bsize + 1 - 8;
-                uint32_t crc, isize;
-                memcpy(&crc, tail, 4); memcpy(&isize, tail + 4, 4);
-                if (isize > 65536) { ok = false; why = "BGZF block larger than 64 KiB"; break; }
+                if (o == got) { if (got < sp.range_bytes[r]) { ok = false; why = "short read"; } break; }
+                BgzfFrame fr;
+                if (parse_bgzf_block(dst + o, got - o, &fr, &why) != 1) { ok = false; break; }
                 BlockDesc d;
-                d.in_off = sp.range_comp_off[r] + o + 12 + xlen;
-                d.out_off = cursor; d.clen = (uint32_t)clen; d.isize = isize; d.crc = crc; d.pad_ = 0;
+                d.in_off = sp.range_comp_off[r] + o + 12 + fr.xlen;
+                d.out_off = cursor; d.clen = (uint32_t)fr.clen; d.isize = fr.isize; d.crc = fr.crc; d.pad_ = 0;
                 sample_blocks[s].push_back(d);
-                lb.push_back(LoadedBlock{sp.ranges[r].first + o, cursor, isize, 0});
-                cursor += isize;
-                o += bsize + 1;
+                lb.push_back(LoadedBlock{sp.ranges[r].first + o, cursor, fr.isize, 0});
+                cursor += fr.isize;
+                o += fr.bsize;
             }
             for (size_t k = first_block; k < lb.size(); ++k) lb[k].run_end = cursor;
         }
@@ -640,6 +672,35 @@ int run_pipeline(B &be, tredsw_ingest_batch *out, tredsw_bam *const *bams, const
     out->n_records = nrec;
     int64_t *d_rpos = static_cast<int64_t *>(be.alloc(sizeof(int64_t) * (size_t)std::max<int64_t>(1, nrec)));
     int32_t *d_rfetch = static_cast<int32_t *>(be.alloc(sizeof(int32_t) * (size_t)std::max<int64_t>(1, nrec)));
+    if (be.rc) return be.rc;
+    {
+        const uint8_t *ibuf = d_ibuf; const Fetch *fe = d_fetches; const Chunk *ch = d_chunks;
+        const uint32_t *fbase = d_fbase;
+        int64_t *rpos = d_rpos; int32_t *rfetch = d_rfetch;
+        const int64_t ibuf_len = ((ibuf_total + 16) / 16) * 16;
+        be.template for_each_warp_window<WalkFillTag>(nfetch, [=] __host__ __device__(int64_t i, int lane, uint32_t *win) {
+            uint32_t k = fbase[i];                               // (a fetch flagged by the count pass yields the same prefix)
+            const uint32_t stop = fbase[i + 1];
+            walk_fetch_lanes(ibuf, ibuf_len, fe[i], ch, lane, win, [&](int64_t p) {
+                if (k < stop && lane == 0) { rpos[k] = p; rfetch[k] = (int32_t)i; }
+                ++k;
+            });
+        });
+    }
+    return select_and_pair(be, out, d_ibuf, d_fetches, d_rpos, d_rfetch, d_fbase, nrec, fetch_first, params, d_params,
+                           d_counts, want_names, t_begin);
+}
+
+// Steps (5) to (7), shared by both front ends (the indexed walk above, the scan of an unindexed BAM below): per-record
+// selection, ordered compaction, pairing by name, results.  rpos[i] is where record i starts in `rbytes`, rfetch[i] its
+// fetch; the records are grouped by fetch (fetch f owns [fbase[f], fbase[f + 1])) and are in file order within a fetch.
+template <class B>
+int select_and_pair(B &be, tredsw_ingest_batch *out, const uint8_t *d_rbytes, const Fetch *d_fetches, const int64_t *d_rpos,
+                    const int32_t *d_rfetch, const uint32_t *d_fbase, int64_t nrec, const std::vector<int32_t> &fetch_first,
+                    const std::vector<ProblemParams> &params, const ProblemParams *d_params, ProblemCounts *d_counts,
+                    bool want_names, double t_begin) {
+    const int32_t nq = out->nproblems;
+    const uint8_t *d_ibuf = d_rbytes;
     uint32_t *d_emit = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)(nrec + 1)));
     uint32_t *d_bases = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)(nrec + 1)));
     uint32_t *d_nameb = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)(nrec + 1)));
@@ -656,19 +717,9 @@ int run_pipeline(B &be, tredsw_ingest_batch *out, tredsw_bam *const *bams, const
     if (be.rc) return be.rc;
     be.upload(d_ffirst, fetch_first.data(), sizeof(int32_t) * (size_t)(nq + 1));
     {
-        const uint8_t *ibuf = d_ibuf; const Fetch *fe = d_fetches; const Chunk *ch = d_chunks;
-        const uint32_t *fbase = d_fbase;
-        int64_t *rpos = d_rpos; int32_t *rfetch = d_rfetch;
-        const int64_t ibuf_len = ((ibuf_total + 16) / 16) * 16;
-        be.template for_each_warp_window<WalkFillTag>(nfetch, [=] __host__ __device__(int64_t i, int lane, uint32_t *win) {
-            uint32_t k = fbase[i];                               // (a fetch flagged by the count pass yields the same prefix)
-            const uint32_t stop = fbase[i + 1];
-            walk_fetch_lanes(ibuf, ibuf_len, fe[i], ch, lane, win, [&](int64_t p) {
-                if (k < stop && lane == 0) { rpos[k] = p; rfetch[k] = (int32_t)i; }
-                ++k;
-            });
-        });
         // ---- (5) per-record selection --------------------------------------------------------------------------------
+        const uint8_t *ibuf = d_ibuf; const Fetch *fe = d_fetches;
+        const int64_t *rpos = d_rpos; const int32_t *rfetch = d_rfetch;
         const ProblemParams *pp = d_params; ProblemCounts *pc = d_counts;
         uint32_t *emit = d_emit, *bases = d_bases, *nameb = d_nameb, *pe = d_pe;
         Mate *mates = d_mates;
@@ -862,7 +913,459 @@ int run_pipeline(B &be, tredsw_ingest_batch *out, tredsw_bam *const *bams, const
     return TREDSW_OK;
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// the scan of a BAM without an index: one streaming pass per sample (ingest_device.cuh: record boundaries, matching)
+// ---------------------------------------------------------------------------------------------------------------
+namespace {
+
+constexpr int64_t SCAN_DEFAULT_SLAB = 128ll << 20;     // compressed bytes per slab when the caller passes 0
+constexpr int64_t SCAN_MIN_SLAB = 65536;               // a slab holds at least one whole BGZF block
+constexpr int64_t SCAN_MAX_INFLATED = 1ll << 30;       // inflated bytes per slab: its record offsets are scanned in 32 bits
+
+struct ScanSlab {                   // the compressed bytes of one slab (page-locked) and their BGZF framing
+    uint8_t *comp = nullptr;
+    std::vector<BlockDesc> blocks;  // in_off into comp, out_off from the slab's first inflated byte
+    int64_t begin = 0, next = 0, inflated = 0;
+    const char *why = nullptr;      // I/O or framing error
+    double ms = 0;                  // host time: pread + framing
+};
+
+// Reads up to `want` bytes of the file from `off` and frames the whole blocks among them.  A block cut by the end of
+// the read is left to the next slab (`next` is its offset); one cut by the end of the file is an error.
+void read_slab(int fd, int64_t file_size, int64_t off, int64_t want, ScanSlab *sl) {
+    const double t0 = now_ms();
+    sl->blocks.clear(); sl->begin = sl->next = off; sl->inflated = 0; sl->why = nullptr;
+    const int64_t n = std::max<int64_t>(0, std::min(want, file_size - off));
+    int64_t got = 0;
+    while (got < n) {
+        const ssize_t k = pread(fd, sl->comp + got, (size_t)(n - got), (off_t)(off + got));
+        if (k <= 0) break;
+        got += k;
+    }
+    if (got < n) sl->why = "short read";
+    int64_t o = 0;
+    while (!sl->why && o < got) {
+        BgzfFrame fr;
+        const char *why = nullptr;
+        const int rc = parse_bgzf_block(sl->comp + o, got - o, &fr, &why);
+        if (rc < 0 || (rc == 0 && off + got >= file_size)) { sl->why = why; break; }
+        if (rc == 0 || (sl->inflated + fr.isize > SCAN_MAX_INFLATED && !sl->blocks.empty())) break;
+        BlockDesc d;
+        d.in_off = o + 12 + fr.xlen; d.out_off = sl->inflated; d.clen = (uint32_t)fr.clen; d.isize = fr.isize; d.crc = fr.crc; d.pad_ = 0;
+        sl->blocks.push_back(d);
+        sl->inflated += fr.isize;
+        o += fr.bsize;
+    }
+    sl->next = off + o;
+    sl->ms = now_ms() - t0;
+}
+
+// a device buffer that is reused from slab to slab and grows geometrically (the old one is released with the batch)
+template <class B> void *grow(B &be, void *&p, size_t &cap, size_t bytes) {
+    if (!p || bytes > cap) { cap = std::max(bytes, 2 * cap); p = be.alloc(cap); }
+    return p;
+}
+
+}  // namespace
+
+template <class B>
+int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locus_query *queries, int32_t nq,
+             const int32_t *depth_regions, int32_t n_depth, double *depth_out, int64_t slab_bytes, uint32_t flags) {
+    const double t_begin = now_ms();
+    const bool want_names = (flags & TREDSW_INGEST_NO_NAMES) == 0;
+    const int check_crc = (flags & TREDSW_INGEST_NO_CRC) == 0;
+    constexpr int NL = B::on_device ? 32 : 1;
+    out->nproblems = nq;
+    out->summaries.assign(nq, tredsw_locus_summary{});
+    out->status.assign(nq, 0);
+    out->spans.assign(nq, tredsw_problem_span{});
+    memset(&out->view, 0, sizeof(out->view));
+    const int32_t n_ref = (int32_t)bam->names.size();
+
+    // ---- (1) the fetches (problem-major, like run_pipeline), then the depth regions; their elementary segments -----
+    std::vector<ProblemParams> params(nq);
+    std::vector<Fetch> fetches;
+    std::vector<int32_t> fetch_first(nq + 1, 0);
+    std::vector<int32_t> id_tid;
+    std::vector<int64_t> id_start, id_end;
+    auto add_id = [&](int32_t tid, int64_t s, int64_t e) { id_tid.push_back(tid); id_start.push_back(s < 0 ? 0 : s); id_end.push_back(e); };
+    for (int p = 0; p < nq; ++p) {
+        fetch_first[p] = (int32_t)fetches.size();
+        const tredsw_locus_query &q = queries[p];
+        if (q.tid < 0 || q.tid >= n_ref) { out->status[p] = 1; continue; }
+        const ProblemParams pp = params[p] = problem_params(q);
+        auto add_fetch = [&](int kind, int32_t tid, int64_t s, int64_t e) {
+            Fetch f;
+            f.problem = p; f.kind = kind; f.tid = tid; f.start = s < 0 ? 0 : s; f.end = e;
+            f.chunk_begin = f.chunk_end = 0; f.pad_ = 0;
+            fetches.push_back(f);
+            add_id(tid, s, e);
+        };
+        add_fetch(0, q.tid, std::min(pp.win_s, pp.pe_s), std::max(pp.win_e, pp.pe_e));
+        for (int a = 0; a < q.n_alts && q.alts; ++a) {
+            const int32_t atid = q.alts[3 * a], as = q.alts[3 * a + 1], ae = q.alts[3 * a + 2];
+            if (atid < 0 || atid >= n_ref) continue;
+            add_fetch(1, atid, as, ae);
+        }
+    }
+    fetch_first[nq] = (int32_t)fetches.size();
+    const int32_t nfetch = (int32_t)fetches.size();
+    for (int d = 0; d < n_depth; ++d) {
+        const int32_t tid = depth_regions[3 * d], s = depth_regions[3 * d + 1], e = depth_regions[3 * d + 2];
+        if (tid < 0 || tid >= n_ref) { tredsw_set_error("depth region %d: contig id %d out of range", d, tid); return TREDSW_ERR_ARG; }
+        if (e < s) { tredsw_set_error("depth region %d is empty", d); return TREDSW_ERR_ARG; }
+        add_id(tid, s, e);
+    }
+    const int nids = (int)id_tid.size();
+    std::vector<int32_t> tid_x0(n_ref + 1, 0), seg_f0, seg_ids;
+    std::vector<int64_t> xs, id_lo(nids), id_hi(nids);
+    for (int i = 0; i < nids; ++i) {                        // the interval every fetch is listed on (MatchTables)
+        id_lo[i] = id_start[i] < id_end[i] ? id_start[i] : id_end[i] - 1;
+        id_hi[i] = id_start[i] < id_end[i] ? id_end[i] : id_end[i];
+    }
+    {
+        std::vector<std::vector<int64_t>> pts(n_ref);
+        for (int i = 0; i < nids; ++i) { pts[id_tid[i]].push_back(id_lo[i]); pts[id_tid[i]].push_back(id_hi[i]); }
+        for (int t = 0; t < n_ref; ++t) {
+            std::sort(pts[t].begin(), pts[t].end());
+            pts[t].erase(std::unique(pts[t].begin(), pts[t].end()), pts[t].end());
+            tid_x0[t] = (int32_t)xs.size();
+            xs.insert(xs.end(), pts[t].begin(), pts[t].end());
+        }
+        tid_x0[n_ref] = (int32_t)xs.size();
+        std::vector<std::vector<int32_t>> lists(xs.size());
+        for (int i = 0; i < nids; ++i) {
+            const auto b0 = xs.begin() + tid_x0[id_tid[i]], b1 = xs.begin() + tid_x0[id_tid[i] + 1];
+            const int j0 = (int)(std::lower_bound(b0, b1, id_lo[i]) - xs.begin()), j1 = (int)(std::lower_bound(b0, b1, id_hi[i]) - xs.begin());
+            for (int j = j0; j < j1; ++j) lists[j].push_back(i);
+        }
+        seg_f0.assign(xs.size() + 1, 0);
+        for (size_t j = 0; j < xs.size(); ++j) { seg_f0[j + 1] = seg_f0[j] + (int32_t)lists[j].size(); seg_ids.insert(seg_ids.end(), lists[j].begin(), lists[j].end()); }
+    }
+    int32_t *d_tid_x0 = static_cast<int32_t *>(be.alloc(sizeof(int32_t) * (size_t)(n_ref + 1)));
+    int64_t *d_xs = static_cast<int64_t *>(be.alloc(sizeof(int64_t) * std::max<size_t>(1, xs.size())));
+    int32_t *d_seg_f0 = static_cast<int32_t *>(be.alloc(sizeof(int32_t) * seg_f0.size()));
+    int32_t *d_seg_ids = static_cast<int32_t *>(be.alloc(sizeof(int32_t) * std::max<size_t>(1, seg_ids.size())));
+    int64_t *d_id_start = static_cast<int64_t *>(be.alloc(sizeof(int64_t) * 3 * (size_t)std::max(1, nids)));
+    unsigned long long *d_depth = static_cast<unsigned long long *>(be.alloc(sizeof(unsigned long long) * (size_t)std::max(1, n_depth)));
+    uint32_t *d_err = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * 2));
+    int64_t *d_small = static_cast<int64_t *>(be.alloc(sizeof(int64_t) * 2));     // last record's order key; repair stop
+    if (be.rc) return be.rc;
+    be.upload(d_tid_x0, tid_x0.data(), sizeof(int32_t) * tid_x0.size());
+    be.upload(d_xs, xs.data(), sizeof(int64_t) * xs.size());
+    be.upload(d_seg_f0, seg_f0.data(), sizeof(int32_t) * seg_f0.size());
+    be.upload(d_seg_ids, seg_ids.data(), sizeof(int32_t) * seg_ids.size());
+    be.upload(d_id_start, id_start.data(), sizeof(int64_t) * (size_t)nids);
+    be.upload(d_id_start + nids, id_end.data(), sizeof(int64_t) * (size_t)nids);
+    be.upload(d_id_start + 2 * nids, id_lo.data(), sizeof(int64_t) * (size_t)nids);
+    be.fill(d_depth, 0, sizeof(unsigned long long) * (size_t)std::max(1, n_depth));
+    be.fill(d_err, 0, sizeof(uint32_t) * 2);
+    const MatchTables mt{d_tid_x0, d_xs, d_seg_f0, d_seg_ids, d_id_start + 2 * nids, d_id_start, d_id_start + nids, n_ref, nfetch};
+
+    // ---- (2) slab by slab: read (the next slab on a host thread), inflate, record boundaries, match, keep ------------
+    const int fd = fileno(bam->bgzf.fh);
+    struct stat st;
+    const int64_t file_size = fstat(fd, &st) == 0 ? (int64_t)st.st_size : 0;
+    const int64_t want = std::max(std::min(slab_bytes > 0 ? slab_bytes : SCAN_DEFAULT_SLAB, file_size), SCAN_MIN_SLAB);
+    ScanSlab slabs[2];
+    for (ScanSlab &sl : slabs) sl.comp = static_cast<uint8_t *>(be.alloc_host((size_t)want + 64));
+    if (be.rc) return be.rc;
+    void *ibuf[2] = {nullptr, nullptr}; size_t ibuf_cap[2] = {0, 0};
+    void *d_comp = nullptr, *d_blocks = nullptr, *d_bstatus = nullptr, *d_sblk = nullptr, *d_cand = nullptr, *d_land = nullptr;
+    void *d_first = nullptr, *d_rcnt = nullptr, *d_rbase = nullptr, *d_recpos = nullptr, *d_nm = nullptr, *d_kb = nullptr;
+    void *d_ebase = nullptr, *d_kbase = nullptr, *d_efetch = nullptr, *d_epos = nullptr, *d_kept = nullptr;
+    size_t c_comp = 0, c_blocks = 0, c_bstatus = 0, c_sblk = 0, c_cand = 0, c_land = 0, c_first = 0, c_rcnt = 0, c_rbase = 0;
+    size_t c_recpos = 0, c_nm = 0, c_kb = 0, c_ebase = 0, c_kbase = 0, c_efetch = 0, c_epos = 0, c_kept = 0;
+    std::vector<int32_t> ent_fetch;         // (record, fetch) entries of the whole file, in file order
+    std::vector<int64_t> ent_pos;           // where the record is in the kept-record stream
+    int64_t kept_total = 0, carry_len = 0, carry_at = 0, prev_key = INT64_MIN;
+    int64_t s0 = (int64_t)(bam->first_record & 0xffff);
+    int32_t status = 0;
+    int64_t *stats = out->scan_stats;
+    std::thread reader;
+    struct Join { std::thread &t; ~Join() { if (t.joinable()) t.join(); } } join_reader{reader};
+    read_slab(fd, file_size, (int64_t)(bam->first_record >> 16), want, &slabs[0]);
+    for (int cur = 0;; cur ^= 1) {
+        ScanSlab &sl = slabs[cur];
+        stats[6] += (int64_t)(sl.ms * 1e3);
+        if (sl.why) { status = 1; tredsw_set_error("%s: %s", bam->path.c_str(), sl.why); break; }
+        const int nb = (int)sl.blocks.size();
+        if (nb == 0) break;                                                  // end of file
+        if (sl.next < file_size) reader = std::thread(read_slab, fd, file_size, sl.next, want, &slabs[cur ^ 1]);
+        else { slabs[cur ^ 1].blocks.clear(); slabs[cur ^ 1].why = nullptr; slabs[cur ^ 1].ms = 0; }
+        const double t_dev = now_ms();
+        const int64_t len = carry_len + sl.inflated;
+        uint8_t *s = static_cast<uint8_t *>(grow(be, ibuf[cur], ibuf_cap[cur], (size_t)len + 64));
+        if (be.rc) return be.rc;
+        be.copy(s, static_cast<uint8_t *>(ibuf[cur ^ 1]) + carry_at, (size_t)carry_len);
+        std::vector<ScanBlock> sblk(nb);
+        for (int b = 0; b < nb; ++b) {
+            sl.blocks[b].out_off += carry_len;
+            sblk[b].begin = b ? sl.blocks[b].out_off : 0;
+            sblk[b].end = sl.blocks[b].out_off + sl.blocks[b].isize;
+        }
+        // inflate; candidates and landings
+        uint8_t *comp = static_cast<uint8_t *>(grow(be, d_comp, c_comp, (size_t)(sl.next - sl.begin) + 64));
+        BlockDesc *blocks = static_cast<BlockDesc *>(grow(be, d_blocks, c_blocks, sizeof(BlockDesc) * nb));
+        uint8_t *bstatus = static_cast<uint8_t *>(grow(be, d_bstatus, c_bstatus, (size_t)nb));
+        ScanBlock *blk = static_cast<ScanBlock *>(grow(be, d_sblk, c_sblk, sizeof(ScanBlock) * nb));
+        int64_t *cand = static_cast<int64_t *>(grow(be, d_cand, c_cand, sizeof(int64_t) * nb));
+        int64_t *land = static_cast<int64_t *>(grow(be, d_land, c_land, sizeof(int64_t) * nb));
+        if (be.rc) return be.rc;
+        be.upload(comp, sl.comp, (size_t)(sl.next - sl.begin));
+        be.upload(blocks, sl.blocks.data(), sizeof(BlockDesc) * nb);
+        be.upload(blk, sblk.data(), sizeof(ScanBlock) * nb);
+        be.inflate(comp, s, blocks, nb, bstatus, check_crc);
+        {
+            const int64_t first0 = s0;
+            be.template for_each_warp<ScanCandidateTag>(nb, [=] __host__ __device__(int64_t b, int lane) {
+                const int64_t c = b == 0 ? first0 : scan_find_candidate<NL>(s, len, blk[b].begin, blk[b].end, n_ref, lane);
+                if (lane == 0) { cand[b] = c; land[b] = c < 0 ? c : scan_chain(s, len, c, blk[b].end); }
+            });
+        }
+        std::vector<uint8_t> h_bstatus(nb);
+        std::vector<int64_t> h_cand(nb), h_land(nb), h_first(nb);
+        be.download(h_bstatus.data(), bstatus, (size_t)nb);
+        be.download(h_cand.data(), cand, sizeof(int64_t) * nb);
+        be.download(h_land.data(), land, sizeof(int64_t) * nb);
+        be.sync();
+        if (be.rc) return be.rc;
+        if (std::any_of(h_bstatus.begin(), h_bstatus.end(), [](uint8_t v) { return v != 0; })) { status = 2; tredsw_set_error("%s: a BGZF block failed to inflate", bam->path.c_str()); break; }
+        // verification: the chain entering every block from the known start of block 0; repair where it disagrees
+        int64_t tf = s0;
+        for (int b = 0; b < nb && tf != SCAN_BAD;) {
+            h_first[b] = tf;
+            if (scan_agrees(sblk[b], h_cand[b], tf)) {
+                if (tf >= sblk[b].begin && tf < sblk[b].end) tf = h_land[b];
+                ++b;
+                continue;
+            }
+            int64_t *stop = d_small + 1;
+            const int b0 = b; const int64_t t0 = tf;
+            be.template for_each<ScanRepairTag>(1, [=] __host__ __device__(int64_t) { *stop = scan_repair_run(s, len, blk, cand, nb, b0, t0, land); });
+            int64_t h_stop = 0;
+            be.download(&h_stop, stop, sizeof(int64_t));
+            be.sync();
+            if (be.rc) return be.rc;
+            be.download(h_land.data() + b0, land + b0, sizeof(int64_t) * (size_t)(h_stop - b0));
+            be.sync();
+            for (int k = b0 + 1; k < (int)h_stop; ++k) h_first[k] = h_land[k - 1];
+            stats[3] += h_stop - b0;
+            tf = h_land[h_stop - 1];
+            b = (int)h_stop;
+        }
+        if (tf == SCAN_BAD) { status = 3; tredsw_set_error("%s: corrupt BAM records (implausible block_size)", bam->path.c_str()); break; }
+        // the records that start in every block, in file order
+        int64_t *first = static_cast<int64_t *>(grow(be, d_first, c_first, sizeof(int64_t) * nb));
+        uint32_t *rcnt = static_cast<uint32_t *>(grow(be, d_rcnt, c_rcnt, sizeof(uint32_t) * (nb + 1)));
+        uint32_t *rbase = static_cast<uint32_t *>(grow(be, d_rbase, c_rbase, sizeof(uint32_t) * (nb + 2)));
+        if (be.rc) return be.rc;
+        be.upload(first, h_first.data(), sizeof(int64_t) * nb);
+        be.template for_each<ScanCountTag>(nb, [=] __host__ __device__(int64_t b) {
+            uint32_t n = 0;
+            scan_block_records(s, len, first[b], blk[b].end, [&](int64_t) { ++n; });
+            rcnt[b] = n;
+        });
+        be.scan(rcnt, nb, rbase);
+        uint32_t h_nrec = 0;
+        be.download(&h_nrec, rbase + nb, sizeof(uint32_t));
+        be.sync();
+        if (be.rc) return be.rc;
+        const int64_t nrec = h_nrec;
+        int64_t *recpos = static_cast<int64_t *>(grow(be, d_recpos, c_recpos, sizeof(int64_t) * (size_t)std::max<int64_t>(1, nrec)));
+        uint32_t *nm = static_cast<uint32_t *>(grow(be, d_nm, c_nm, sizeof(uint32_t) * (size_t)(nrec + 1)));
+        uint32_t *kb = static_cast<uint32_t *>(grow(be, d_kb, c_kb, sizeof(uint32_t) * (size_t)(nrec + 1)));
+        uint32_t *ebase = static_cast<uint32_t *>(grow(be, d_ebase, c_ebase, sizeof(uint32_t) * (size_t)(nrec + 2)));
+        uint32_t *kbase = static_cast<uint32_t *>(grow(be, d_kbase, c_kbase, sizeof(uint32_t) * (size_t)(nrec + 2)));
+        if (be.rc) return be.rc;
+        {
+            const int64_t pk = prev_key;
+            int64_t *last = d_small;
+            uint32_t *err = d_err;
+            unsigned long long *depth = d_depth;
+            be.template for_each<ScanFillTag>(nb, [=] __host__ __device__(int64_t b) {
+                uint32_t k = rbase[b];
+                scan_block_records(s, len, first[b], blk[b].end, [&](int64_t p) { recpos[k++] = p; });
+            });
+            be.template for_each<ScanMatchTag>(nrec, [=] __host__ __device__(int64_t i) {
+                const uint32_t n = scan_record(s, recpos, i, pk, mt, depth, err);
+                nm[i] = n;
+                kb[i] = n ? 4u + (uint32_t)ld_i32(s, recpos[i]) : 0u;
+                if (i == nrec - 1) *last = order_key(ld_i32(s, recpos[i] + 4), ld_i32(s, recpos[i] + 8));
+            });
+        }
+        be.scan(nm, nrec, ebase);
+        be.scan(kb, nrec, kbase);
+        uint32_t h_tot[2] = {0, 0}, h_err = 0;
+        int64_t h_last = prev_key;
+        be.download(&h_tot[0], ebase + nrec, sizeof(uint32_t));
+        be.download(&h_tot[1], kbase + nrec, sizeof(uint32_t));
+        be.download(&h_err, d_err, sizeof(uint32_t));
+        if (nrec) be.download(&h_last, d_small, sizeof(int64_t));
+        be.sync();
+        if (be.rc) return be.rc;
+        if (h_err & SCAN_ERR_RECORD) { status = 3; tredsw_set_error("%s: corrupt BAM record", bam->path.c_str()); break; }
+        if (h_err & SCAN_ERR_ORDER) { status = 4; tredsw_set_error("%s is not sorted by coordinate", bam->path.c_str()); break; }
+        // copy the kept records once into the kept-record stream; one (fetch, position) entry per (record, fetch)
+        const int64_t nent = h_tot[0], kbytes = h_tot[1];
+        if (nent) {
+            if (kept_total + kbytes + 64 > (int64_t)c_kept) {
+                void *old = d_kept;
+                void *nw = be.alloc(std::max<size_t>((size_t)(kept_total + kbytes + 64), 2 * c_kept));
+                if (be.rc) return be.rc;
+                be.copy(nw, old, (size_t)kept_total);
+                d_kept = nw; c_kept = std::max<size_t>((size_t)(kept_total + kbytes + 64), 2 * c_kept);
+            }
+            int32_t *efetch = static_cast<int32_t *>(grow(be, d_efetch, c_efetch, sizeof(int32_t) * (size_t)nent));
+            int64_t *epos = static_cast<int64_t *>(grow(be, d_epos, c_epos, sizeof(int64_t) * (size_t)nent));
+            if (be.rc) return be.rc;
+            uint8_t *kept = static_cast<uint8_t *>(d_kept) + kept_total;
+            const int64_t k0 = kept_total;
+            be.template for_each_warp<ScanKeepTag>(nrec, [=] __host__ __device__(int64_t i, int lane) {
+                if (!nm[i]) return;
+                const int64_t p = recpos[i];
+                const uint32_t nbytes = kb[i], at = kbase[i];
+                for (uint32_t k = (uint32_t)lane; k < nbytes; k += NL) kept[at + k] = s[p + k];
+                if (lane) return;
+                const RecFields r = parse_record(s, p);
+                uint32_t e = ebase[i];
+                scan_matches(mt, r.tid, r.pos, record_fetch_end(r), [&](int32_t id) {
+                    if (id < mt.nfetch) { efetch[e] = id; epos[e] = k0 + at; ++e; }
+                });
+            });
+            const size_t e0 = ent_fetch.size();
+            ent_fetch.resize(e0 + nent); ent_pos.resize(e0 + nent);
+            be.download(ent_fetch.data() + e0, efetch, sizeof(int32_t) * (size_t)nent);
+            be.download(ent_pos.data() + e0, epos, sizeof(int64_t) * (size_t)nent);
+            be.sync();
+            if (be.rc) return be.rc;
+            kept_total += kbytes;
+        }
+        prev_key = h_last;
+        carry_at = tf; carry_len = len - tf; s0 = 0;
+        stats[0] += 1; stats[1] += nb; stats[2] += nrec;
+        stats[4] += sl.next - sl.begin; stats[5] += sl.inflated;
+        stats[7] += (int64_t)((now_ms() - t_dev) * 1e3);
+        if (reader.joinable()) reader.join();
+    }
+    if (reader.joinable()) reader.join();
+    if (!status && carry_len > 0) { status = 3; tredsw_set_error("%s ends inside a BAM record", bam->path.c_str()); }
+    stats[9] = status;
+
+    // ---- (3) depth regions; the entries grouped by fetch (stable counting sort: file order within a fetch) ----------
+    std::vector<unsigned long long> h_depth((size_t)std::max(1, n_depth));
+    be.download(h_depth.data(), d_depth, sizeof(unsigned long long) * (size_t)std::max(1, n_depth));
+    be.sync();
+    if (be.rc) return be.rc;
+    for (int d = 0; d < n_depth; ++d)
+        depth_out[d] = status ? NAN : (double)h_depth[d] * 1.0 / (double)(depth_regions[3 * d + 2] - depth_regions[3 * d + 1] + 1);
+    if (status) {
+        for (int p = 0; p < nq; ++p) if (!out->status[p]) out->status[p] = status;
+        ent_fetch.clear(); ent_pos.clear();
+    }
+    const int64_t nrec = (int64_t)ent_fetch.size();
+    if (nrec >= (1ll << 32)) { tredsw_set_error("too many selected records"); return TREDSW_ERR_IO; }
+    std::vector<uint32_t> fbase(nfetch + 2, 0);
+    for (int32_t f : ent_fetch) ++fbase[f + 1];
+    for (int f = 0; f < nfetch; ++f) fbase[f + 1] += fbase[f];
+    std::vector<int64_t> rpos((size_t)std::max<int64_t>(1, nrec));
+    std::vector<int32_t> rfetch((size_t)std::max<int64_t>(1, nrec));
+    {
+        std::vector<uint32_t> at(fbase.begin(), fbase.begin() + nfetch + 1);
+        for (int64_t e = 0; e < nrec; ++e) { const uint32_t k = at[ent_fetch[e]]++; rpos[k] = ent_pos[e]; rfetch[k] = ent_fetch[e]; }
+    }
+    out->n_blocks = stats[1]; out->n_records = stats[2];
+    out->comp_bytes = stats[4]; out->inflated_bytes = stats[5];
+    out->ms_host_stage = stats[6] * 1e-3;
+    out->ms_marks[0] = now_ms() - t_begin;
+    if (nq == 0) {
+        be.release_intermediates();
+        out->ms_total = now_ms() - t_begin;
+        stats[8] = (int64_t)(out->ms_total * 1e3);
+        tredsw_ingest_view &v = out->view;
+        v.n_blocks = out->n_blocks; v.n_records = out->n_records; v.comp_bytes = out->comp_bytes; v.inflated_bytes = out->inflated_bytes;
+        v.ms_host_stage = out->ms_host_stage; v.ms_total = out->ms_total; v.ms_marks[0] = out->ms_marks[0];
+        return TREDSW_OK;
+    }
+    Fetch *d_fetches = static_cast<Fetch *>(be.alloc(sizeof(Fetch) * (size_t)std::max(1, nfetch)));
+    ProblemParams *d_params = static_cast<ProblemParams *>(be.alloc(sizeof(ProblemParams) * (size_t)nq));
+    ProblemCounts *d_counts = static_cast<ProblemCounts *>(be.alloc(sizeof(ProblemCounts) * (size_t)nq));
+    int64_t *d_rpos = static_cast<int64_t *>(be.alloc(sizeof(int64_t) * rpos.size()));
+    int32_t *d_rfetch = static_cast<int32_t *>(be.alloc(sizeof(int32_t) * rfetch.size()));
+    uint32_t *d_fbase = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * fbase.size()));
+    if (!d_kept) d_kept = be.alloc(64);
+    if (be.rc) return be.rc;
+    be.upload(d_fetches, fetches.data(), sizeof(Fetch) * (size_t)nfetch);
+    be.upload(d_params, params.data(), sizeof(ProblemParams) * (size_t)nq);
+    be.fill(d_counts, 0, sizeof(ProblemCounts) * (size_t)nq);
+    be.upload(d_rpos, rpos.data(), sizeof(int64_t) * (size_t)nrec);
+    be.upload(d_rfetch, rfetch.data(), sizeof(int32_t) * (size_t)nrec);
+    be.upload(d_fbase, fbase.data(), sizeof(uint32_t) * fbase.size());
+    const int rc = select_and_pair(be, out, static_cast<const uint8_t *>(d_kept), d_fetches, d_rpos, d_rfetch, d_fbase, nrec,
+                                   fetch_first, params, d_params, d_counts, want_names, t_begin);
+    stats[8] = (int64_t)(out->ms_total * 1e3);
+    return rc;
+}
+
+namespace {
+// (once per device) keep freed blocks in the stream-ordered pool: the buffers of consecutive batches have similar sizes
+void keep_pool(int device) {
+    static bool pool_set[64] = {false};
+    if (device < 64 && !pool_set[device]) {
+        cudaMemPool_t pool;
+        if (cudaDeviceGetDefaultMemPool(&pool, device) == cudaSuccess) {
+            unsigned long long thr = ~0ull;
+            cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &thr);
+        }
+        pool_set[device] = true;
+    }
+}
+}  // namespace
+
 extern "C" {
+
+int tredsw_ingest_scan_run(tredsw_ctx *ctx, tredsw_bam *bam, const tredsw_locus_query *queries, int32_t nqueries,
+                           const int32_t *depth_regions, int32_t n_depth, double *depth_out, int64_t slab_bytes,
+                           uint32_t flags, tredsw_ingest_batch **out) {
+    if (!ctx || !bam || !out || nqueries < 0 || (nqueries > 0 && !queries) || n_depth < 0 ||
+        (n_depth > 0 && (!depth_regions || !depth_out)) || slab_bytes < 0) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
+    *out = nullptr;
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    keep_pool(ctx->device);
+    std::unique_ptr<tredsw_ingest_batch> b(new tredsw_ingest_batch());
+    b->cuda.stream = ctx->stream;
+    int rc;
+    try { rc = run_scan(b->cuda, b.get(), bam, queries, nqueries, depth_regions, n_depth, depth_out, slab_bytes, flags); }
+    catch (const std::exception &e) { tredsw_set_error("tredsw_ingest_scan_run: %s", e.what()); rc = TREDSW_ERR_IO; }
+    ctx->launches += b->cuda.launches;
+    if (rc) { b->cuda.release(); return rc; }
+    *out = b.release();
+    return TREDSW_OK;
+}
+
+// TEST INFRASTRUCTURE: tredsw_ingest_scan_run with every kernel body run serially on the host.  Not used by the package.
+int tredsw_ingest_scan_emulate(tredsw_bam *bam, const tredsw_locus_query *queries, int32_t nqueries,
+                               const int32_t *depth_regions, int32_t n_depth, double *depth_out, int64_t slab_bytes,
+                               uint32_t flags, tredsw_ingest_batch **out) {
+    if (!bam || !out || nqueries < 0 || (nqueries > 0 && !queries) || n_depth < 0 ||
+        (n_depth > 0 && (!depth_regions || !depth_out)) || slab_bytes < 0) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
+    *out = nullptr;
+    std::unique_ptr<tredsw_ingest_batch> b(new tredsw_ingest_batch());
+    b->emulated = true;
+    int rc;
+    try { rc = run_scan(b->host, b.get(), bam, queries, nqueries, depth_regions, n_depth, depth_out, slab_bytes, flags); }
+    catch (const std::exception &e) { tredsw_set_error("tredsw_ingest_scan_emulate: %s", e.what()); rc = TREDSW_ERR_IO; }
+    if (rc) { b->host.release(); return rc; }
+    *out = b.release();
+    return TREDSW_OK;
+}
+
+int tredsw_ingest_scan_stats(const tredsw_ingest_batch *b, int64_t *stats) {
+    if (!b || !stats) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
+    memcpy(stats, b->scan_stats, sizeof(b->scan_stats));
+    return TREDSW_OK;
+}
 
 int tredsw_ingest_batch_run(tredsw_ctx *ctx, tredsw_bam *const *bams, const int32_t *sample_of,
                             const tredsw_locus_query *queries, int32_t nqueries, uint32_t flags, tredsw_ingest_batch **out) {
@@ -870,16 +1373,7 @@ int tredsw_ingest_batch_run(tredsw_ctx *ctx, tredsw_bam *const *bams, const int3
     *out = nullptr;
     std::lock_guard<std::mutex> lock(ctx->mu);
     CUDA_TRY(cudaSetDevice(ctx->device));
-    static bool pool_set[64] = {false};
-    if (ctx->device < 64 && !pool_set[ctx->device]) {
-        // keep freed blocks in the stream-ordered pool: the buffers of consecutive batches have similar sizes
-        cudaMemPool_t pool;
-        if (cudaDeviceGetDefaultMemPool(&pool, ctx->device) == cudaSuccess) {
-            unsigned long long thr = ~0ull;
-            cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &thr);
-        }
-        pool_set[ctx->device] = true;
-    }
+    keep_pool(ctx->device);
     std::unique_ptr<tredsw_ingest_batch> b(new tredsw_ingest_batch());
     b->cuda.stream = ctx->stream;
     int rc;

@@ -30,7 +30,8 @@ using namespace tredsw_ingest;
 
 extern "C" {
 
-tredsw_bam *tredsw_bam_open(const char *bam_path, const char *bai_path) {
+// the handle with its header read (reference dictionary, first record), no index yet
+static tredsw_bam *open_header(const char *bam_path) {
     if (!bam_path) { tredsw_set_error("null path"); return nullptr; }
     tredsw_bam *b = new tredsw_bam();
     b->bgzf.fh = fopen(bam_path, "rb");
@@ -54,6 +55,14 @@ tredsw_bam *tredsw_bam_open(const char *bam_path, const char *bai_path) {
     }
     b->first_record = b->bgzf.tell();
     b->path = bam_path;
+    return b;
+}
+
+tredsw_bam *tredsw_bam_open_unindexed(const char *bam_path) { return open_header(bam_path); }
+
+tredsw_bam *tredsw_bam_open(const char *bam_path, const char *bai_path) {
+    tredsw_bam *b = open_header(bam_path);
+    if (!b) return nullptr;
     // index: <bam>.bai, then <bam without extension>.bai (bamio.AlignmentFile)
     std::string cands[2];
     if (bai_path) cands[0] = bai_path;
@@ -165,6 +174,7 @@ int32_t tredsw_bam_tid(tredsw_bam *b, const char *name) {
 // (same restatement as bamio.region_depth).
 int tredsw_bam_region_depth(tredsw_bam *b, int32_t tid, int64_t start, int64_t end, double *depth) {
     if (!b || !depth) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
+    if (!b->has_index) { tredsw_set_error("%s has no index", b->path.c_str()); return TREDSW_ERR_UNSUPPORTED; }
     if (tid < 0 || tid >= (int)b->names.size()) { tredsw_set_error("contig id %d out of range", tid); return TREDSW_ERR_ARG; }
     if (end < start) { tredsw_set_error("empty region"); return TREDSW_ERR_ARG; }
     int64_t total = 0;
@@ -211,6 +221,7 @@ int tredsw_bam_extract_locus(tredsw_bam *b, const tredsw_locus_query *q, int8_t 
                              int32_t *target_lens, int32_t target_cap, char *names, int64_t names_cap,
                              tredsw_locus_summary *out) {
     if (!b || !q || !out || !roff || reads_cap < 0) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
+    if (!b->has_index) { tredsw_set_error("%s has no index", b->path.c_str()); return TREDSW_ERR_UNSUPPORTED; }
     b->bgzf.err = nullptr;
     int rc;
     try {

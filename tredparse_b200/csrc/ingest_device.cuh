@@ -673,4 +673,153 @@ TG_HD int pair_eval(const Mate &x, const Mate &y, const ProblemParams &q, int32_
     return (x.pos < q.tstart && y.ref_end > q.tend) ? 2 : 1;
 }
 
+// ---- scan of a BAM without an index (tredsw_ingest_scan_run) ---------------------------------------------------------
+// A slab of the file is inflated into one stream: the carry (the bytes of the last record of the previous slab that was
+// not complete there) followed by the slab's blocks.  Nothing says where a record starts inside a block, so:
+//   1. candidate: the first offset of every block where a record header passes a strict predicate, and so do the next
+//      two records of the chain it starts (one warp per block, 32 offsets per step);
+//   2. landing: from its candidate, the chain (block_size only) to the first record at or after the block's end;
+//   3. the true start of block 0 is known (after the header / the carry); wherever a block's landing equals the next
+//      block's candidate, that candidate is a true record start, by induction.  Where they differ, the landing is the
+//      true start and the chain is walked again from it (scan_repair_run, on the few such blocks).
+// Every record position the later steps use therefore comes from a chain that starts at a known record.
+constexpr int64_t SCAN_NONE = -1;           // no candidate in the block
+constexpr int64_t SCAN_BAD = -2;            // the chain met an implausible block_size: corrupt records
+struct ScanBlock { int64_t begin, end; };   // a block's bytes in the slab stream (block 0 includes the carry)
+
+// strict record predicate at p (offsets relative to the stream s[0, len)); *bs: its block_size
+TG_HD bool scan_plausible(const uint8_t *s, int64_t len, int64_t p, int32_t n_ref, int32_t *bs) {
+    if (p + 36 > len) return false;
+    const int32_t b = ld_i32(s, p), tid = ld_i32(s, p + 4), pos = ld_i32(s, p + 8), l_seq = ld_i32(s, p + 20);
+    const int32_t next_tid = ld_i32(s, p + 24);
+    const int l_name = s[p + 12];
+    const int n_cigar = (int)ld_u16(s, p + 16);
+    if (b < 33 || b > (64 << 20)) return false;
+    if (tid < -1 || tid >= n_ref || next_tid < -1 || next_tid >= n_ref || pos < -1) return false;
+    if (l_name < 1 || l_seq < 0 || p + 36 + l_name > len || s[p + 35 + l_name] != 0) return false;
+    if (32LL + l_name + 4LL * n_cigar + ((int64_t)l_seq + 1) / 2 + l_seq > (int64_t)b) return false;
+    *bs = b;
+    return true;
+}
+// p passes the predicate, and so do the next two records of its chain as far as they lie in the stream
+TG_HD bool scan_candidate_ok(const uint8_t *s, int64_t len, int64_t p, int32_t n_ref) {
+    for (int k = 0; k < 3; ++k) {
+        if (k > 0 && p + 36 > len) return true;
+        int32_t bs;
+        if (!scan_plausible(s, len, p, n_ref, &bs)) return false;
+        p += 4 + (int64_t)bs;
+    }
+    return true;
+}
+// first offset of [begin, end) that passes scan_candidate_ok, or SCAN_NONE; NL lanes test NL consecutive offsets a step
+template <int NL>
+TG_HD int64_t scan_find_candidate(const uint8_t *s, int64_t len, int64_t begin, int64_t end, int32_t n_ref, int lane) {
+    for (int64_t o0 = begin; o0 < end; o0 += NL) {
+        const int64_t o = o0 + lane;
+        const bool ok = o < end && scan_candidate_ok(s, len, o, n_ref);
+#if defined(__CUDA_ARCH__)
+        const uint32_t m = __ballot_sync(0xffffffffu, ok);
+        if (m) return o0 + __ffs(m) - 1;
+#else
+        if (ok) return o;
+#endif
+    }
+    return SCAN_NONE;
+}
+// Follows the chain from the record at p to the first record at or after `end`.  Stops early at a record that is not
+// complete in the stream (it is carried into the next slab) and returns its start; SCAN_BAD at an implausible size.
+TG_HD int64_t scan_chain(const uint8_t *s, int64_t len, int64_t p, int64_t end) {
+    while (p < end) {
+        if (p + 4 > len) return p;
+        const int32_t bs = ld_i32(s, p);
+        if (bs < 32 || bs > (64 << 20)) return SCAN_BAD;
+        if (p + 4 + (int64_t)bs > len) return p;
+        p += 4 + (int64_t)bs;
+    }
+    return p;
+}
+// Where the chain entering block b at `tf` stands relative to the block's candidate: true when the block needs no walk
+// from tf (no record starts in it, or its candidate is tf and so its landing is right).
+TG_HD bool scan_agrees(const ScanBlock &blk, int64_t cand, int64_t tf) {
+    return tf < blk.begin || tf >= blk.end || cand == tf;
+}
+// The repair of a run of blocks whose candidates were wrong: walk from the true start tf of block b on, block after
+// block, until the chain agrees with a block's candidate again.  land[k] receives the true landing of every block
+// walked; returns the first block not walked.
+TG_HD int scan_repair_run(const uint8_t *s, int64_t len, const ScanBlock *blk, const int64_t *cand, int nblocks, int b,
+                          int64_t tf, int64_t *land) {
+    for (;;) {
+        tf = scan_chain(s, len, tf, blk[b].end);
+        land[b] = tf;
+        ++b;
+        if (b >= nblocks || tf == SCAN_BAD || scan_agrees(blk[b], cand[b], tf)) return b;
+    }
+}
+// records that start in a block: from its true first record, while they start before the block's end and are complete
+template <class F>
+TG_HD void scan_block_records(const uint8_t *s, int64_t len, int64_t p, int64_t end, F &&f) {
+    while (p < end && p + 4 <= len) {
+        const int64_t next = p + 4 + (int64_t)ld_i32(s, p);
+        if (next > len) return;
+        f(p);
+        p = next;
+    }
+}
+
+// Records -> fetches.  A record [pos, rend) belongs to a fetch [start, end) of its contig when pos < end and
+// rend > start (tredsw_bam::fetch).  The fetches of a scan (locus windows, alt regions, then depth regions: ids >=
+// nfetch) are cut, per contig, into elementary segments between consecutive fetch boundaries; segment j =
+// [xs[j], xs[j + 1]) lists the fetches that cover it.  A record meets every fetch that covers a segment it overlaps; a
+// fetch is reported once, at the first such segment (the record's first segment, or the one where the fetch starts).
+// (A fetch with end <= start holds the records that contain [end - 1, start + 1): it is listed on [end - 1, end) and
+// the rule above is checked for every fetch reported.)
+struct MatchTables {
+    const int32_t *tid_x0;      // n_ref + 1: contig t owns xs[tid_x0[t], tid_x0[t + 1])
+    const int64_t *xs;          // segment boundaries
+    const int32_t *seg_f0;      // segment j lists seg_ids[seg_f0[j], seg_f0[j + 1])
+    const int32_t *seg_ids;
+    const int64_t *id_lo;       // first boundary of every fetch / depth region in xs
+    const int64_t *id_start, *id_end;
+    int32_t n_ref, nfetch;
+};
+template <class F>
+TG_HD void scan_matches(const MatchTables &m, int32_t tid, int64_t pos, int64_t rend, F &&f) {
+    if (tid < 0 || tid >= m.n_ref) return;
+    const int k0 = m.tid_x0[tid], k1 = m.tid_x0[tid + 1];
+    int lo = k0, hi = k1;                                   // first boundary > pos
+    while (lo < hi) { const int mid = (lo + hi) >> 1; if (m.xs[mid] <= pos) lo = mid + 1; else hi = mid; }
+    const int j0 = lo > k0 ? lo - 1 : k0;
+    for (int j = j0; j < k1 - 1 && m.xs[j] < rend; ++j)
+        for (int e = m.seg_f0[j]; e < m.seg_f0[j + 1]; ++e) {
+            const int32_t id = m.seg_ids[e];
+            if ((j == j0 || m.id_lo[id] >= m.xs[j]) && pos < m.id_end[id] && rend > m.id_start[id]) f(id);
+        }
+}
+// the overlap interval of a record as tredsw_bam::fetch tests it
+TG_HD int64_t record_fetch_end(const RecFields &r) {
+    int64_t rend = (int64_t)r.pos + r.ref_len;
+    if ((r.flag & 4) || !r.has_cigar || rend <= r.pos) rend = (int64_t)r.pos + 1;
+    return rend;
+}
+TG_HD int64_t order_key(int32_t tid, int32_t pos) {         // coordinate order: unmapped records (tid -1) last
+    return ((int64_t)(tid < 0 ? 0x7fffffff : tid) << 32) + ((int64_t)pos + 1);
+}
+enum : uint32_t { SCAN_ERR_RECORD = 1u, SCAN_ERR_ORDER = 2u };
+// per record: matched fetches (depth regions are summed here, with the pileup filter of select_record), order check
+TG_HD uint32_t scan_record(const uint8_t *s, const int64_t *rec_pos, int64_t i, int64_t prev_key, const MatchTables &m,
+                           unsigned long long *depth_sum, uint32_t *err) {
+    const int64_t p = rec_pos[i];
+    const RecFields r = parse_record(s, p);
+    if (!r.ok) { atomic_or_u32(err, SCAN_ERR_RECORD); return 0; }
+    const int64_t before = i ? order_key(ld_i32(s, rec_pos[i - 1] + 4), ld_i32(s, rec_pos[i - 1] + 8)) : prev_key;
+    if (order_key(r.tid, r.pos) < before) atomic_or_u32(err, SCAN_ERR_ORDER);
+    uint32_t n = 0;
+    const bool counted = !(r.flag & (4 | 256 | 512 | 1024)) && r.has_cigar;
+    scan_matches(m, r.tid, r.pos, record_fetch_end(r), [&](int32_t id) {
+        if (id < m.nfetch) ++n;
+        else if (counted) atomic_add_u64(&depth_sum[id - m.nfetch], (unsigned long long)r.ref_len);
+    });
+    return n;
+}
+
 }  // namespace tredsw_gi

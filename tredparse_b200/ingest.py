@@ -7,6 +7,9 @@ layout ``cohort.CohortBatch`` / ``tredsw_genotype_batch`` consume.  Host code on
     with BamIngest("sample.bam") as bam:
         ev = bam.extract_locus(repo["HD"], readlen=150)          # reads (codes), pair lengths, depth
         problem = bam.problem(repo["HD"], readlen=150)           # ready for cohort.CohortBatch([...])
+
+A BAM without a usable index is read on the GPU in one pass per sample: ``scan_sample(ctx, BamIngest.unindexed(path),
+...)``.
 """
 import ctypes
 
@@ -38,6 +41,8 @@ def _bind(lib):
         return
     lib.tredsw_bam_open.restype = ctypes.c_void_p
     lib.tredsw_bam_open.argtypes = [ctypes.c_char_p, ctypes.c_char_p]
+    lib.tredsw_bam_open_unindexed.restype = ctypes.c_void_p
+    lib.tredsw_bam_open_unindexed.argtypes = [ctypes.c_char_p]
     lib.tredsw_bam_inflate_stats.restype = None
     lib.tredsw_bam_inflate_stats.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_int64)]
     lib.tredsw_inflate_raw.restype = ctypes.c_int
@@ -98,6 +103,20 @@ class BamIngest:
         if not self.handle:
             raise IOError("tredsw_bam_open({}): {}".format(path, _lib.last_error()))
         self._caps = dict(reads=512, bases=512 * 256, pairs=8192, names=512 * 48)
+
+    @classmethod
+    def unindexed(cls, path):
+        """A handle on a BAM without a usable index: header, contig ids and read length only (``scan_sample`` reads
+        its evidence in one pass over the file; ``extract_locus`` and ``region_depth`` refuse it)."""
+        self = object.__new__(cls)
+        self.lib = _lib.load()
+        _bind(self.lib)
+        self.path = path
+        self.handle = self.lib.tredsw_bam_open_unindexed(path.encode())
+        if not self.handle:
+            raise IOError("tredsw_bam_open_unindexed({}): {}".format(path, _lib.last_error()))
+        self._caps = dict(reads=512, bases=512 * 256, pairs=8192, names=512 * 48)
+        return self
 
     def inflate_stats(self):
         """(blocks inflated by the library's own decoder, blocks that fell back to zlib) for this handle."""
@@ -267,6 +286,14 @@ def _bind_batch(lib):
     lib.tredsw_ingest_batch_view.argtypes = [ctypes.c_void_p, ctypes.POINTER(IngestView)]
     lib.tredsw_ingest_batch_free.restype = None
     lib.tredsw_ingest_batch_free.argtypes = [ctypes.c_void_p]
+    lib.tredsw_ingest_scan_run.restype = ctypes.c_int
+    lib.tredsw_ingest_scan_run.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.POINTER(LocusQuery), ctypes.c_int32,
+                                           ctypes.c_void_p, ctypes.c_int32, ctypes.c_void_p, ctypes.c_int64,
+                                           ctypes.c_uint32, ctypes.POINTER(ctypes.c_void_p)]
+    lib.tredsw_ingest_scan_emulate.restype = ctypes.c_int
+    lib.tredsw_ingest_scan_emulate.argtypes = lib.tredsw_ingest_scan_run.argtypes[1:]
+    lib.tredsw_ingest_scan_stats.restype = ctypes.c_int
+    lib.tredsw_ingest_scan_stats.argtypes = [ctypes.c_void_p, ctypes.c_void_p]
     lib.tredsw_inflate_raw_device_code.restype = ctypes.c_int
     lib.tredsw_inflate_raw_device_code.argtypes = [ctypes.c_char_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_int64]
     lib._ingest_batch_bound = True
@@ -323,6 +350,10 @@ class IngestBatch:
         else:
             rc = self.lib.tredsw_ingest_batch_run(ctx.handle, hs, so.ctypes.data, qs, n, flags, ctypes.byref(out))
         _lib.check(rc, "tredsw_ingest_batch_run")
+        self._attach(out, n, want_names)
+
+    def _attach(self, out, n, want_names):
+        """take over the tredsw_ingest_batch `out` of n problems"""
         self.handle = out
         self.view = IngestView()
         _lib.check(self.lib.tredsw_ingest_batch_view(self.handle, ctypes.byref(self.view)), "tredsw_ingest_batch_view")
@@ -384,3 +415,50 @@ class IngestBatch:
             self.close()
         except Exception:
             pass
+
+
+SCAN_NSTATS = 10
+
+
+class ScanBatch(IngestBatch):
+    """The evidence of one sample read in ONE pass over a BAM without an index (``tredsw_ingest_scan_run``): an
+    ``IngestBatch`` (``.status``, ``.evidence(i)``, the device buffers), plus ``.depths`` (the depth of every
+    requested region) and the scan's statistics.  Build it with ``scan_sample``."""
+
+    def __init__(self, ctx, handle, queries, keep=(), depth_regions=(), slab_bytes=None, want_names=True, check_crc=True):
+        self.lib = _lib.load()
+        _bind(self.lib)
+        _bind_batch(self.lib)
+        n = len(queries)
+        self._keep = (list(keep), [handle])
+        qs = (LocusQuery * max(1, n))(*queries)
+        dr = np.ascontiguousarray(np.array(depth_regions, dtype=np.int32).reshape(-1, 3))
+        depths = np.zeros(max(1, len(dr)), dtype=np.float64)
+        flags = (0 if want_names else INGEST_NO_NAMES) | (0 if check_crc else INGEST_NO_CRC)
+        out = ctypes.c_void_p()
+        args = (handle.handle, qs, n, dr.ctypes.data if len(dr) else None, len(dr), depths.ctypes.data,
+                int(slab_bytes or 0), flags, ctypes.byref(out))
+        if ctx is None:
+            rc = self.lib.tredsw_ingest_scan_emulate(*args)
+        else:
+            rc = self.lib.tredsw_ingest_scan_run(ctx.handle, *args)
+        _lib.check(rc, "tredsw_ingest_scan_run")
+        self._attach(out, n, want_names)
+        self.depths = depths[:len(dr)]
+        st = np.zeros(SCAN_NSTATS, dtype=np.int64)
+        _lib.check(self.lib.tredsw_ingest_scan_stats(self.handle, st.ctypes.data), "tredsw_ingest_scan_stats")
+        self.scan_status = int(st[9])
+        self._scan = dict(zip(("slabs", "blocks", "records", "repaired_blocks", "compressed_bytes", "inflated_bytes"),
+                              (int(x) for x in st[:6])))
+        self._scan.update(ms_host_read=st[6] * 1e-3, ms_device=st[7] * 1e-3, ms_total=st[8] * 1e-3)
+
+    def stats(self):
+        return dict(self._scan)
+
+
+def scan_sample(ctx, handle, queries, keep, depth_regions, slab_bytes=None):
+    """Every locus of one sample (``queries``: ``LocusQuery`` records, alt regions included) and the depth of
+    ``depth_regions`` ((tid, start, end) rows) in one streaming pass over a BAM opened with ``BamIngest.unindexed``.
+    ``slab_bytes``: compressed bytes read per step (None: 128 MiB).  ``ctx=None`` runs the serial host emulation of
+    the device code — test infrastructure only.  -> ScanBatch"""
+    return ScanBatch(ctx, handle, queries, keep=keep, depth_regions=depth_regions, slab_bytes=slab_bytes)

@@ -327,10 +327,51 @@ def ingest_chunk_gpu(samples, ctx=None, keep_batch=None):
         return {}
 
 
-def presteps(bam, repo, tredNames, logger, ing=None):
-    """The per-sample pre-steps of tred.run (tred.py:195-223): gender from the chrY depth — only when an X-linked
-    locus is requested; 'Unknown' / -1 when the lookup fails — and the read length (150 when it cannot be read).
-    They decide ploidy (bam_parser.py:58-61) and the number of templates (:73), so they gate parity on real BAMs."""
+def ingest_sample_scan(arg, wanted, READLEN, h, with_gender, ctx=None):
+    """Evidence of every wanted locus of one sample whose BAM has no usable index, and its chrY depth when
+    ``with_gender``, in ONE streaming pass over the file on the GPU (``ingest.scan_sample``).
+    :param h: the sample's handle from ``ingest.BamIngest.unindexed``
+    :return: ({tredName: LocusEvidence}, (gender, depthY) or None) — loci the scan could not serve (contig missing,
+             a corrupt or unsorted file) are left out, and so is the gender: the caller reads them with the Python
+             reader."""
+    from . import _lib
+    from .ingest import locus_query, scan_sample
+    samplekey, bam, repo, tredNames, maxinsert, fullsearch, clip, alts, repeatpairs, log = arg
+    qs, keep, names = [], [], []
+    for t in wanted:
+        xtred = repo[t]
+        q = locus_query(h, xtred, READLEN, alts=alt_regions(xtred, repo.ref, alts, clip))
+        if q is None:
+            continue
+        qs.append(q[0]); keep.append(q[1]); names.append(t)
+    yreg = []
+    if with_gender:
+        rows = BamDepth.y_regions(repo.ref)
+        tids = [h.tid(c) for c, s, e in rows]
+        if rows and min(tids) >= 0:
+            yreg = [(t, s, e) for t, (c, s, e) in zip(tids, rows)]
+    got, gender = {}, None
+    if not qs and not yreg:
+        return got, gender
+    try:
+        with scan_sample(ctx or _lib.default_context(), h, qs, keep, yreg) as b:
+            for i, t in enumerate(names):
+                if b.status[i]:
+                    logger.debug("GPU scan handed {} / {} back (status {})".format(samplekey, t, int(b.status[i])))
+                    continue
+                got[t] = b.evidence(i)
+            if yreg and not b.scan_status:
+                ydepth = float(np.median(b.depths))
+                gender = ("Male" if ydepth > 1 else "Female", ydepth)
+    except Exception as e:
+        logger.error("GPU scan of `{}` failed ({}); reading with the Python reader".format(bam, e))
+        return {}, None
+    return got, gender
+
+
+def infer_gender(bam, repo, tredNames, logger, ing=None):
+    """Gender from the chrY depth (tred.py:195-211) — only when an X-linked locus is requested; 'Unknown' / -1 when
+    the lookup fails.  -> (gender, depthY)"""
     gender, ydepth = "Unknown", -1
     if any(repo[tred].is_xlinked for tred in tredNames):
         try:
@@ -339,6 +380,14 @@ def presteps(bam, repo, tredNames, logger, ing=None):
         except Exception:
             pass
         logger.debug("Inferred gender: {} (depthY={})".format(gender, ydepth))
+    return gender, ydepth
+
+
+def presteps(bam, repo, tredNames, logger, ing=None, with_gender=True):
+    """The per-sample pre-steps of tred.run (tred.py:195-223): gender (``infer_gender``; 'Unknown' / -1 without
+    ``with_gender``) and the read length (150 when it cannot be read).  They decide ploidy (bam_parser.py:58-61) and
+    the number of templates (:73), so they gate parity on real BAMs."""
+    gender, ydepth = infer_gender(bam, repo, tredNames, logger, ing=ing) if with_gender else ("Unknown", -1)
     READLEN = 150
     try:
         READLEN = BamReadLen(bam, logger, ing=ing).readlen
@@ -365,39 +414,61 @@ def prepare_chunk(args, only=None, ctx=None):
         out.append({"samplekey": samplekey, "bam": bam, "tredCalls": tredCalls, "_fields": {}, "_names": list(tredNames)})
     # per sample: one native handle (validity check, pre-steps, GPU ingest), the pre-steps (gender looks at every
     # requested locus); the samples are dealt to host threads
+    # a BAM without a usable index is scanned once on the GPU (unless the GPU ingest is off): its gender comes from
+    # that scan, so its pre-steps here read only the read length
     def pre(si):
         samplekey, bam, repo, tredNames = args[si][:4]
+        from .ingest import BamIngest
         ing = None
         try:
-            from .ingest import BamIngest
             ing = BamIngest(bam_path(bam))
         except Exception as e:
             logger.debug("native BAM ingest unavailable for `{}` ({})".format(bam, e))
             if check_bam(bam) is None:
                 return None
-        return ing, presteps(bam, repo, tredNames, logger, ing=ing)
+            if GPU_INGEST:
+                try:
+                    uh = BamIngest.unindexed(bam_path(bam))
+                    return uh, presteps(bam, repo, tredNames, logger, ing=uh, with_gender=False), True
+                except Exception as e2:
+                    logger.debug("GPU scan unavailable for `{}` ({})".format(bam, e2))
+        return ing, presteps(bam, repo, tredNames, logger, ing=ing), False
     if len(args) > 1 and INGEST_THREADS > 1:
         from concurrent.futures import ThreadPoolExecutor
         with ThreadPoolExecutor(max_workers=min(INGEST_THREADS, len(args))) as pool:
             pres = list(pool.map(pre, range(len(args))))
     else:
         pres = [pre(si) for si in range(len(args))]
-    wanted_of, handle_of = {}, {}
+    wanted_of, handle_of, unindexed = {}, {}, set()
     for si, ps in enumerate(pres):
         if ps is None:
             continue
         todo.append(si)
         handle_of[si] = ps[0]
+        if ps[2]:
+            unindexed.add(si)
         out[si]["tredCalls"].update(ps[1])
         tredNames = args[si][3]
         wanted_of[si] = [t for t in tredNames if only is None or t in only[si]]
         out[si]["_names"] = wanted_of[si]
-    # evidence: the GPU ingest for every (sample, locus) of the chunk in one pass; the host reader for what it
-    # hands back (no index, corrupt blocks, unknown contig) or when it is switched off (TREDSW_GPU_INGEST=0)
+    # evidence: the GPU ingest for every (sample, locus) of the chunk in one pass, one GPU scan per sample without an
+    # index; the host reader for what they hand back (corrupt blocks, unsorted files, unknown contig) or when they are
+    # switched off (TREDSW_GPU_INGEST=0)
     kept = []
     try:
-        got = ingest_chunk_gpu([(si, args[si], wanted_of[si], out[si]["tredCalls"]["readLen"], handle_of[si])
-                                for si in todo], ctx=ctx, keep_batch=kept if DEVICE_HANDOFF else None) if GPU_INGEST else {}
+        got = ingest_chunk_gpu([(si, args[si], wanted_of[si], out[si]["tredCalls"]["readLen"],
+                                 None if si in unindexed else handle_of[si]) for si in todo],
+                               ctx=ctx, keep_batch=kept if DEVICE_HANDOFF else None) if GPU_INGEST else {}
+        for si in sorted(unindexed):
+            samplekey, bam, repo, tredNames = args[si][:4]
+            with_gender = any(repo[t].is_xlinked for t in tredNames)
+            got[si], gender = ingest_sample_scan(args[si], wanted_of[si], out[si]["tredCalls"]["readLen"],
+                                                 handle_of[si], with_gender, ctx=ctx)
+            if gender is None and with_gender:
+                gender = infer_gender(bam, repo, tredNames, logger)
+            if gender is not None:
+                logger.debug("Inferred gender: {} (depthY={})".format(*gender))
+                out[si]["tredCalls"].update({"inferredGender": gender[0], "depthY": gender[1]})
     finally:
         for h in handle_of.values():
             if h is not None:
