@@ -455,10 +455,22 @@ tredsw_bam *tredsw_bam_open_unindexed(const char *bam_path);
  * every block, finds the record boundaries without an index (a candidate per block, verified by chaining from the
  * known first record), keeps the records that overlap a fetch of `queries` (locus windows and alt regions) and sums
  * the depth of `depth_regions` (n_depth x (tid, start, end); depth_out[d] = what tredsw_bam_region_depth returns for
- * region d, NaN when the scan failed).  The result is an ordinary batch (tredsw_ingest_batch_view / _free), with the
+ * region d, NaN when the scan failed).  On a stream handle the slabs are read in order with read() (a slab of slab_bytes
+ * is not capped by a size) and the end of the input is read() returning 0.  The result is an ordinary batch (tredsw_ingest_batch_view / _free), with the
  * same evidence as tredsw_ingest_batch_run on an indexed copy, problem by problem.  Its status is per scan: every
  * problem gets 1 (I/O, BGZF framing), 2 (a block failed to inflate), 3 (corrupt or truncated records) or 4 (the file is
  * not sorted by coordinate: tid non-decreasing with -1 last, pos non-decreasing within a tid). */
+/* A BAM read strictly in order with read(): a pipe, a FIFO, a socket, or stdin when bam_path is "-" (a regular file works
+ * too, read the same way).  No seek, no size.  The handle parses the header from the bytes it has read and keeps every
+ * byte from the block of the first record on; tredsw_bam_read_length reads the first records ahead and answers from
+ * them.  tredsw_bam_tid, tredsw_bam_header_signature and tredsw_bam_header_text work on it; tredsw_bam_clone,
+ * tredsw_bam_extract_locus, tredsw_bam_region_depth and tredsw_ingest_batch_run refuse it (TREDSW_ERR_UNSUPPORTED).  The
+ * stream can be scanned ONCE (tredsw_ingest_scan_run / _emulate): a second scan, or a read length after the scan, is
+ * TREDSW_ERR_ARG.  NULL + tredsw_last_error() on failure. */
+tredsw_bam *tredsw_bam_open_stream(const char *bam_path);
+/* The SAM header text of any handle: copies at most cap - 1 bytes and a NUL into buf (buf may be NULL); returns the
+ * length of the whole text. */
+int64_t tredsw_bam_header_text(tredsw_bam *bam, char *buf, int64_t cap);
 int tredsw_ingest_scan_run(tredsw_ctx *ctx, tredsw_bam *bam, const tredsw_locus_query *queries, int32_t nqueries,
                            const int32_t *depth_regions, int32_t n_depth, double *depth_out, int64_t slab_bytes,
                            uint32_t flags, tredsw_ingest_batch **out);

@@ -37,6 +37,7 @@ EXPORTS = [
     "tredsw_inflate_raw_device_code",
     # BAMs without an index: one streaming pass per sample
     "tredsw_bam_open_unindexed", "tredsw_ingest_scan_run", "tredsw_ingest_scan_emulate", "tredsw_ingest_scan_stats",
+    "tredsw_bam_open_stream", "tredsw_bam_header_text",
 ]
 
 

@@ -455,6 +455,7 @@ int run_pipeline(B &be, tredsw_ingest_batch *out, tredsw_bam *const *bams, const
         SamplePlan &sp = plans[sample_of[i]];
         sp.bam = bams[sample_of[i]];
         if (!sp.bam) { tredsw_set_error("null BAM handle for sample %d", sample_of[i]); return TREDSW_ERR_ARG; }
+        if (sp.bam->is_stream()) { tredsw_set_error("%s is a stream: scan it (tredsw_ingest_scan_run)", sp.bam->path.c_str()); return TREDSW_ERR_UNSUPPORTED; }
         if (!sp.bam->has_index) { tredsw_set_error("%s has no index: scan it (tredsw_ingest_scan_run)", sp.bam->path.c_str()); return TREDSW_ERR_UNSUPPORTED; }
         sp.problems.push_back(i);
     }
@@ -926,29 +927,58 @@ struct ScanSlab {                   // the compressed bytes of one slab (page-lo
     uint8_t *comp = nullptr;
     std::vector<BlockDesc> blocks;  // in_off into comp, out_off from the slab's first inflated byte
     int64_t begin = 0, next = 0, inflated = 0;
+    int64_t got = 0;                // bytes in comp (the whole blocks end at next - begin)
     const char *why = nullptr;      // I/O or framing error
-    double ms = 0;                  // host time: pread + framing
+    double ms = 0;                  // host time: read + framing
 };
 
-// Reads up to `want` bytes of the file from `off` and frames the whole blocks among them.  A block cut by the end of
-// the read is left to the next slab (`next` is its offset); one cut by the end of the file is an error.
-void read_slab(int fd, int64_t file_size, int64_t off, int64_t want, ScanSlab *sl) {
+// Where the slabs come from.  A file is read with pread at absolute offsets; its size caps the slab and tells a block
+// cut by the end of the file.  A stream is read strictly in order with read(), its size unknown: a slab starts with the
+// bytes the slab before it read past its last whole block (the first slab: what the handle buffered while it read the
+// header and the read length), and the end of the input is read() returning 0.
+struct ScanSource {
+    int fd = -1;
+    bool stream = false;
+    int64_t file_size = 0;                  // file
+    bool eof = false;                       // stream: read() returned 0
+    const uint8_t *head = nullptr;          // stream: the first slab's leading bytes
+    int64_t head_len = 0;
+};
+
+// Reads up to `want` bytes from `off` and frames the whole blocks among them.  A block cut by the end of the read is
+// left to the next slab (`next` is its offset); one cut by the end of the input is an error.  prev: the slab before
+// (a stream's next slab starts with its unframed tail).
+void read_slab(ScanSource *src, int64_t off, int64_t want, const ScanSlab *prev, ScanSlab *sl) {
     const double t0 = now_ms();
     sl->blocks.clear(); sl->begin = sl->next = off; sl->inflated = 0; sl->why = nullptr;
-    const int64_t n = std::max<int64_t>(0, std::min(want, file_size - off));
     int64_t got = 0;
-    while (got < n) {
-        const ssize_t k = pread(fd, sl->comp + got, (size_t)(n - got), (off_t)(off + got));
-        if (k <= 0) break;
-        got += k;
+    if (!src->stream) {
+        const int64_t n = std::max<int64_t>(0, std::min(want, src->file_size - off));
+        while (got < n) {
+            const ssize_t k = pread(src->fd, sl->comp + got, (size_t)(n - got), (off_t)(off + got));
+            if (k <= 0) break;
+            got += k;
+        }
+        if (got < n) sl->why = "short read";
+    } else {
+        const uint8_t *lead = prev ? prev->comp + (prev->next - prev->begin) : src->head;
+        got = prev ? prev->got - (prev->next - prev->begin) : src->head_len;
+        if (got > 0) memcpy(sl->comp, lead, (size_t)got);
+        while (got < want && !src->eof) {
+            const ssize_t k = read(src->fd, sl->comp + got, (size_t)(want - got));
+            if (k > 0) got += k;
+            else if (k == 0) src->eof = true;
+            else if (errno != EINTR) { sl->why = "read failed"; break; }
+        }
     }
-    if (got < n) sl->why = "short read";
+    sl->got = got;
+    const bool at_end = src->stream ? src->eof : off + got >= src->file_size;
     int64_t o = 0;
     while (!sl->why && o < got) {
         BgzfFrame fr;
         const char *why = nullptr;
         const int rc = parse_bgzf_block(sl->comp + o, got - o, &fr, &why);
-        if (rc < 0 || (rc == 0 && off + got >= file_size)) { sl->why = why; break; }
+        if (rc < 0 || (rc == 0 && at_end)) { sl->why = why; break; }
         if (rc == 0 || (sl->inflated + fr.isize > SCAN_MAX_INFLATED && !sl->blocks.empty())) break;
         BlockDesc d;
         d.in_off = o + 12 + fr.xlen; d.out_off = sl->inflated; d.clen = (uint32_t)fr.clen; d.isize = fr.isize; d.crc = fr.crc; d.pad_ = 0;
@@ -1063,10 +1093,20 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
     const MatchTables mt{d_tid_x0, d_xs, d_seg_f0, d_seg_ids, d_id_start + 2 * nids, d_id_start, d_id_start + nids, n_ref, nfetch};
 
     // ---- (2) slab by slab: read (the next slab on a host thread), inflate, record boundaries, match, keep ------------
-    const int fd = fileno(bam->bgzf.fh);
-    struct stat st;
-    const int64_t file_size = fstat(fd, &st) == 0 ? (int64_t)st.st_size : 0;
-    const int64_t want = std::max(std::min(slab_bytes > 0 ? slab_bytes : SCAN_DEFAULT_SLAB, file_size), SCAN_MIN_SLAB);
+    ScanSource src;
+    int64_t want;
+    if (!bam->is_stream()) {
+        src.fd = fileno(bam->bgzf.fh);
+        struct stat st;
+        src.file_size = fstat(src.fd, &st) == 0 ? (int64_t)st.st_size : 0;
+        want = std::max(std::min(slab_bytes > 0 ? slab_bytes : SCAN_DEFAULT_SLAB, src.file_size), SCAN_MIN_SLAB);
+    } else {
+        tredsw_bam::Bgzf &z = bam->bgzf;
+        const int64_t at = (int64_t)(bam->first_record >> 16) - z.sbase;
+        src.fd = z.sfd; src.stream = true; src.eof = z.seof;
+        src.head = z.sbuf.data() + at; src.head_len = (int64_t)z.sbuf.size() - at;
+        want = std::max({slab_bytes > 0 ? slab_bytes : SCAN_DEFAULT_SLAB, SCAN_MIN_SLAB, src.head_len});
+    }
     ScanSlab slabs[2];
     for (ScanSlab &sl : slabs) sl.comp = static_cast<uint8_t *>(be.alloc_host((size_t)want + 64));
     if (be.rc) return be.rc;
@@ -1084,14 +1124,17 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
     int64_t *stats = out->scan_stats;
     std::thread reader;
     struct Join { std::thread &t; ~Join() { if (t.joinable()) t.join(); } } join_reader{reader};
-    read_slab(fd, file_size, (int64_t)(bam->first_record >> 16), want, &slabs[0]);
+    bam->consumed = bam->is_stream();
+    read_slab(&src, (int64_t)(bam->first_record >> 16), want, nullptr, &slabs[0]);
+    if (src.stream) { bam->bgzf.sbuf = std::vector<unsigned char>(); src.head = nullptr; }
     for (int cur = 0;; cur ^= 1) {
         ScanSlab &sl = slabs[cur];
         stats[6] += (int64_t)(sl.ms * 1e3);
         if (sl.why) { status = 1; tredsw_set_error("%s: %s", bam->path.c_str(), sl.why); break; }
         const int nb = (int)sl.blocks.size();
         if (nb == 0) break;                                                  // end of file
-        if (sl.next < file_size) reader = std::thread(read_slab, fd, file_size, sl.next, want, &slabs[cur ^ 1]);
+        const bool more = src.stream ? !(src.eof && sl.next == sl.begin + sl.got) : sl.next < src.file_size;
+        if (more) reader = std::thread(read_slab, &src, sl.next, want, &slabs[cur], &slabs[cur ^ 1]);
         else { slabs[cur ^ 1].blocks.clear(); slabs[cur ^ 1].why = nullptr; slabs[cur ^ 1].ms = 0; }
         const double t_dev = now_ms();
         const int64_t len = carry_len + sl.inflated;
@@ -1330,6 +1373,7 @@ int tredsw_ingest_scan_run(tredsw_ctx *ctx, tredsw_bam *bam, const tredsw_locus_
     if (!ctx || !bam || !out || nqueries < 0 || (nqueries > 0 && !queries) || n_depth < 0 ||
         (n_depth > 0 && (!depth_regions || !depth_out)) || slab_bytes < 0) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
     *out = nullptr;
+    if (bam->consumed) { tredsw_set_error("%s: stream already consumed", bam->path.c_str()); return TREDSW_ERR_ARG; }
     std::lock_guard<std::mutex> lock(ctx->mu);
     CUDA_TRY(cudaSetDevice(ctx->device));
     keep_pool(ctx->device);
@@ -1351,6 +1395,7 @@ int tredsw_ingest_scan_emulate(tredsw_bam *bam, const tredsw_locus_query *querie
     if (!bam || !out || nqueries < 0 || (nqueries > 0 && !queries) || n_depth < 0 ||
         (n_depth > 0 && (!depth_regions || !depth_out)) || slab_bytes < 0) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
     *out = nullptr;
+    if (bam->consumed) { tredsw_set_error("%s: stream already consumed", bam->path.c_str()); return TREDSW_ERR_ARG; }
     std::unique_ptr<tredsw_ingest_batch> b(new tredsw_ingest_batch());
     b->emulated = true;
     int rc;

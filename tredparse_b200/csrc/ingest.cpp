@@ -13,6 +13,8 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <fcntl.h>
+#include <unistd.h>
 #include <zlib.h>
 
 #include <algorithm>
@@ -30,19 +32,22 @@ using namespace tredsw_ingest;
 
 extern "C" {
 
-// the handle with its header read (reference dictionary, first record), no index yet
-static tredsw_bam *open_header(const char *bam_path) {
+// the handle with its header read (reference dictionary, first record), no index yet.  stream: read the input strictly
+// in order ("-" is stdin)
+static tredsw_bam *open_header(const char *bam_path, bool stream = false) {
     if (!bam_path) { tredsw_set_error("null path"); return nullptr; }
     tredsw_bam *b = new tredsw_bam();
-    b->bgzf.fh = fopen(bam_path, "rb");
-    if (!b->bgzf.fh) { tredsw_set_error("cannot open %s", bam_path); delete b; return nullptr; }
+    if (!stream) b->bgzf.fh = fopen(bam_path, "rb");
+    else b->bgzf.sfd = strcmp(bam_path, "-") == 0 ? dup(STDIN_FILENO) : open(bam_path, O_RDONLY | O_CLOEXEC);
+    if (!b->bgzf.fh && b->bgzf.sfd < 0) { tredsw_set_error("cannot open %s", bam_path); delete b; return nullptr; }
     char magic[4];
     int32_t l_text = 0, n_ref = 0;
     if (b->bgzf.read(magic, 4) != 4 || memcmp(magic, "BAM\1", 4) != 0 || b->bgzf.read(&l_text, 4) != 4 || l_text < 0) {
         tredsw_set_error("%s is not a BAM file", bam_path); delete b; return nullptr;
     }
-    std::vector<char> text(l_text);
-    if (l_text && b->bgzf.read(text.data(), l_text) != (size_t)l_text) { tredsw_set_error("truncated BAM header"); delete b; return nullptr; }
+    b->text.resize(l_text);
+    if (l_text && b->bgzf.read(&b->text[0], l_text) != (size_t)l_text) { tredsw_set_error("truncated BAM header"); delete b; return nullptr; }
+    b->text.resize(strnlen(b->text.c_str(), b->text.size()));          // (the text may end in NULs)
     if (b->bgzf.read(&n_ref, 4) != 4 || n_ref < 0) { tredsw_set_error("truncated BAM header"); delete b; return nullptr; }
     for (int i = 0; i < n_ref; ++i) {
         int32_t l_name = 0, l_ref = 0;
@@ -55,10 +60,31 @@ static tredsw_bam *open_header(const char *bam_path) {
     }
     b->first_record = b->bgzf.tell();
     b->path = bam_path;
+    if (stream) {
+        if (b->path == "-") b->path = "(stdin)";
+        // the header's blocks are not needed again: keep the stream from the block of the first record on
+        Bgzf &z = b->bgzf;
+        const int64_t drop = std::min<int64_t>((int64_t)(b->first_record >> 16) - z.sbase, (int64_t)z.sbuf.size());
+        if (drop > 0) { z.sbuf.erase(z.sbuf.begin(), z.sbuf.begin() + drop); z.sbase += drop; }
+    }
     return b;
 }
 
 tredsw_bam *tredsw_bam_open_unindexed(const char *bam_path) { return open_header(bam_path); }
+
+// A BAM read strictly in order (a pipe, stdin as "-", a socket; a regular file works the same way): no seek, no size.
+// The handle keeps the compressed bytes it has read from the block of the first record on; the scan starts with them.
+tredsw_bam *tredsw_bam_open_stream(const char *path) { return open_header(path, true); }
+
+int64_t tredsw_bam_header_text(tredsw_bam *b, char *buf, int64_t cap) {
+    if (!b) { tredsw_set_error("null handle"); return TREDSW_ERR_ARG; }
+    if (buf && cap > 0) {
+        const size_t n = std::min<size_t>(b->text.size(), (size_t)cap - 1);
+        memcpy(buf, b->text.data(), n);
+        buf[n] = 0;
+    }
+    return (int64_t)b->text.size();
+}
 
 tredsw_bam *tredsw_bam_open(const char *bam_path, const char *bai_path) {
     tredsw_bam *b = open_header(bam_path);
@@ -123,12 +149,13 @@ tredsw_bam *tredsw_bam_open(const char *bam_path, const char *bai_path) {
 // header tables copied, the parsed index shared.  Handles are not thread-safe; clones are independent.
 tredsw_bam *tredsw_bam_clone(tredsw_bam *src) {
     if (!src) { tredsw_set_error("null handle"); return nullptr; }
+    if (src->is_stream()) { tredsw_set_error("%s is a stream: it can be read only once, by one handle", src->path.c_str()); return nullptr; }
     tredsw_bam *b = new tredsw_bam();
     b->bgzf.fh = fopen(src->path.c_str(), "rb");
     if (!b->bgzf.fh) { tredsw_set_error("cannot open %s", src->path.c_str()); delete b; return nullptr; }
     b->names = src->names; b->lengths = src->lengths; b->tid_of = src->tid_of;
     b->index_ptr = src->index_ptr; b->has_index = src->has_index;
-    b->first_record = src->first_record; b->path = src->path;
+    b->first_record = src->first_record; b->path = src->path; b->text = src->text;
     return b;
 }
 
@@ -174,6 +201,7 @@ int32_t tredsw_bam_tid(tredsw_bam *b, const char *name) {
 // (same restatement as bamio.region_depth).
 int tredsw_bam_region_depth(tredsw_bam *b, int32_t tid, int64_t start, int64_t end, double *depth) {
     if (!b || !depth) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
+    if (b->is_stream()) { tredsw_set_error("%s is a stream: region queries need an indexed file", b->path.c_str()); return TREDSW_ERR_UNSUPPORTED; }
     if (!b->has_index) { tredsw_set_error("%s has no index", b->path.c_str()); return TREDSW_ERR_UNSUPPORTED; }
     if (tid < 0 || tid >= (int)b->names.size()) { tredsw_set_error("contig id %d out of range", tid); return TREDSW_ERR_ARG; }
     if (end < start) { tredsw_set_error("empty region"); return TREDSW_ERR_ARG; }
@@ -191,9 +219,11 @@ int tredsw_bam_region_depth(tredsw_bam *b, int32_t tid, int64_t start, int64_t e
 }
 
 // BamReadLen.readlen (bam_parser.py:372-391): the longest query among the first `first_n` + 1 records of the
-// file (the reference breaks after len(rls) > firstN); min_out may be NULL.
+// file (the reference breaks after len(rls) > firstN); min_out may be NULL.  On a stream these records are read ahead
+// and stay buffered for the scan.
 int tredsw_bam_read_length(tredsw_bam *b, int32_t first_n, int32_t *max_out, int32_t *min_out) {
     if (!b || !max_out || first_n < 0) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
+    if (b->consumed) { tredsw_set_error("%s: stream already consumed", b->path.c_str()); return TREDSW_ERR_ARG; }
     int32_t n = 0, mx = -1, mn = 0x7fffffff;
     b->bgzf.err = nullptr;
     try {
@@ -221,6 +251,7 @@ int tredsw_bam_extract_locus(tredsw_bam *b, const tredsw_locus_query *q, int8_t 
                              int32_t *target_lens, int32_t target_cap, char *names, int64_t names_cap,
                              tredsw_locus_summary *out) {
     if (!b || !q || !out || !roff || reads_cap < 0) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
+    if (b->is_stream()) { tredsw_set_error("%s is a stream: region queries need an indexed file", b->path.c_str()); return TREDSW_ERR_UNSUPPORTED; }
     if (!b->has_index) { tredsw_set_error("%s has no index", b->path.c_str()); return TREDSW_ERR_UNSUPPORTED; }
     b->bgzf.err = nullptr;
     int rc;

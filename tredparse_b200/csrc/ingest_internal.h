@@ -5,6 +5,8 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <errno.h>
+#include <unistd.h>
 #include <zlib.h>
 
 #include <algorithm>
@@ -23,6 +25,13 @@ namespace tredsw_ingest {
 
 struct Bgzf {
     FILE *fh = nullptr;
+    // A stream (pipe, stdin, socket) instead of a file: read strictly in order with read(), never seeked.  `sbuf` keeps
+    // the compressed bytes read so far from stream offset `sbase` on, so that load() can go back to any block from there
+    // on; it reads further as it needs.
+    int sfd = -1;
+    bool seof = false;                                // read() returned 0
+    std::vector<unsigned char> sbuf;
+    int64_t sbase = 0, spos = 0;
     std::vector<unsigned char> cbuf, block;
     const unsigned char *cur = nullptr;               // inflated bytes of the current block
     int64_t block_coffset = -1, next_coffset = 0;
@@ -37,18 +46,38 @@ struct Bgzf {
     const char *err = nullptr;
     bool fail(const char *why) { if (!err) err = why; return false; }
 
+    // n bytes at the current position: fread on a file; from sbuf on a stream, reading the stream further first
+    size_t get(void *dst, size_t n) {
+        if (sfd < 0) return fread(dst, 1, n, fh);
+        while (!seof && spos + (int64_t)n > sbase + (int64_t)sbuf.size()) {
+            const size_t have = sbuf.size(), want = std::max<size_t>(spos + n - sbase - have, 1 << 16);
+            sbuf.resize(have + want);
+            const ssize_t k = ::read(sfd, sbuf.data() + have, want);
+            sbuf.resize(have + (k > 0 ? (size_t)k : 0));
+            if (k == 0) seof = true;
+            else if (k < 0 && errno != EINTR) { fail("read failed"); break; }
+        }
+        const int64_t avail = std::max<int64_t>(0, sbase + (int64_t)sbuf.size() - spos);
+        const size_t take = std::min<size_t>(n, (size_t)avail);
+        if (take) memcpy(dst, sbuf.data() + (spos - sbase), take);
+        spos += (int64_t)take;
+        return take;
+    }
+    bool at_eof() { return sfd < 0 ? feof(fh) != 0 : seof && spos >= sbase + (int64_t)sbuf.size(); }
+
     bool load(int64_t coffset) {
         blen = 0; pos = 0; block_coffset = coffset; next_coffset = coffset;
-        if (fseeko(fh, coffset, SEEK_SET) != 0) return fail("seek failed");
+        if (sfd >= 0) { if (coffset < sbase) return fail("the stream has moved past this block"); spos = coffset; }
+        else if (fseeko(fh, coffset, SEEK_SET) != 0) return fail("seek failed");
         unsigned char head[18];
-        const size_t nhead = fread(head, 1, 18, fh);
-        if (nhead == 0 && feof(fh)) return false;                          // clean end of file
+        const size_t nhead = get(head, 18);
+        if (nhead == 0 && at_eof()) return false;                          // clean end of file
         if (nhead != 18) return fail("truncated BGZF block header");
         if (head[0] != 31 || head[1] != 139 || !(head[3] & 4)) return fail("not a BGZF block");
         const int xlen = head[10] | (head[11] << 8);
         std::vector<unsigned char> extra(xlen);
         memcpy(extra.data(), head + 12, std::min(6, xlen));
-        if (xlen > 6 && fread(extra.data() + 6, 1, xlen - 6, fh) != (size_t)(xlen - 6)) return fail("truncated BGZF block header");
+        if (xlen > 6 && get(extra.data() + 6, xlen - 6) != (size_t)(xlen - 6)) return fail("truncated BGZF block header");
         int bsize = -1;
         for (int off = 0; off + 4 <= xlen;) {
             const int slen = extra[off + 2] | (extra[off + 3] << 8);
@@ -59,9 +88,9 @@ struct Bgzf {
         const int clen = bsize - xlen - 19;
         if (clen < 0) return fail("bad BGZF block size");
         cbuf.resize(clen > 0 ? clen : 0);
-        if (clen > 0 && fread(cbuf.data(), 1, clen, fh) != (size_t)clen) return fail("truncated BGZF block");
+        if (clen > 0 && get(cbuf.data(), clen) != (size_t)clen) return fail("truncated BGZF block");
         unsigned char tail[8];
-        if (fread(tail, 1, 8, fh) != 8) return fail("truncated BGZF block");
+        if (get(tail, 8) != 8) return fail("truncated BGZF block");
         const uint32_t crc = tail[0] | (tail[1] << 8) | (tail[2] << 16) | ((uint32_t)tail[3] << 24);
         const uint32_t isize = tail[4] | (tail[5] << 8) | (tail[6] << 16) | ((uint32_t)tail[7] << 24);
         if (isize > 65536) return fail("BGZF block larger than 64 KiB");   // (the format's limit; also bounds the resize)
@@ -118,7 +147,7 @@ struct Bgzf {
         }
         return got;
     }
-    ~Bgzf() { if (zs_init) inflateEnd(&zs); if (fh) fclose(fh); delete fast; }
+    ~Bgzf() { if (zs_init) inflateEnd(&zs); if (fh) fclose(fh); if (sfd >= 0) close(sfd); delete fast; }
 };
 
 struct RefIndex {
@@ -149,8 +178,11 @@ struct tredsw_bam {
     // the parsed .bai (tens of MB for a whole-genome BAM) is immutable and shared by the clones of a handle
     std::shared_ptr<const std::vector<RefIndex>> index_ptr;
     std::string path;
+    std::string text;                // the header text (SAM header lines)
     bool has_index = false;
+    bool consumed = false;           // a stream handle whose scan has read the stream (it can be read only once)
     uint64_t first_record = 0;       // virtual offset of the first alignment record
+    bool is_stream() const { return bgzf.sfd >= 0; }
     std::vector<unsigned char> rec;
 
     bool read_record(Record &r) {

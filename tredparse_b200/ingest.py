@@ -9,8 +9,11 @@ layout ``cohort.CohortBatch`` / ``tredsw_genotype_batch`` consume.  Host code on
         problem = bam.problem(repo["HD"], readlen=150)           # ready for cohort.CohortBatch([...])
 
 A BAM without a usable index is read on the GPU in one pass per sample: ``scan_sample(ctx, BamIngest.unindexed(path),
-...)``.
+...)``.  So is a BAM that can be read only once, in order (a pipe, a FIFO, stdin as ``-``): ``scan_sample(ctx,
+BamIngest.stream(path), ...)``.
 """
+import os
+import stat
 import ctypes
 
 import numpy as np
@@ -43,6 +46,10 @@ def _bind(lib):
     lib.tredsw_bam_open.argtypes = [ctypes.c_char_p, ctypes.c_char_p]
     lib.tredsw_bam_open_unindexed.restype = ctypes.c_void_p
     lib.tredsw_bam_open_unindexed.argtypes = [ctypes.c_char_p]
+    lib.tredsw_bam_open_stream.restype = ctypes.c_void_p
+    lib.tredsw_bam_open_stream.argtypes = [ctypes.c_char_p]
+    lib.tredsw_bam_header_text.restype = ctypes.c_int64
+    lib.tredsw_bam_header_text.argtypes = [ctypes.c_void_p, ctypes.c_char_p, ctypes.c_int64]
     lib.tredsw_bam_inflate_stats.restype = None
     lib.tredsw_bam_inflate_stats.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_int64)]
     lib.tredsw_inflate_raw.restype = ctypes.c_int
@@ -69,6 +76,17 @@ def _bind(lib):
     lib.tredsw_bam_read_length.argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.POINTER(ctypes.c_int32),
                                            ctypes.POINTER(ctypes.c_int32)]
     lib._ingest_bound = True
+
+
+def is_stream(path):
+    """True when `path` can be read only once, in order: ``-`` (stdin), a FIFO, a character device or a socket."""
+    if path == "-":
+        return True
+    try:
+        mode = os.stat(path).st_mode
+    except OSError:
+        return False
+    return stat.S_ISFIFO(mode) or stat.S_ISCHR(mode) or stat.S_ISSOCK(mode)
 
 
 class LocusEvidence:
@@ -108,15 +126,42 @@ class BamIngest:
     def unindexed(cls, path):
         """A handle on a BAM without a usable index: header, contig ids and read length only (``scan_sample`` reads
         its evidence in one pass over the file; ``extract_locus`` and ``region_depth`` refuse it)."""
+        return cls._open_header_only(path, "tredsw_bam_open_unindexed")
+
+    @classmethod
+    def stream(cls, path):
+        """A handle on a BAM that is read strictly in order, once (``is_stream``; ``-`` is stdin): header, contig ids and
+        read length, then ONE ``scan_sample``.  ``clone``, ``extract_locus`` and ``region_depth`` refuse it."""
+        return cls._open_header_only(path, "tredsw_bam_open_stream")
+
+    @classmethod
+    def _open_header_only(cls, path, opener):
         self = object.__new__(cls)
         self.lib = _lib.load()
         _bind(self.lib)
         self.path = path
-        self.handle = self.lib.tredsw_bam_open_unindexed(path.encode())
+        self.handle = getattr(self.lib, opener)(path.encode())
         if not self.handle:
-            raise IOError("tredsw_bam_open_unindexed({}): {}".format(path, _lib.last_error()))
+            raise IOError("{}({}): {}".format(opener, path, _lib.last_error()))
         self._caps = dict(reads=512, bases=512 * 256, pairs=8192, names=512 * 48)
         return self
+
+    def header_text(self):
+        """the SAM header text (@HD, @SQ, @RG, ... lines)"""
+        n = int(self.lib.tredsw_bam_header_text(self.handle, None, 0))
+        buf = ctypes.create_string_buffer(n + 1)
+        self.lib.tredsw_bam_header_text(self.handle, buf, n + 1)
+        return buf.value.decode("utf-8", "replace")
+
+    def read_group_sample(self):
+        """the SM field of the header's first @RG line; None when there is none"""
+        for line in self.header_text().splitlines():
+            if line.startswith("@RG"):
+                for field in line.split("\t")[1:]:
+                    if field.startswith("SM:"):
+                        return field[3:]
+                return None
+        return None
 
     def inflate_stats(self):
         """(blocks inflated by the library's own decoder, blocks that fell back to zlib) for this handle."""
@@ -458,7 +503,8 @@ class ScanBatch(IngestBatch):
 
 def scan_sample(ctx, handle, queries, keep, depth_regions, slab_bytes=None):
     """Every locus of one sample (``queries``: ``LocusQuery`` records, alt regions included) and the depth of
-    ``depth_regions`` ((tid, start, end) rows) in one streaming pass over a BAM opened with ``BamIngest.unindexed``.
+    ``depth_regions`` ((tid, start, end) rows) in one streaming pass over a BAM opened with ``BamIngest.unindexed`` or
+    ``BamIngest.stream`` (a stream can be scanned once).
     ``slab_bytes``: compressed bytes read per step (None: 128 MiB).  ``ctx=None`` runs the serial host emulation of
     the device code — test infrastructure only.  -> ScanBatch"""
     return ScanBatch(ctx, handle, queries, keep=keep, depth_regions=depth_regions, slab_bytes=slab_bytes)

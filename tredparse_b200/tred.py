@@ -16,7 +16,9 @@ Differences that are the point of this build:
     results).  If that call fails, the chunk fails: ``run_chunks(..., isolate=True)`` turns that into error records
     for its samples;
   * samples are sharded over GPUs (``--gpus``), one worker process per GPU, instead of over CPU cores
-    with ``multiprocessing.Pool`` (tred.py:528-532).  No collective: workers return their dicts.
+    with ``multiprocessing.Pool`` (tred.py:528-532).  No collective: workers return their dicts;
+  * a BAM that can be read only once, in order (``-`` for stdin, a FIFO; e.g. ``samtools view -u x.cram | ... -``) is
+    read by one GPU scan that serves its read length, gender and every locus; there is no fallback reader for it.
 S3 / ``@HLI-id`` inputs are out of scope (SURVEY.md §2 row 5).
 """
 import argparse
@@ -102,7 +104,7 @@ def set_argparse():
 
 
 def bam_path(bam):
-    if bam.startswith(("s3://", "http://", "ftp://", "https://")):
+    if bam == "-" or bam.startswith(("s3://", "http://", "ftp://", "https://")):
         return bam
     return op.abspath(bam)
 
@@ -327,13 +329,15 @@ def ingest_chunk_gpu(samples, ctx=None, keep_batch=None):
         return {}
 
 
-def ingest_sample_scan(arg, wanted, READLEN, h, with_gender, ctx=None):
+def ingest_sample_scan(arg, wanted, READLEN, h, with_gender, ctx=None, stream=False):
     """Evidence of every wanted locus of one sample whose BAM has no usable index, and its chrY depth when
     ``with_gender``, in ONE streaming pass over the file on the GPU (``ingest.scan_sample``).
-    :param h: the sample's handle from ``ingest.BamIngest.unindexed``
+    :param h: the sample's handle from ``ingest.BamIngest.unindexed`` or ``ingest.BamIngest.stream``
+    :param stream: `h` is a stream, which can be read only once: a scan that fails raises (no partial evidence, no
+                   second reader), and a header without the chrY regions gives gender ('Unknown', -1)
     :return: ({tredName: LocusEvidence}, (gender, depthY) or None) — loci the scan could not serve (contig missing,
              a corrupt or unsorted file) are left out, and so is the gender: the caller reads them with the Python
-             reader."""
+             reader (not a stream's: a locus whose contig the header lacks gets no call)."""
     from . import _lib
     from .ingest import locus_query, scan_sample
     samplekey, bam, repo, tredNames, maxinsert, fullsearch, clip, alts, repeatpairs, log = arg
@@ -350,11 +354,13 @@ def ingest_sample_scan(arg, wanted, READLEN, h, with_gender, ctx=None):
         tids = [h.tid(c) for c, s, e in rows]
         if rows and min(tids) >= 0:
             yreg = [(t, s, e) for t, (c, s, e) in zip(tids, rows)]
-    got, gender = {}, None
+    got, gender = {}, (("Unknown", -1) if stream and with_gender and not yreg else None)
     if not qs and not yreg:
         return got, gender
     try:
         with scan_sample(ctx or _lib.default_context(), h, qs, keep, yreg) as b:
+            if stream and b.scan_status:
+                raise IOError("the GPU scan of `{}` failed (status {}): {}".format(bam, b.scan_status, _lib.last_error()))
             for i, t in enumerate(names):
                 if b.status[i]:
                     logger.debug("GPU scan handed {} / {} back (status {})".format(samplekey, t, int(b.status[i])))
@@ -364,9 +370,31 @@ def ingest_sample_scan(arg, wanted, READLEN, h, with_gender, ctx=None):
                 ydepth = float(np.median(b.depths))
                 gender = ("Male" if ydepth > 1 else "Female", ydepth)
     except Exception as e:
+        if stream:
+            raise
         logger.error("GPU scan of `{}` failed ({}); reading with the Python reader".format(bam, e))
         return {}, None
     return got, gender
+
+
+OPEN_STREAMS = {}       # stream path -> ingest.BamIngest whose header was read early (the sample key of `-`)
+
+
+def stream_presteps(bam):
+    """(handle, pre-steps) of a stream sample: its handle (``ingest.BamIngest.stream``) and the read length from the
+    records the handle reads ahead; gender comes later, from the chrY regions of the sample's one scan."""
+    from .ingest import BamIngest
+    from . import _lib
+    if not GPU_INGEST:
+        raise IOError("`{}` is a stream: only the GPU scan reads it (TREDSW_GPU_INGEST=0)".format(bam))
+    h = OPEN_STREAMS.pop(bam, None) or BamIngest.stream(bam)
+    READLEN = 150
+    try:
+        READLEN = h.read_length()[0]
+    except _lib.TredswError:
+        pass                    # no records (the scan finds none either) or a damaged stream (the scan reports it)
+    logger.debug("Read length: {}bp".format(READLEN))
+    return h, {"inferredGender": "Unknown", "depthY": -1, "readLen": READLEN}
 
 
 def infer_gender(bam, repo, tredNames, logger, ing=None):
@@ -415,10 +443,16 @@ def prepare_chunk(args, only=None, ctx=None):
     # per sample: one native handle (validity check, pre-steps, GPU ingest), the pre-steps (gender looks at every
     # requested locus); the samples are dealt to host threads
     # a BAM without a usable index is scanned once on the GPU (unless the GPU ingest is off): its gender comes from
-    # that scan, so its pre-steps here read only the read length
+    # that scan, so its pre-steps here read only the read length.  So is a stream, which nothing else may read: a
+    # stream that cannot be scanned makes its sample an error
     def pre(si):
         samplekey, bam, repo, tredNames = args[si][:4]
-        from .ingest import BamIngest
+        from .ingest import BamIngest, is_stream
+        if is_stream(bam):
+            try:
+                return stream_presteps(bam) + ("stream",)
+            except Exception as e:
+                return e
         ing = None
         try:
             ing = BamIngest(bam_path(bam))
@@ -439,14 +473,24 @@ def prepare_chunk(args, only=None, ctx=None):
             pres = list(pool.map(pre, range(len(args))))
     else:
         pres = [pre(si) for si in range(len(args))]
-    wanted_of, handle_of, unindexed = {}, {}, set()
+    wanted_of, handle_of, unindexed, streams, failed = {}, {}, set(), set(), set()
+
+    def fail(si, e):
+        logger.error("Sample `{}`: {}".format(args[si][0], e))
+        failed.add(si)
+        out[si].update({"tredCalls": {}, "error": repr(e), "_names": []})
     for si, ps in enumerate(pres):
         if ps is None:
+            continue
+        if isinstance(ps, Exception):
+            fail(si, ps)
             continue
         todo.append(si)
         handle_of[si] = ps[0]
         if ps[2]:
             unindexed.add(si)
+        if ps[2] == "stream":
+            streams.add(si)
         out[si]["tredCalls"].update(ps[1])
         tredNames = args[si][3]
         wanted_of[si] = [t for t in tredNames if only is None or t in only[si]]
@@ -462,8 +506,14 @@ def prepare_chunk(args, only=None, ctx=None):
         for si in sorted(unindexed):
             samplekey, bam, repo, tredNames = args[si][:4]
             with_gender = any(repo[t].is_xlinked for t in tredNames)
-            got[si], gender = ingest_sample_scan(args[si], wanted_of[si], out[si]["tredCalls"]["readLen"],
-                                                 handle_of[si], with_gender, ctx=ctx)
+            try:
+                got[si], gender = ingest_sample_scan(args[si], wanted_of[si], out[si]["tredCalls"]["readLen"],
+                                                     handle_of[si], with_gender, ctx=ctx, stream=si in streams)
+            except Exception as e:
+                if si not in streams:
+                    raise
+                fail(si, e)
+                continue
             if gender is None and with_gender:
                 gender = infer_gender(bam, repo, tredNames, logger)
             if gender is not None:
@@ -474,12 +524,14 @@ def prepare_chunk(args, only=None, ctx=None):
             if h is not None:
                 h.close()
     for si in todo:
+        if si in failed:
+            continue
         samplekey, bam, repo, tredNames, maxinsert, fullsearch, clip, alts, repeatpairs, log = args[si]
         gender, READLEN = out[si]["tredCalls"]["inferredGender"], out[si]["tredCalls"]["readLen"]
         wanted = wanted_of[si]
         evidence = got.get(si, {})
         rest = [t for t in wanted if t not in evidence]
-        if rest:
+        if rest and si not in streams:              # (a stream's bytes are gone: its missing loci get no call)
             evidence.update(ingest_loci(bam, repo, rest, READLEN, alts, clip, logger, want_names=True))
         for t in wanted:
             if t in evidence:
@@ -661,6 +713,12 @@ def to_vcf(results, ref, repo, treds=("HD",), store=None):
 
 
 def read_csv(csvfile, args):
+    if csvfile == "-":
+        # one sample on stdin: its key is the SM of the header's first @RG line (the header is read here and the
+        # handle kept for the run)
+        from .ingest import BamIngest
+        h = OPEN_STREAMS["-"] = BamIngest.stream("-")
+        return [(h.read_group_sample() or "stdin", "-", None)]
     if csvfile[0] == "@":
         raise ValueError("@HLI-id inputs are not supported by this build")
     if csvfile.endswith(".bam") or csvfile.endswith(".cram"):
@@ -747,7 +805,14 @@ def main(args):
     infile = args.infile
     if not infile:
         sys.exit(not p.print_help())
+    # ranks scan their own loci of every sample, and a stream can be read only once
+    multi_gpu_stream = "--gpus {} with a stream input: a stream can be read only once, by one GPU".format(args.gpus)
+    if args.gpus > 1 and infile == "-":
+        p.error(multi_gpu_stream)
     samples = read_csv(infile, args)
+    from .ingest import is_stream
+    if args.gpus > 1 and any(is_stream(bam) for _, bam, _ in samples):
+        p.error(multi_gpu_stream)
     logger.debug("Total samples: {}".format(len(samples)))
 
     task_args = []
@@ -763,6 +828,8 @@ def main(args):
         jsonfile = ".".join((samplekey, "json"))
         if args.checkexists and op.exists(jsonfile):
             logger.debug("File `{}` exists. Skipped computation.".format(jsonfile))
+            if bam in OPEN_STREAMS:
+                OPEN_STREAMS.pop(bam).close()
             continue
         _treds = [tred] if tred else treds
         task_args.append((samplekey, bam, repo, _treds, args.maxinsert, args.fullsearch,
