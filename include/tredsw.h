@@ -97,6 +97,13 @@ int tredsw_synchronize(tredsw_ctx *ctx);
 int tredsw_sm_count(tredsw_ctx *ctx);
 /* Kernels launched through this context so far (bench.py's gpu_launches claim). */
 int64_t tredsw_launch_count(tredsw_ctx *ctx);
+/* Main strips of the packed family kernel skipped at the fixed point of their boundary column (DESIGN.md §4.1),
+ * summed over every call on this context so far; synchronises the stream.  out (TREDSW_STRIP_SKIP_STATS x int64):
+ * [0] skipped phase-1 cell updates (stats[1] of tredsw_classify_reads counts them as planned), then for each loop
+ * instantiation period p = 1..12 at [1 + 4 (p - 1)]: main strips planned, main strips skipped, warp items, items
+ * that skipped nothing.  TREDSW_NO_STRIP_SKIP set in the environment turns the skipping off (read on every call). */
+#define TREDSW_STRIP_SKIP_STATS 49
+int tredsw_strip_skip_stats(tredsw_ctx *ctx, int64_t *out);
 /* Stage timing with CUDA events on the context's stream: enable, run calls, then read the device time
  * of the LAST call's stages in ms: [0] Smith-Waterman classify kernels, [1] likelihood grid (surface +
  * reduce), [2] KDE, [3] whole call.  Reading synchronises the stream. */

@@ -25,7 +25,7 @@ EXPORTS = [
     "ssw_init", "init_destroy", "ssw_align", "align_destroy", "cigar_int_to_op", "cigar_int_to_len",
     # batched API
     "tredsw_version", "tredsw_device_count", "tredsw_last_error", "tredsw_create", "tredsw_destroy",
-    "tredsw_synchronize", "tredsw_sm_count", "tredsw_launch_count", "tredsw_enable_timing",
+    "tredsw_synchronize", "tredsw_sm_count", "tredsw_launch_count", "tredsw_strip_skip_stats", "tredsw_enable_timing",
     "tredsw_get_timing", "tredsw_get_timeline", "tredsw_int_pipe_peak", "tredsw_align_pairs", "tredsw_classify_reads",
     "tredsw_likelihood_grid", "tredsw_pe_kde", "tredsw_genotype_batch", "tredsw_genotype_batch_ex", "tredsw_pack_reads4", "tredsw_narrow_i16",
     # native BAM ingest
@@ -118,6 +118,8 @@ def load():
         lib.tredsw_sm_count.argtypes = [_vp]
         lib.tredsw_launch_count.restype = ctypes.c_int64
         lib.tredsw_launch_count.argtypes = [_vp]
+        lib.tredsw_strip_skip_stats.restype = ctypes.c_int
+        lib.tredsw_strip_skip_stats.argtypes = [_vp, _vp]
         lib.tredsw_enable_timing.argtypes = [_vp, ctypes.c_int]
         lib.tredsw_get_timing.argtypes = [_vp, _vp]
         lib.tredsw_get_timeline.argtypes = [_vp, _vp]
@@ -198,6 +200,17 @@ class Context:
     @property
     def launches(self):
         return int(self.lib.tredsw_launch_count(self.handle))
+
+    def strip_skip_stats(self):
+        """Main strips of the packed family kernel skipped at the fixed point of their boundary column, summed over
+        this context's calls so far: dict(cells_skipped, by_period={p: dict(planned, skipped, items, items_no_skip)})
+        for the loop instantiation periods p that ran (tredsw_strip_skip_stats)."""
+        a = np.zeros(49, dtype=np.int64)
+        check(self.lib.tredsw_strip_skip_stats(self.handle, ptr(a)), "tredsw_strip_skip_stats")
+        per = a[1:].reshape(12, 4)
+        return {"cells_skipped": int(a[0]),
+                "by_period": {p + 1: dict(zip(("planned", "skipped", "items", "items_no_skip"), map(int, per[p])))
+                              for p in range(12) if per[p, 2]}}
 
     def enable_timing(self, on=True):
         check(self.lib.tredsw_enable_timing(self.handle, int(on)), "tredsw_enable_timing")

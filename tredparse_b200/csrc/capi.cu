@@ -27,7 +27,7 @@ tredsw_ctx::~tredsw_ctx() {
     }
     DevBuf *all[] = {&d_q, &d_qoff, &d_t, &d_toff, &d_qidx, &d_tidx, &d_out, &d_cigar, &d_scratch, &d_misc,
                      &d_fam, &d_rfam, &d_stats, &d_work, &d_prob, &d_ipool, &d_dpool, &d_surface, &d_marg,
-                     &d_res, &d_counter, &d_tiles, &d_pk, &d_pe16, &d_ftab};
+                     &d_res, &d_counter, &d_tiles, &d_pk, &d_pe16, &d_ftab, &d_skip};
     for (DevBuf *b : all) b->release();
     h_in.release(); h_out.release(); h_tab.release();
     for (int i = 0; i < 10; ++i) if (ev[i]) cudaEventDestroy(ev[i]);
@@ -101,6 +101,17 @@ int tredsw_synchronize(tredsw_ctx *ctx) {
 int tredsw_sm_count(tredsw_ctx *ctx) { return ctx ? ctx->sm_count : 0; }
 
 int64_t tredsw_launch_count(tredsw_ctx *ctx) { return ctx ? ctx->launches : 0; }
+
+int tredsw_strip_skip_stats(tredsw_ctx *ctx, int64_t *out) {
+    if (!ctx || !out) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    memset(out, 0, TREDSW_STRIP_SKIP_STATS * sizeof(int64_t));
+    if (!ctx->d_skip.p) return TREDSW_OK;          // no packed-kernel call yet
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    CUDA_TRY(cudaMemcpyAsync(out, ctx->d_skip.p, TREDSW_STRIP_SKIP_STATS * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    return TREDSW_OK;
+}
 
 int tredsw_enable_timing(tredsw_ctx *ctx, int on) {
     if (!ctx) return TREDSW_ERR_ARG;

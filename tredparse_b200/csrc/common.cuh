@@ -69,7 +69,8 @@ struct tredsw_ctx {
     size_t smem_optin = 0;
     // staging buffers (host-pointer mode)
     DevBuf d_q, d_qoff, d_t, d_toff, d_qidx, d_tidx, d_out, d_cigar, d_scratch, d_misc, d_fam,
-        d_rfam, d_stats, d_work, d_prob, d_ipool, d_dpool, d_surface, d_marg, d_res, d_counter, d_tiles, d_pk, d_pe16, d_ftab;
+        d_rfam, d_stats, d_work, d_prob, d_ipool, d_dpool, d_surface, d_marg, d_res, d_counter, d_tiles, d_pk, d_pe16, d_ftab,
+        d_skip;   // strip-skip counters of the packed family kernel, accumulated over the context's calls
     PinnedBuf h_in, h_out, h_tab;
     // compute token (see DeviceToken): this context's "whole call finished" event, and the event the next
     // Smith-Waterman launch on this context has to wait for (consumed by tredsw_internal_classify)

@@ -37,6 +37,9 @@
 #include <type_traits>
 #include <algorithm>
 #include <vector>
+#ifdef TREDSW_DEBUG
+#include <assert.h>
+#endif
 
 namespace {
 
@@ -74,6 +77,8 @@ struct ClassifyParams {
     int32_t *counter;              // [2] work counters (generic, fast), zeroed before the launches
     int32_t *out;
     unsigned long long *stats;     // 4 counters
+    int strip_skip;                // phase1_packed stops at the fixed point of the strip boundary
+    unsigned long long *skip_stats;  // [TREDSW_STRIP_SKIP_STATS] context counters (tredsw_strip_skip_stats)
 };
 
 __constant__ int8_t c_fmat25[25];
@@ -197,11 +202,13 @@ __host__ __device__ constexpr int instance_period(int P) { return P == 6 ? 3 : P
 //           bytes per half, one word per row and lane in this CTA's global scratch (L1/L2 resident,
 //           requested one iteration ahead); every strip keeps its own slot, phase 2 restarts from them
 //   pot     suffix potentials of this warp's reads in global scratch, one word per row and lane
+//   diff    (HAS_IN and HAS_OUT) OR of bout ^ bin over the lane's rows: 0 when the strip left exactly the column it
+//           received, so that every later strip of the same table would repeat it (phase1_packed's fixed point)
 template <int NC, int PER, bool HAS_IN, bool HAS_OUT, bool HOOK>
 __device__ __forceinline__ void strip_pass(const uint32_t *stab, const uint8_t *codes, int lane, int m, int rows2,
                                            const uint32_t *bin, uint32_t *bout, const uint32_t *pot,
                                            uint32_t (&seg)[NC / PER], uint32_t (&mu)[NC / PER], uint32_t mgo2,
-                                           uint32_t mge2, uint32_t one) {
+                                           uint32_t mge2, uint32_t one, uint32_t &diff) {
     constexpr int K = NC / PER;
     static_assert(K * PER == NC, "strip = whole units");
     constexpr int NG = (NC + 3) / 4;
@@ -267,7 +274,11 @@ __device__ __forceinline__ void strip_pass(const uint32_t *stab, const uint8_t *
                     mu[u] = __viaddmax_s16x2(hdA, potHA, mu[u]);
                     mu[u] = __viaddmax_s16x2(eA, potEA, mu[u]);
                 }
-                if (HAS_OUT && s == NC - 1) bout[j * 32 + lane] = sw_prmt(hA, eA, 0x6420);
+                if (HAS_OUT && s == NC - 1) {
+                    const uint32_t w = sw_prmt(hA, eA, 0x6420);
+                    bout[j * 32 + lane] = w;
+                    if (HAS_IN) diff |= w ^ bA;                          // bA: row j's entering word
+                }
             }
             if (s >= 1) {
                 PACKED_CELL(hdB, eB, sB[s - 1], s - 1, hB)
@@ -277,7 +288,11 @@ __device__ __forceinline__ void strip_pass(const uint32_t *stab, const uint8_t *
                     mu[u] = __viaddmax_s16x2(hdB, potHB, mu[u]);
                     mu[u] = __viaddmax_s16x2(eB, potEB, mu[u]);
                 }
-                if (HAS_OUT && s - 1 == NC - 1) bout[(j + 1) * 32 + lane] = sw_prmt(hB, eB, 0x6420);
+                if (HAS_OUT && s - 1 == NC - 1) {
+                    const uint32_t w = sw_prmt(hB, eB, 0x6420);
+                    bout[(j + 1) * 32 + lane] = w;
+                    if (HAS_IN) diff |= w ^ bB;
+                }
             }
         }
         rowA = rowA2; rowB = rowB2; codeA2 = codeA3; codeB2 = codeB3;
@@ -436,7 +451,7 @@ __device__ __noinline__ void locate_packed(const FamilySmem &F, const SwLut *lut
                                            uint32_t *colsel, bool &suffix_table_ready, const uint8_t *codes, int lane,
                                            int m, int m_warp, uint32_t *bnd, const uint32_t *gbnd, int R, int go, int ge,
                                            uint32_t one, int G, int cs, int u, int u_main, int half, int sa, int sb,
-                                           int *end_ref, int *end_read, unsigned long long &cells) {
+                                           int last_slot, int *end_ref, int *end_read, unsigned long long &cells) {
     constexpr int K = strip_units(P);
     constexpr int NC = P * K;
     const uint32_t mgo2 = (uint32_t)((-go) & 0xffff) | ((uint32_t)((-go) & 0xffff) << 16);
@@ -445,6 +460,12 @@ __device__ __noinline__ void locate_packed(const FamilySmem &F, const SwLut *lut
     const int rows2 = (m_warp + 1) & ~1;
     const int su = G * (u_main > 0 ? u_main : u) - 1;        // last sub-unit of the unit of interest (idle lanes: u = 1)
     const int tstar = su / K, kstar = su % K;                // (K is a multiple of G: units do not straddle strips)
+    // Phase 1 stopped after writing slot last_slot when the strips reached their fixed point: every later strip
+    // enters with that same column.  The running main maximum does not grow in a skipped strip, so u_main (the
+    // first unit attaining cs) never lies in one — only the suffix case reads an aliased slot.
+#ifdef TREDSW_DEBUG
+    assert(u_main <= 0 || tstar < last_slot);
+#endif
     const int sh = half ? 16 : 0;
     int found_col = -1, found_row = 0;
     {
@@ -452,7 +473,7 @@ __device__ __noinline__ void locate_packed(const FamilySmem &F, const SwLut *lut
         // own strip's stored boundary column: stage it into shared memory first — 2 x rows independent,
         // sector-sized loads per lane in flight at once instead of an L2 round trip per row pair in the loop.
         {
-            const uint32_t *src = gbnd + (size_t)tstar * R * 32 + lane;
+            const uint32_t *src = gbnd + (size_t)min(tstar, last_slot) * R * 32 + lane;
             for (int j = 0; j < rows2; ++j) bnd[j * 32 + lane] = src[j * 32];
         }
         uint32_t colkey[NC];
@@ -496,11 +517,13 @@ __device__ __noinline__ void locate_packed(const FamilySmem &F, const SwLut *lut
     *end_ref = found_col; *end_read = found_row;
 }
 
+// Returns the index of the last boundary slot written (warp-uniform); *planned = main strips of the full plan.
 template <int P>
-__device__ __noinline__ void phase1_packed(const FamilySmem &F, const SwLut *lut, uint32_t *stab, uint32_t *colsel,
-                                           const uint8_t *codes, int lane, int m, int m_warp, uint32_t *pot,
-                                           uint32_t *gbnd, int R, uint8_t *scores, uint8_t *runs, int go, int ge,
-                                           uint32_t one, int G, int sa, int sb, unsigned long long &cells) {
+__device__ __noinline__ int phase1_packed(const FamilySmem &F, const SwLut *lut, uint32_t *stab, uint32_t *colsel,
+                                          const uint8_t *codes, int lane, int m, int m_warp, uint32_t *pot,
+                                          uint32_t *gbnd, int R, uint8_t *scores, uint8_t *runs, int go, int ge,
+                                          uint32_t one, int G, int sa, int sb, bool skip, int *planned,
+                                          unsigned long long &cells, unsigned long long &skipped_cells) {
     constexpr int K = strip_units(P);
     constexpr int NC = P * K;
     static_assert(NC <= STAB_PAD && FLANK <= STAB_PAD, "strip wider than the score table");
@@ -523,8 +546,9 @@ __device__ __noinline__ void phase1_packed(const FamilySmem &F, const SwLut *lut
     __syncwarp();
     uint32_t run;                   // running maximum over the main columns so far, per half
     {
-        uint32_t seg0[1] = {0u}, mu0[1] = {0u};
-        strip_pass<FLANK, FLANK, false, true, false>(stab, codes, lane, m, rows2, nullptr, gbnd, pot, seg0, mu0, mgo2, mge2, one);
+        uint32_t seg0[1] = {0u}, mu0[1] = {0u}, unused = 0u;
+        strip_pass<FLANK, FLANK, false, true, false>(stab, codes, lane, m, rows2, nullptr, gbnd, pot, seg0, mu0, mgo2, mge2,
+                                                     one, unused);
         run = seg0[0];
     }
     __syncwarp();
@@ -533,30 +557,52 @@ __device__ __noinline__ void phase1_packed(const FamilySmem &F, const SwLut *lut
     __syncwarp();
     build_stab<NPAIR>(stab, lut, lane, NC, colsel, go2);
     __syncwarp();
+    // scores and running main maxima of the template with sub-units su (when su ends a real unit)
+    auto put = [&](int su, uint32_t mu_u) {
+        if (su % G == 0 && su <= F.U * G) {
+            const int ur = su / G - 1;                              // 0-based real unit
+            const uint32_t best = __vimax3_s16x2(run, mu_u, fresh);
+            // slot 2 * ur + h: half h of the lane (strand h of a "both" item's read, read h of a pair item)
+            scores[(2 * ur + 0) * 32 + lane] = (uint8_t)(best & 0xffu);
+            scores[(2 * ur + 1) * 32 + lane] = (uint8_t)((best >> 16) & 0xffu);
+            runs[(2 * ur + 0) * 32 + lane] = (uint8_t)(run & 0xffu);          // running maximum of the main columns
+            runs[(2 * ur + 1) * 32 + lane] = (uint8_t)((run >> 16) & 0xffu);
+        }
+    };
+    // Every main strip runs the same table and potentials, so its outputs (seg, mu, leaving column) are a function
+    // of its entering column alone.  A strip that leaves exactly the column it received (every row, both halves, all
+    // lanes) is therefore repeated verbatim by every later strip: the running maximum stays `run`, unit u of a later
+    // strip scores max(run, mu[u], fresh), and every later boundary slot equals the one just written.  The loop
+    // stops there; phase 2 reads that slot for any later strip (locate_packed's last_slot).
+    const int nplan = (F.U * G + K - 1) / K;                        // main strips of the full nested plan
     int nstrips = 0;
-    for (int u0 = 0; u0 < F.U * G; u0 += K, ++nstrips) {        // u0, u: sub-units of P columns
-        uint32_t seg[K], mu[K];
+    for (int u0 = 0; u0 < F.U * G; u0 += K) {                       // u0, u: sub-units of P columns
+        uint32_t seg[K], mu[K], diff = 0u;
 #pragma unroll
         for (int u = 0; u < K; ++u) { seg[u] = 0; mu[u] = 0; }
         // (slot t of the scratch = boundary entering main strip t; the strip writes slot t+1)
         strip_pass<NC, P, true, true, true>(stab, codes, lane, m, rows2, gbnd + (size_t)nstrips * R * 32,
-                                            gbnd + (size_t)(nstrips + 1) * R * 32, pot, seg, mu, mgo2, mge2, one);
+                                            gbnd + (size_t)(nstrips + 1) * R * 32, pot, seg, mu, mgo2, mge2, one, diff);
+        ++nstrips;
 #pragma unroll
         for (int u = 0; u < K; ++u) {
             run = __vmaxs2(run, seg[u]);
-            const int su = u0 + u + 1;                              // sub-units completed
-            if (su % G == 0 && su <= F.U * G) {
-                const int ur = su / G - 1;                          // 0-based real unit
-                const uint32_t best = __vimax3_s16x2(run, mu[u], fresh);
-                // slot 2 * ur + h: half h of the lane (strand h of a "both" item's read, read h of a pair item)
-                scores[(2 * ur + 0) * 32 + lane] = (uint8_t)(best & 0xffu);
-                scores[(2 * ur + 1) * 32 + lane] = (uint8_t)((best >> 16) & 0xffu);
-                runs[(2 * ur + 0) * 32 + lane] = (uint8_t)(run & 0xffu);      // running maximum of the main columns
-                runs[(2 * ur + 1) * 32 + lane] = (uint8_t)((run >> 16) & 0xffu);
+            put(u0 + u + 1, mu[u]);                                 // (sub-units completed)
+        }
+        if (skip && __all_sync(0xffffffffu, diff == 0u)) {
+            for (int v0 = u0 + K; v0 < F.U * G; v0 += K) {
+#pragma unroll
+                for (int u = 0; u < K; ++u) put(v0 + u + 1, mu[u]);
             }
+            break;
         }
     }
-    cells += (unsigned long long)m * 2ull * (unsigned long long)(2 * FLANK + nstrips * NC);
+    // (cells: the full plan, whether or not strips were skipped — the executed-cell statistic keeps its meaning;
+    //  the skipped ones are counted apart)
+    cells += (unsigned long long)m * 2ull * (unsigned long long)(2 * FLANK + nplan * NC);
+    skipped_cells += (unsigned long long)m * 2ull * (unsigned long long)((nplan - nstrips) * NC);
+    *planned = nplan;
+    return nstrips;                 // the last boundary slot written
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -593,9 +639,11 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
     uint32_t *pot = FAST ? bnd : p.pot_buf + (size_t)blockIdx.x * R * 32;
     uint32_t *gbnd = p.gbnd_buf + (size_t)blockIdx.x * (p.nslots + 1) * R * 32;    // [nslots + 1][R][32]
     const uint32_t one = p.one;
+    __shared__ unsigned long long skip_acc[TREDSW_STRIP_SKIP_STATS];   // this CTA's share, added up at the end
+    for (int i = lane; i < TREDSW_STRIP_SKIP_STATS; i += 32) skip_acc[i] = 0ull;
     sw_build_lut(&lut, c_fmat25, lane, 32);
     const int nitems = p.chunk_start[p.ngroups];
-    unsigned long long alg = 0, cells1 = 0, cells2 = 0;
+    unsigned long long alg = 0, cells1 = 0, cells2 = 0, cells_skipped = 0;
     unsigned nal = 0;
 
     for (;;) {
@@ -647,13 +695,21 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
         const int m_warp = __reduce_max_sync(0xffffffffu, m_lane);
         __syncwarp();
 
+        int last_slot = 0;              // last boundary slot phase 1 wrote (packed kernel)
         if constexpr (!FAST) {
             phase1_generic(F, &lut, codes, lane, m0, m_warp, bnd, scores, p.go, p.ge, cells1);
         } else {
-            switch (instance_period(F.P)) {
-#define PCASE(PP) case PP: phase1_packed<PP>(F, &lut, stab, colsel, codes, lane, m_lane, m_warp, pot, gbnd, R, scores, runs, p.go, p.ge, one, F.P / PP, sa, sb, cells1); break;
+            const int pi = instance_period(F.P);
+            int planned = 0;
+            switch (pi) {
+#define PCASE(PP) case PP: last_slot = phase1_packed<PP>(F, &lut, stab, colsel, codes, lane, m_lane, m_warp, pot, gbnd, R, scores, runs, p.go, p.ge, one, F.P / PP, sa, sb, p.strip_skip != 0, &planned, cells1, cells_skipped); break;
                 PCASE(1) PCASE(2) PCASE(3) PCASE(4) PCASE(5) PCASE(7) PCASE(8) PCASE(9) PCASE(10) PCASE(11) PCASE(12)
 #undef PCASE
+            }
+            if (lane == 0) {            // per instance period: planned / skipped main strips, items, items without a skip
+                unsigned long long *a = skip_acc + 1 + 4 * (pi - 1);
+                a[0] += (unsigned long long)planned; a[1] += (unsigned long long)(planned - last_slot);
+                a[2] += 1ull; a[3] += last_slot == planned ? 1ull : 0ull;
             }
         }
         __syncwarp();
@@ -699,7 +755,7 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
                         int u_main = 0;                      // first unit whose running main maximum equals cs
                         if (pending) for (int k = 1; k <= u; ++k) if ((int)runs[(2 * (k - 1) + half) * 32 + lane] == cs) { u_main = k; break; }
                         switch (instance_period(F.P)) {
-#define PCASE(PP) case PP: locate_packed<PP>(F, &lut, stab, stab2, colsel, suffix_table_ready, codes, lane, m, m_warp, bnd, gbnd, R, p.go, p.ge, one, F.P / PP, pending ? cs : 0x7fff, u, u_main, half, sa, sb, &fast_end_ref, &fast_end_read, cells2); break;
+#define PCASE(PP) case PP: locate_packed<PP>(F, &lut, stab, stab2, colsel, suffix_table_ready, codes, lane, m, m_warp, bnd, gbnd, R, p.go, p.ge, one, F.P / PP, pending ? cs : 0x7fff, u, u_main, half, sa, sb, last_slot, &fast_end_ref, &fast_end_read, cells2); break;
                             PCASE(1) PCASE(2) PCASE(3) PCASE(4) PCASE(5) PCASE(7) PCASE(8) PCASE(9) PCASE(10) PCASE(11) PCASE(12)
 #undef PCASE
                         }
@@ -782,6 +838,13 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
             atomicAdd(&p.stats[0], alg); atomicAdd(&p.stats[1], c1); atomicAdd(&p.stats[2], c2);
             atomicAdd(&p.stats[3], na);
         }
+    }
+    if (FAST) {
+        for (int d = 16; d > 0; d >>= 1) cells_skipped += __shfl_down_sync(0xffffffffu, cells_skipped, d);
+        if (lane == 0) skip_acc[0] = cells_skipped;
+        __syncwarp();
+        for (int i = lane; i < TREDSW_STRIP_SKIP_STATS; i += 32)
+            if (skip_acc[i]) atomicAdd(&p.skip_stats[i], skip_acc[i]);
     }
 }
 
@@ -989,6 +1052,13 @@ int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_
     p.allow_fast = allow_fast ? 1 : 0;
     p.match = max_match > 0 ? max_match : 1;
     p.stats = d_stats;
+    // (read on every call, so that one process can compare both modes)
+    p.strip_skip = getenv("TREDSW_NO_STRIP_SKIP") == nullptr ? 1 : 0;
+    if (!ctx->d_skip.p) {
+        if ((rc = ctx->d_skip.ensure(TREDSW_STRIP_SKIP_STATS * sizeof(unsigned long long)))) return rc;
+        CUDA_TRY(cudaMemsetAsync(ctx->d_skip.p, 0, TREDSW_STRIP_SKIP_STATS * sizeof(unsigned long long), ctx->stream));
+    }
+    p.skip_stats = ctx->d_skip.as<unsigned long long>();
     const int nitems_bound = nreads / 32 + ngroups + 1;
     int nctas = 0;
     if ((rc = persistent_ctas(ctx, smem, static_smem, need_fast, need_generic, &nctas))) return rc;
