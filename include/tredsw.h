@@ -101,8 +101,11 @@ int64_t tredsw_launch_count(tredsw_ctx *ctx);
  * summed over every call on this context so far; synchronises the stream.  out (TREDSW_STRIP_SKIP_STATS x int64):
  * [0] skipped phase-1 cell updates (stats[1] of tredsw_classify_reads counts them as planned), then for each loop
  * instantiation period p = 1..12 at [1 + 4 (p - 1)]: main strips planned, main strips skipped, warp items, items
- * that skipped nothing.  TREDSW_NO_STRIP_SKIP set in the environment turns the skipping off (read on every call). */
-#define TREDSW_STRIP_SKIP_STATS 49
+ * that skipped nothing; then at [49 + 3 (p - 1)], summed over the lanes that hold a read: main strips planned, main
+ * strips their warp skipped, and main strips the lane could skip on its own (from the first strip that leaves the
+ * lane's own column unchanged: the bound that no grouping of reads into items can beat).  TREDSW_NO_STRIP_SKIP set
+ * in the environment turns the skipping off (read on every call). */
+#define TREDSW_STRIP_SKIP_STATS 85
 int tredsw_strip_skip_stats(tredsw_ctx *ctx, int64_t *out);
 /* Stage timing with CUDA events on the context's stream: enable, run calls, then read the device time
  * of the LAST call's stages in ms: [0] Smith-Waterman classify kernels, [1] likelihood grid (surface +

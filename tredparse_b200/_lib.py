@@ -203,13 +203,18 @@ class Context:
 
     def strip_skip_stats(self):
         """Main strips of the packed family kernel skipped at the fixed point of their boundary column, summed over
-        this context's calls so far: dict(cells_skipped, by_period={p: dict(planned, skipped, items, items_no_skip)})
-        for the loop instantiation periods p that ran (tredsw_strip_skip_stats)."""
-        a = np.zeros(49, dtype=np.int64)
+        this context's calls so far: dict(cells_skipped, by_period={p: dict(planned, skipped, items, items_no_skip,
+        lane_planned, lane_skipped, lane_skippable)}) for the loop instantiation periods p that ran
+        (tredsw_strip_skip_stats).  The lane_ counters sum over the lanes holding a read: planned strips, strips their
+        warp skipped, and strips the lane could skip on its own — lane_skippable / lane_planned bounds
+        lane_skipped / lane_planned whatever the order of the reads."""
+        a = np.zeros(85, dtype=np.int64)
         check(self.lib.tredsw_strip_skip_stats(self.handle, ptr(a)), "tredsw_strip_skip_stats")
-        per = a[1:].reshape(12, 4)
+        per = a[1:49].reshape(12, 4)
+        lanes = a[49:85].reshape(12, 3)
         return {"cells_skipped": int(a[0]),
-                "by_period": {p + 1: dict(zip(("planned", "skipped", "items", "items_no_skip"), map(int, per[p])))
+                "by_period": {p + 1: dict(zip(("planned", "skipped", "items", "items_no_skip", "lane_planned",
+                                               "lane_skipped", "lane_skippable"), map(int, (*per[p], *lanes[p]))))
                               for p in range(12) if per[p, 2]}}
 
     def enable_timing(self, on=True):

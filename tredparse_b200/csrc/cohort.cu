@@ -515,7 +515,7 @@ extern "C" int tredsw_genotype_batch_ex(tredsw_ctx *ctx, const tredsw_cohort *c,
                  o_stats = carve(4 * sizeof(unsigned long long)), o_drop = carve((size_t)nr + 1);
     if ((rc = ctx->d_misc.ensure(off))) return rc;
     unsigned char *mb = ctx->d_misc.as<unsigned char>();
-    if ((rc = ctx->d_work.ensure(((size_t)12 * nf + 2 + nr + 1) * sizeof(int32_t)))) return rc;
+    if ((rc = ctx->d_work.ensure((tredsw_classify_work_words(c->families, nf, nr) + 1) * sizeof(int32_t)))) return rc;
     CohortDev cd{};
     cd.problems = d_prob; cd.families = d_fam; cd.loci = d_loci; cd.read_problem = d_rp;
     cd.nreads = nr; cd.nproblems = np_; cd.HU = HU; cd.KC = KC; cd.HL = HL;

@@ -4,8 +4,11 @@
 #include "common.cuh"
 
 // Smith-Waterman + classification of every read against its family (sw_family.cu).
-// h_families: host copy (shape decisions); d_* : device buffers.  d_work needs
-// (12*nfamilies + 2 + nreads) int32: counts, offsets and cursors per (family, strand class), the read order.  d_stats: 4 x u64 or NULL (must be zeroed by the caller).
+// h_families: host copy (shape decisions); d_* : device buffers.  d_work needs tredsw_classify_work_words int32:
+// counts and cursors per bin (family, strand class, predicted strips), offsets per (family, strand class), the read
+// order.  d_stats: 4 x u64 or NULL (must be zeroed by the caller).
+int tredsw_classify_bins(const tredsw_family *h_families, int nfamilies);
+size_t tredsw_classify_work_words(const tredsw_family *h_families, int nfamilies, int nreads);
 int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_t *d_roff, int nreads,
                              const int32_t *d_read_family, const tredsw_family *d_families,
                              const tredsw_family *h_families, int nfamilies, int max_read_len,

@@ -517,12 +517,14 @@ __device__ __noinline__ void locate_packed(const FamilySmem &F, const SwLut *lut
     *end_ref = found_col; *end_read = found_row;
 }
 
-// Returns the index of the last boundary slot written (warp-uniform); *planned = main strips of the full plan.
+// Returns the index of the last boundary slot written (warp-uniform); *planned = main strips of the full plan;
+// *lane_conv = main strips this lane needed: the first strip that left the lane's own column unchanged (its outputs
+// depend on that column alone, so the lane stays at the fixed point), or the strips run when it never got there.
 template <int P>
 __device__ __noinline__ int phase1_packed(const FamilySmem &F, const SwLut *lut, uint32_t *stab, uint32_t *colsel,
                                           const uint8_t *codes, int lane, int m, int m_warp, uint32_t *pot,
                                           uint32_t *gbnd, int R, uint8_t *scores, uint8_t *runs, int go, int ge,
-                                          uint32_t one, int G, int sa, int sb, bool skip, int *planned,
+                                          uint32_t one, int G, int sa, int sb, bool skip, int *planned, int *lane_conv,
                                           unsigned long long &cells, unsigned long long &skipped_cells) {
     constexpr int K = strip_units(P);
     constexpr int NC = P * K;
@@ -575,7 +577,7 @@ __device__ __noinline__ int phase1_packed(const FamilySmem &F, const SwLut *lut,
     // strip scores max(run, mu[u], fresh), and every later boundary slot equals the one just written.  The loop
     // stops there; phase 2 reads that slot for any later strip (locate_packed's last_slot).
     const int nplan = (F.U * G + K - 1) / K;                        // main strips of the full nested plan
-    int nstrips = 0;
+    int nstrips = 0, conv = 0;
     for (int u0 = 0; u0 < F.U * G; u0 += K) {                       // u0, u: sub-units of P columns
         uint32_t seg[K], mu[K], diff = 0u;
 #pragma unroll
@@ -584,6 +586,7 @@ __device__ __noinline__ int phase1_packed(const FamilySmem &F, const SwLut *lut,
         strip_pass<NC, P, true, true, true>(stab, codes, lane, m, rows2, gbnd + (size_t)nstrips * R * 32,
                                             gbnd + (size_t)(nstrips + 1) * R * 32, pot, seg, mu, mgo2, mge2, one, diff);
         ++nstrips;
+        if (conv == 0 && diff == 0u) conv = nstrips;
 #pragma unroll
         for (int u = 0; u < K; ++u) {
             run = __vmaxs2(run, seg[u]);
@@ -602,6 +605,7 @@ __device__ __noinline__ int phase1_packed(const FamilySmem &F, const SwLut *lut,
     cells += (unsigned long long)m * 2ull * (unsigned long long)(2 * FLANK + nplan * NC);
     skipped_cells += (unsigned long long)m * 2ull * (unsigned long long)((nplan - nstrips) * NC);
     *planned = nplan;
+    *lane_conv = conv ? conv : nstrips;
     return nstrips;                 // the last boundary slot written
 }
 
@@ -700,9 +704,9 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
             phase1_generic(F, &lut, codes, lane, m0, m_warp, bnd, scores, p.go, p.ge, cells1);
         } else {
             const int pi = instance_period(F.P);
-            int planned = 0;
+            int planned = 0, conv = 0;
             switch (pi) {
-#define PCASE(PP) case PP: last_slot = phase1_packed<PP>(F, &lut, stab, colsel, codes, lane, m_lane, m_warp, pot, gbnd, R, scores, runs, p.go, p.ge, one, F.P / PP, sa, sb, p.strip_skip != 0, &planned, cells1, cells_skipped); break;
+#define PCASE(PP) case PP: last_slot = phase1_packed<PP>(F, &lut, stab, colsel, codes, lane, m_lane, m_warp, pot, gbnd, R, scores, runs, p.go, p.ge, one, F.P / PP, sa, sb, p.strip_skip != 0, &planned, &conv, cells1, cells_skipped); break;
                 PCASE(1) PCASE(2) PCASE(3) PCASE(4) PCASE(5) PCASE(7) PCASE(8) PCASE(9) PCASE(10) PCASE(11) PCASE(12)
 #undef PCASE
             }
@@ -710,6 +714,16 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
                 unsigned long long *a = skip_acc + 1 + 4 * (pi - 1);
                 a[0] += (unsigned long long)planned; a[1] += (unsigned long long)(planned - last_slot);
                 a[2] += 1ull; a[3] += last_slot == planned ? 1ull : 0ull;
+            }
+            // per lane holding a read: the strips of the plan, those its warp skipped, and those it could skip on its
+            // own (the bound that no grouping of reads into items can beat)
+            const bool busy = m_lane > 0;
+            const unsigned lane_planned = __reduce_add_sync(0xffffffffu, busy ? (unsigned)planned : 0u);
+            const unsigned lane_skipped = __reduce_add_sync(0xffffffffu, busy ? (unsigned)(planned - last_slot) : 0u);
+            const unsigned lane_skippable = __reduce_add_sync(0xffffffffu, busy ? (unsigned)(planned - conv) : 0u);
+            if (lane == 0) {
+                unsigned long long *b = skip_acc + 1 + 4 * 12 + 3 * (pi - 1);
+                b[0] += lane_planned; b[1] += lane_skipped; b[2] += lane_skippable;
             }
         }
         __syncwarp();
@@ -862,35 +876,47 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
 // The same bound per strand gives the read's strand class: when only one strand reaches the threshold, no
 // template of the other strand can score min_score, so that strand can never be a candidate (pick() skips scores
 // below max(min_len, 30)) and the packed kernel computes the read on one strand only, two reads per lane.
+//
+// Convergence key.  A lane's main strips reach their fixed point (phase1_packed) about one strip after the template
+// columns have passed the read's own repeat stretch, so the q-grams of the read that occur in the pure repeat (repeat^k,
+// either strand) predict the strips the read needs: min(nplan, ceil((hits + q - 1) / NC) + 1), NC = strip columns.
+// Reads are grouped by (family, strand class, predicted strips), so that the reads of an item stop at about the same
+// strip instead of all waiting for the one with the longest repeat stretch.
 struct QgramInfo {
     int q;                         // 0: filter off for this family (N in the templates)
     int min_score;
     int pair;                      // single-strand classes allowed (packed-kernel family, pairing not switched off)
+    int nplan;                     // main strips of the packed plan; 0: reads keep predicted strips 0 (no ordering)
+    int nc;                        // columns per main strip
 };
-constexpr int QTAB_WORDS = 256;                   // 4096 six-mers x 2 bits (forward / reverse-complement templates)
+// per family: 4096 six-mers x 2 bits (forward / reverse-complement templates), then the same for the pure repeat
+constexpr int QTAB_WORDS = 256;
 
-// eff_group[r] = f * NCLASS + strand class, -2 when the read has no candidate, -1 when it has no family
+// eff_bin[r] = (f * NCLASS + strand class) * nb + nb - 1 - predicted strips (the bins of a group in descending
+// predicted strips), -2 when the read has no candidate, -1 when it has no family
 __global__ void prefilter_kernel(const int8_t *rbuf, const int64_t *roff, int nreads, const int32_t *read_family,
                                  int nfam, const tredsw_family *families, const uint32_t *qtab, const QgramInfo *qinfo,
-                                 int b_minus, int32_t *eff_group, unsigned long long *stats) {
+                                 int nb, int32_t *eff_bin, unsigned long long *stats) {
     const int r = blockIdx.x * blockDim.x + threadIdx.x;
     unsigned long long alg = 0; unsigned nal = 0;
     if (r < nreads) {
-        int f = read_family[r], cls = CLASS_BOTH;
+        int f = read_family[r], cls = CLASS_BOTH, strips = 0;
         if (f < 0 || f >= nfam) f = -1;
         if (f >= 0 && qinfo[f].q > 0) {
             const int q = qinfo[f].q;
             const uint32_t mask = (1u << (2 * q)) - 1u;
-            const uint32_t *tab = qtab + (size_t)f * QTAB_WORDS;
+            const uint32_t *tab = qtab + (size_t)f * 2 * QTAB_WORDS, *rtab = tab + QTAB_WORDS;
             const int8_t *s = rbuf + roff[r];
             const int m = (int)(roff[r + 1] - roff[r]);
-            uint32_t code = 0; int run = 0, nN = 0, hf = 0, hr = 0;
+            uint32_t code = 0; int run = 0, nN = 0, hf = 0, hr = 0, rf = 0, rr = 0;
             for_each_base(s, m, [&](int, int c) {
                 if (c < 0 || c > 3) { ++nN; run = 0; return; }
                 code = ((code << 2) | (uint32_t)c) & mask;
                 if (++run >= q) {
-                    const uint32_t e = (tab[code >> 4] >> ((code & 15u) * 2u)) & 3u;
+                    const uint32_t sh = (code & 15u) * 2u;
+                    const uint32_t e = (tab[code >> 4] >> sh) & 3u, er = (rtab[code >> 4] >> sh) & 3u;
                     hf += e & 1u; hr += e >> 1;
+                    rf += er & 1u; rr += er >> 1;
                 }
             });
             const int thr = qinfo[f].min_score - (q - 1) * (nN + 1);
@@ -905,8 +931,12 @@ __global__ void prefilter_kernel(const int8_t *rbuf, const int64_t *roff, int nr
             } else if (qinfo[f].pair && (hf < thr || hr < thr)) {
                 cls = hf >= thr ? CLASS_FWD : CLASS_RC;
             }
+            if (f >= 0 && qinfo[f].nplan > 0) {
+                const int key = cls == CLASS_FWD ? rf : cls == CLASS_RC ? rr : max(rf, rr);
+                strips = min(qinfo[f].nplan, (key + q - 1 + qinfo[f].nc - 1) / qinfo[f].nc + 1);
+            }
         }
-        eff_group[r] = f >= 0 ? f * NCLASS + cls : f;
+        eff_bin[r] = f >= 0 ? (f * NCLASS + cls) * nb + nb - 1 - strips : f;
     }
     if (stats) {
         for (int d = 16; d > 0; d >>= 1) { alg += __shfl_down_sync(0xffffffffu, alg, d); nal += __shfl_down_sync(0xffffffffu, nal, d); }
@@ -914,36 +944,74 @@ __global__ void prefilter_kernel(const int8_t *rbuf, const int64_t *roff, int nr
     }
 }
 
-// (reads arrive grouped by problem, so the lanes of a warp mostly share one family: the atomics are
-//  aggregated per warp and distinct family — one atomic instead of up to 32 on the same counter)
-__global__ void fam_count_kernel(const int32_t *read_group, int nreads, int ngroups, int32_t *count) {
+// Counting sort of the reads into bins (group, predicted strips), nb bins per (family, strand class) group.
+// (reads arrive grouped by problem, so the lanes of a warp mostly share one bin: the atomics are aggregated per warp
+//  and distinct bin — one atomic instead of up to 32 on the same counter)
+__global__ void fam_count_kernel(const int32_t *read_bin, int nreads, int nbins, int32_t *count) {
     const int r = blockIdx.x * blockDim.x + threadIdx.x;
-    int f = r < nreads ? read_group[r] : -1;
-    if (f >= ngroups) f = -1;
+    int f = r < nreads ? read_bin[r] : -1;
+    if (f >= nbins) f = -1;
     const unsigned peers = __match_any_sync(0xffffffffu, f);
     if (f >= 0 && (threadIdx.x & 31) == __ffs(peers) - 1) atomicAdd(&count[f], __popc(peers));
 }
-// single block: exclusive scans -> grp_start, chunk_start; cursor := grp_start.  An item holds 32 reads of a
-// "both" group, 64 of a single-strand group (two per lane).
-__global__ void fam_scan_kernel(const int32_t *count, int ngroups, const int32_t *perm, int32_t *grp_start,
-                                int32_t *chunk_start, int32_t *cursor) {
-    if (threadIdx.x == 0 && blockIdx.x == 0) {
-        int a = 0, b = 0;
-        for (int g = 0; g < ngroups; ++g) { grp_start[g] = a; cursor[g] = a; a += count[g]; }
-        grp_start[ngroups] = a;
-        for (int i = 0; i < ngroups; ++i) {
-            const int per = perm[i] % NCLASS == CLASS_BOTH ? 32 : 64;
-            chunk_start[i] = b; b += (count[perm[i]] + per - 1) / per;
+constexpr int SCAN_THREADS = 1024;
+// exclusive prefix sums of load(0..n-1), handed to store(i, sum); returns the total (one block of SCAN_THREADS)
+template <class Load, class Store>
+__device__ int block_exclusive_scan(int n, Load load, Store store, int *warp_sums) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    int carry = 0;
+    for (int base = 0; base < n; base += SCAN_THREADS) {
+        const int i = base + threadIdx.x;
+        const int v = i < n ? load(i) : 0;
+        int x = v;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) { const int y = __shfl_up_sync(0xffffffffu, x, d); if (lane >= d) x += y; }
+        if (lane == 31) warp_sums[warp] = x;
+        __syncthreads();
+        if (warp == 0) {
+            int w = warp_sums[lane];
+#pragma unroll
+            for (int d = 1; d < 32; d <<= 1) { const int y = __shfl_up_sync(0xffffffffu, w, d); if (lane >= d) w += y; }
+            warp_sums[lane] = w;
         }
-        chunk_start[ngroups] = b;
+        __syncthreads();
+        if (i < n) store(i, carry + (warp ? warp_sums[warp - 1] : 0) + x - v);
+        carry += warp_sums[31];
+        __syncthreads();
     }
+    return carry;
 }
-__global__ void fam_scatter_kernel(const int32_t *read_group, int nreads, int ngroups, int32_t *cursor,
-                                   int32_t *order, int32_t *out) {
+// An item holds 32 reads of a "both" group, 64 of a single-strand group (two per lane).
+__host__ __device__ constexpr int item_reads(int grp) { return grp % NCLASS == CLASS_BOTH ? 32 : 64; }
+// one block of SCAN_THREADS: cursor[bin] := start of the bin, grp_start[g] = start of group g's first bin, and
+// chunk_start (items, groups in perm order).  A group that fits one item gains nothing from the order of its reads:
+// fam_scatter_kernel sends all its reads to its last bin, in arrival order, so its cursor is the group's start.
+__global__ void __launch_bounds__(SCAN_THREADS) fam_scan_kernel(const int32_t *count, int ngroups, int nb,
+                                                                 const int32_t *perm, int32_t *grp_start,
+                                                                 int32_t *chunk_start, int32_t *cursor) {
+    __shared__ int warp_sums[32];
+    const int total = block_exclusive_scan(ngroups * nb, [&](int i) { return count[i]; },
+                                           [&](int i, int v) { cursor[i] = v; }, warp_sums);
+    for (int g = threadIdx.x; g < ngroups; g += SCAN_THREADS) grp_start[g] = cursor[g * nb];
+    if (threadIdx.x == 0) grp_start[ngroups] = total;
+    __syncthreads();
+    for (int g = threadIdx.x; g < ngroups; g += SCAN_THREADS)
+        if (grp_start[g + 1] - grp_start[g] <= item_reads(g)) cursor[g * nb + nb - 1] = grp_start[g];
+    const int items = block_exclusive_scan(ngroups, [&](int i) {
+        const int g = perm[i], per = item_reads(g);
+        return (grp_start[g + 1] - grp_start[g] + per - 1) / per; }, [&](int i, int v) { chunk_start[i] = v; }, warp_sums);
+    if (threadIdx.x == 0) chunk_start[ngroups] = items;
+}
+__global__ void fam_scatter_kernel(const int32_t *read_bin, int nreads, int nbins, int nb, const int32_t *grp_start,
+                                   int32_t *cursor, int32_t *order, int32_t *out) {
     const int r = blockIdx.x * blockDim.x + threadIdx.x;
     const int lane = threadIdx.x & 31;
-    int f = r < nreads ? read_group[r] : -1;
-    if (f >= ngroups) f = -1;
+    int f = r < nreads ? read_bin[r] : -1;
+    if (f >= nbins) f = -1;
+    if (f >= 0) {
+        const int g = f / nb;
+        if (grp_start[g + 1] - grp_start[g] <= item_reads(g)) f = g * nb + nb - 1;
+    }
     const unsigned peers = __match_any_sync(0xffffffffu, f);
     const int leader = __ffs(peers) - 1;
     int base = 0;
@@ -1002,7 +1070,34 @@ int persistent_ctas(tredsw_ctx *ctx, size_t smem, size_t static_smem, bool need_
     return TREDSW_OK;
 }
 
+// packed plan of a family: main strips and columns per strip (0 strips: the family runs the generic kernel)
+void packed_plan(const tredsw_family &g, bool allow_fast, int *nplan, int *nc) {
+    *nplan = 0; *nc = 0;
+    if (!(allow_fast && g.prefix_len == FLANK && g.suffix_len == FLANK && g.period >= 1 && g.period <= 12)) return;
+    const int pi = instance_period(g.period), k = strip_units(pi);
+    *nplan = (g.max_units * (g.period / pi) + k - 1) / k;
+    *nc = pi * k;
+}
+
 }  // namespace
+
+// bins per (family, strand class) group of the read order: predicted strips 0..nplan of the longest packed plan
+int tredsw_classify_bins(const tredsw_family *h_families, int nfamilies) {
+    int nb = 1;
+    for (int f = 0; f < nfamilies; ++f) {
+        const tredsw_family &g = h_families[f];
+        if (g.period < 1 || g.period > 12 || g.max_units < 1 || g.max_units > 4096) continue;
+        int nplan, nc;
+        packed_plan(g, true, &nplan, &nc);
+        nb = std::max(nb, nplan + 1);
+    }
+    return nb;
+}
+
+size_t tredsw_classify_work_words(const tredsw_family *h_families, int nfamilies, int nreads) {
+    const size_t ngroups = (size_t)NCLASS * nfamilies, nbins = ngroups * tredsw_classify_bins(h_families, nfamilies);
+    return 2 * nbins + 2 * (ngroups + 1) + (size_t)nreads;
+}
 
 int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_t *d_roff, int nreads,
                              const int32_t *d_read_family, const tredsw_family *d_families,
@@ -1024,9 +1119,9 @@ int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_
         bool fast = allow_fast && g.prefix_len == FLANK && g.suffix_len == FLANK && g.period <= 12;
         if (fast) {
             need_fast = true;
-            const int pi = instance_period(g.period), sub = g.period / pi;      // sub-units per unit
-            const int k = strip_units(pi), slots = (g.max_units * sub + k - 1) / k + 1;
-            if (slots > nslots) nslots = slots;
+            int nplan, nc;
+            packed_plan(g, allow_fast, &nplan, &nc);
+            if (nplan + 1 > nslots) nslots = nplan + 1;
         } else need_generic = true;
     }
     const int max_rows = max_m > 0 ? max_m : 1;
@@ -1042,11 +1137,15 @@ int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_
     ClassifyParams p{};
     p.rbuf = d_rbuf; p.roff = d_roff; p.families = d_families; p.out = d_out;
     const int ngroups = NCLASS * nfamilies;
+    // read order: bins of predicted strips per group (one bin when the order is switched off; read on every call, so
+    // that one process can compare both modes).  d_work is sized for tredsw_classify_bins bins per group.
+    const bool conv_order = getenv("TREDSW_NO_CONVERGENCE_ORDER") == nullptr;
+    const int nb = conv_order ? tredsw_classify_bins(h_families, nfamilies) : 1, nbins = ngroups * nb;
     int32_t *w = d_work;
-    int32_t *d_count = w, *d_grp_start = w + ngroups, *d_chunk_start = d_grp_start + ngroups + 1,
-            *d_cursor = d_chunk_start + ngroups + 1, *d_order = d_cursor + ngroups;
-    CUDA_TRY(cudaMemsetAsync(d_count, 0, ngroups * sizeof(int32_t), ctx->stream));
-    const int tb = 256, nb = (nreads + tb - 1) / tb;
+    int32_t *d_count = w, *d_grp_start = w + nbins, *d_chunk_start = d_grp_start + ngroups + 1,
+            *d_cursor = d_chunk_start + ngroups + 1, *d_order = d_cursor + nbins;
+    CUDA_TRY(cudaMemsetAsync(d_count, 0, nbins * sizeof(int32_t), ctx->stream));
+    const int tb = 256, nblk = (nreads + tb - 1) / tb;
     p.order = d_order; p.grp_start = d_grp_start; p.chunk_start = d_chunk_start;
     p.ngroups = ngroups; p.go = gap_open; p.ge = gap_extend; p.max_rows = max_rows;
     p.allow_fast = allow_fast ? 1 : 0;
@@ -1068,7 +1167,7 @@ int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_
     const size_t pot_bytes = (size_t)nctas * rows_alloc * 32 * sizeof(uint32_t);
     const size_t gbnd_bytes = pot_bytes * (nslots + 1);
     const size_t perm_bytes = (((size_t)ngroups * sizeof(int32_t)) + 15) & ~(size_t)15;
-    const size_t qtab_bytes = (size_t)nfamilies * QTAB_WORDS * sizeof(uint32_t);
+    const size_t qtab_bytes = (size_t)nfamilies * 2 * QTAB_WORDS * sizeof(uint32_t);
     const size_t qinfo_bytes = (((size_t)nfamilies * sizeof(QgramInfo)) + 15) & ~(size_t)15;
     const size_t eff_bytes = (((size_t)nreads * sizeof(int32_t)) + 15) & ~(size_t)15;
     if ((rc = ctx->d_scratch.ensure(score_bytes + pot_bytes + gbnd_bytes + 16 + perm_bytes + qtab_bytes + qinfo_bytes + eff_bytes))) return rc;
@@ -1096,11 +1195,11 @@ int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_
         h_perm.swap(perm);
     }
     p.grp_perm = d_perm;
-    // q-gram pre-filter tables: per family 4096 x 2 bits (q-grams of all forward / all reverse-complement templates)
+    // q-gram pre-filter tables: per family 4096 x 2 bits (q-grams of all forward / all reverse-complement templates),
+    // then 4096 x 2 bits for the pure repeat (convergence key)
     uint32_t *d_qtab = reinterpret_cast<uint32_t *>(reinterpret_cast<unsigned char *>(d_perm) + perm_bytes);
     QgramInfo *d_qinfo = reinterpret_cast<QgramInfo *>(reinterpret_cast<unsigned char *>(d_qtab) + qtab_bytes);
     int32_t *d_eff = reinterpret_cast<int32_t *>(reinterpret_cast<unsigned char *>(d_qinfo) + qinfo_bytes);
-    int b_minus = 0;
     {
         // q - 1 <= min(mismatch penalty, gap open); only for match == 1 and N scoring <= 0 everywhere
         int max_off = -128; bool n_ok = true, diag_ok = true;
@@ -1110,7 +1209,7 @@ int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_
             else if (i == j) { if (v != 1) diag_ok = false; }
             else if (v > max_off) max_off = v;
         }
-        b_minus = -max_off;
+        const int b_minus = -max_off;
         int q = 6;
         if (q > b_minus + 1) q = b_minus + 1;
         if (q > gap_open + 1) q = gap_open + 1;
@@ -1118,31 +1217,17 @@ int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_
         const bool usable = n_ok && diag_ok && q >= 4 && !env_off;
         // (read on every call, so that one process can compare both modes)
         const bool pairing = getenv("TREDSW_NO_STRAND_PAIRING") == nullptr;
-        std::vector<uint32_t> tab((size_t)nfamilies * QTAB_WORDS, 0u);
+        std::vector<uint32_t> tab((size_t)nfamilies * 2 * QTAB_WORDS, 0u);
         std::vector<QgramInfo> info(nfamilies);
         std::vector<int8_t> t;
-        for (int f = 0; f < nfamilies; ++f) {
-            const tredsw_family &g = h_families[f];
-            // N in a template (GCN / NGC motifs) scores 0 against every base: such a pair neither breaks the
-            // score nor earns it.  Count it as "compatible": runs of compatible pairs are broken by mismatches
-            // and gaps only, so the same bound holds for q-grams compared with N as a wildcard — every template
-            // q-gram with N's is expanded to the concrete q-grams it is compatible with.
-            info[f].q = usable ? q : 0;
-            info[f].min_score = 30;                         // bam_parser.py:134: min_score = max(min_len, 30)
-            info[f].pair = pairing && allow_fast && g.prefix_len == FLANK && g.suffix_len == FLANK && g.period <= 12;
-            if (!info[f].q) continue;
-            bool too_many_n = false;
-            // every q-gram of a template with u >= u0 units already occurs in the template with u0 units
-            const int u0 = (q - 1 + g.period - 1) / g.period + 1;
-            const uint32_t mask = (1u << (2 * q)) - 1u;
-            uint32_t *tf = tab.data() + (size_t)f * QTAB_WORDS;
-            for (int u = 1; u <= std::min(g.max_units, u0 + 1); ++u) {
-                t.clear();
-                for (int i = 0; i < g.prefix_len; ++i) t.push_back(g.prefix[i]);
-                for (int k = 0; k < u; ++k) for (int i = 0; i < g.period; ++i) t.push_back(g.repeat[i]);
-                for (int i = 0; i < g.suffix_len; ++i) t.push_back(g.suffix[i]);
-                const int n = (int)t.size();
-                for (int i = 0; i + q <= n; ++i) {
+        const uint32_t mask = (1u << (2 * q)) - 1u;
+        // N in a template (GCN / NGC motifs) scores 0 against every base: such a pair neither breaks the score nor
+        // earns it.  Count it as "compatible": runs of compatible pairs are broken by mismatches and gaps only, so the
+        // same bound holds for q-grams compared with N as a wildcard — every q-gram of t with N's is expanded to the
+        // concrete q-grams it is compatible with.  False when a q-gram holds too many N.
+        auto add_grams = [&](uint32_t *tf) {
+            const int n = (int)t.size();
+            for (int i = 0; i + q <= n; ++i) {
                     // forward q-gram t[i..i+q) and the reverse complement's q-gram that covers the same bases
                     int npos[8], nn = 0;
                     uint32_t cf = 0, cr = 0;
@@ -1154,7 +1239,7 @@ int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_
                         cf |= (uint32_t)(isn ? 0 : c) << (2 * (q - 1 - k));
                         cr |= (uint32_t)(isn ? 0 : 3 - c) << (2 * k);       // position k of the forward gram = q-1-k from the right
                     }
-                    if (nn > 4) { too_many_n = true; break; }
+                    if (nn > 4) return false;
                     for (uint32_t e = 0; e < (1u << (2 * nn)); ++e) {       // all fillings of the N positions
                         uint32_t xf = cf, xr = cr;
                         for (int z = 0; z < nn; ++z) {
@@ -1166,10 +1251,32 @@ int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_
                         tf[xf >> 4] |= 1u << ((xf & 15u) * 2u);
                         tf[xr >> 4] |= 2u << ((xr & 15u) * 2u);
                     }
-                }
-                if (too_many_n) break;
             }
-            if (too_many_n) info[f].q = 0;
+            return true;
+        };
+        for (int f = 0; f < nfamilies; ++f) {
+            const tredsw_family &g = h_families[f];
+            info[f].q = usable ? q : 0;
+            info[f].min_score = 30;                         // bam_parser.py:134: min_score = max(min_len, 30)
+            info[f].pair = pairing && allow_fast && g.prefix_len == FLANK && g.suffix_len == FLANK && g.period <= 12;
+            packed_plan(g, allow_fast && conv_order, &info[f].nplan, &info[f].nc);
+            if (!info[f].q) continue;
+            bool ok = true;
+            // every q-gram of a template with u >= u0 units already occurs in the template with u0 units
+            const int u0 = (q - 1 + g.period - 1) / g.period + 1;
+            uint32_t *tf = tab.data() + (size_t)f * 2 * QTAB_WORDS;
+            for (int u = 1; ok && u <= std::min(g.max_units, u0 + 1); ++u) {
+                t.clear();
+                for (int i = 0; i < g.prefix_len; ++i) t.push_back(g.prefix[i]);
+                for (int k = 0; k < u; ++k) for (int i = 0; i < g.period; ++i) t.push_back(g.repeat[i]);
+                for (int i = 0; i < g.suffix_len; ++i) t.push_back(g.suffix[i]);
+                ok = add_grams(tf);
+            }
+            // the pure repeat repeat^(u0 + 1): every q-gram of any run of the repeat
+            t.clear();
+            for (int k = 0; k <= u0; ++k) for (int i = 0; i < g.period; ++i) t.push_back(g.repeat[i]);
+            if (ok && info[f].nplan) ok = add_grams(tf + QTAB_WORDS);
+            if (!ok) info[f].q = 0;
         }
         // perm | qtab | qinfo through the page-locked table staging (see stage_small): no pageable copy sits
         // between the input transfer and the kernels of a call
@@ -1184,11 +1291,12 @@ int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_
         CUDA_TRY(cudaMemcpyAsync(d_qinfo, ht + offs[2], sizes[2], cudaMemcpyHostToDevice, ctx->stream));
     }
     ctx->mark(0);
-    prefilter_kernel<<<nb, tb, 0, ctx->stream>>>(d_rbuf, d_roff, nreads, d_read_family, nfamilies, d_families, d_qtab,
-                                                 d_qinfo, b_minus, d_eff, d_stats);
-    fam_count_kernel<<<nb, tb, 0, ctx->stream>>>(d_eff, nreads, ngroups, d_count);
-    fam_scan_kernel<<<1, 32, 0, ctx->stream>>>(d_count, ngroups, d_perm, d_grp_start, d_chunk_start, d_cursor);
-    fam_scatter_kernel<<<nb, tb, 0, ctx->stream>>>(d_eff, nreads, ngroups, d_cursor, d_order, p.out);
+    prefilter_kernel<<<nblk, tb, 0, ctx->stream>>>(d_rbuf, d_roff, nreads, d_read_family, nfamilies, d_families, d_qtab,
+                                                   d_qinfo, nb, d_eff, d_stats);
+    fam_count_kernel<<<nblk, tb, 0, ctx->stream>>>(d_eff, nreads, nbins, d_count);
+    fam_scan_kernel<<<1, SCAN_THREADS, 0, ctx->stream>>>(d_count, ngroups, nb, d_perm, d_grp_start, d_chunk_start,
+                                                         d_cursor);
+    fam_scatter_kernel<<<nblk, tb, 0, ctx->stream>>>(d_eff, nreads, nbins, nb, d_grp_start, d_cursor, d_order, p.out);
     CUDA_TRY(cudaGetLastError());
     ctx->launches += 4;
     CUDA_TRY(cudaMemsetAsync(p.counter, 0, 2 * sizeof(int32_t), ctx->stream));
@@ -1225,7 +1333,7 @@ extern "C" int tredsw_classify_reads(tredsw_ctx *ctx, const int8_t *rbuf, const 
     if ((rc = stage_in(ctx, ctx->d_rfam, read_family, (size_t)nreads, flags, &d_rfam))) return rc;
     if ((rc = stage_in(ctx, ctx->d_fam, families, (size_t)nfamilies, flags, &d_fam))) return rc;
     if ((rc = ctx->d_out.ensure((size_t)nreads * 8 * sizeof(int32_t)))) return rc;
-    if ((rc = ctx->d_work.ensure(((size_t)4 * NCLASS * nfamilies + 2 + nreads) * sizeof(int32_t)))) return rc;
+    if ((rc = ctx->d_work.ensure(tredsw_classify_work_words(families, nfamilies, nreads) * sizeof(int32_t)))) return rc;
     if ((rc = ctx->d_stats.ensure(4 * sizeof(unsigned long long)))) return rc;
     CUDA_TRY(cudaMemsetAsync(ctx->d_stats.p, 0, 4 * sizeof(unsigned long long), ctx->stream));
     if ((rc = tredsw_internal_classify(ctx, d_rbuf, d_roff, nreads, d_rfam, d_fam, families, nfamilies, max_m, mat25,
