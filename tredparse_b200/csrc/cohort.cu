@@ -374,6 +374,8 @@ extern "C" int tredsw_genotype_batch_ex(tredsw_ctx *ctx, const tredsw_cohort *c,
     if (c->norepeatpairs && c->nreads > 0 && !c->read_name) { tredsw_set_error("norepeatpairs needs read_name"); return TREDSW_ERR_ARG; }
     if (c->nproblems <= 0 || c->nreads < 0 || c->nfamilies <= 0 || !c->families || !c->loci || !c->step_pmf ||
         c->max_read_len <= 0 || c->maxinsert < 1) { tredsw_set_error("bad cohort descriptor"); return TREDSW_ERR_ARG; }
+    int grid_tables;
+    if (int rc0 = tredsw_internal_grid_tables(&grid_tables)) return rc0;
     const bool dev = dev_ptrs(flags);
     // TREDSW_DEVICE_INPUTS: the bulk evidence (rbuf, roff, read_problem, pe_lens) already lies in device memory — e.g.
     // where tredsw_ingest_batch_run left it — while `problems`, `read_name` and every output are host buffers that
@@ -575,7 +577,7 @@ extern "C" int tredsw_genotype_batch_ex(tredsw_ctx *ctx, const tredsw_cohort *c,
     unsigned long long *d_tab_flag = nullptr;
     if ((rc = tredsw_internal_grid(ctx, cd.gp, np_, d_ipool, d_dpool, ctx->d_surface.as<double>(), cd.marg,
                                    ctx->d_res.as<tredsw_grid_result>(), c->fullsearch ? per_problem : 4LL * HL, 0,
-                                   d_post, post_cap, cd.post_cursor, &d_tab_flag))) return rc;
+                                   d_post, post_cap, cd.post_cursor, &d_tab_flag, grid_tables))) return rc;
     finalize_kernel<<<(np_ + 7) / 8, 256, 0, ctx->stream>>>(cd, ctx->d_res.as<tredsw_grid_result>(), d_calls);
     CUDA_TRY(cudaGetLastError());
     ctx->mark(7);

@@ -87,6 +87,7 @@ struct GridParams {
     double small_value, log_small;
     int nproblems;
     int materialise;             // write every point (and -inf where h1 > h2) into the surface slots
+    int tables;                  // best table tier a large surface may take: 0 full, 1 without PE operands, 2 none
     BigInfo *big;                // [nproblems]
     int *lists;                  // [0] number of large surfaces, [1 + i] their problem indices
     int *items;                  // point items of the small surfaces: (problem, chunk, nitems) triples
@@ -408,13 +409,15 @@ __global__ void __launch_bounds__(256) grid_classify_kernel(GridParams g) {
         const int npe = (P.run_pe && P.n_target > 0) ? P.n_target : 0;
         const Tab full = tab_layout(n1, n2, B.nd, npe, B.nc, true), nope = tab_layout(n1, n2, B.nd, 0, B.nc, true),
                   bare = tab_layout(n1, n2, B.nd, 0, B.nc, false);
-        // the reduction scratch is mandatory; the tables are taken when the arena has room for them
+        // the reduction scratch is mandatory; the tables are taken when the arena has room for them (and the
+        // caller allows that tier)
         bool fail = false;
-        unsigned long long off = atomicAdd(&g.fcursor[0], (unsigned long long)full.end);
-        if ((long long)(off + full.end) <= g.ftab_cap) { B.ok = 1; B.npe = npe; }
+        unsigned long long off = 0;
+        if (g.tables == 0) off = atomicAdd(&g.fcursor[0], (unsigned long long)full.end);
+        if (g.tables == 0 && (long long)(off + full.end) <= g.ftab_cap) { B.ok = 1; B.npe = npe; }
         else {
-            off = atomicAdd(&g.fcursor[0], (unsigned long long)nope.end);
-            if ((long long)(off + nope.end) <= g.ftab_cap) { B.ok = 1; B.npe = 0; }
+            if (g.tables <= 1) off = atomicAdd(&g.fcursor[0], (unsigned long long)nope.end);
+            if (g.tables <= 1 && (long long)(off + nope.end) <= g.ftab_cap) { B.ok = 1; B.npe = 0; }
             else {
                 off = atomicAdd(&g.fcursor[0], (unsigned long long)bare.end);
                 if ((long long)(off + bare.end) > g.ftab_cap) { fail = true; atomicExch(&g.fcursor[1], 1ULL); off = 0; }
@@ -1111,6 +1114,18 @@ __global__ void __launch_bounds__(KDE_THREADS) pe_kde_kernel(const int32_t *lens
 
 }  // namespace
 
+// TREDSW_GRID_TABLES=nope | none: large surfaces evaluate the paired-end term point by point, or every term (the
+// tiers a full arena falls back to; same results).  Read on every call.
+int tredsw_internal_grid_tables(int *tables) {
+    *tables = 0;
+    if (const char *tier = getenv("TREDSW_GRID_TABLES")) {
+        if (strcmp(tier, "nope") == 0) *tables = 1;
+        else if (strcmp(tier, "none") == 0) *tables = 2;
+        else { tredsw_set_error("TREDSW_GRID_TABLES must be nope or none, not '%s'", tier); return TREDSW_ERR_ARG; }
+    }
+    return TREDSW_OK;
+}
+
 // device-side bookkeeping area of one grid call, at the start of ctx->d_ftab
 struct GridArea {
     size_t big_bytes, ctr_off, list_off, item_off, row_off, tab_off;
@@ -1130,12 +1145,12 @@ int tredsw_internal_grid(tredsw_ctx *ctx, const tredsw_grid_problem *d_prob, int
                          const int32_t *d_ipool, const double *d_dpool, double *d_surface, double *d_marg,
                          tredsw_grid_result *d_res, long long points_hint, int materialise,
                          tredsw_posterior *d_post, long long post_cap, unsigned long long *d_post_cursor,
-                         unsigned long long **d_overflow_flag) {
+                         unsigned long long **d_overflow_flag, int tables) {
     GridParams g{};
     g.prob = d_prob; g.ipool = d_ipool; g.dpool = d_dpool; g.surface = d_surface; g.marg = d_marg; g.res = d_res;
     g.small_value = exp(-10.0);
     g.log_small = log(g.small_value);
-    g.nproblems = nproblems; g.materialise = materialise;
+    g.nproblems = nproblems; g.materialise = materialise; g.tables = tables;
     g.post = d_post; g.post_cap = post_cap; g.post_cursor = d_post_cursor;
     int rc;
     ctx->mark(2);
@@ -1194,12 +1209,13 @@ extern "C" int tredsw_likelihood_grid(tredsw_ctx *ctx, const tredsw_grid_problem
     if (nproblems == 0) return TREDSW_OK;
     const bool dev = dev_ptrs(flags);
     if (dev && !surface) { tredsw_set_error("device mode needs the surface buffer (it is the kernels' scratch)"); return TREDSW_ERR_ARG; }
+    int tables, rc;
+    if ((rc = tredsw_internal_grid_tables(&tables))) return rc;
     std::lock_guard<std::mutex> lock(ctx->mu);
     CUDA_TRY(cudaSetDevice(ctx->device));
     // host mode: the surface is materialised iff the caller wants it back; device mode: unless TREDSW_GRID_NO_SURFACE
     const int materialise = dev ? ((flags & TREDSW_GRID_NO_SURFACE) ? 0 : 1) : ((surface && n_surface > 0) ? 1 : 0);
     GridParams g{};
-    int rc;
     long long max_points = 0;
     if (!dev) {
         for (int i = 0; i < nproblems; ++i) {
@@ -1227,7 +1243,7 @@ extern "C" int tredsw_likelihood_grid(tredsw_ctx *ctx, const tredsw_grid_problem
     for (int attempt = 0; attempt < 2; ++attempt) {
         unsigned long long *d_flag = nullptr;
         if ((rc = tredsw_internal_grid(ctx, g.prob, nproblems, g.ipool, g.dpool, g.surface, g.marg, g.res, max_points,
-                                       materialise, nullptr, 0, nullptr, &d_flag))) return rc;
+                                       materialise, nullptr, 0, nullptr, &d_flag, tables))) return rc;
         if (dev) return TREDSW_OK;
         unsigned long long h_flag[2] = {0, 0};
         CUDA_TRY(cudaMemcpyAsync(h_flag, d_flag, sizeof(h_flag), cudaMemcpyDeviceToHost, ctx->stream));

@@ -23,4 +23,7 @@ int tredsw_internal_grid(tredsw_ctx *ctx, const tredsw_grid_problem *d_prob, int
                          const int32_t *d_ipool, const double *d_dpool, double *d_surface, double *d_marg,
                          tredsw_grid_result *d_res, long long points_hint, int materialise,
                          tredsw_posterior *d_post, long long post_cap, unsigned long long *d_post_cursor,
-                         unsigned long long **d_overflow_flag);
+                         unsigned long long **d_overflow_flag, int tables);
+// TREDSW_GRID_TABLES -> the best table tier a large likelihood surface may take (0 full, 1 without the paired-end
+// operands, 2 none); an unknown value is an argument error.  Parsed by the public entry points before they launch.
+int tredsw_internal_grid_tables(int *tables);
