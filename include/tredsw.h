@@ -381,6 +381,9 @@ tredsw_bam *tredsw_bam_open(const char *bam_path, const char *bai_path);
 tredsw_bam *tredsw_bam_clone(tredsw_bam *bam);
 void tredsw_bam_close(tredsw_bam *bam);
 int32_t tredsw_bam_nref(tredsw_bam *bam);
+/* contig `tid` of the binary reference dictionary: its length (-1: no such contig); its name, NUL-terminated and cut to
+ * cap - 1 bytes, into name when name is not NULL */
+int64_t tredsw_bam_ref(tredsw_bam *bam, int32_t tid, char *name, int64_t cap);
 int32_t tredsw_bam_tid(tredsw_bam *bam, const char *contig);     /* -1 when unknown */
 /* signature of the reference dictionary (names + lengths, in order): equal signatures = equal contig numbering */
 uint64_t tredsw_bam_header_signature(tredsw_bam *bam);
@@ -495,6 +498,51 @@ int tredsw_ingest_scan_emulate(tredsw_bam *bam, const tredsw_locus_query *querie
  * (us), [9] status of the scan (the per-problem code above; 0 ok). */
 #define TREDSW_SCAN_NSTATS 10
 int tredsw_ingest_scan_stats(const tredsw_ingest_batch *batch, int64_t *stats);
+
+/* The STR profile of a scan: in-repeat reads (IRRs), found in the same streaming pass (DESIGN §4.5).  Records
+ * considered are the primary ones (flags 0x100, 0x200, 0x400, 0x800 unset), mapped or not, with l_seq >= min_read_len.
+ * A read s of length L is an IRR of period k when, of the L - k positions i with s[i] == s[i + k] (N never equal), at
+ * least purity_num / purity_den agree (m * den >= num * (L - k)); its period is the smallest such k in
+ * [min_period, max_period].  Its motif: the majority base of every phase (ties: the smallest of A < C < G < T; an
+ * all-N phase: A), reduced to its primitive root (a root of one base is a homopolymer: not an IRR), in canonical
+ * form (the smallest rotation of the root and of its reverse complement), 2 bits a base, first base most significant.
+ * Valid parameters: 2 <= min_period <= max_period <= 20, 0 < purity_num <= purity_den <= 1000, min_read_len >=
+ * 2 max_period; anything else is TREDSW_ERR_ARG. */
+typedef struct { int32_t min_period, max_period, purity_num, purity_den, min_read_len; } tredsw_irr_params;
+typedef struct {                /* one IRR record, in file order */
+    int32_t tid, pos, next_tid, next_pos;
+    int32_t flag, mapq, mq, period;   /* mq: the record's MQ tag (integer types c C s S i I), -1 without one */
+    uint64_t motif;             /* canonical motif, `period` bases of 2 bits */
+    int64_t name_off;           /* its name: name_len bytes (no NUL) at names + name_off */
+    int32_t name_len, mate;     /* mate: the entry with the same name and the other segment flag (0x40 / 0x80), -1 none */
+} tredsw_irr_entry;
+typedef struct {                /* host arrays, valid until tredsw_ingest_batch_free; a failed scan (status 1-4) has no
+                                   entries and every counter 0 */
+    int64_t n_entries;
+    const tredsw_irr_entry *entries;
+    const char *names; int64_t name_bytes;
+    int64_t records_considered, irr_records;
+    int64_t depth_bases;        /* sum of l_seq over primary, mapped, non-duplicate, non-QC-fail records */
+    int64_t max_l_seq;          /* over the primary records */
+    int64_t anchors_without_mq; /* IRRs that are paired (0x1), whose mate is mapped (0x8 unset, next_tid >= 0) and not
+                                   an IRR, and that carry no MQ tag */
+    int64_t unparsed_aux;       /* IRR records whose aux area could not be parsed (taken as without MQ) */
+} tredsw_irr_view;
+/* tredsw_ingest_scan_run / _emulate with an IRR profile: irr = NULL is exactly those calls; nqueries = 0 and no depth
+ * regions with irr set is a profile-only scan.  The profile's kernels do not change the evidence, depths or
+ * statistics of the scan. */
+int tredsw_ingest_scan_run_ex(tredsw_ctx *ctx, tredsw_bam *bam, const tredsw_locus_query *queries, int32_t nqueries,
+                              const int32_t *depth_regions, int32_t n_depth, double *depth_out, int64_t slab_bytes,
+                              uint32_t flags, const tredsw_irr_params *irr, tredsw_ingest_batch **out);
+/* TEST INFRASTRUCTURE: the same with every kernel body run serially on the host.  The package never calls it. */
+int tredsw_ingest_scan_emulate_ex(tredsw_bam *bam, const tredsw_locus_query *queries, int32_t nqueries,
+                                  const int32_t *depth_regions, int32_t n_depth, double *depth_out, int64_t slab_bytes,
+                                  uint32_t flags, const tredsw_irr_params *irr, tredsw_ingest_batch **out);
+/* The profile of a batch scanned with irr set (TREDSW_ERR_ARG otherwise). */
+int tredsw_ingest_scan_irr(const tredsw_ingest_batch *batch, tredsw_irr_view *view);
+/* Test hook: the classifier body on the host.  codes: 0..3 = A C G T, anything else N.  *period = 0: not an IRR. */
+int tredsw_irr_classify_host(const int8_t *codes, int32_t len, const tredsw_irr_params *params, int32_t *period,
+                             uint64_t *motif);
 
 #ifdef __cplusplus
 }

@@ -91,12 +91,13 @@ def encode(r):
     body = struct.pack("<iiBBHHHiiii", r.reference_id, r.reference_start, len(nm), r.mapping_quality,
                        int(reg2bin(np.array([r.reference_start]), np.array([rend]))[0]), len(r.cigartuples), r.flag,
                        len(seq), r.next_reference_id, r.next_reference_start, r.template_length)
-    body += nm + b"".join(struct.pack("<I", (l << 4) | op) for op, l in r.cigartuples) + packed + b"\xff" * len(seq)
+    body += nm + b"".join(struct.pack("<I", (l << 4) | op) for op, l in r.cigartuples) + packed + b"\xff" * len(seq) + r.aux
     return struct.pack("<i", len(body)) + body, rend
 
 
-def write_sample(path, gb, seed=5):
-    """-> (records, inflated bytes); writes path and path.bai"""
+def write_sample(path, gb, seed=5, extra=()):
+    """-> (records, inflated bytes); writes path and path.bai.  extra: more bamio.AlignedSegment records (placed by
+    contig and position; records without a contig go to the unmapped tail)"""
     from tredparse_b200 import bamio, simulate
     from tredparse_b200.meta import TREDsRepo
     repo = TREDsRepo()
@@ -121,6 +122,9 @@ def write_sample(path, gb, seed=5):
                                         seed=sp["seed"], tag="l{}".format(li)):
             raw, rend = encode(r)
             loci.setdefault(r.reference_id, []).append((r.reference_start, rend, raw))
+    for r in extra:
+        raw, rend = encode(r)
+        loci.setdefault(r.reference_id, []).append((r.reference_start, rend, raw))
     # the stream, contig by contig: (per record) position, end, bytes in file order
     parts, meta = [header], []                     # meta: (tid, pos array, end array, lengths array)
     first_name = 0
@@ -145,6 +149,7 @@ def write_sample(path, gb, seed=5):
             P.append(pos[prev:]); E.append(pos[prev:] + READLEN); L.append(np.full(len(pos) - prev, REC_BYTES))
         meta.append((tid, np.concatenate(P) if P else np.zeros(0, np.int64), np.concatenate(E) if E else np.zeros(0, np.int64),
                      np.concatenate(L) if L else np.zeros(0, np.int64)))
+    parts += [raw for _, _, raw in loci.get(-1, [])]          # the unmapped tail (not in the index)
     stream = b"".join(parts)
     del parts
     nblocks = (len(stream) + BLOCK - 1) // BLOCK
@@ -205,7 +210,7 @@ def write_sample(path, gb, seed=5):
                 else:
                     nxt = lin[k]
             fh.write(struct.pack("<i", nwin) + lin.astype("<u8").tobytes())
-    return sum(len(m[1]) for m in meta), len(stream)
+    return sum(len(m[1]) for m in meta) + len(loci.get(-1, [])), len(stream)
 
 
 def main():

@@ -31,13 +31,15 @@ EXPORTS = [
     # native BAM ingest
     "tredsw_bam_open", "tredsw_bam_close", "tredsw_bam_nref", "tredsw_bam_tid", "tredsw_bam_extract_locus",
     "tredsw_bam_region_depth", "tredsw_bam_read_length", "tredsw_bam_clone", "tredsw_bam_inflate_stats", "tredsw_inflate_raw",
-    "tredsw_bam_header_signature",
+    "tredsw_bam_header_signature", "tredsw_bam_ref",
     # BAM ingest on the GPU (batched); *_emulate / *_device_code run the device code on the host for the CPU tests
     "tredsw_ingest_batch_run", "tredsw_ingest_batch_view", "tredsw_ingest_batch_free", "tredsw_ingest_batch_emulate",
     "tredsw_inflate_raw_device_code",
     # BAMs without an index: one streaming pass per sample
     "tredsw_bam_open_unindexed", "tredsw_ingest_scan_run", "tredsw_ingest_scan_emulate", "tredsw_ingest_scan_stats",
     "tredsw_bam_open_stream", "tredsw_bam_header_text",
+    # the STR profile of a scan (in-repeat reads)
+    "tredsw_ingest_scan_run_ex", "tredsw_ingest_scan_emulate_ex", "tredsw_ingest_scan_irr", "tredsw_irr_classify_host",
 ]
 
 

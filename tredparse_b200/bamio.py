@@ -42,10 +42,10 @@ class AlignedSegment:
 
     __slots__ = ("query_name", "flag", "reference_id", "reference_start", "mapping_quality",
                  "cigartuples", "next_reference_id", "next_reference_start", "template_length",
-                 "query_sequence", "_qual", "_ref_end")
+                 "query_sequence", "_qual", "_ref_end", "aux")
 
     def __init__(self, query_name, flag, reference_id, reference_start, mapping_quality, cigartuples,
-                 next_reference_id, next_reference_start, template_length, query_sequence, qual=None):
+                 next_reference_id, next_reference_start, template_length, query_sequence, qual=None, aux=b""):
         self.query_name = query_name
         self.flag = flag
         self.reference_id = reference_id
@@ -58,6 +58,7 @@ class AlignedSegment:
         self.query_sequence = query_sequence
         self._qual = qual
         self._ref_end = None
+        self.aux = aux          # the raw optional fields (tag, type, value ...) as stored in the record
 
     # flags -------------------------------------------------------------------------------------
     @property
@@ -72,6 +73,42 @@ class AlignedSegment:
     def is_secondary(self): return bool(self.flag & FSECONDARY)
     @property
     def is_qcfail(self): return bool(self.flag & FQCFAIL)
+
+    # optional fields -----------------------------------------------------------------------------
+    def integer_tag(self, tag):
+        """The value of the first field `tag` of an integer type (c C s S i I) in the raw aux bytes, None when there is
+        none (fields of the types A Z H B f are skipped).  Raises ValueError when the aux area cannot be parsed."""
+        a, data, want = 0, self.aux, tag.encode("latin-1")
+        sizes = {b"A": 1, b"c": 1, b"C": 1, b"s": 2, b"S": 2, b"i": 4, b"I": 4, b"f": 4}
+        ints = {b"c": "<b", b"C": "<B", b"s": "<h", b"S": "<H", b"i": "<i", b"I": "<I"}
+        while a < len(data):
+            if a + 3 > len(data):
+                raise ValueError("truncated aux field")
+            t = data[a + 2:a + 3]
+            hit = data[a:a + 2] == want
+            a += 3
+            if t in sizes:
+                if a + sizes[t] > len(data):
+                    raise ValueError("truncated aux field")
+                if hit and t in ints:
+                    return struct.unpack_from(ints[t], data, a)[0]
+                a += sizes[t]
+            elif t in (b"Z", b"H"):
+                end = data.find(b"\0", a)
+                if end < 0:
+                    raise ValueError("unterminated aux string")
+                a = end + 1
+            elif t == b"B":
+                if a + 5 > len(data):
+                    raise ValueError("truncated aux array")
+                sub = data[a:a + 1]
+                (n,) = struct.unpack_from("<I", data, a + 1)
+                if sub not in sizes or sub == b"A" or a + 5 + n * sizes[sub] > len(data):
+                    raise ValueError("bad aux array")
+                a += 5 + n * sizes[sub]
+            else:
+                raise ValueError("unknown aux type {!r}".format(t))
+        return None
 
     # geometry ----------------------------------------------------------------------------------
     @property
@@ -355,7 +392,7 @@ class AlignmentFile:
         seq = "".join(_NIB2[packed].tolist())[:l_seq] if l_seq else ""
         qual = data[off:off + l_seq]
         return AlignedSegment(name, flag, refID, pos, mapq, cigartuples, next_refID, next_pos, tlen,
-                              seq, qual)
+                              seq, qual, aux=bytes(data[off + l_seq:]))
 
     # iteration -----------------------------------------------------------------------------------
     def fetch(self, contig: Optional[str] = None, start: Optional[int] = None,
@@ -460,9 +497,10 @@ def _reg2bin(beg: int, end: int) -> int:
 
 
 def write_bam(path: str, references: List[Tuple[str, int]], records: List[AlignedSegment],
-              header_text: Optional[str] = None, level: int = 6, index: bool = True):
+              header_text: Optional[str] = None, level: int = 6, index: bool = True, aux: bool = False):
     """Write a coordinate-sorted BAM (records must already be in file order) and, by default, its
-    ``.bai`` index."""
+    ``.bai`` index.  aux: write each record's raw optional fields (``AlignedSegment.aux``); without it records are
+    written without any, as they always were."""
     w = BGZFWriter(path, level=level)
     bins = [dict() for _ in references]
     linear = [dict() for _ in references]
@@ -491,7 +529,7 @@ def write_bam(path: str, references: List[Tuple[str, int]], records: List[Aligne
                            r.mapping_quality, _reg2bin(max(r.reference_start, 0), max(rend, 1)),
                            len(r.cigartuples), r.flag, l_seq, r.next_reference_id,
                            r.next_reference_start, r.template_length)
-        body += nm + cig + packed + qual
+        body += nm + cig + packed + qual + ((r.aux or b"") if aux else b"")
         vbeg = w.tell()
         w.write(struct.pack("<i", len(body)) + body)
         vend = w.tell()

@@ -50,6 +50,8 @@ struct WalkCountTag; struct WalkFillTag; struct SelectTag; struct SummaryTag; st
 struct PairInsertTag; struct PairSecondTag; struct PairEvalTag; struct PairCountTag; struct PairScatterTag;
 // the scan of an unindexed BAM
 struct ScanCandidateTag; struct ScanRepairTag; struct ScanCountTag; struct ScanFillTag; struct ScanMatchTag; struct ScanKeepTag;
+// its STR profile (in-repeat reads)
+struct ScanIrrTag; struct ScanIrrFillTag;
 }
 using namespace tredsw_gi;
 
@@ -368,7 +370,12 @@ struct tredsw_ingest_batch {
     long long n_blocks = 0, n_records = 0;
     long long comp_bytes = 0, inflated_bytes = 0;
     int64_t scan_stats[TREDSW_SCAN_NSTATS] = {0};   // tredsw_ingest_scan_stats
+    bool irr_on = false;                            // the scan profiled in-repeat reads (tredsw_ingest_scan_irr)
+    std::vector<IrrEntry> irr_entries;
+    std::vector<char> irr_names;
+    tredsw_irr_view irr_view;
 };
+static_assert(sizeof(IrrEntry) == sizeof(tredsw_irr_entry), "IrrEntry mirrors tredsw_irr_entry");
 
 namespace {
 
@@ -998,9 +1005,12 @@ template <class B> void *grow(B &be, void *&p, size_t &cap, size_t bytes) {
 
 }  // namespace
 
+namespace { void irr_join(tredsw_ingest_batch *out, const unsigned long long *st); }
+
 template <class B>
 int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locus_query *queries, int32_t nq,
-             const int32_t *depth_regions, int32_t n_depth, double *depth_out, int64_t slab_bytes, uint32_t flags) {
+             const int32_t *depth_regions, int32_t n_depth, double *depth_out, int64_t slab_bytes, uint32_t flags,
+             const tredsw_irr_params *irr) {
     const double t_begin = now_ms();
     const bool want_names = (flags & TREDSW_INGEST_NO_NAMES) == 0;
     const int check_crc = (flags & TREDSW_INGEST_NO_CRC) == 0;
@@ -1080,7 +1090,13 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
     unsigned long long *d_depth = static_cast<unsigned long long *>(be.alloc(sizeof(unsigned long long) * (size_t)std::max(1, n_depth)));
     uint32_t *d_err = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * 2));
     int64_t *d_small = static_cast<int64_t *>(be.alloc(sizeof(int64_t) * 2));     // last record's order key; repair stop
+    // the STR profile: counters over the whole scan; per slab the IRR flags / name bytes, their scans, the entries
+    out->irr_on = irr != nullptr;
+    const IrrParams ip = irr ? IrrParams{irr->min_period, irr->max_period, irr->purity_num, irr->purity_den, irr->min_read_len}
+                             : IrrParams{0, 0, 0, 1, 0};
+    unsigned long long *d_irr_stats = irr ? static_cast<unsigned long long *>(be.alloc(sizeof(unsigned long long) * IRR_NSTATS)) : nullptr;
     if (be.rc) return be.rc;
+    if (irr) be.fill(d_irr_stats, 0, sizeof(unsigned long long) * IRR_NSTATS);
     be.upload(d_tid_x0, tid_x0.data(), sizeof(int32_t) * tid_x0.size());
     be.upload(d_xs, xs.data(), sizeof(int64_t) * xs.size());
     be.upload(d_seg_f0, seg_f0.data(), sizeof(int32_t) * seg_f0.size());
@@ -1114,6 +1130,8 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
     void *d_comp = nullptr, *d_blocks = nullptr, *d_bstatus = nullptr, *d_sblk = nullptr, *d_cand = nullptr, *d_land = nullptr;
     void *d_first = nullptr, *d_rcnt = nullptr, *d_rbase = nullptr, *d_recpos = nullptr, *d_nm = nullptr, *d_kb = nullptr;
     void *d_ebase = nullptr, *d_kbase = nullptr, *d_efetch = nullptr, *d_epos = nullptr, *d_kept = nullptr;
+    void *d_iflag = nullptr, *d_inb = nullptr, *d_ibase = nullptr, *d_inbase = nullptr, *d_ient = nullptr, *d_iname = nullptr;
+    size_t c_iflag = 0, c_inb = 0, c_ibase = 0, c_inbase = 0, c_ient = 0, c_iname = 0;
     size_t c_comp = 0, c_blocks = 0, c_bstatus = 0, c_sblk = 0, c_cand = 0, c_land = 0, c_first = 0, c_rcnt = 0, c_rbase = 0;
     size_t c_recpos = 0, c_nm = 0, c_kb = 0, c_ebase = 0, c_kbase = 0, c_efetch = 0, c_epos = 0, c_kept = 0;
     std::vector<int32_t> ent_fetch;         // (record, fetch) entries of the whole file, in file order
@@ -1239,6 +1257,27 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
         }
         be.scan(nm, nrec, ebase);
         be.scan(kb, nrec, kbase);
+        // the profile: classify every record (one thread each), IRR flags and name bytes -> their exclusive scans
+        uint32_t *iflag = nullptr, *inb = nullptr, *ibase = nullptr, *inbase = nullptr;
+        uint32_t h_itot[2] = {0, 0};
+        if (irr) {
+            iflag = static_cast<uint32_t *>(grow(be, d_iflag, c_iflag, sizeof(uint32_t) * (size_t)(nrec + 1)));
+            inb = static_cast<uint32_t *>(grow(be, d_inb, c_inb, sizeof(uint32_t) * (size_t)(nrec + 1)));
+            ibase = static_cast<uint32_t *>(grow(be, d_ibase, c_ibase, sizeof(uint32_t) * (size_t)(nrec + 2)));
+            inbase = static_cast<uint32_t *>(grow(be, d_inbase, c_inbase, sizeof(uint32_t) * (size_t)(nrec + 2)));
+            if (be.rc) return be.rc;
+            unsigned long long *ist = d_irr_stats;
+            be.template for_each<ScanIrrTag>(nrec, [=] __host__ __device__(int64_t i) {
+                uint64_t motif; RecFields r;
+                const int per = scan_irr_record(s, recpos[i], ip, ist, &motif, &r);
+                iflag[i] = per ? 1u : 0u;
+                inb[i] = per && r.l_name > 1 ? (uint32_t)(r.l_name - 1) : 0u;
+            });
+            be.scan(iflag, nrec, ibase);
+            be.scan(inb, nrec, inbase);
+            be.download(&h_itot[0], ibase + nrec, sizeof(uint32_t));
+            be.download(&h_itot[1], inbase + nrec, sizeof(uint32_t));
+        }
         uint32_t h_tot[2] = {0, 0}, h_err = 0;
         int64_t h_last = prev_key;
         be.download(&h_tot[0], ebase + nrec, sizeof(uint32_t));
@@ -1249,6 +1288,37 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
         if (be.rc) return be.rc;
         if (h_err & SCAN_ERR_RECORD) { status = 3; tredsw_set_error("%s: corrupt BAM record", bam->path.c_str()); break; }
         if (h_err & SCAN_ERR_ORDER) { status = 4; tredsw_set_error("%s is not sorted by coordinate", bam->path.c_str()); break; }
+        // the slab's IRR entries and names, appended to the host lists (IRRs are rare: the join by name is host work)
+        if (h_itot[0]) {
+            const int64_t nirr = h_itot[0], nnb = h_itot[1];
+            IrrEntry *ient = static_cast<IrrEntry *>(grow(be, d_ient, c_ient, sizeof(IrrEntry) * (size_t)nirr));
+            char *iname = static_cast<char *>(grow(be, d_iname, c_iname, (size_t)nnb + 1));
+            if (be.rc) return be.rc;
+            unsigned long long *ist = d_irr_stats;
+            be.template for_each<ScanIrrFillTag>(nrec, [=] __host__ __device__(int64_t i) {
+                if (!iflag[i]) return;
+                const int64_t p = recpos[i];
+                const RecFields r = parse_record(s, p);
+                IrrEntry e;
+                e.period = irr_classify(PackedSeq{s + record_seq(p, r)}, r.l_seq, ip, &e.motif);
+                bool unparsed;
+                e.mq = aux_mq(s, record_aux(p, r), p + 4 + (int64_t)ld_i32(s, p), &unparsed);
+                if (unparsed) atomic_add_u64(&ist[IRR_UNPARSED_AUX], 1ull);
+                e.tid = r.tid; e.pos = r.pos; e.next_tid = r.next_tid; e.next_pos = r.next_pos;
+                e.flag = r.flag; e.mapq = s[p + 13];
+                e.name_off = inbase[i]; e.name_len = (int32_t)inb[i]; e.mate = -1;
+                ient[ibase[i]] = e;
+                for (uint32_t k = 0; k < inb[i]; ++k) iname[inbase[i] + k] = (char)s[p + 36 + k];
+            });
+            const size_t e0 = out->irr_entries.size(), n0 = out->irr_names.size();
+            out->irr_entries.resize(e0 + (size_t)nirr);
+            out->irr_names.resize(n0 + (size_t)nnb);
+            be.download(out->irr_entries.data() + e0, ient, sizeof(IrrEntry) * (size_t)nirr);
+            be.download(out->irr_names.data() + n0, iname, (size_t)nnb);
+            be.sync();
+            if (be.rc) return be.rc;
+            for (size_t k = e0; k < out->irr_entries.size(); ++k) out->irr_entries[k].name_off += (int64_t)n0;
+        }
         // copy the kept records once into the kept-record stream; one (fetch, position) entry per (record, fetch)
         const int64_t nent = h_tot[0], kbytes = h_tot[1];
         if (nent) {
@@ -1294,6 +1364,14 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
     if (reader.joinable()) reader.join();
     if (!status && carry_len > 0) { status = 3; tredsw_set_error("%s ends inside a BAM record", bam->path.c_str()); }
     stats[9] = status;
+    if (irr) {
+        unsigned long long h_ist[IRR_NSTATS];
+        be.download(h_ist, d_irr_stats, sizeof(h_ist));
+        be.sync();
+        if (be.rc) return be.rc;
+        if (status) { out->irr_entries.clear(); out->irr_names.clear(); memset(h_ist, 0, sizeof(h_ist)); }
+        irr_join(out, h_ist);
+    }
 
     // ---- (3) depth regions; the entries grouped by fetch (stable counting sort: file order within a fetch) ----------
     std::vector<unsigned long long> h_depth((size_t)std::max(1, n_depth));
@@ -1351,6 +1429,46 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
 }
 
 namespace {
+// The mates among the IRR entries: the records of one name with segment flags 0x40 and 0x80 (the first of each, in
+// file order), and the profile's counters.  An anchored IRR without an MQ tag (paired, mate mapped and not an IRR)
+// is counted in anchors_without_mq.
+void irr_join(tredsw_ingest_batch *out, const unsigned long long *st) {
+    std::vector<IrrEntry> &e = out->irr_entries;
+    const char *names = out->irr_names.data();
+    std::unordered_map<std::string, std::pair<int32_t, int32_t>> seg;     // name -> (first 0x40 entry, first 0x80 entry)
+    seg.reserve(e.size());
+    for (size_t k = 0; k < e.size(); ++k) {
+        const int f = e[k].flag & 0xc0;
+        if (f != 0x40 && f != 0x80) continue;
+        auto it = seg.emplace(std::string(names + e[k].name_off, (size_t)e[k].name_len), std::make_pair(-1, -1)).first;
+        int32_t &slot = f == 0x40 ? it->second.first : it->second.second;
+        if (slot < 0) slot = (int32_t)k;
+    }
+    for (auto &kv : seg)
+        if (kv.second.first >= 0 && kv.second.second >= 0) { e[kv.second.first].mate = kv.second.second; e[kv.second.second].mate = kv.second.first; }
+    tredsw_irr_view &v = out->irr_view;
+    memset(&v, 0, sizeof(v));
+    v.n_entries = (int64_t)e.size();
+    v.entries = reinterpret_cast<const tredsw_irr_entry *>(e.data());
+    v.names = names; v.name_bytes = (int64_t)out->irr_names.size();
+    v.records_considered = (int64_t)st[IRR_CONSIDERED]; v.irr_records = (int64_t)e.size();
+    v.depth_bases = (int64_t)st[IRR_DEPTH_BASES]; v.max_l_seq = (int64_t)st[IRR_MAX_LSEQ];
+    v.unparsed_aux = (int64_t)st[IRR_UNPARSED_AUX];
+    for (const IrrEntry &x : e)
+        v.anchors_without_mq += (x.flag & 1) && !(x.flag & 8) && x.next_tid >= 0 && x.mate < 0 && x.mq < 0;
+}
+
+bool irr_params_ok(const tredsw_irr_params *p) {
+    if (!p) return true;
+    if (p->min_period < 2 || p->min_period > p->max_period || p->max_period > 20 || p->purity_num <= 0 ||
+        p->purity_num > p->purity_den || p->purity_den > 1000 || p->min_read_len < 2 * p->max_period) {
+        tredsw_set_error("IRR parameters out of range (2 <= min_period <= max_period <= 20, 0 < num <= den <= 1000, "
+                         "min_read_len >= 2 max_period)");
+        return false;
+    }
+    return true;
+}
+
 // (once per device) keep freed blocks in the stream-ordered pool: the buffers of consecutive batches have similar sizes
 void keep_pool(int device) {
     static bool pool_set[64] = {false};
@@ -1370,8 +1488,15 @@ extern "C" {
 int tredsw_ingest_scan_run(tredsw_ctx *ctx, tredsw_bam *bam, const tredsw_locus_query *queries, int32_t nqueries,
                            const int32_t *depth_regions, int32_t n_depth, double *depth_out, int64_t slab_bytes,
                            uint32_t flags, tredsw_ingest_batch **out) {
+    return tredsw_ingest_scan_run_ex(ctx, bam, queries, nqueries, depth_regions, n_depth, depth_out, slab_bytes, flags, nullptr, out);
+}
+
+int tredsw_ingest_scan_run_ex(tredsw_ctx *ctx, tredsw_bam *bam, const tredsw_locus_query *queries, int32_t nqueries,
+                              const int32_t *depth_regions, int32_t n_depth, double *depth_out, int64_t slab_bytes,
+                              uint32_t flags, const tredsw_irr_params *irr, tredsw_ingest_batch **out) {
     if (!ctx || !bam || !out || nqueries < 0 || (nqueries > 0 && !queries) || n_depth < 0 ||
         (n_depth > 0 && (!depth_regions || !depth_out)) || slab_bytes < 0) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
+    if (!irr_params_ok(irr)) return TREDSW_ERR_ARG;
     *out = nullptr;
     if (bam->consumed) { tredsw_set_error("%s: stream already consumed", bam->path.c_str()); return TREDSW_ERR_ARG; }
     std::lock_guard<std::mutex> lock(ctx->mu);
@@ -1380,7 +1505,7 @@ int tredsw_ingest_scan_run(tredsw_ctx *ctx, tredsw_bam *bam, const tredsw_locus_
     std::unique_ptr<tredsw_ingest_batch> b(new tredsw_ingest_batch());
     b->cuda.stream = ctx->stream;
     int rc;
-    try { rc = run_scan(b->cuda, b.get(), bam, queries, nqueries, depth_regions, n_depth, depth_out, slab_bytes, flags); }
+    try { rc = run_scan(b->cuda, b.get(), bam, queries, nqueries, depth_regions, n_depth, depth_out, slab_bytes, flags, irr); }
     catch (const std::exception &e) { tredsw_set_error("tredsw_ingest_scan_run: %s", e.what()); rc = TREDSW_ERR_IO; }
     ctx->launches += b->cuda.launches;
     if (rc) { b->cuda.release(); return rc; }
@@ -1392,17 +1517,40 @@ int tredsw_ingest_scan_run(tredsw_ctx *ctx, tredsw_bam *bam, const tredsw_locus_
 int tredsw_ingest_scan_emulate(tredsw_bam *bam, const tredsw_locus_query *queries, int32_t nqueries,
                                const int32_t *depth_regions, int32_t n_depth, double *depth_out, int64_t slab_bytes,
                                uint32_t flags, tredsw_ingest_batch **out) {
+    return tredsw_ingest_scan_emulate_ex(bam, queries, nqueries, depth_regions, n_depth, depth_out, slab_bytes, flags, nullptr, out);
+}
+
+int tredsw_ingest_scan_emulate_ex(tredsw_bam *bam, const tredsw_locus_query *queries, int32_t nqueries,
+                                  const int32_t *depth_regions, int32_t n_depth, double *depth_out, int64_t slab_bytes,
+                                  uint32_t flags, const tredsw_irr_params *irr, tredsw_ingest_batch **out) {
     if (!bam || !out || nqueries < 0 || (nqueries > 0 && !queries) || n_depth < 0 ||
         (n_depth > 0 && (!depth_regions || !depth_out)) || slab_bytes < 0) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
+    if (!irr_params_ok(irr)) return TREDSW_ERR_ARG;
     *out = nullptr;
     if (bam->consumed) { tredsw_set_error("%s: stream already consumed", bam->path.c_str()); return TREDSW_ERR_ARG; }
     std::unique_ptr<tredsw_ingest_batch> b(new tredsw_ingest_batch());
     b->emulated = true;
     int rc;
-    try { rc = run_scan(b->host, b.get(), bam, queries, nqueries, depth_regions, n_depth, depth_out, slab_bytes, flags); }
+    try { rc = run_scan(b->host, b.get(), bam, queries, nqueries, depth_regions, n_depth, depth_out, slab_bytes, flags, irr); }
     catch (const std::exception &e) { tredsw_set_error("tredsw_ingest_scan_emulate: %s", e.what()); rc = TREDSW_ERR_IO; }
     if (rc) { b->host.release(); return rc; }
     *out = b.release();
+    return TREDSW_OK;
+}
+
+int tredsw_ingest_scan_irr(const tredsw_ingest_batch *b, tredsw_irr_view *v) {
+    if (!b || !v) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
+    if (!b->irr_on) { tredsw_set_error("the scan did not profile in-repeat reads (tredsw_ingest_scan_run_ex with irr)"); return TREDSW_ERR_ARG; }
+    *v = b->irr_view;
+    return TREDSW_OK;
+}
+
+// The IRR classifier on its own (test hook, host execution of the device code)
+int tredsw_irr_classify_host(const int8_t *codes, int32_t len, const tredsw_irr_params *p, int32_t *period, uint64_t *motif) {
+    if (!p || !period || !motif || len < 0 || (len > 0 && !codes)) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
+    if (!irr_params_ok(p)) return TREDSW_ERR_ARG;
+    const IrrParams ip{p->min_period, p->max_period, p->purity_num, p->purity_den, p->min_read_len};
+    *period = irr_classify(CodeSeq{codes}, len, ip, motif);
     return TREDSW_OK;
 }
 

@@ -189,6 +189,17 @@ int tredsw_inflate_raw(const uint8_t *in, int64_t in_len, uint8_t *out, int64_t 
 
 int32_t tredsw_bam_nref(tredsw_bam *b) { return b ? (int32_t)b->names.size() : 0; }
 
+int64_t tredsw_bam_ref(tredsw_bam *b, int32_t tid, char *name, int64_t cap) {
+    if (!b || tid < 0 || tid >= (int32_t)b->names.size()) return -1;
+    const std::string &n = b->names[tid];
+    if (name && cap > 0) {
+        const size_t k = std::min<size_t>(n.size(), (size_t)cap - 1);
+        memcpy(name, n.data(), k);
+        name[k] = 0;
+    }
+    return b->lengths[tid];
+}
+
 int32_t tredsw_bam_tid(tredsw_bam *b, const char *name) {
     if (!b || !name) return -1;
     auto it = b->tid_of.find(name);

@@ -822,4 +822,195 @@ TG_HD uint32_t scan_record(const uint8_t *s, const int64_t *rec_pos, int64_t i, 
     return n;
 }
 
+// ---- in-repeat reads: the STR profile of a scan (tredsw_ingest_scan_run_ex, DESIGN §4.5) ---------------------------
+// A read is an in-repeat read (IRR) when, for some period k in [min_period, max_period], the bases k apart agree (N
+// never agrees) on at least num / den of its L - k comparisons; the smallest such k is its period.  Its motif is the
+// per-phase majority base, reduced to its primitive root (a root of one base is a homopolymer: not an IRR), in the
+// canonical form: the smallest rotation of the root and of its reverse complement, 2 bits a base, first base in the
+// most significant bits.  All integer arithmetic: the kernel, the host hook and the Python oracle agree bit for bit.
+struct IrrParams { int32_t min_period, max_period, num, den, min_read_len; };
+struct IrrEntry {               // one IRR record (tredsw_irr_entry)
+    int32_t tid, pos, next_tid, next_pos;
+    int32_t flag, mapq, mq, period;     // mq: the MQ:i tag, -1 without one
+    uint64_t motif;
+    int64_t name_off;
+    int32_t name_len, mate;             // mate: filled by the host join (index of the mate's entry, -1 none)
+};
+enum : int { IRR_CONSIDERED = 0, IRR_DEPTH_BASES = 1, IRR_MAX_LSEQ = 2, IRR_UNPARSED_AUX = 3, IRR_NSTATS = 4 };
+constexpr uint32_t IRR_SKIP_FLAGS = 0x100u | 0x200u | 0x400u | 0x800u;      // secondary, QC fail, duplicate, supplementary
+
+struct PackedSeq {              // base i of a record's 4-bit sequence as a code 0..4 (A C G T, anything else N)
+    const uint8_t *p;
+    TG_HD int operator()(int i) const { return nib_code((p[i >> 1] >> ((i & 1) ? 0 : 4)) & 15u); }
+};
+struct CodeSeq {                // a sequence of codes (the host test hook)
+    const int8_t *p;
+    TG_HD int operator()(int i) const { const int c = p[i]; return (c >= 0 && c < 4) ? c : 4; }
+};
+
+TG_HD int popc64(uint64_t x) {
+#if defined(__CUDA_ARCH__)
+    return __popcll(x);
+#else
+    return __builtin_popcountll(x);
+#endif
+}
+
+// -> the period of the IRR (0: not one); *motif its canonical motif
+template <class Seq>
+TG_HD int irr_classify(const Seq &sq, int L, const IrrParams &pr, uint64_t *motif) {
+    *motif = 0;
+    if (L < pr.min_read_len) return 0;                  // (min_read_len >= 2 max_period: L - k >= k for every k)
+    // Prefilter: the first W <= 64 bases as 2-bit codes (base i at bits 2i) and their N flags (bit 2i).  The
+    // disagreements of period k among the first W - k comparisons are counted at once (shift, xor, popcount); they are
+    // a subset of the read's, so more than the allowance rejects k exactly.  Most reads are rejected here at every k
+    // from one pass over 32 bytes instead of per-period walks over the sequence.
+    const int W = L < 64 ? L : 64;
+    unsigned __int128 codes = 0, nflag = 0;
+    for (int i = 0; i < W; ++i) {
+        const int a = sq(i);
+        if (a == 4) nflag |= (unsigned __int128)1 << (2 * i);
+        else codes |= (unsigned __int128)a << (2 * i);
+    }
+    const unsigned __int128 low = ((unsigned __int128)0x5555555555555555ull << 64) | 0x5555555555555555ull;
+    int P = 0;
+    for (int k = pr.min_period; k <= pr.max_period; ++k) {
+        const int n = L - k;
+        const int64_t need = ((int64_t)pr.num * n + pr.den - 1) / pr.den;    // ceil(num n / den) agreements
+        const int64_t allow = n - need;                  // disagreements a passing read can have: exact early exit
+        {
+            const unsigned __int128 d = codes ^ (codes >> (2 * k));
+            const unsigned __int128 window = ((unsigned __int128)1 << (2 * (W - k))) - 1;      // comparisons i < W - k
+            const unsigned __int128 mis = (d | (d >> 1) | nflag | (nflag >> (2 * k))) & low & window;
+            if (popc64((uint64_t)mis) + popc64((uint64_t)(mis >> 64)) > allow) continue;
+        }
+        int64_t miss = 0;
+        int i = 0;
+        for (; i < n; ++i) {
+            const int a = sq(i);
+            if ((a == 4 || a != sq(i + k)) && ++miss > allow) break;
+        }
+        if (i == n) { P = k; break; }
+    }
+    if (!P) return 0;
+    uint64_t cons = 0;                                  // phase j's majority base at bits 2j
+    for (int j = 0; j < P; ++j) {
+        int c0 = 0, c1 = 0, c2 = 0, c3 = 0;
+        for (int i = j; i < L; i += P) {
+            const int a = sq(i);
+            c0 += a == 0; c1 += a == 1; c2 += a == 2; c3 += a == 3;
+        }
+        int best = 0, bc = c0;                          // ties: the smallest code; all N: A
+        if (c1 > bc) { best = 1; bc = c1; }
+        if (c2 > bc) { best = 2; bc = c2; }
+        if (c3 > bc) { best = 3; }
+        cons |= (uint64_t)best << (2 * j);
+    }
+    int d = P;                                          // primitive root: the smallest period that divides P
+    for (int e = 1; e < P; ++e) {
+        if (P % e) continue;
+        bool rep = true;
+        for (int i = e; i < P && rep; ++i) rep = ((cons >> (2 * i)) & 3u) == ((cons >> (2 * (i - e))) & 3u);
+        if (rep) { d = e; break; }
+    }
+    if (d == 1) return 0;                               // homopolymer
+    uint64_t f = 0, r = 0;
+    for (int i = 0; i < d; ++i) f = (f << 2) | ((cons >> (2 * i)) & 3u);
+    for (int i = d - 1; i >= 0; --i) r = (r << 2) | (3u - ((cons >> (2 * i)) & 3u));
+    const uint64_t mask = (1ull << (2 * d)) - 1ull;
+    uint64_t best = f < r ? f : r;
+    for (int t = 1; t < d; ++t) {                       // the other rotations, one base to the left at a time
+        f = ((f << 2) | (f >> (2 * d - 2))) & mask;
+        r = ((r << 2) | (r >> (2 * d - 2))) & mask;
+        if (f < best) best = f;
+        if (r < best) best = r;
+    }
+    *motif = best;
+    return d;
+}
+
+// The MQ tag of the aux area [a, end): its value (negative values read as 0), -1 when there is none.  Only the integer
+// types c C s S i I count; A Z H B f fields are skipped.  An area the walk cannot parse (a field running past the end,
+// an unknown type) is "no MQ" and sets *unparsed.
+TG_HD int32_t aux_mq(const uint8_t *s, int64_t a, int64_t end, bool *unparsed) {
+    *unparsed = false;
+    while (a < end) {
+        if (a + 3 > end) { *unparsed = true; return -1; }
+        const bool mq = s[a] == 'M' && s[a + 1] == 'Q';
+        const uint8_t t = s[a + 2];
+        a += 3;
+        int size = 0;
+        if (t == 'A' || t == 'c' || t == 'C') size = 1;
+        else if (t == 's' || t == 'S') size = 2;
+        else if (t == 'i' || t == 'I' || t == 'f') size = 4;
+        if (size) {
+            if (a + size > end) { *unparsed = true; return -1; }
+            if (mq && t != 'A' && t != 'f') {
+                int64_t v;
+                if (t == 'c') v = (int8_t)s[a];
+                else if (t == 'C') v = s[a];
+                else if (t == 's') v = (int16_t)ld_u16(s, a);
+                else if (t == 'S') v = ld_u16(s, a);
+                else if (t == 'i') v = ld_i32(s, a);
+                else v = ld_u32(s, a);
+                return v < 0 ? 0 : v > 0x7fffffff ? 0x7fffffff : (int32_t)v;
+            }
+            a += size;
+        } else if (t == 'Z' || t == 'H') {
+            while (a < end && s[a] != 0) ++a;
+            if (a >= end) { *unparsed = true; return -1; }
+            ++a;
+        } else if (t == 'B') {
+            if (a + 5 > end) { *unparsed = true; return -1; }
+            const uint8_t st = s[a];
+            const int es = (st == 'c' || st == 'C') ? 1 : (st == 's' || st == 'S') ? 2 : (st == 'i' || st == 'I' || st == 'f') ? 4 : 0;
+            const int64_t cnt = ld_u32(s, a + 1);
+            if (!es || a + 5 + cnt * es > end) { *unparsed = true; return -1; }
+            a += 5 + cnt * es;
+        } else {
+            *unparsed = true; return -1;
+        }
+    }
+    return -1;
+}
+
+// where a record's sequence and aux area lie (it passed parse_record)
+TG_HD int64_t record_seq(int64_t p, const RecFields &r) { return p + 36 + r.l_name + 4 * (int64_t)r.n_cigar; }
+TG_HD int64_t record_aux(int64_t p, const RecFields &r) { return record_seq(p, r) + ((int64_t)r.l_seq + 1) / 2 + r.l_seq; }
+
+// sum / max over the lanes that call it together, one atomic per warp (every record of a slab adds its depth bases)
+TG_HD void warp_add_u64(unsigned long long *p, uint32_t v) {
+#if defined(__CUDA_ARCH__)
+    const unsigned m = __activemask();
+    const uint32_t t = __reduce_add_sync(m, v);
+    if ((threadIdx.x & 31u) == (unsigned)(__ffs(m) - 1) && t) atomicAdd(p, (unsigned long long)t);
+#else
+    *p += v;
+#endif
+}
+TG_HD void warp_max_u64(unsigned long long *p, uint32_t v) {
+#if defined(__CUDA_ARCH__)
+    const unsigned m = __activemask();
+    const uint32_t t = __reduce_max_sync(m, v);
+    if ((threadIdx.x & 31u) == (unsigned)(__ffs(m) - 1) && t) atomicMax(p, (unsigned long long)t);
+#else
+    if (v > *p) *p = v;
+#endif
+}
+
+// per record of a scan: the profile's counters; -> its IRR period (0: not an IRR) and motif
+TG_HD int scan_irr_record(const uint8_t *s, int64_t p, const IrrParams &pr, unsigned long long *stats, uint64_t *motif,
+                          RecFields *fields) {
+    const RecFields r = parse_record(s, p);
+    *fields = r;
+    const bool primary = r.ok && !(r.flag & IRR_SKIP_FLAGS);
+    const bool considered = primary && r.l_seq >= pr.min_read_len;
+    warp_add_u64(&stats[IRR_CONSIDERED], considered ? 1u : 0u);
+    warp_add_u64(&stats[IRR_DEPTH_BASES], primary && !(r.flag & 4) ? (uint32_t)r.l_seq : 0u);
+    warp_max_u64(&stats[IRR_MAX_LSEQ], primary ? (uint32_t)r.l_seq : 0u);
+    *motif = 0;
+    if (!considered) return 0;
+    return irr_classify(PackedSeq{s + record_seq(p, r)}, r.l_seq, pr, motif);
+}
+
 }  // namespace tredsw_gi

@@ -60,6 +60,8 @@ def _bind(lib):
     lib.tredsw_bam_close.argtypes = [ctypes.c_void_p]
     lib.tredsw_bam_nref.restype = ctypes.c_int32
     lib.tredsw_bam_nref.argtypes = [ctypes.c_void_p]
+    lib.tredsw_bam_ref.restype = ctypes.c_int64
+    lib.tredsw_bam_ref.argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.c_char_p, ctypes.c_int64]
     lib.tredsw_bam_tid.restype = ctypes.c_int32
     lib.tredsw_bam_tid.argtypes = [ctypes.c_void_p, ctypes.c_char_p]
     lib.tredsw_bam_header_signature.restype = ctypes.c_uint64
@@ -145,6 +147,14 @@ class BamIngest:
             raise IOError("{}({}): {}".format(opener, path, _lib.last_error()))
         self._caps = dict(reads=512, bases=512 * 256, pairs=8192, names=512 * 48)
         return self
+
+    def references(self):
+        """[(contig, length)] of the binary reference dictionary, in tid order (the @SQ text of the header may be absent)"""
+        out, buf = [], ctypes.create_string_buffer(8192)                # (the header reader takes names up to 4 KiB)
+        for t in range(int(self.lib.tredsw_bam_nref(self.handle))):
+            n = int(self.lib.tredsw_bam_ref(self.handle, t, buf, len(buf)))
+            out.append((buf.value.decode("latin-1"), n))
+        return out
 
     def header_text(self):
         """the SAM header text (@HD, @SQ, @RG, ... lines)"""
@@ -318,6 +328,41 @@ class IngestView(ctypes.Structure):
                 ("ms_marks", ctypes.c_double * 4)]
 
 
+class IrrParams(ctypes.Structure):
+    """tredsw_irr_params (include/tredsw.h): what makes a read an in-repeat read (IRR)"""
+    _fields_ = [(n, ctypes.c_int32) for n in ("min_period", "max_period", "purity_num", "purity_den", "min_read_len")]
+
+    def __init__(self, min_period=2, max_period=20, purity_num=9, purity_den=10, min_read_len=50):
+        super().__init__(min_period, max_period, purity_num, purity_den, min_read_len)
+
+    def as_dict(self):
+        return {n: int(getattr(self, n)) for n, _ in self._fields_}
+
+
+IRR_STATS = ("records_considered", "irr_records", "depth_bases", "max_l_seq", "anchors_without_mq", "unparsed_aux")
+
+
+class IrrView(ctypes.Structure):
+    """tredsw_irr_view (include/tredsw.h)"""
+    _fields_ = [("n_entries", ctypes.c_int64), ("entries", ctypes.c_void_p), ("names", ctypes.c_void_p),
+                ("name_bytes", ctypes.c_int64)] + [(n, ctypes.c_int64) for n in IRR_STATS]
+IRR_ENTRY_DTYPE = np.dtype([("tid", "<i4"), ("pos", "<i4"), ("next_tid", "<i4"), ("next_pos", "<i4"), ("flag", "<i4"),
+                            ("mapq", "<i4"), ("mq", "<i4"), ("period", "<i4"), ("motif", "<u8"), ("name_off", "<i8"),
+                            ("name_len", "<i4"), ("mate", "<i4")])
+
+
+def irr_classify_host(codes, params=None):
+    """The IRR classifier body run on the host (test hook): codes 0..3 = A C G T, anything else N -> (period, motif);
+    period 0: not an IRR."""
+    lib = _lib.load()
+    _bind_batch(lib)
+    a = np.ascontiguousarray(np.asarray(codes, dtype=np.int8))
+    per, mot = ctypes.c_int32(), ctypes.c_uint64()
+    _lib.check(lib.tredsw_irr_classify_host(a.ctypes.data if len(a) else None, len(a), ctypes.byref(params or IrrParams()),
+                                            ctypes.byref(per), ctypes.byref(mot)), "tredsw_irr_classify_host")
+    return int(per.value), int(mot.value)
+
+
 def _bind_batch(lib):
     if getattr(lib, "_ingest_batch_bound", False):
         return
@@ -341,6 +386,16 @@ def _bind_batch(lib):
     lib.tredsw_ingest_scan_stats.argtypes = [ctypes.c_void_p, ctypes.c_void_p]
     lib.tredsw_inflate_raw_device_code.restype = ctypes.c_int
     lib.tredsw_inflate_raw_device_code.argtypes = [ctypes.c_char_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_int64]
+    lib.tredsw_ingest_scan_run_ex.restype = ctypes.c_int
+    lib.tredsw_ingest_scan_run_ex.argtypes = (lib.tredsw_ingest_scan_run.argtypes[:-1] + [ctypes.POINTER(IrrParams)]
+                                              + lib.tredsw_ingest_scan_run.argtypes[-1:])
+    lib.tredsw_ingest_scan_emulate_ex.restype = ctypes.c_int
+    lib.tredsw_ingest_scan_emulate_ex.argtypes = lib.tredsw_ingest_scan_run_ex.argtypes[1:]
+    lib.tredsw_ingest_scan_irr.restype = ctypes.c_int
+    lib.tredsw_ingest_scan_irr.argtypes = [ctypes.c_void_p, ctypes.POINTER(IrrView)]
+    lib.tredsw_irr_classify_host.restype = ctypes.c_int
+    lib.tredsw_irr_classify_host.argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.POINTER(IrrParams),
+                                             ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_uint64)]
     lib._ingest_batch_bound = True
 
 
@@ -470,7 +525,8 @@ class ScanBatch(IngestBatch):
     ``IngestBatch`` (``.status``, ``.evidence(i)``, the device buffers), plus ``.depths`` (the depth of every
     requested region) and the scan's statistics.  Build it with ``scan_sample``."""
 
-    def __init__(self, ctx, handle, queries, keep=(), depth_regions=(), slab_bytes=None, want_names=True, check_crc=True):
+    def __init__(self, ctx, handle, queries, keep=(), depth_regions=(), slab_bytes=None, want_names=True, check_crc=True,
+                 irr=None):
         self.lib = _lib.load()
         _bind(self.lib)
         _bind_batch(self.lib)
@@ -482,13 +538,19 @@ class ScanBatch(IngestBatch):
         flags = (0 if want_names else INGEST_NO_NAMES) | (0 if check_crc else INGEST_NO_CRC)
         out = ctypes.c_void_p()
         args = (handle.handle, qs, n, dr.ctypes.data if len(dr) else None, len(dr), depths.ctypes.data,
-                int(slab_bytes or 0), flags, ctypes.byref(out))
-        if ctx is None:
-            rc = self.lib.tredsw_ingest_scan_emulate(*args)
+                int(slab_bytes or 0), flags)
+        if irr is None:
+            if ctx is None:
+                rc = self.lib.tredsw_ingest_scan_emulate(*args, ctypes.byref(out))
+            else:
+                rc = self.lib.tredsw_ingest_scan_run(ctx.handle, *args, ctypes.byref(out))
+        elif ctx is None:
+            rc = self.lib.tredsw_ingest_scan_emulate_ex(*args, ctypes.byref(irr), ctypes.byref(out))
         else:
-            rc = self.lib.tredsw_ingest_scan_run(ctx.handle, *args)
+            rc = self.lib.tredsw_ingest_scan_run_ex(ctx.handle, *args, ctypes.byref(irr), ctypes.byref(out))
         _lib.check(rc, "tredsw_ingest_scan_run")
         self._attach(out, n, want_names)
+        self.irr = self._irr() if irr is not None else None
         self.depths = depths[:len(dr)]
         st = np.zeros(SCAN_NSTATS, dtype=np.int64)
         _lib.check(self.lib.tredsw_ingest_scan_stats(self.handle, st.ctypes.data), "tredsw_ingest_scan_stats")
@@ -500,11 +562,24 @@ class ScanBatch(IngestBatch):
     def stats(self):
         return dict(self._scan)
 
+    def _irr(self):
+        """the STR profile's records: dict(entries = numpy array of IRR_ENTRY_DTYPE in file order, names = their query
+        names, stats = the counters of tredsw_irr_view)"""
+        v = IrrView()
+        _lib.check(self.lib.tredsw_ingest_scan_irr(self.handle, ctypes.byref(v)), "tredsw_ingest_scan_irr")
+        n = int(v.n_entries)
+        raw = ctypes.string_at(v.entries, n * IRR_ENTRY_DTYPE.itemsize) if n else b""
+        ent = np.frombuffer(raw, dtype=IRR_ENTRY_DTYPE).copy()
+        text = ctypes.string_at(v.names, int(v.name_bytes)) if v.name_bytes else b""
+        names = [text[o:o + k].decode("latin-1") for o, k in zip(ent["name_off"].tolist(), ent["name_len"].tolist())]
+        return {"entries": ent, "names": names, "stats": {k: int(getattr(v, k)) for k in IRR_STATS}}
 
-def scan_sample(ctx, handle, queries, keep, depth_regions, slab_bytes=None):
+
+def scan_sample(ctx, handle, queries, keep, depth_regions, slab_bytes=None, irr=None):
     """Every locus of one sample (``queries``: ``LocusQuery`` records, alt regions included) and the depth of
     ``depth_regions`` ((tid, start, end) rows) in one streaming pass over a BAM opened with ``BamIngest.unindexed`` or
     ``BamIngest.stream`` (a stream can be scanned once).
-    ``slab_bytes``: compressed bytes read per step (None: 128 MiB).  ``ctx=None`` runs the serial host emulation of
-    the device code — test infrastructure only.  -> ScanBatch"""
-    return ScanBatch(ctx, handle, queries, keep=keep, depth_regions=depth_regions, slab_bytes=slab_bytes)
+    ``slab_bytes``: compressed bytes read per step (None: 128 MiB).  ``irr``: an ``IrrParams`` to find the in-repeat
+    reads of the whole file in the same pass (``ScanBatch.irr``; ``strprofile`` builds the STR profile from them).
+    ``ctx=None`` runs the serial host emulation of the device code — test infrastructure only.  -> ScanBatch"""
+    return ScanBatch(ctx, handle, queries, keep=keep, depth_regions=depth_regions, slab_bytes=slab_bytes, irr=irr)

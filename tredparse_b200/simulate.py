@@ -268,3 +268,81 @@ def write_sample_bam(path, repo, names, references, sample, readlen=150, seed=20
     recs.sort(key=lambda r: (r.reference_id, r.reference_start))
     write_bam(path, references, recs, level=1)
     return truth
+
+
+# ---------------------------------------------------------------------------------------------------------
+# planted expansions anywhere: the in-repeat reads of the STR profile (strprofile)
+# ---------------------------------------------------------------------------------------------------------
+def _mq_aux(mq):
+    """the raw aux bytes of an MQ:i tag (stored as type C, as aligners write small values)"""
+    return b"MQC" + bytes([mq])
+
+
+def expansion_records(tid, pos, motif, units, readlen=150, cov=15.0, flank=2000, error=0.005, seed=0, tag="x",
+                      mq_tags=True, mismap_fraction=0.0, mismap_to=None):
+    """Paired reads of a haplotype with `units` copies of `motif` inserted at 0-based reference position `pos` of contig
+    `tid` (random flanks of `flank` bases on either side, mapped one to one onto [pos - flank, pos + flank)), placed as
+    an aligner places reads around an expansion longer than a read:
+      * pairs with no read inside the repeat: proper pairs, MAPQ 60, ``<readlen>M``;
+      * a read wholly inside the repeat (an in-repeat read) whose mate is not: unmapped, placed at its mate's position
+        (tid / pos / next = the mate's), its mate flagged 0x8; with probability `mismap_fraction` it is instead mismapped
+        at MAPQ 0 at a random position of ``mismap_to = (tid, start, end)``, its mate pointing there;
+      * both reads inside the repeat: both unmapped, in the unmapped tail (tid -1).
+    The in-repeat read carries its mate's MAPQ as an ``MQ`` tag (mapped mates carry one too) unless ``mq_tags`` is
+    False.  Records are bamio.AlignedSegment, not sorted (``coordinate_sort``); write them with
+    ``bamio.write_bam(..., aux=True)`` to keep the MQ tags."""
+    from .bamio import AlignedSegment
+    rng = np.random.default_rng(seed)
+    m = encode(motif)
+    rep = np.tile(m, units).astype(np.int8)
+    hap = np.concatenate([rng.integers(0, 4, flank).astype(np.int8), rep, rng.integers(0, 4, flank).astype(np.int8)])
+    rep_start, rep_end, L = flank, flank + len(rep), len(hap)
+    lut = np.array(list("ACGTN"))
+    nfrag = int(round(cov * L / (2.0 * readlen)))
+    frag = _fragment_lengths(rng, nfrag)
+    frag = frag[frag >= readlen]
+    start = rng.integers(0, L - frag + 1)
+
+    def to_ref(x):
+        return pos - (rep_start - x) if x < rep_start else (pos if x < rep_end else pos + (x - rep_end))
+    aux = (lambda q: _mq_aux(q)) if mq_tags else (lambda q: b"")
+    recs = []
+    for k in range(len(frag)):
+        s1, s2 = int(start[k]), int(start[k] + frag[k] - readlen)
+        seqs = []
+        for s_ in (s1, s2):
+            r = hap[s_:s_ + readlen].copy()
+            err = rng.random(readlen) < error
+            r[err] = rng.integers(0, 4, int(err.sum()))
+            seqs.append("".join(lut[r]))
+        irr = [s_ >= rep_start and s_ + readlen <= rep_end for s_ in (s1, s2)]
+        p = [to_ref(s1), to_ref(s2)]
+        seg, strand = (0x40, 0x80), (0x20, 0x10)
+        name = "{}f{}".format(tag, k)
+        if not irr[0] and not irr[1]:
+            for i in (0, 1):
+                recs.append(AlignedSegment(name, 0x1 | 0x2 | seg[i] | strand[i], tid, p[i], 60, [(0, readlen)], tid,
+                                           p[1 - i], 0, seqs[i], aux=aux(60)))
+        elif irr[0] and irr[1]:
+            for i in (0, 1):
+                recs.append(AlignedSegment(name, 0x1 | 0x4 | 0x8 | seg[i] | strand[i], -1, -1, 0, [], -1, -1, 0, seqs[i]))
+        else:
+            i, j = (0, 1) if irr[0] else (1, 0)              # i: the in-repeat read, j: its anchor
+            if mismap_to is not None and rng.random() < mismap_fraction:
+                mt, ms, me = mismap_to
+                mp = int(rng.integers(ms, me))
+                recs.append(AlignedSegment(name, 0x1 | seg[i] | strand[i], mt, mp, 0, [(0, readlen)], tid, p[j], 0,
+                                           seqs[i], aux=aux(60)))
+                recs.append(AlignedSegment(name, 0x1 | seg[j] | strand[j], tid, p[j], 60, [(0, readlen)], mt, mp, 0,
+                                           seqs[j], aux=aux(0)))
+            else:
+                recs.append(AlignedSegment(name, 0x1 | 0x4 | seg[i] | strand[i], tid, p[j], 0, [], tid, p[j], 0,
+                                           seqs[i], aux=aux(60)))
+                recs.append(AlignedSegment(name, 0x1 | 0x8 | seg[j] | strand[j], tid, p[j], 60, [(0, readlen)], tid,
+                                           p[j], 0, seqs[j]))
+    return recs
+
+
+def coordinate_sort(recs):
+    """records in coordinate order: by contig, then position; unmapped records without a contig (tid -1) last"""
+    return sorted(recs, key=lambda r: (r.reference_id if r.reference_id >= 0 else 1 << 31, r.reference_start))
