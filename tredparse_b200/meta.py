@@ -23,6 +23,23 @@ def get_region(location):
     return chr, int(start), int(end)
 
 
+def location_field(ref=REF):
+    """the row field that holds a locus' location on reference `ref` (hg38: repeat_location, hg19:
+    repeat_location.hg19; the _nochr variants use the field of their build)"""
+    return "repeat_location" if ref == REF else "repeat_location." + ref.split("_")[0]
+
+
+def locus_names(sites=SITES):
+    """the names of the catalogue loci and of the user loci in <sites>/*.json, in TREDsRepo's order, without reading
+    their rows (a user locus may carry the location of one reference build only)"""
+    with open(datafile("loci.tsv")) as fp:
+        names = [row["name"] for row in csv.DictReader(fp, delimiter="\t")]
+    for s in sorted(glob("{}/*.json".format(sites))):
+        with open(s) as fp:
+            names += [str(name) for name in json.load(fp)]
+    return names
+
+
 def _num(x):
     try:
         f = float(x)
@@ -37,10 +54,7 @@ class TRED(object):
         self.name = name
         self.alt = list(alt)
         self.repeat = row["repeat"]
-        field = "repeat_location"
-        if ref != REF:
-            field += "." + ref.split("_")[0]
-        location = row[field]
+        location = row[location_field(ref)]
         if "_nochr" in ref:
             location = location.replace("chr", "")
         self.chr, self.repeat_start, self.repeat_end = get_region(location)

@@ -28,6 +28,7 @@ from .utils import datafile, listify
 SPAN = 1000
 FLANKMATCH = 9
 MAX_PERIOD = 6
+MAX_LOCUS_PERIOD = 20        # the longest motif the STR profile reports (IrrParams.max_period): discovered loci
 SMALL_VALUE = math.exp(-10)
 REALLY_SMALL_VALUE = math.exp(-100)
 MODEL_PREFIX = "illumina_v3.pcrfree"
@@ -52,7 +53,8 @@ class StepModel:
         self.non_unit_step_by_period = {i + 1: v for i, v in enumerate(md["non_unit_step_by_period"])}
         self.prob_increase = md["prob_increase"]
         self.step_size_by_period = {int(k): np.array(v) for k, v in md["step_size_by_period"].items()}
-        for i in range(MAX_PERIOD, 3 * MAX_PERIOD):
+        # longer periods share the period-6 distribution (models.py:59-60 stops at 17; discovered loci reach 20)
+        for i in range(MAX_PERIOD, MAX_LOCUS_PERIOD + 1):
             self.step_size_by_period[i] = self.step_size_by_period[MAX_PERIOD]
 
 

@@ -346,3 +346,101 @@ def expansion_records(tid, pos, motif, units, readlen=150, cov=15.0, flank=2000,
 def coordinate_sort(recs):
     """records in coordinate order: by contig, then position; unmapped records without a contig (tid -1) last"""
     return sorted(recs, key=lambda r: (r.reference_id if r.reference_id >= 0 else 1 << 31, r.reference_start))
+
+
+# ---------------------------------------------------------------------------------------------------------
+# a reference and reads that agree with it: discovered loci (strprofile.locus_for) end to end
+# ---------------------------------------------------------------------------------------------------------
+def planted_reference(lengths, sites, seed=0):
+    """Random contigs {name: bases} of `lengths` [(name, length)] with repeat tracts planted: a site (contig, pos,
+    unit, copies) writes `copies` back-to-back copies of `unit` from 0-based `pos` on.  The base before a tract is
+    not the unit's last base and the base after it not its first, so no rotation of the unit runs longer: the tract is
+    exactly the planted one."""
+    rng = np.random.default_rng(seed)
+    seqs = {n: rng.choice(list("ACGT"), L) for n, L in lengths}
+    for contig, pos, unit, copies in sites:
+        s, end = seqs[contig], pos + len(unit) * copies
+        s[pos:end] = list(unit * copies)
+        if pos > 0 and s[pos - 1] == unit[-1]:
+            s[pos - 1] = "ACGT"[("ACGT".index(unit[-1]) + 1) % 4]
+        if end < len(s) and s[end] == unit[0]:
+            s[end] = "ACGT"[("ACGT".index(unit[0]) + 1) % 4]
+    return {n: "".join(s) for n, s in seqs.items()}
+
+
+def write_fasta(path, contigs, width=60, fai=False):
+    """contigs {name: bases} as a FASTA of `width` bases a line; with `fai`, its samtools-style index at path.fai"""
+    rows, offset = [], 0
+    with open(path, "w") as fp:
+        for name, seq in contigs.items():
+            head = ">{}\n".format(name)
+            fp.write(head)
+            lb = min(width, len(seq))                        # (a record of one short line: its own width)
+            rows.append("{}\t{}\t{}\t{}\t{}\n".format(name, len(seq), offset + len(head), lb, lb + 1 if lb else 0))
+            body = "".join(seq[i:i + width] + "\n" for i in range(0, len(seq), width))
+            fp.write(body)
+            offset += len(head) + len(body)
+    if fai:
+        with open(path + ".fai", "w") as fp:
+            fp.writelines(rows)
+    return path
+
+
+def reference_records(seq, tid, rep_start, rep_end, motif, alleles, readlen=150, cov_per_hap=15.0, flank=2000,
+                      error=0.005, seed=0, tag=""):
+    """Paired reads of a locus whose reference tract is seq[rep_start:rep_end] (0-based): haplotype h = the reference's
+    `flank` bases before the tract, h copies of `motif`, its `flank` bases after the tract.  Fragment lengths and
+    errors follow ``locus_records``; reads are placed as ``locus_records`` and ``expansion_records`` place them:
+      * pairs with no read wholly inside the repeat: ``<readlen>M`` proper pairs, MAPQ 60, flanks mapped one to one
+        and the repeat clamped to the reference's tract;
+      * an in-repeat read whose mate is not one: unmapped at its mate's position, the mate flagged 0x8;
+      * both reads inside the repeat: both unmapped, in the unmapped tail (tid -1).
+    Records with a mapped mate carry its MAPQ as an ``MQ`` tag.  Not sorted (``coordinate_sort``); write them with
+    ``bamio.write_bam(..., aux=True)``."""
+    from .bamio import AlignedSegment
+    rng = np.random.default_rng(seed)
+    lut = np.array(list("ACGTN"))
+    ref_len = rep_end - rep_start
+    left = encode(seq[max(0, rep_start - flank):rep_start])
+    right = encode(seq[rep_end:rep_end + flank])
+    recs = []
+    for hap_idx, h in enumerate(alleles):
+        hap = np.concatenate([left, np.tile(encode(motif), h), right]).astype(np.int8)
+        hrs, hre, L = len(left), len(left) + len(motif) * h, len(left) + len(motif) * h + len(right)
+
+        def to_ref(x):
+            if x < hrs:
+                return rep_start - (hrs - x)
+            return rep_start + min(x - hrs, ref_len - 1) if x < hre else rep_end + (x - hre)
+        nfrag = int(round(cov_per_hap * L / (2.0 * readlen)))
+        frag = _fragment_lengths(rng, nfrag)
+        frag = frag[(frag >= readlen) & (frag <= L)]
+        start = rng.integers(0, L - frag + 1)
+        for k in range(len(frag)):
+            s = (int(start[k]), int(start[k] + frag[k] - readlen))
+            seqs = []
+            for s_ in s:
+                r = hap[s_:s_ + readlen].copy()
+                err = rng.random(readlen) < error
+                r[err] = rng.integers(0, 4, int(err.sum()))
+                seqs.append("".join(lut[r]))
+            irr = [hrs <= s_ and s_ + readlen <= hre for s_ in s]
+            p = [to_ref(s_) for s_ in s]
+            seg, strand = (0x40, 0x80), (0x20, 0x10)
+            name = "{}h{}f{}".format(tag, hap_idx, k)
+            if not irr[0] and not irr[1]:
+                tl = to_ref(s[1] + readlen - 1) + 1 - p[0]
+                for i in (0, 1):
+                    recs.append(AlignedSegment(name, 0x1 | 0x2 | seg[i] | strand[i], tid, p[i], 60, [(0, readlen)],
+                                               tid, p[1 - i], tl if i == 0 else -tl, seqs[i], aux=_mq_aux(60)))
+            elif irr[0] and irr[1]:
+                for i in (0, 1):
+                    recs.append(AlignedSegment(name, 0x1 | 0x4 | 0x8 | seg[i] | strand[i], -1, -1, 0, [], -1, -1, 0,
+                                               seqs[i]))
+            else:
+                i, j = (0, 1) if irr[0] else (1, 0)          # i: the in-repeat read, j: its anchor
+                recs.append(AlignedSegment(name, 0x1 | 0x4 | seg[i] | strand[i], tid, p[j], 0, [], tid, p[j], 0,
+                                           seqs[i], aux=_mq_aux(60)))
+                recs.append(AlignedSegment(name, 0x1 | 0x8 | seg[j] | strand[j], tid, p[j], 60, [(0, readlen)], tid,
+                                           p[j], 0, seqs[j]))
+    return recs

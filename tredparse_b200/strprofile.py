@@ -9,6 +9,8 @@ with more anchored IRRs in a region than the rest of the cohort — expansions o
 
     python -m tredparse_b200.strprofile profile x.bam [y.bam ... | -] --workdir w
     python -m tredparse_b200.strprofile outliers w/*.str_profile.json --tsv out.tsv
+    python -m tredparse_b200.strprofile loci out.tsv --fasta ref.fa --profiles w/*.str_profile.json
+    python -m tredparse_b200.tred samples.csv --tred <name> ...          # from the directory that holds sites/
 
 Definitions (include/tredsw.h, tredsw_irr_params):
   * an IRR record is primary (0x100, 0x200, 0x400, 0x800 unset), mapped or not, at least ``min_read_len`` long, and
@@ -33,6 +35,10 @@ from .ingest import BamIngest, IrrParams, is_stream, scan_sample
 MIN_ANCHOR_MAPQ = 50
 MERGE_DISTANCE = 500
 NORM_DEPTH = 40.0
+LOCUS_WINDOW = 1000
+MIN_REF_UNITS = 3
+LOCUS_FLANK = 18
+_RC = str.maketrans("ACGT", "TGCA")
 
 
 def motif_string(period, bits):
@@ -166,6 +172,105 @@ def write_tsv(rows, samples, fp):
         fp.write("\t".join(cells) + "\n")
 
 
+def read_tsv(fp):
+    """the rows of an ``outliers`` table (``write_tsv``): contig, start, end (None for a motif-only row), motif,
+    top_sample, z and the per-sample counts"""
+    header = fp.readline().rstrip("\n").split("\t")
+    if header[:6] != ["contig", "start", "end", "motif", "top_sample", "z"]:
+        raise ValueError("not an outliers table (header {})".format(header[:6]))
+    rows = []
+    for line in fp:
+        c = line.rstrip("\n").split("\t")
+        if len(c) < 6:
+            continue
+        rows.append({"contig": c[0], "start": None if c[1] == "-" else int(c[1]), "end": None if c[2] == "-" else int(c[2]),
+                     "motif": c[3], "top_sample": c[4], "z": float(c[5]),
+                     "counts": {s: float(x) for s, x in zip(header[6:], c[6:])}})
+    return rows
+
+
+class Skip(ValueError):
+    """an outlier row that gives no locus; str() is the reason"""
+
+
+def locus_for(row, fasta, read_length, window=LOCUS_WINDOW, min_ref_units=MIN_REF_UNITS, ref=None):
+    """The locus behind a region row of ``outliers`` -> (name, locus row for ``meta.TRED``); raises Skip(reason).
+
+    Candidate units are the k rotations of the row's canonical motif (period k) and the k rotations of its reverse
+    complement.  The tract is the longest run of exact, back-to-back copies of one candidate unit in the reference
+    window [start - window, end + window) clipped to the contig: the region spans the anchors, mates that lie up to a
+    fragment from the tract.  Ties go to the run whose centre is closest to the region's centre, then to the leftmost
+    run.  Reasons to skip: ``no position`` (a motif-only row), ``contig not in FASTA``, ``no reference tract`` (fewer
+    than `min_ref_units` copies), ``flank outside contig``, ``N in flank`` (any base but A, C, G, T in the 18 bases
+    either side).
+
+    The row: ``repeat`` = the unit as it reads on the reference at the tract's first base; the location
+    ``contig:first-last`` (1-based, inclusive, the contig named as in the BAM header) under the field of `ref`
+    (``meta.location_field``, default hg38); 18-base ``prefix`` / ``suffix``; inheritance AD, mutation_nature
+    increase; ``cutoff_prerisk`` = ``cutoff_risk`` = ceil(read_length / k).  A discovered locus has no clinical
+    cut-off: with this one, label ``risk`` and PP state that an allele is longer than a read, which is what an excess
+    of anchored in-repeat reads supports.  The name is ``<contig>_<first>_<repeat>``."""
+    from .meta import REF, location_field
+    contig, motif = row["contig"], row["motif"]
+    if contig == "-" or row.get("start") is None:
+        raise Skip("no position")
+    if contig not in fasta:
+        raise Skip("contig not in FASTA")
+    k = len(motif)
+    length = fasta.lengths()[contig]
+    lo, hi = max(0, row["start"] - window), min(length, row["end"] + window)
+    seq = fasta.fetch(contig, lo, hi)
+    rc = motif.translate(_RC)[::-1]
+    units = {m[i:] + m[:i] for m in (motif, rc) for i in range(k)}
+    # copies[i]: back-to-back copies of the candidate unit seq[i:i+k] from i on (right to left: one pass)
+    copies = [0] * (len(seq) + k)
+    for i in range(len(seq) - k, -1, -1):
+        u = seq[i:i + k]
+        if u in units:
+            copies[i] = 1 + (copies[i + k] if seq[i + k:i + 2 * k] == u else 0)
+    centre2 = row["start"] + row["end"] - 2 * lo         # twice the region's centre, in window coordinates
+    best = None
+    for i in range(len(seq) - k + 1):
+        c = copies[i]
+        if c and not (i >= k and seq[i - k:i] == seq[i:i + k]):          # the first copy of a run
+            key = (-c, abs(2 * i + c * k - centre2), i)
+            if best is None or key < best:
+                best = key
+    if best is None or -best[0] < min_ref_units:
+        raise Skip("no reference tract")
+    first, n = lo + best[2], -best[0]
+    last = first + n * k                                 # exclusive
+    if first - LOCUS_FLANK < 0 or last + LOCUS_FLANK > length:
+        raise Skip("flank outside contig")
+    prefix, suffix = fasta.fetch(contig, first - LOCUS_FLANK, first), fasta.fetch(contig, last, last + LOCUS_FLANK)
+    if any(b not in "ACGT" for b in prefix + suffix):
+        raise Skip("N in flank")
+    repeat = seq[first - lo:first - lo + k]
+    name = "{}_{}_{}".format(contig, first + 1, repeat)
+    cut = -(-int(read_length) // k)
+    return name, {"title": "Discovered {} repeat".format(motif), "gene_name": "", "id": name, "motif": motif,
+                  "repeat": repeat, location_field(ref or REF): "{}:{}-{}".format(contig, first + 1, last),
+                  "prefix": prefix, "suffix": suffix, "inheritance": "AD", "mutation_nature": "increase",
+                  "cutoff_prerisk": cut, "cutoff_risk": cut}
+
+
+def discover_loci(rows, fasta, read_length, min_z=3.0, window=LOCUS_WINDOW, min_ref_units=MIN_REF_UNITS, ref=None):
+    """The loci of the outlier rows with z >= min_z, in row order -> ({name: locus row}, [(row, reason)] of the rows
+    skipped).  Rows that resolve to one (contig, first base, repeat) — the left and right anchors of a long expansion
+    can make two regions — give one locus, the first row's."""
+    sites, skipped = {}, []
+    for row in rows:
+        if row["z"] < min_z:
+            continue
+        try:
+            name, locus = locus_for(row, fasta, read_length, window, min_ref_units, ref)
+        except Skip as e:
+            skipped.append((row, str(e)))
+            continue
+        sites.setdefault(name, locus)
+    return sites, skipped
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(prog="python -m tredparse_b200.strprofile",
                                  description="STR profiles of whole BAMs (in-repeat reads found on the GPU) and their "
@@ -186,7 +291,52 @@ def main(argv=None):
     po.add_argument("profiles", nargs="+", help="<sample>.str_profile.json files")
     po.add_argument("--tsv", default=None, help="output table (default: stdout)")
     po.add_argument("--merge-distance", type=int, default=None)
+    pl = sub.add_parser("loci", help="a sites JSON of the loci behind the outlier regions, for tred.py --tred NAME",
+                        description="Build a locus from the reference at every outlier region with z >= --min-z and "
+                                    "write them as one sites JSON. Genotype them with python -m tredparse_b200.tred "
+                                    "samples.csv --tred NAME ... run from the directory that holds sites/ (indexed "
+                                    "or unindexed BAMs, one or more GPUs). A BAM streamed through a pipe or stdin "
+                                    "was read once by `profile`: genotyping needs it streamed again.")
+    pl.add_argument("tsv", help="the table `outliers` wrote")
+    pl.add_argument("--fasta", required=True, help="the reference the BAMs are aligned to (plain text; its .fai is "
+                                                   "used when present)")
+    pl.add_argument("--profiles", nargs="+", required=True,
+                    help="<sample>.str_profile.json files: the read length is the largest among them")
+    pl.add_argument("--min-z", type=float, default=3.0)
+    pl.add_argument("--ref", default="hg38", choices=("hg38", "hg38_nochr", "hg19", "hg19_nochr"),
+                    help="the tred.py --ref the loci are for (selects the location field)")
+    pl.add_argument("--window", type=int, default=LOCUS_WINDOW, help="bases searched either side of a region")
+    pl.add_argument("--min-ref-units", type=int, default=MIN_REF_UNITS)
+    pl.add_argument("--out", default=os.path.join("sites", "discovered.json"))
     a = ap.parse_args(argv)
+    if a.cmd == "loci":
+        from .fasta import Fasta
+        with open(a.tsv) as fp:
+            rows = read_tsv(fp)
+        read_length = 0
+        for f in a.profiles:
+            with open(f) as fp:
+                read_length = max(read_length, int(json.load(fp)["read_length"]))
+        if read_length <= 0:
+            ap.error("the profiles give no read length")
+        try:
+            fasta = Fasta(a.fasta)
+        except (IOError, ValueError) as e:
+            ap.error(str(e))
+        sites, skipped = discover_loci(rows, fasta, read_length, a.min_z, a.window, a.min_ref_units, a.ref)
+        below = sum(1 for r in rows if r["z"] < a.min_z)
+        for r, why in skipped:
+            where = r["contig"] if r["start"] is None else "{}:{}-{}".format(r["contig"], r["start"], r["end"])
+            print("skipped {} {} (z {:.4f}): {}".format(where, r["motif"], r["z"], why), file=sys.stderr)
+        print("{} rows below --min-z {}".format(below, a.min_z), file=sys.stderr)
+        if os.path.dirname(a.out):
+            os.makedirs(os.path.dirname(a.out), exist_ok=True)
+        with open(a.out, "w") as fp:
+            json.dump(sites, fp, indent=1, sort_keys=True)
+            fp.write("\n")
+        for name in sites:
+            print(name)
+        return 0
     if a.cmd == "profile":
         # one file per sample key: keys that repeat would overwrite each other (stdin's key is known once it is open)
         keys = [sample_key(b, None) for b in a.bams if b != "-"]

@@ -38,7 +38,7 @@ from . import __version__
 from .utils import DefaultHelpParser, mkdir
 from .bam_parser import BamDepth, BamReadLen, BamParser, BamParserResults, extract_locus, read_alignment
 from .models import IntegratedCaller, mean_std, histogram
-from .meta import TREDsRepo
+from .meta import TREDsRepo, locus_names
 
 logging.basicConfig()
 logger = logging.getLogger(__name__)
@@ -69,7 +69,7 @@ INFO = """##INFO=<ID=RPA,Number=1,Type=String,Description="Repeats per allele">
 
 
 def set_argparse():
-    TRED_NAMES = TREDsRepo().names
+    TRED_NAMES = locus_names()
     p = DefaultHelpParser(description=__doc__, prog=op.basename(__file__),
                           formatter_class=argparse.ArgumentDefaultsHelpFormatter)
     p.add_argument("infile", nargs="?", help="Input path (BAM, list of BAMs, or csv format)")
