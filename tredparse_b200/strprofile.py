@@ -8,6 +8,7 @@ with more anchored IRRs in a region than the rest of the cohort — expansions o
     rows = strprofile.outliers([prof_a, prof_b, ...])  # highest z first
 
     python -m tredparse_b200.strprofile profile x.bam [y.bam ... | -] --workdir w
+    python -m tredparse_b200.tred samples.csv --workdir w --str-profile     # or: catalogue calls and profiles, one read
     python -m tredparse_b200.strprofile outliers w/*.str_profile.json --tsv out.tsv
     python -m tredparse_b200.strprofile loci out.tsv --fasta ref.fa --profiles w/*.str_profile.json
     python -m tredparse_b200.tred samples.csv --tred <name> ...          # from the directory that holds sites/
@@ -117,6 +118,13 @@ def profile(path, ctx=None, sample=None, min_period=2, max_period=20, purity_num
     finally:
         h.close()
     return build_profile(irr, refs, params, min_anchor_mapq, merge_distance, sample=sample, bam=path)
+
+
+def write_profile(prof, path):
+    """a profile as a <sample>.str_profile.json file (what ``outliers`` and ``loci --profiles`` read)"""
+    with open(path, "w") as fp:
+        json.dump(prof, fp, indent=1, sort_keys=True)
+        fp.write("\n")
 
 
 def _zscore(xs, i):
@@ -296,7 +304,9 @@ def main(argv=None):
                                     "write them as one sites JSON. Genotype them with python -m tredparse_b200.tred "
                                     "samples.csv --tred NAME ... run from the directory that holds sites/ (indexed "
                                     "or unindexed BAMs, one or more GPUs). A BAM streamed through a pipe or stdin "
-                                    "was read once by `profile`: genotyping needs it streamed again.")
+                                    "has to be streamed again to genotype the discovered loci; `python -m "
+                                    "tredparse_b200.tred - --str-profile` gives its catalogue calls and its profile "
+                                    "from one read.")
     pl.add_argument("tsv", help="the table `outliers` wrote")
     pl.add_argument("--fasta", required=True, help="the reference the BAMs are aligned to (plain text; its .fai is "
                                                    "used when present)")
@@ -352,9 +362,7 @@ def main(argv=None):
                 ap.error("{}: its sample key `{}` is that of another input".format(bam, prof["sample"]))
             written.add(prof["sample"])
             out = os.path.join(a.workdir, "{}.str_profile.json".format(prof["sample"]))
-            with open(out, "w") as fp:
-                json.dump(prof, fp, indent=1, sort_keys=True)
-                fp.write("\n")
+            write_profile(prof, out)
             print(out)
         return 0
     profs = []

@@ -18,7 +18,9 @@ Differences that are the point of this build:
   * samples are sharded over GPUs (``--gpus``), one worker process per GPU, instead of over CPU cores
     with ``multiprocessing.Pool`` (tred.py:528-532).  No collective: workers return their dicts;
   * a BAM that can be read only once, in order (``-`` for stdin, a FIFO; e.g. ``samtools view -u x.cram | ... -``) is
-    read by one GPU scan that serves its read length, gender and every locus; there is no fallback reader for it.
+    read by one GPU scan that serves its read length, gender and every locus; there is no fallback reader for it;
+  * ``--str-profile`` makes that one scan (indexed BAMs included) also find the in-repeat reads of the whole file and
+    writes each sample's STR profile (``strprofile``) beside its JSON: catalogue calls and profile from one read.
 S3 / ``@HLI-id`` inputs are out of scope (SURVEY.md §2 row 5).
 """
 import argparse
@@ -98,8 +100,14 @@ def set_argparse():
     g = p.add_argument_group("I/O options")
     g.add_argument("--workdir", default=os.getcwd(), help="Specify work dir")
     g.add_argument("--cleanup", default=False, action="store_true", help="Cleanup the workdir after done")
-    g.add_argument("--checkexists", default=False, action="store_true", help="Do not run if JSON output exists")
+    g.add_argument("--checkexists", default=False, action="store_true",
+                   help="Do not run if JSON output exists (such a sample gets no STR profile either)")
     g.add_argument("--no-output", default=False, action="store_true", help="Do not write JSON and VCF output")
+    g.add_argument("--str-profile", default=False, action="store_true",
+                   help="Also write <samplekey>.str_profile.json, the STR profile of `python -m "
+                        "tredparse_b200.strprofile profile` with its default parameters, from the same GPU scan of the "
+                        "BAM that serves the loci (an indexed BAM is scanned whole instead of read by the indexed "
+                        "ingest; a stream is still read once)")
     return p
 
 
@@ -329,18 +337,23 @@ def ingest_chunk_gpu(samples, ctx=None, keep_batch=None):
         return {}
 
 
-def ingest_sample_scan(arg, wanted, READLEN, h, with_gender, ctx=None, stream=False):
-    """Evidence of every wanted locus of one sample whose BAM has no usable index, and its chrY depth when
-    ``with_gender``, in ONE streaming pass over the file on the GPU (``ingest.scan_sample``).
+def ingest_sample_scan(arg, wanted, READLEN, h, with_gender, ctx=None, stream=False, str_profile=False):
+    """Evidence of every wanted locus of one sample whose BAM has no usable index (or whose STR profile is wanted),
+    and its chrY depth when ``with_gender``, in ONE streaming pass over the file on the GPU (``ingest.scan_sample``).
     :param h: the sample's handle from ``ingest.BamIngest.unindexed`` or ``ingest.BamIngest.stream``
     :param stream: `h` is a stream, which can be read only once: a scan that fails raises (no partial evidence, no
                    second reader), and a header without the chrY regions gives gender ('Unknown', -1)
-    :return: ({tredName: LocusEvidence}, (gender, depthY) or None) — loci the scan could not serve (contig missing,
-             a corrupt or unsorted file) are left out, and so is the gender: the caller reads them with the Python
-             reader (not a stream's: a locus whose contig the header lacks gets no call)."""
+    :param str_profile: the same pass also finds the in-repeat reads of the whole file (``IrrParams()``, the defaults
+                        of ``strprofile profile``) and the sample's STR profile is built from them
+                        (``strprofile.build_profile``; its sample is the sample key, its bam the path of the run)
+    :return: ({tredName: LocusEvidence}, (gender, depthY) or None, STR profile or None) — loci the scan could not
+             serve (contig missing, a corrupt or unsorted file) are left out, and so are the gender and the profile:
+             the caller reads the loci with the Python reader (not a stream's: a locus whose contig the header lacks
+             gets no call).  A file whose scan fails gets no profile, and the failure is logged as an error."""
     from . import _lib
-    from .ingest import locus_query, scan_sample
+    from .ingest import IrrParams, locus_query, scan_sample
     samplekey, bam, repo, tredNames, maxinsert, fullsearch, clip, alts, repeatpairs, log = arg
+    irr = IrrParams() if str_profile else None
     qs, keep, names = [], [], []
     for t in wanted:
         xtred = repo[t]
@@ -354,11 +367,11 @@ def ingest_sample_scan(arg, wanted, READLEN, h, with_gender, ctx=None, stream=Fa
         tids = [h.tid(c) for c, s, e in rows]
         if rows and min(tids) >= 0:
             yreg = [(t, s, e) for t, (c, s, e) in zip(tids, rows)]
-    got, gender = {}, (("Unknown", -1) if stream and with_gender and not yreg else None)
-    if not qs and not yreg:
-        return got, gender
+    got, gender, prof = {}, (("Unknown", -1) if stream and with_gender and not yreg else None), None
+    if not qs and not yreg and irr is None:
+        return got, gender, prof
     try:
-        with scan_sample(ctx or _lib.default_context(), h, qs, keep, yreg) as b:
+        with scan_sample(ctx or _lib.default_context(), h, qs, keep, yreg, irr=irr) as b:
             if stream and b.scan_status:
                 raise IOError("the GPU scan of `{}` failed (status {}): {}".format(bam, b.scan_status, _lib.last_error()))
             for i, t in enumerate(names):
@@ -369,12 +382,21 @@ def ingest_sample_scan(arg, wanted, READLEN, h, with_gender, ctx=None, stream=Fa
             if yreg and not b.scan_status:
                 ydepth = float(np.median(b.depths))
                 gender = ("Male" if ydepth > 1 else "Female", ydepth)
+            if irr is not None:
+                if b.scan_status:
+                    logger.error("Sample `{}`: the GPU scan of `{}` failed (status {}): no STR profile".format(
+                        samplekey, bam, b.scan_status))
+                else:
+                    from .strprofile import build_profile
+                    prof = build_profile(b.irr, h.references(), irr, sample=samplekey, bam=bam)
     except Exception as e:
         if stream:
             raise
         logger.error("GPU scan of `{}` failed ({}); reading with the Python reader".format(bam, e))
-        return {}, None
-    return got, gender
+        if irr is not None:
+            logger.error("Sample `{}`: no STR profile (the GPU scan of `{}` raised: {})".format(samplekey, bam, e))
+        return {}, None, None
+    return got, gender, prof
 
 
 OPEN_STREAMS = {}       # stream path -> ingest.BamIngest whose header was read early (the sample key of `-`)
@@ -430,11 +452,23 @@ def run(arg):
     return run_chunk([arg])[0]
 
 
-def prepare_chunk(args, only=None, ctx=None):
+STR_PROFILE = "_str_profile"       # key of a result's STR profile (not part of the JSON: ``main`` writes it apart)
+
+
+def _per_sample(flag, n):
+    """a ``str_profile`` argument (one bool for all the samples, or one per sample) as a list of n bools"""
+    return [bool(flag)] * n if isinstance(flag, bool) else [bool(x) for x in flag]
+
+
+def prepare_chunk(args, only=None, ctx=None, str_profile=False):
     """First half of ``run_chunk``: per-sample pre-steps and the evidence of every (sample, locus) — the GPU ingest,
     the host reader for what it hands back.  Touches no state of the genotyping context, so the next chunk can be
     prepared (on ``ctx``, a context of its own) while the previous one is genotyped.
+    :param str_profile: True, or one bool per sample: the sample's STR profile is made by its one GPU scan (an indexed
+                        BAM is then scanned instead of read by the indexed ingest) and its result carries it under
+                        ``STR_PROFILE``; a sample whose scan fails has none
     :return: an opaque state for ``finish_chunk``"""
+    profile_of = _per_sample(str_profile, len(args))
     out, items, where, todo = [], [], [], []
     for si, arg in enumerate(args):
         samplekey, bam, repo, tredNames, maxinsert, fullsearch, clip, alts, repeatpairs, log = arg
@@ -444,7 +478,8 @@ def prepare_chunk(args, only=None, ctx=None):
     # requested locus); the samples are dealt to host threads
     # a BAM without a usable index is scanned once on the GPU (unless the GPU ingest is off): its gender comes from
     # that scan, so its pre-steps here read only the read length.  So is a stream, which nothing else may read: a
-    # stream that cannot be scanned makes its sample an error
+    # stream that cannot be scanned makes its sample an error.  So is an indexed BAM whose STR profile is wanted: the
+    # profile needs a pass over every record, and that pass serves the loci and gender as well
     def pre(si):
         samplekey, bam, repo, tredNames = args[si][:4]
         from .ingest import BamIngest, is_stream
@@ -466,6 +501,14 @@ def prepare_chunk(args, only=None, ctx=None):
                     return uh, presteps(bam, repo, tredNames, logger, ing=uh, with_gender=False), True
                 except Exception as e2:
                     logger.debug("GPU scan unavailable for `{}` ({})".format(bam, e2))
+        if ing is not None and profile_of[si] and GPU_INGEST:
+            try:
+                uh = BamIngest.unindexed(bam_path(bam))
+            except Exception as e2:
+                logger.error("Sample `{}`: GPU scan unavailable for `{}` ({}): no STR profile".format(samplekey, bam, e2))
+            else:
+                ing.close()
+                return uh, presteps(bam, repo, tredNames, logger, ing=uh, with_gender=False), True
         return ing, presteps(bam, repo, tredNames, logger, ing=ing), False
     if len(args) > 1 and INGEST_THREADS > 1:
         from concurrent.futures import ThreadPoolExecutor
@@ -507,13 +550,16 @@ def prepare_chunk(args, only=None, ctx=None):
             samplekey, bam, repo, tredNames = args[si][:4]
             with_gender = any(repo[t].is_xlinked for t in tredNames)
             try:
-                got[si], gender = ingest_sample_scan(args[si], wanted_of[si], out[si]["tredCalls"]["readLen"],
-                                                     handle_of[si], with_gender, ctx=ctx, stream=si in streams)
+                got[si], gender, prof = ingest_sample_scan(args[si], wanted_of[si], out[si]["tredCalls"]["readLen"],
+                                                           handle_of[si], with_gender, ctx=ctx, stream=si in streams,
+                                                           str_profile=profile_of[si])
             except Exception as e:
                 if si not in streams:
                     raise
                 fail(si, e)
                 continue
+            if prof is not None:
+                out[si][STR_PROFILE] = prof
             if gender is None and with_gender:
                 gender = infer_gender(bam, repo, tredNames, logger)
             if gender is not None:
@@ -582,23 +628,26 @@ def finish_chunk(state, ctx=None):
     return out
 
 
-def run_chunk(args, only=None):
+def run_chunk(args, only=None, str_profile=False):
     """Several samples at once: per-sample pre-steps, then the evidence of every (sample, locus) of the chunk in one
     pass of the GPU ingest, then the loci of ALL the samples through ONE fused device call.  Same results as ``run``
     sample by sample.
     :param args: list of ``run`` argument tuples (same maxinsert / fullsearch / clip / repeatpairs for all)
     :param only: optional list, per sample, of the TRED names to process (a rank's share of a sharded cohort);
                  the other requested names of that sample are left out of its tredCalls
-    :return: list of {"samplekey", "bam", "tredCalls"}"""
-    return finish_chunk(prepare_chunk(args, only))
+    :param str_profile: True, or one bool per sample: see ``prepare_chunk``
+    :return: list of {"samplekey", "bam", "tredCalls"} (and ``STR_PROFILE`` where a profile was made)"""
+    return finish_chunk(prepare_chunk(args, only, str_profile=str_profile))
 
 
-def run_chunks(args, only=None, chunk=None, isolate=False):
+def run_chunks(args, only=None, chunk=None, isolate=False, str_profile=False):
     """``run_chunk`` over a long list of samples, ``chunk`` samples at a time, two stages deep: a helper thread
     prepares chunk k + 1 (file reads and the GPU ingest, on a context and stream of its own; the C calls release the
     GIL) while this thread genotypes chunk k and assembles its JSON fields.  Yields the per-sample results in order.
     isolate: a chunk that raises yields {"samplekey", "bam", "tredCalls": {}, "error"} for its samples instead of
-    ending the run."""
+    ending the run.
+    str_profile: True, or one bool per sample: the result of such a sample carries its STR profile under
+    ``STR_PROFILE`` when its scan made one (``prepare_chunk``)."""
     from concurrent.futures import ThreadPoolExecutor
     from . import _lib
     chunk = chunk or CHUNK_SAMPLES
@@ -614,7 +663,10 @@ def run_chunks(args, only=None, chunk=None, isolate=False):
 
     def prep(k):
         a, b = spans[k]
-        return prepare_chunk(args[a:b], None if only is None else only[a:b], ctx=ictx)
+        if not str_profile:
+            return prepare_chunk(args[a:b], None if only is None else only[a:b], ctx=ictx)
+        return prepare_chunk(args[a:b], None if only is None else only[a:b], ctx=ictx,
+                             str_profile=_per_sample(str_profile, len(args))[a:b])
     try:
         with ThreadPoolExecutor(max_workers=1) as pool:
             fut = pool.submit(prep, 0)
@@ -752,6 +804,15 @@ def write_vcf_json(results, ref, repo, treds, store):
         print("Error writing: {} ({})".format(results.get("samplekey"), e), file=sys.stderr)
 
 
+def write_str_profile(samplekey, prof):
+    """<samplekey>.str_profile.json, as ``strprofile profile`` writes it (``strprofile outliers`` reads both)"""
+    from .strprofile import write_profile
+    try:
+        write_profile(prof, ".".join((samplekey, "str_profile.json")))
+    except Exception as e:
+        print("Error writing: {} ({})".format(samplekey, e), file=sys.stderr)
+
+
 CHUNK_SAMPLES = int(os.environ.get("TREDSW_CHUNK_SAMPLES", "16"))     # samples per fused device call
 
 
@@ -769,25 +830,93 @@ def locus_costs(repo, task_args, readlen=150):
     return np.array(costs), keys
 
 
-def _worker(rank, ngpus, task_args, queue):
-    """One process per GPU.  The (sample, locus) problems are dealt by cost (dist.shard_by_cost: every rank computes
-    the same partition, no communication); a rank ingests only the windows of its own problems and sends back, per
-    chunk of samples, the per-locus fields it produced.  The parent merges them into the per-sample JSON."""
+def deal(task_args, ngpus):
+    """The (sample, locus) problems of a task list dealt to `ngpus` ranks by cost (dist.shard_by_cost: every rank
+    computes the same partition, no communication) -> (owner rank per problem, [(sample index, tred)])"""
+    from .dist import shard_by_cost
+    costs, keys = locus_costs(task_args[0][2], task_args)
+    return shard_by_cost(costs, ngpus), keys
+
+
+def profile_ranks(owner, keys, nsamples):
+    """The rank that makes each sample's STR profile under ``--gpus N``: the rank that owns the most of its loci,
+    ties to the lowest rank; None for a sample no rank owns a locus of.  Every rank computes the same answer from the
+    same deal.  -> list of nsamples ranks"""
+    count = {}
+    for (si, _), o in zip(keys, np.asarray(owner).tolist()):
+        count[si, o] = count.get((si, o), 0) + 1
+    best = [None] * nsamples
+    for (si, o), c in sorted(count.items()):                       # (ranks in ascending order within a sample)
+        if best[si] is None or c > count[si, best[si]]:
+            best[si] = o
+    return best
+
+
+def _worker(rank, ngpus, task_args, queue, str_profile=False):
+    """One process per GPU.  The (sample, locus) problems are dealt by cost (``deal``); a rank ingests only the
+    windows of its own problems and sends back, per chunk of samples, the per-locus fields it produced.  With
+    ``str_profile`` the rank also profiles the samples ``profile_ranks`` gives it; only those of its indexed samples
+    are scanned instead of read by the indexed ingest.  The parent merges the parts (``PartMerge``)."""
     try:
         os.environ["TREDSW_DEVICE"] = str(rank)
-        from .dist import shard_by_cost
-        costs, keys = locus_costs(task_args[0][2], task_args)
-        owner = shard_by_cost(costs, ngpus)
+        owner, keys = deal(task_args, ngpus)
         mine = {}
         for (si, t), o in zip(keys, owner):
             if o == rank:
                 mine.setdefault(si, []).append(t)
         order = sorted(mine)
-        got = run_chunks([task_args[i] for i in order], only=[mine[i] for i in order], isolate=True)
+        if str_profile:
+            prof_rank = profile_ranks(owner, keys, len(task_args))
+            str_profile = [prof_rank[i] == rank for i in order]
+        got = run_chunks([task_args[i] for i in order], only=[mine[i] for i in order], isolate=True,
+                         str_profile=str_profile)
         for i, r in zip(order, got):                                # (a failed chunk must not hang the parent)
-            queue.put(("part", i, r, len(mine[i])))
+            queue.put(("part", rank, i, r, len(mine[i])))
     finally:
-        queue.put(("done", rank, None, 0))
+        queue.put(("done", rank, None, None, 0))
+
+
+class PartMerge:
+    """The parent's side of ``--gpus N``: the "part" messages of the ranks (per sample, the fields of the loci a rank
+    owns) merged into one result per sample, released in input order (like Pool.imap) once all the sample's loci
+    have arrived and, when ``profile_rank`` is given (``profile_ranks``), the part of the rank that profiles it —
+    that part carries the profile (``STR_PROFILE``) unless its scan failed."""
+
+    def __init__(self, need, profile_rank=None):
+        """:param need: per sample, the number of its loci"""
+        self.need = list(need)
+        self.got = [0] * len(self.need)
+        self.merged = [None] * len(self.need)
+        self.profiled = [profile_rank is None or profile_rank[i] is None for i in range(len(self.need))]
+        self.profile_rank = profile_rank
+        self.nxt = 0
+
+    def add(self, rank, i, res, n):
+        """one part: sample i's results from `rank`, covering n of its loci -> the samples now complete, in order"""
+        if self.merged[i] is None:
+            self.merged[i] = {"samplekey": res["samplekey"], "bam": res["bam"], "tredCalls": {}}
+        m = self.merged[i]
+        m["tredCalls"].update(res["tredCalls"])
+        if "error" in res:
+            logger.error("Sample `{}`: {}".format(res["samplekey"], res["error"]))
+        if STR_PROFILE in res:
+            m[STR_PROFILE] = res[STR_PROFILE]
+        self.got[i] += n
+        if self.profile_rank is not None and rank == self.profile_rank[i]:
+            self.profiled[i] = True
+        out = []
+        while self.nxt < len(self.need) and self.got[self.nxt] >= self.need[self.nxt] and self.profiled[self.nxt]:
+            out.append(self.merged[self.nxt])
+            self.merged[self.nxt] = None
+            self.nxt += 1
+        return out
+
+    def rest(self):
+        """once every rank is done: the samples still held (no rank owned a locus of them, or a part never came)"""
+        out = [m for m in self.merged[self.nxt:] if m is not None]
+        self.merged[self.nxt:] = [None] * (len(self.need) - self.nxt)
+        self.nxt = len(self.need)
+        return out
 
 
 def main(args):
@@ -805,6 +934,8 @@ def main(args):
     infile = args.infile
     if not infile:
         sys.exit(not p.print_help())
+    if args.str_profile and not GPU_INGEST:
+        p.error("--str-profile with TREDSW_GPU_INGEST=0: only the GPU scan makes an STR profile")
     # ranks scan their own loci of every sample, and a stream can be read only once
     multi_gpu_stream = "--gpus {} with a stream input: a stream can be read only once, by one GPU".format(args.gpus)
     if args.gpus > 1 and infile == "-":
@@ -840,29 +971,32 @@ def main(args):
         return
 
     def emit(results):
+        prof = results.pop(STR_PROFILE, None)
         if not args.no_output:
             write_vcf_json(results, ref, repo, treds, None)
+            if prof is not None:
+                write_str_profile(results["samplekey"], prof)
 
     ngpus = max(1, args.gpus)
     if ngpus == 1:
         # chunks of samples: one fused device call per chunk (all loci of all its samples)
-        for results in run_chunks(task_args):
+        for results in (run_chunks(task_args, str_profile=True) if args.str_profile else run_chunks(task_args)):
             emit(results)
     else:
         import multiprocessing as mp
         import queue as pyqueue
         ctx = mp.get_context("spawn")
         queue = ctx.Queue()
-        procs = [ctx.Process(target=_worker, args=(r, ngpus, task_args, queue)) for r in range(ngpus)]
+        procs = [ctx.Process(target=_worker, args=(r, ngpus, task_args, queue), kwargs={"str_profile": args.str_profile})
+                 for r in range(ngpus)]
         for pr in procs:
             pr.start()
-        merged = [None] * len(task_args)
-        got = [0] * len(task_args)
-        need = [len(ta[3]) for ta in task_args]
-        done, nxt = 0, 0
+        merge = PartMerge([len(ta[3]) for ta in task_args],
+                          profile_ranks(*deal(task_args, ngpus), len(task_args)) if args.str_profile else None)
+        done = 0
         while done < ngpus:
             try:
-                kind, i, res, n = queue.get(timeout=30)
+                kind, rank, i, res, n = queue.get(timeout=30)
             except pyqueue.Empty:
                 # a worker that died without its sentinel (segfault, OOM kill) must not hang the run
                 dead = [pr for pr in procs if not pr.is_alive() and pr.exitcode not in (0, None)]
@@ -872,22 +1006,12 @@ def main(args):
             if kind == "done":
                 done += 1
                 continue
-            if merged[i] is None:
-                merged[i] = {"samplekey": res["samplekey"], "bam": res["bam"], "tredCalls": {}}
-            merged[i]["tredCalls"].update(res["tredCalls"])
-            if "error" in res:
-                logger.error("Sample `{}`: {}".format(res["samplekey"], res["error"]))
-            got[i] += n
-            while nxt < len(task_args) and got[nxt] >= need[nxt]:          # emit in input order, like Pool.imap
-                emit(merged[nxt])
-                merged[nxt] = None
-                nxt += 1
+            for results in merge.add(rank, i, res, n):
+                emit(results)
         for pr in procs:
             pr.join()
-        while nxt < len(task_args):                                         # (samples no rank owned a locus of)
-            if merged[nxt] is not None:
-                emit(merged[nxt])
-            nxt += 1
+        for results in merge.rest():
+            emit(results)
 
     print("Elapsed time={}".format(timedelta(seconds=time.time() - start)), file=sys.stderr)
     os.chdir(cwd)
