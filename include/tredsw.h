@@ -544,6 +544,44 @@ int tredsw_ingest_scan_irr(const tredsw_ingest_batch *batch, tredsw_irr_view *vi
 int tredsw_irr_classify_host(const int8_t *codes, int32_t len, const tredsw_irr_params *params, int32_t *period,
                              uint64_t *motif);
 
+/* ------------------------------------------------------------------------------------------------
+ * (E) Reference tract scan (csrc/ref_tracts_device.cuh, bgzf_gpu.cu; DESIGN §4.5): every tract of the requested
+ * motifs in a plain-text FASTA, for the alt regions of discovered loci.  For a period k (2..20), a maximal stretch
+ * [a, b) of bases in ACGTacgt (compared case-insensitively; N, IUPAC codes and anything else break it) with
+ * s[j] == s[j + k] for every j in [a, b - k) gives the tract [a, a + c k), c = floor((b - a) / k), unit s[a, a + k) in
+ * upper case.  It is kept when the unit's primitive root has period k, c >= min_units, c k >= min_len and the unit's
+ * canonical code (as tredsw_irr_entry.motif: the smallest rotation of the unit and of its reverse complement, 2 bits a
+ * base, first base most significant) is among the motifs of period k.
+ *
+ * The host preads whole contigs as FASTA text (their .fai layout) into two page-locked buffers, in steps of at most
+ * step_bytes of text (0: 256 MiB; a larger contig is a step of its own), the read of step k + 1 on a host thread
+ * while the device packs and scans step k.  A base position holding '\n', '\r' or '>' (the index does not fit the
+ * file) or a file shorter than its index is TREDSW_ERR_IO; every error leaves no result.  No CPU fallback.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct { int64_t length, offset; int32_t line_bases, line_width; } tredsw_fai_entry;   /* a .fai row */
+typedef struct { int32_t period, reserved_; uint64_t code; } tredsw_motif;     /* a canonical code of `period` bases */
+typedef struct { int32_t min_units, min_len; int64_t step_bytes; } tredsw_tract_params;   /* min_units >= 2 */
+typedef struct { int64_t start, length; uint64_t code; int32_t contig, period; } tredsw_tract;   /* 0-based start */
+typedef struct tredsw_tracts tredsw_tracts;
+typedef struct {                /* host arrays, valid until tredsw_ref_tracts_free */
+    int64_t n_tracts;
+    const tredsw_tract *tracts; /* by (contig, start, period); contig indexes the `contigs` of the call */
+    int64_t steps, bytes, bases, invalid_bases;   /* bytes: FASTA text read; invalid: bases not in ACGTacgt */
+    const double *step_read_ms, *step_device_ms;  /* per step: host read (overlaps the previous step's device work),
+                                                     device work (upload, kernels, copies back) */
+    double ms_total;
+} tredsw_tracts_view;
+int tredsw_ref_tracts(tredsw_ctx *ctx, const char *fasta_path, const tredsw_fai_entry *contigs, int32_t ncontigs,
+                      const tredsw_motif *motifs, int32_t nmotifs, const tredsw_tract_params *params,
+                      tredsw_tracts **result);
+/* TEST INFRASTRUCTURE: the same with every kernel body run serially on the host (ctx is not used and may be NULL).
+ * The package never calls it. */
+int tredsw_ref_tracts_emulate(tredsw_ctx *ctx, const char *fasta_path, const tredsw_fai_entry *contigs,
+                              int32_t ncontigs, const tredsw_motif *motifs, int32_t nmotifs,
+                              const tredsw_tract_params *params, tredsw_tracts **result);
+int tredsw_ref_tracts_view(const tredsw_tracts *result, tredsw_tracts_view *view);
+void tredsw_ref_tracts_free(tredsw_tracts *result);
+
 #ifdef __cplusplus
 }
 #endif

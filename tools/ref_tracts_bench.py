@@ -1,0 +1,134 @@
+#!/usr/bin/env python
+"""The reference tract scan (Fasta.tracts, tredsw_ref_tracts) on a whole synthetic genome: a seeded FASTA with the
+contig sizes of hg38 scaled to --gbp, 60-base lines, half of every contig soft-masked (lowercase) in 4 KiB blocks, an
+N run at either end of every contig and one in its middle (~3 % of its length), and planted tracts of the motifs it
+scans for.  The motifs are those of 20 loci of periods 2 to 20 (what `strprofile loci --alts` asks for after a cohort
+with that many discovered loci).
+
+One context, then --reps + 1 calls: the first call on its own (pinned buffers allocated, modules loaded) and the best
+of the later ones.  The card's name, power limit and max SM clock are read in the same run.  The file is written to a
+temporary directory, never into the repository, and is read from the page cache (the run writes it just before): a
+cold-cache read and a real reference genome are not measured.
+
+    python tools/ref_tracts_bench.py [--gbp 3.1] [--reps 3] [--step-mib 256] [--out profiles/r3_ref_tracts_bench.json]
+(without --out the result line is only printed)
+"""
+import argparse
+import json
+import os
+import shutil
+import subprocess
+import sys
+import tempfile
+import time
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+HG38_MBP = [248.96, 242.19, 198.30, 190.21, 181.54, 170.81, 159.35, 145.14, 138.39, 133.80, 135.09, 133.28, 114.36,
+            107.04, 101.99, 90.34, 83.26, 80.37, 58.62, 64.44, 46.71, 50.82, 156.04, 57.23]
+NAMES = ["chr{}".format(i) for i in range(1, 23)] + ["chrX", "chrY"]
+MOTIFS = ["AC", "AT", "AG", "CAG", "AAG", "ATC", "AAAG", "AATG", "AAGGG", "AAAAT", "AACCCT", "AAGGCC", "AGCGGCG",
+          "AACCTGG", "ACCGGAGCG", "AGGTTCCAGC", "AAGGTACCGTT", "ACGTTGCAAGCT", "TGCTTACCGTCAA",
+          "GATCCAGTTAGCCTGAAAGT"]
+
+
+def card():
+    try:
+        return subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                              capture_output=True, text=True).stdout.strip().splitlines()[0]
+    except Exception as e:
+        return "unknown ({})".format(e)
+
+
+def write_genome(path, gbp, seed=0, width=60):
+    rng = np.random.default_rng(seed)
+    lut = np.frombuffer(b"ACGT", np.uint8)
+    scale = gbp * 1e3 / sum(HG38_MBP)
+    total, fai = 0, []
+    with open(path, "wb") as fp:
+        for name, mbp in zip(NAMES, HG38_MBP):
+            L = int(mbp * 1e6 * scale)
+            s = lut[rng.integers(0, 4, L, dtype=np.uint8)]
+            for _ in range(L // 50000):                     # planted tracts, 3 to 40 copies
+                u = MOTIFS[int(rng.integers(len(MOTIFS)))]
+                t = np.frombuffer((u * int(rng.integers(3, 41))).encode(), np.uint8)
+                a = int(rng.integers(0, L - len(t)))
+                s[a:a + len(t)] = t
+            nb = L // 4096                                  # soft-masking: half of the 4 KiB blocks in lowercase
+            blocks = s[:nb * 4096].reshape(nb, 4096)
+            blocks[rng.random(nb) < 0.5] += 32
+            for a, n in ((0, 10000), (L // 2, L // 33), (L - 10000, 10000)):
+                s[a:a + n] = ord("N")
+            fp.write(">{}\n".format(name).encode())
+            fai.append("{}\t{}\t{}\t{}\t{}\n".format(name, L, fp.tell(), width, width + 1))
+            n = (L + width - 1) // width
+            body = np.full((n, width + 1), ord("\n"), np.uint8)
+            pad = np.full(n * width, ord("\n"), np.uint8)
+            pad[:L] = s
+            body[:, :width] = pad.reshape(n, width)
+            fp.write(body.tobytes()[:L + n])
+            total += L
+    with open(path + ".fai", "w") as fp:
+        fp.writelines(fai)
+    return total
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--gbp", type=float, default=3.1)
+    ap.add_argument("--reps", type=int, default=3)
+    ap.add_argument("--step-mib", type=int, default=256)
+    ap.add_argument("--out", default=None)
+    a = ap.parse_args()
+    from tredparse_b200 import _lib
+    from tredparse_b200.fasta import Fasta
+    ctx = _lib.default_context()
+    d = tempfile.mkdtemp(prefix="ref_tracts_bench_")
+    try:
+        path = os.path.join(d, "genome.fa")
+        t0 = time.time()
+        bases = write_genome(path, a.gbp)
+        t_write = time.time() - t0
+        fa = Fasta(path)
+        calls = []
+        for _ in range(a.reps + 1):
+            t0 = time.perf_counter()
+            r = fa.tracts(MOTIFS, step_bytes=a.step_mib << 20, ctx=ctx)
+            calls.append((time.perf_counter() - t0, r))
+        first, later = calls[0], calls[1:]
+        best = min(later, key=lambda c: c[0]) if later else first
+        if later:
+            for _, r in later:
+                assert np.array_equal(r["tracts"], first[1]["tracts"])
+        st = best[1]["stats"]
+
+        def summary(wall, res):
+            s = res["stats"]
+            return {"wall_s": round(wall, 4), "lib_ms_total": round(s["ms_total"], 2),
+                    "text_GB_per_s": round(s["bytes"] / wall / 1e9, 3),
+                    "host_read_ms_sum": round(sum(s["step_read_ms"]), 2),
+                    "device_ms_sum": round(sum(s["step_device_ms"]), 2)}
+        out = {"bench": "ref_tracts", "card": card(), "gbp": a.gbp, "bases": bases, "file_bytes": os.path.getsize(path),
+               "write_s": round(t_write, 1), "motifs": len(MOTIFS), "step_mib": a.step_mib,
+               "steps": st["steps"], "text_bytes": st["bytes"], "invalid_bases": st["invalid_bases"],
+               "tracts": st["tracts"], "first_call": summary(*first), "best_later_call": summary(*best),
+               "later_walls_s": [round(w, 4) for w, _ in later],
+               "per_step_best": [{"read_ms": round(x, 2), "device_ms": round(y, 2)}
+                                 for x, y in zip(st["step_read_ms"], st["step_device_ms"])],
+               "page_cache": "warm (file written in the same run); cold cache not measured"}
+    finally:
+        shutil.rmtree(d, ignore_errors=True)
+    line = json.dumps(out)
+    print(line)
+    if a.out:
+        os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
+        with open(a.out, "w") as fp:
+            json.dump(out, fp, indent=1)
+            fp.write("\n")
+
+
+if __name__ == "__main__":
+    main()

@@ -40,6 +40,8 @@ EXPORTS = [
     "tredsw_bam_open_stream", "tredsw_bam_header_text",
     # the STR profile of a scan (in-repeat reads)
     "tredsw_ingest_scan_run_ex", "tredsw_ingest_scan_emulate_ex", "tredsw_ingest_scan_irr", "tredsw_irr_classify_host",
+    # the reference tract scan (alt regions of discovered loci); *_emulate runs the device code on the host
+    "tredsw_ref_tracts", "tredsw_ref_tracts_emulate", "tredsw_ref_tracts_view", "tredsw_ref_tracts_free",
 ]
 
 
@@ -88,6 +90,24 @@ POST_H1, POST_H2, POST_JOINT, POST_JOINT_TOTAL = 1, 2, 3, 4
 FAMILY_DTYPE = np.dtype([("prefix", "i1", 32), ("suffix", "i1", 32), ("repeat", "i1", 32),
                          ("prefix_len", "<i4"), ("suffix_len", "<i4"), ("period", "<i4"),
                          ("max_units", "<i4"), ("clip", "<i4"), ("reserved", "<i4", 3)])
+FAI_ENTRY_DTYPE = np.dtype([("length", "<i8"), ("offset", "<i8"), ("line_bases", "<i4"), ("line_width", "<i4")])
+MOTIF_DTYPE = np.dtype([("period", "<i4"), ("reserved", "<i4"), ("code", "<u8")])
+TRACT_DTYPE = np.dtype([("start", "<i8"), ("length", "<i8"), ("code", "<u8"), ("contig", "<i4"), ("period", "<i4")])
+
+
+class TractParams(ctypes.Structure):
+    """tredsw_tract_params (include/tredsw.h)"""
+    _fields_ = [("min_units", ctypes.c_int32), ("min_len", ctypes.c_int32), ("step_bytes", ctypes.c_int64)]
+
+
+class TractsView(ctypes.Structure):
+    """tredsw_tracts_view (include/tredsw.h)"""
+    _fields_ = [("n_tracts", ctypes.c_int64), ("tracts", ctypes.c_void_p), ("steps", ctypes.c_int64),
+                ("bytes", ctypes.c_int64), ("bases", ctypes.c_int64), ("invalid_bases", ctypes.c_int64),
+                ("step_read_ms", ctypes.POINTER(ctypes.c_double)), ("step_device_ms", ctypes.POINTER(ctypes.c_double)),
+                ("ms_total", ctypes.c_double)]
+
+
 assert GRID_PROBLEM_DTYPE.itemsize == ctypes.sizeof(GridProblem)
 assert GRID_RESULT_DTYPE.itemsize == ctypes.sizeof(GridResult)
 assert FAMILY_DTYPE.itemsize == ctypes.sizeof(Family)
@@ -143,6 +163,14 @@ def load():
         lib.tredsw_pack_reads4.argtypes = [_vp, ctypes.c_int64, _vp, ctypes.c_int]
         lib.tredsw_narrow_i16.restype = ctypes.c_int
         lib.tredsw_narrow_i16.argtypes = [_vp, ctypes.c_int64, _vp, ctypes.c_int]
+        for f in (lib.tredsw_ref_tracts, lib.tredsw_ref_tracts_emulate):
+            f.restype = ctypes.c_int
+            f.argtypes = [_vp, ctypes.c_char_p, _vp, ctypes.c_int32, _vp, ctypes.c_int32,
+                          ctypes.POINTER(TractParams), ctypes.POINTER(_vp)]
+        lib.tredsw_ref_tracts_view.restype = ctypes.c_int
+        lib.tredsw_ref_tracts_view.argtypes = [_vp, ctypes.POINTER(TractsView)]
+        lib.tredsw_ref_tracts_free.restype = None
+        lib.tredsw_ref_tracts_free.argtypes = [_vp]
         _lib = lib
         return lib
 
@@ -154,6 +182,42 @@ def last_error():
 def check(rc, what):
     if rc != 0:
         raise TredswError("{} failed (code {}): {}".format(what, rc, last_error()))
+
+
+def ref_tracts(path, contigs, motifs, min_units, min_len, step_bytes=0, ctx=None, emulate=False):
+    """Every tract of `motifs` in the FASTA at `path` (tredsw_ref_tracts, DESIGN §4.5).  contigs: FAI_ENTRY_DTYPE rows
+    in FASTA order; motifs: (period, canonical code) pairs.  -> (TRACT_DTYPE array by (contig, start, period), stats
+    dict).  ``ctx``: a Context (default the process's); ``emulate`` runs the serial host emulation of the device code
+    instead — test infrastructure only.  Raises TredswError (no device, I/O, an index that does not fit the file)."""
+    lib = load()
+    cs = np.ascontiguousarray(contigs, dtype=FAI_ENTRY_DTYPE)
+    ms = np.zeros(len(motifs), dtype=MOTIF_DTYPE)
+    for i, (k, code) in enumerate(motifs):
+        ms[i]["period"], ms[i]["code"] = k, code
+    prm = TractParams(int(min_units), int(min_len), int(step_bytes))
+    res = ctypes.c_void_p()
+    if emulate:
+        rc = lib.tredsw_ref_tracts_emulate(None, path.encode(), ptr(cs), len(cs), ptr(ms), len(ms), ctypes.byref(prm),
+                                           ctypes.byref(res))
+    else:
+        handle = (ctx or default_context()).handle
+        rc = lib.tredsw_ref_tracts(handle, path.encode(), ptr(cs), len(cs), ptr(ms), len(ms), ctypes.byref(prm),
+                                   ctypes.byref(res))
+    check(rc, "tredsw_ref_tracts")
+    try:
+        v = TractsView()
+        check(lib.tredsw_ref_tracts_view(res, ctypes.byref(v)), "tredsw_ref_tracts_view")
+        n = int(v.n_tracts)
+        tracts = np.zeros(n, dtype=TRACT_DTYPE)
+        if n:
+            ctypes.memmove(tracts.ctypes.data, v.tracts, n * TRACT_DTYPE.itemsize)
+        stats = {"steps": int(v.steps), "bytes": int(v.bytes), "bases": int(v.bases),
+                 "invalid_bases": int(v.invalid_bases), "tracts": n, "ms_total": float(v.ms_total),
+                 "step_read_ms": [float(v.step_read_ms[i]) for i in range(v.steps)],
+                 "step_device_ms": [float(v.step_device_ms[i]) for i in range(v.steps)]}
+    finally:
+        lib.tredsw_ref_tracts_free(res)
+    return tracts, stats
 
 
 def ptr(a):

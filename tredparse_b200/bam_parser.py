@@ -130,7 +130,7 @@ class BamParser:
                     if self.clip:
                         continue
                     try:
-                        if "nochr" in self.ref:
+                        if "nochr" in self.ref and c.startswith("chr"):
                             c = c[3:]
                         for read in samfile.fetch(c, s, e):
                             rid = read.next_reference_id

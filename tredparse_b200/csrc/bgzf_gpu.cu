@@ -22,6 +22,9 @@
 // sample, slab by slab, that finds the record boundaries on the device and hands the records of every fetch to the
 // same selection / compaction / pairing steps (select_and_pair) — see the scan_* bodies of ingest_device.cuh.
 //
+// A third front end, run_ref_tracts (tredsw_ref_tracts), scans a plain-text FASTA for the tracts of requested motifs
+// with the same backend and the same staging (page-locked steps read by a host thread): ref_tracts_device.cuh.
+//
 // The per-thread bodies live in ingest_device.cuh as __host__ __device__ functions; the pipeline below is written
 // once against a small backend (allocate / copy / for_each / scan) with a CUDA implementation and a serial host
 // implementation.  The host one is TEST INFRASTRUCTURE (tredsw_ingest_batch_emulate): it lets the CPU suite compare
@@ -30,6 +33,7 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <fcntl.h>
 #include <unistd.h>
 #include <sys/stat.h>
 
@@ -44,6 +48,7 @@
 #include "common.cuh"
 #include "ingest_internal.h"
 #include "ingest_device.cuh"
+#include "ref_tracts_device.cuh"
 
 namespace tredsw_gi {       // kernel name tags (they show up in profiler listings: for_each_kernel<tredsw_gi::SelectTag, ...>)
 struct WalkCountTag; struct WalkFillTag; struct SelectTag; struct SummaryTag; struct CompactTag; struct EmitTag;
@@ -52,6 +57,8 @@ struct PairInsertTag; struct PairSecondTag; struct PairEvalTag; struct PairCount
 struct ScanCandidateTag; struct ScanRepairTag; struct ScanCountTag; struct ScanFillTag; struct ScanMatchTag; struct ScanKeepTag;
 // its STR profile (in-repeat reads)
 struct ScanIrrTag; struct ScanIrrFillTag;
+// the reference tract scan
+struct TractPackTag; struct TractRunsTag;
 }
 using namespace tredsw_gi;
 
@@ -1616,5 +1623,258 @@ int tredsw_inflate_raw_device_code(const uint8_t *in, int64_t in_len, uint8_t *o
     // (offset 4 + a caller-chosen misalignment would also work: the reader handles any start address)
     return inflate_block<1>(padded.data() + 4, in_len, out, out_len, TabRef{tabs.data(), 1, true}, lens, sub_need, sub_base, 0) ? 0 : 1;
 }
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------------------------
+// the reference tract scan: every tract of the requested motifs in a plain-text FASTA (ref_tracts_device.cuh)
+// ---------------------------------------------------------------------------------------------------------------
+struct tredsw_tracts {
+    std::vector<TractOut> tracts;
+    std::vector<double> read_ms, device_ms;
+    tredsw_tracts_view view;
+};
+static_assert(sizeof(TractOut) == sizeof(tredsw_tract), "TractOut mirrors tredsw_tract");
+
+namespace {
+
+constexpr int64_t TRACT_DEFAULT_STEP = 256ll << 20;    // bytes of FASTA text per step when the caller passes 0
+
+int64_t fai_text_bytes(const tredsw_fai_entry &c) {     // bytes from a contig's first base to its last
+    if (c.length <= 0) return 0;
+    const int64_t last = c.length - 1;
+    return last / c.line_bases * c.line_width + last % c.line_bases + 1;
+}
+
+struct TractStep {                  // contigs [c0, c1) of the call, their text in one page-locked buffer
+    int32_t c0 = 0, c1 = 0;
+    int64_t bytes = 0;
+    uint8_t *text = nullptr;
+    const char *why = nullptr;      // I/O error
+    double ms = 0;                  // host read time
+};
+
+void read_tract_step(int fd, const tredsw_fai_entry *cs, TractStep *st) {
+    const double t0 = now_ms();
+    st->why = nullptr;
+    int64_t at = 0;
+    for (int32_t c = st->c0; c < st->c1 && !st->why; ++c) {
+        const int64_t n = fai_text_bytes(cs[c]);
+        int64_t got = 0;
+        while (got < n) {
+            const ssize_t k = pread(fd, st->text + at + got, (size_t)(n - got), (off_t)(cs[c].offset + got));
+            if (k <= 0) break;
+            got += k;
+        }
+        if (got < n) st->why = "the file is shorter than its index says";
+        at += n;
+    }
+    st->ms = now_ms() - t0;
+}
+
+template <class B>
+int run_ref_tracts(B &be, tredsw_tracts *out, const char *path, const tredsw_fai_entry *cs, int32_t nc,
+                   const tredsw_motif *ms, int32_t nm, const tredsw_tract_params &prm) {
+    const double t_begin = now_ms();
+    // the requested codes by period, ascending
+    std::vector<std::pair<int32_t, uint64_t>> mv;
+    for (int32_t i = 0; i < nm; ++i) mv.emplace_back(ms[i].period, ms[i].code);
+    std::sort(mv.begin(), mv.end());
+    mv.erase(std::unique(mv.begin(), mv.end()), mv.end());
+    std::vector<int32_t> periods, mfirst;
+    std::vector<uint64_t> mcodes;
+    for (const auto &m : mv) {
+        if (periods.empty() || periods.back() != m.first) { periods.push_back(m.first); mfirst.push_back((int32_t)mcodes.size()); }
+        mcodes.push_back(m.second);
+    }
+    mfirst.push_back((int32_t)mcodes.size());
+    const int32_t nper = (int32_t)periods.size();
+    // steps: consecutive contigs under the byte budget (a larger contig alone)
+    const int64_t budget = prm.step_bytes > 0 ? prm.step_bytes : TRACT_DEFAULT_STEP;
+    std::vector<TractStep> steps;
+    int64_t max_bytes = 0, bases = 0;
+    for (int32_t c = 0; c < nc && nper; ++c) {
+        const int64_t n = fai_text_bytes(cs[c]);
+        bases += cs[c].length;
+        if (steps.empty() || (steps.back().bytes + n > budget && steps.back().c1 > steps.back().c0)) {
+            steps.push_back(TractStep());
+            steps.back().c0 = c;
+        }
+        steps.back().c1 = c + 1;
+        steps.back().bytes += n;
+        max_bytes = std::max(max_bytes, steps.back().bytes);
+    }
+    const int fd = steps.empty() ? -1 : open(path, O_RDONLY);
+    if (!steps.empty() && fd < 0) { tredsw_set_error("%s: cannot open: %s", path, strerror(errno)); return TREDSW_ERR_IO; }
+    struct Close { int fd; ~Close() { if (fd >= 0) close(fd); } } close_fd{fd};
+    uint8_t *pinned[2] = {nullptr, nullptr};
+    for (uint8_t *&p : pinned) if (!steps.empty()) p = static_cast<uint8_t *>(be.alloc_host((size_t)max_bytes + 64));
+    int32_t *d_per = static_cast<int32_t *>(be.alloc(sizeof(int32_t) * (size_t)(2 * nper + 1)));
+    uint64_t *d_codes = static_cast<uint64_t *>(be.alloc(sizeof(uint64_t) * std::max<size_t>(1, mcodes.size())));
+    unsigned long long *d_small = static_cast<unsigned long long *>(be.alloc(sizeof(unsigned long long) * 3));
+    if (be.rc) return be.rc;
+    be.upload(d_per, periods.data(), sizeof(int32_t) * (size_t)nper);
+    be.upload(d_per + nper, mfirst.data(), sizeof(int32_t) * (size_t)(nper + 1));
+    be.upload(d_codes, mcodes.data(), sizeof(uint64_t) * mcodes.size());
+    const TractQuery q{d_per, d_per + nper, d_codes, nper, prm.min_units, (int64_t)prm.min_len};
+    void *d_text = nullptr, *d_code = nullptr, *d_valid = nullptr, *d_cs = nullptr, *d_out = nullptr;
+    size_t c_text = 0, c_code = 0, c_valid = 0, c_cs = 0, c_out = 0;
+    grow(be, d_out, c_out, sizeof(TractOut) * 65536);
+    int64_t invalid = 0, bytes = 0;
+    std::thread reader;
+    struct Join { std::thread &t; ~Join() { if (t.joinable()) t.join(); } } join_reader{reader};
+    if (!steps.empty()) { steps[0].text = pinned[0]; read_tract_step(fd, cs, &steps[0]); }
+    for (size_t k = 0; k < steps.size(); ++k) {
+        TractStep &st = steps[k];
+        if (st.why) { tredsw_set_error("%s: %s", path, st.why); return TREDSW_ERR_IO; }
+        if (k + 1 < steps.size()) {
+            steps[k + 1].text = pinned[(k + 1) & 1];
+            reader = std::thread(read_tract_step, fd, cs, &steps[k + 1]);
+        }
+        const double t_dev = now_ms();
+        // the step's contigs: text and word offsets
+        const int ncs = st.c1 - st.c0;
+        std::vector<TractContig> tc(ncs);
+        int64_t text_at = 0, words = 0;
+        for (int i = 0; i < ncs; ++i) {
+            const tredsw_fai_entry &f = cs[st.c0 + i];
+            tc[i] = TractContig{f.length, text_at, words, f.line_bases, f.line_width, st.c0 + i, 0};
+            text_at += fai_text_bytes(f);
+            words += tract_words(f.length);
+        }
+        uint8_t *text = static_cast<uint8_t *>(grow(be, d_text, c_text, (size_t)st.bytes + 64));
+        uint64_t *code = static_cast<uint64_t *>(grow(be, d_code, c_code, sizeof(uint64_t) * (size_t)std::max<int64_t>(1, words)));
+        uint32_t *valid = static_cast<uint32_t *>(grow(be, d_valid, c_valid, sizeof(uint32_t) * (size_t)std::max<int64_t>(1, words)));
+        TractContig *dcs = static_cast<TractContig *>(grow(be, d_cs, c_cs, sizeof(TractContig) * (size_t)ncs));
+        if (be.rc) return be.rc;
+        be.upload(text, st.text, (size_t)st.bytes);
+        be.upload(dcs, tc.data(), sizeof(TractContig) * (size_t)ncs);
+        be.fill(d_small, 0, sizeof(unsigned long long) * 3);
+        unsigned long long *cnt = d_small, *inval = d_small + 1, *err = d_small + 2;
+        be.template for_each<TractPackTag>(words, [=] __host__ __device__(int64_t w) {
+            const TractContig c = dcs[tract_contig_of(dcs, ncs, w)];
+            bool bad = false;
+            const int n = tract_pack_word(text, c, w - c.word0, &code[w], &valid[w], &bad);
+            warp_add_u64(inval, (uint32_t)n);
+            if (bad) atomic_add_u64(err, 1ull);
+        });
+        // the runs of every period, one thread per (word, period); more tracts than room: run again with room for all
+        unsigned long long h_small[3] = {0, 0, 0};
+        for (int pass = 0; pass < 2; ++pass) {
+            const unsigned long long cap = c_out / sizeof(TractOut);
+            TractOut *tout = static_cast<TractOut *>(d_out);
+            be.template for_each<TractRunsTag>(words * nper, [=] __host__ __device__(int64_t i) {
+                const int64_t w = i / q.nper;
+                const TractContig &c = dcs[tract_contig_of(dcs, ncs, w)];
+                tract_runs(code, valid, c, w - c.word0, (int)(i - w * q.nper), q, tout, cnt, cap);
+            });
+            be.download(h_small, d_small, sizeof(h_small));
+            be.sync();
+            if (be.rc) return be.rc;
+            if (h_small[2]) { tredsw_set_error("%s: a base position holds a line break or a header: the index does not fit the file", path); return TREDSW_ERR_IO; }
+            if (h_small[0] <= cap) break;
+            if (pass) { tredsw_set_error("tract count changed between passes"); return TREDSW_ERR_CUDA; }
+            c_out = sizeof(TractOut) * (size_t)(h_small[0] + h_small[0] / 4 + 1024);
+            d_out = be.alloc(c_out);
+            be.fill(cnt, 0, sizeof(unsigned long long));
+            if (be.rc) return be.rc;
+        }
+        const size_t t0 = out->tracts.size();
+        out->tracts.resize(t0 + (size_t)h_small[0]);
+        be.download(out->tracts.data() + t0, d_out, sizeof(TractOut) * (size_t)h_small[0]);
+        be.sync();
+        if (be.rc) return be.rc;
+        invalid += (int64_t)h_small[1];
+        bytes += st.bytes;
+        out->read_ms.push_back(st.ms);
+        out->device_ms.push_back(now_ms() - t_dev);
+        if (reader.joinable()) reader.join();
+    }
+    std::sort(out->tracts.begin(), out->tracts.end(), [](const TractOut &x, const TractOut &y) {
+        return x.contig != y.contig ? x.contig < y.contig : x.start != y.start ? x.start < y.start : x.period < y.period;
+    });
+    be.release_intermediates();
+    tredsw_tracts_view &v = out->view;
+    memset(&v, 0, sizeof(v));
+    v.n_tracts = (int64_t)out->tracts.size();
+    v.tracts = reinterpret_cast<const tredsw_tract *>(out->tracts.data());
+    v.steps = (int64_t)out->read_ms.size(); v.bytes = bytes; v.bases = bases; v.invalid_bases = invalid;
+    v.step_read_ms = out->read_ms.data(); v.step_device_ms = out->device_ms.data();
+    v.ms_total = now_ms() - t_begin;
+    return TREDSW_OK;
+}
+
+bool tract_args_ok(const char *path, const tredsw_fai_entry *cs, int32_t nc, const tredsw_motif *ms, int32_t nm,
+                   const tredsw_tract_params *p, tredsw_tracts **out) {
+    if (!path || !out || !p || nc < 0 || nm < 0 || (nc && !cs) || (nm && !ms)) { tredsw_set_error("bad arguments"); return false; }
+    if (p->min_units < 2 || p->min_len < 0 || p->step_bytes < 0) {
+        tredsw_set_error("tract parameters out of range (min_units >= 2, min_len >= 0, step_bytes >= 0)");
+        return false;
+    }
+    for (int32_t i = 0; i < nm; ++i)
+        if (ms[i].period < 2 || ms[i].period > 20 || ms[i].code >> (2 * ms[i].period)) {
+            tredsw_set_error("motif %d: period %d / code %llu out of range (2 <= period <= 20, code < 4^period)", i,
+                             ms[i].period, (unsigned long long)ms[i].code);
+            return false;
+        }
+    for (int32_t c = 0; c < nc; ++c)
+        if (cs[c].length < 0 || cs[c].offset < 0 || (cs[c].length > 0 && (cs[c].line_bases <= 0 || cs[c].line_width < cs[c].line_bases))) {
+            tredsw_set_error("contig %d: bad index entry (length %lld, offset %lld, line %d bases / %d bytes)", c,
+                             (long long)cs[c].length, (long long)cs[c].offset, cs[c].line_bases, cs[c].line_width);
+            return false;
+        }
+    return true;
+}
+
+}  // namespace
+
+extern "C" {
+
+int tredsw_ref_tracts(tredsw_ctx *ctx, const char *fasta_path, const tredsw_fai_entry *contigs, int32_t ncontigs,
+                      const tredsw_motif *motifs, int32_t nmotifs, const tredsw_tract_params *params,
+                      tredsw_tracts **result) {
+    if (!ctx) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
+    if (!tract_args_ok(fasta_path, contigs, ncontigs, motifs, nmotifs, params, result)) return TREDSW_ERR_ARG;
+    *result = nullptr;
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    keep_pool(ctx->device);
+    std::unique_ptr<tredsw_tracts> r(new tredsw_tracts());
+    CudaBackend be;
+    be.stream = ctx->stream;
+    int rc;
+    try { rc = run_ref_tracts(be, r.get(), fasta_path, contigs, ncontigs, motifs, nmotifs, *params); }
+    catch (const std::exception &e) { tredsw_set_error("tredsw_ref_tracts: %s", e.what()); rc = TREDSW_ERR_IO; }
+    ctx->launches += be.launches;
+    be.release();
+    if (rc) return rc;
+    *result = r.release();
+    return TREDSW_OK;
+}
+
+// TEST INFRASTRUCTURE: tredsw_ref_tracts with every kernel body run serially on the host.  Not used by the package.
+int tredsw_ref_tracts_emulate(tredsw_ctx *, const char *fasta_path, const tredsw_fai_entry *contigs, int32_t ncontigs,
+                              const tredsw_motif *motifs, int32_t nmotifs, const tredsw_tract_params *params,
+                              tredsw_tracts **result) {
+    if (!tract_args_ok(fasta_path, contigs, ncontigs, motifs, nmotifs, params, result)) return TREDSW_ERR_ARG;
+    *result = nullptr;
+    std::unique_ptr<tredsw_tracts> r(new tredsw_tracts());
+    HostBackend be;
+    int rc;
+    try { rc = run_ref_tracts(be, r.get(), fasta_path, contigs, ncontigs, motifs, nmotifs, *params); }
+    catch (const std::exception &e) { tredsw_set_error("tredsw_ref_tracts_emulate: %s", e.what()); rc = TREDSW_ERR_IO; }
+    be.release();
+    if (rc) return rc;
+    *result = r.release();
+    return TREDSW_OK;
+}
+
+int tredsw_ref_tracts_view(const tredsw_tracts *r, tredsw_tracts_view *v) {
+    if (!r || !v) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
+    *v = r->view;
+    return TREDSW_OK;
+}
+
+void tredsw_ref_tracts_free(tredsw_tracts *r) { delete r; }
 
 }  // extern "C"

@@ -856,6 +856,33 @@ TG_HD int popc64(uint64_t x) {
 #endif
 }
 
+// A unit of P <= 32 bases (base j at bits 2j): -> the period d of its primitive root (the smallest e dividing P with
+// unit[i] == unit[i - e] for every i >= e); *code the root's canonical code: the smallest rotation of the root and of
+// its reverse complement, 2 bits a base, first base in the most significant bits.  Shared by the IRR classifier and the
+// reference tract scan (ref_tracts_device.cuh), so a profile's motif and a tract's code are one number.
+TG_HD int canonical_root(uint64_t unit, int P, uint64_t *code) {
+    int d = P;
+    for (int e = 1; e < P; ++e) {
+        if (P % e) continue;
+        bool rep = true;
+        for (int i = e; i < P && rep; ++i) rep = ((unit >> (2 * i)) & 3u) == ((unit >> (2 * (i - e))) & 3u);
+        if (rep) { d = e; break; }
+    }
+    uint64_t f = 0, r = 0;
+    for (int i = 0; i < d; ++i) f = (f << 2) | ((unit >> (2 * i)) & 3u);
+    for (int i = d - 1; i >= 0; --i) r = (r << 2) | (3u - ((unit >> (2 * i)) & 3u));
+    const uint64_t mask = d >= 32 ? ~0ull : (1ull << (2 * d)) - 1ull;
+    uint64_t best = f < r ? f : r;
+    for (int t = 1; t < d; ++t) {                       // the other rotations, one base to the left at a time
+        f = ((f << 2) | (f >> (2 * d - 2))) & mask;
+        r = ((r << 2) | (r >> (2 * d - 2))) & mask;
+        if (f < best) best = f;
+        if (r < best) best = r;
+    }
+    *code = best;
+    return d;
+}
+
 // -> the period of the IRR (0: not one); *motif its canonical motif
 template <class Seq>
 TG_HD int irr_classify(const Seq &sq, int L, const IrrParams &pr, uint64_t *motif) {
@@ -906,26 +933,10 @@ TG_HD int irr_classify(const Seq &sq, int L, const IrrParams &pr, uint64_t *moti
         if (c3 > bc) { best = 3; }
         cons |= (uint64_t)best << (2 * j);
     }
-    int d = P;                                          // primitive root: the smallest period that divides P
-    for (int e = 1; e < P; ++e) {
-        if (P % e) continue;
-        bool rep = true;
-        for (int i = e; i < P && rep; ++i) rep = ((cons >> (2 * i)) & 3u) == ((cons >> (2 * (i - e))) & 3u);
-        if (rep) { d = e; break; }
-    }
+    uint64_t code;
+    const int d = canonical_root(cons, P, &code);
     if (d == 1) return 0;                               // homopolymer
-    uint64_t f = 0, r = 0;
-    for (int i = 0; i < d; ++i) f = (f << 2) | ((cons >> (2 * i)) & 3u);
-    for (int i = d - 1; i >= 0; --i) r = (r << 2) | (3u - ((cons >> (2 * i)) & 3u));
-    const uint64_t mask = (1ull << (2 * d)) - 1ull;
-    uint64_t best = f < r ? f : r;
-    for (int t = 1; t < d; ++t) {                       // the other rotations, one base to the left at a time
-        f = ((f << 2) | (f >> (2 * d - 2))) & mask;
-        r = ((r << 2) | (r >> (2 * d - 2))) & mask;
-        if (f < best) best = f;
-        if (r < best) best = r;
-    }
-    *motif = best;
+    *motif = code;
     return d;
 }
 

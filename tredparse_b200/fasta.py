@@ -4,6 +4,7 @@ Random access to a plain-text FASTA file, as `samtools faidx` gives it.
     fa = Fasta("ref.fa")                  # uses ref.fa.fai when it exists, else indexes the file in memory
     fa.fetch("chr4", 3074876, 3074933)    # 0-based, half-open; uppercase bases
     fa.lengths()                          # {contig: length}
+    fa.tracts(["AAGGG", "AGC"])           # every tract of these motifs, found by one GPU scan of the file
 
 The index is the `.fai` format: per record its name (the header up to the first white space), length, the byte
 offset of its first base, and the bases and bytes of each line.  Lines of any width work as long as every line of a
@@ -11,6 +12,23 @@ record but the last has the same width, which is what `samtools faidx` requires 
 memory: nothing is written next to the user's file.  Compressed files (gzip, BGZF) are refused.
 """
 import os
+
+import numpy as np
+
+MIN_REF_UNITS = 3       # copies a reference tract needs (strprofile.locus_for uses the same)
+MIN_TRACT_LEN = 30      # bases a tract needs: BWA-MEM's default minimum alignment score
+
+
+def canonical_code(motif):
+    """the canonical code of a motif: the smallest rotation of it and of its reverse complement, 2 bits a base
+    (A C G T = 0 1 2 3), first base most significant — the code of tredsw_irr_entry.motif and tredsw_tract.code"""
+    motif = motif.upper()
+    rc = motif.translate(str.maketrans("ACGT", "TGCA"))[::-1]
+    best = min(m[i:] + m[:i] for m in (motif, rc) for i in range(len(motif)))
+    code = 0
+    for b in best:
+        code = code * 4 + "ACGT".index(b)
+    return code
 
 
 class Fasta:
@@ -72,6 +90,25 @@ class Fasta:
 
     def lengths(self):
         return {name: e[0] for name, e in self.index.items()}
+
+    def tracts(self, motifs, min_units=MIN_REF_UNITS, min_len=MIN_TRACT_LEN, step_bytes=0, ctx=None, emulate=False):
+        """Every tract of the motifs (strings of 2 to 20 bases; a motif stands for all its rotations on both strands)
+        in the whole file, from one scan on the GPU (``_lib.ref_tracts``, DESIGN §4.5): a maximal stretch of exact
+        back-to-back copies of a unit whose primitive root has the motif's length, at least `min_units` copies and
+        `min_len` bases long, lowercase bases equal to uppercase, anything but ACGT breaking it.  -> dict(contigs:
+        the contig names in FASTA order, tracts: a ``_lib.TRACT_DTYPE`` array by (contig, start, period) with contig
+        an index into contigs, start 0-based, length a whole number of units, code the canonical code; stats: steps,
+        bytes, bases, invalid_bases, tracts, per-step host read and device ms).  ``ctx``: a ``_lib.Context``;
+        ``emulate``: the serial host emulation of the device code (test infrastructure only)."""
+        from . import _lib
+        names = list(self.index)
+        contigs = np.array([self.index[n] for n in names], dtype=np.int64).reshape(-1, 4)
+        fai = np.zeros(len(names), dtype=_lib.FAI_ENTRY_DTYPE)
+        for f, col in zip(("length", "offset", "line_bases", "line_width"), contigs.T):
+            fai[f] = col
+        motifs = sorted({(len(m), canonical_code(m)) for m in motifs})
+        tracts, stats = _lib.ref_tracts(self.path, fai, motifs, min_units, min_len, step_bytes, ctx=ctx, emulate=emulate)
+        return {"contigs": names, "tracts": tracts, "stats": stats}
 
     def fetch(self, contig, start, end):
         """the bases [start, end) of `contig` (0-based), uppercase, clipped to the contig; KeyError for a contig the

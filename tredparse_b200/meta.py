@@ -29,6 +29,18 @@ def location_field(ref=REF):
     return "repeat_location" if ref == REF else "repeat_location." + ref.split("_")[0]
 
 
+def alts_field(ref=REF):
+    """the field that holds a locus' alt regions on reference `ref`, in alts.tsv and in a user row (hg38: alts, hg19:
+    alts.hg19; the _nochr variants use the field of their build): `contig:start-end` regions (0-based, end exclusive)
+    joined by '|', empty for none"""
+    return "alts" if ref == REF else "alts." + ref.split("_")[0]
+
+
+def parse_alts(value):
+    """an alts field -> [(contig, start, end)]"""
+    return [get_region(x) for x in value.split("|")] if value.strip() else []
+
+
 def locus_names(sites=SITES):
     """the names of the catalogue loci and of the user loci in <sites>/*.json, in TREDsRepo's order, without reading
     their rows (a user locus may carry the location of one reference build only)"""
@@ -105,7 +117,8 @@ class TREDsRepo(dict):
             with open(s) as fp:
                 for name, row in json.load(fp).items():
                     name = str(name)
-                    self[name] = TRED(name, row, ref=ref, alt=alts.get(name, []))
+                    alt = parse_alts(row[alts_field(ref)]) if alts_field(ref) in row else alts.get(name, [])
+                    self[name] = TRED(name, row, ref=ref, alt=alt)
                     self.rows[name] = row
                     self.names.append(name)
         if toy:
@@ -132,10 +145,9 @@ class TREDsRepo(dict):
 
     @staticmethod
     def get_alts(ref):
-        field = "alts" if ref == REF else "alts." + ref.split("_")[0]
+        field = alts_field(ref)
         alts = {}
         with open(datafile("alts.tsv")) as fp:
             for row in csv.DictReader(fp, delimiter="\t"):
-                v = row.get(field) or ""
-                alts[row["name"]] = [get_region(x) for x in v.split("|")] if v.strip() else []
+                alts[row["name"]] = parse_alts(row.get(field) or "")
         return alts

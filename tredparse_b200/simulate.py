@@ -387,13 +387,16 @@ def write_fasta(path, contigs, width=60, fai=False):
 
 
 def reference_records(seq, tid, rep_start, rep_end, motif, alleles, readlen=150, cov_per_hap=15.0, flank=2000,
-                      error=0.005, seed=0, tag=""):
+                      error=0.005, seed=0, tag="", mismap_fraction=0.0, mismap_to=()):
     """Paired reads of a locus whose reference tract is seq[rep_start:rep_end] (0-based): haplotype h = the reference's
     `flank` bases before the tract, h copies of `motif`, its `flank` bases after the tract.  Fragment lengths and
     errors follow ``locus_records``; reads are placed as ``locus_records`` and ``expansion_records`` place them:
       * pairs with no read wholly inside the repeat: ``<readlen>M`` proper pairs, MAPQ 60, flanks mapped one to one
         and the repeat clamped to the reference's tract;
-      * an in-repeat read whose mate is not one: unmapped at its mate's position, the mate flagged 0x8;
+      * an in-repeat read whose mate is not one: unmapped at its mate's position, the mate flagged 0x8; with probability
+        `mismap_fraction` it is instead mismapped at MAPQ 0 at a random position of a decoy tract (tid, start, end)
+        drawn from `mismap_to`, its mate pointing there (as ``expansion_records``); without decoys no random number is
+        drawn for it;
       * both reads inside the repeat: both unmapped, in the unmapped tail (tid -1).
     Records with a mapped mate carry its MAPQ as an ``MQ`` tag.  Not sorted (``coordinate_sort``); write them with
     ``bamio.write_bam(..., aux=True)``."""
@@ -439,6 +442,14 @@ def reference_records(seq, tid, rep_start, rep_end, motif, alleles, readlen=150,
                                                seqs[i]))
             else:
                 i, j = (0, 1) if irr[0] else (1, 0)          # i: the in-repeat read, j: its anchor
+                if mismap_to and rng.random() < mismap_fraction:
+                    mt, ms, me = mismap_to[int(rng.integers(len(mismap_to)))]
+                    mp = int(rng.integers(ms, me))
+                    recs.append(AlignedSegment(name, 0x1 | seg[i] | strand[i], mt, mp, 0, [(0, readlen)], tid, p[j], 0,
+                                               seqs[i], aux=_mq_aux(60)))
+                    recs.append(AlignedSegment(name, 0x1 | seg[j] | strand[j], tid, p[j], 60, [(0, readlen)], mt, mp,
+                                               0, seqs[j], aux=_mq_aux(0)))
+                    continue
                 recs.append(AlignedSegment(name, 0x1 | 0x4 | seg[i] | strand[i], tid, p[j], 0, [], tid, p[j], 0,
                                            seqs[i], aux=_mq_aux(60)))
                 recs.append(AlignedSegment(name, 0x1 | 0x8 | seg[j] | strand[j], tid, p[j], 60, [(0, readlen)], tid,

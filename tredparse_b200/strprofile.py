@@ -10,7 +10,7 @@ with more anchored IRRs in a region than the rest of the cohort — expansions o
     python -m tredparse_b200.strprofile profile x.bam [y.bam ... | -] --workdir w
     python -m tredparse_b200.tred samples.csv --workdir w --str-profile     # or: catalogue calls and profiles, one read
     python -m tredparse_b200.strprofile outliers w/*.str_profile.json --tsv out.tsv
-    python -m tredparse_b200.strprofile loci out.tsv --fasta ref.fa --profiles w/*.str_profile.json
+    python -m tredparse_b200.strprofile loci out.tsv --fasta ref.fa --profiles w/*.str_profile.json [--alts]
     python -m tredparse_b200.tred samples.csv --tred <name> ...          # from the directory that holds sites/
 
 Definitions (include/tredsw.h, tredsw_irr_params):
@@ -31,14 +31,16 @@ import os
 import sys
 
 from . import _lib
+from .fasta import MIN_REF_UNITS, MIN_TRACT_LEN
 from .ingest import BamIngest, IrrParams, is_stream, scan_sample
 
 MIN_ANCHOR_MAPQ = 50
 MERGE_DISTANCE = 500
 NORM_DEPTH = 40.0
 LOCUS_WINDOW = 1000
-MIN_REF_UNITS = 3
 LOCUS_FLANK = 18
+ALT_SPAN = 1000         # a locus' own read window: its tract +- this many bases
+MAX_ALTS = 100          # the catalogue's largest count of alt regions (FXTAS)
 _RC = str.maketrans("ACGT", "TGCA")
 
 
@@ -279,6 +281,35 @@ def discover_loci(rows, fasta, read_length, min_z=3.0, window=LOCUS_WINDOW, min_
     return sites, skipped
 
 
+def alt_regions_for(locus_row, tracts, read_length, max_alts=MAX_ALTS, ref=None):
+    """The alt regions of a locus row (``locus_for``), from the tracts of a reference scan (``Fasta.tracts``): the
+    regions an aligner may place its in-repeat reads on, for the `alts` field of the row (``meta.alts_field``).
+
+    The tracts of the row's motif, less those that overlap the locus' own read window (its tract +- ALT_SPAN bases on
+    its contig: those reads are fetched already), merged on a contig while the gap to the next tract is less than
+    `read_length` (a read must not be fetched twice); the `max_alts` regions with the longest tracts are kept (ties:
+    FASTA contig order, then start).  -> the kept regions in (contig, start) order as ``contig:start-end`` (0-based,
+    end exclusive, how ``tred.alt_regions`` hands them to the fetch) joined by '|'; empty when none qualifies."""
+    from .fasta import canonical_code
+    from .meta import REF, get_region, location_field
+    contig, first, last = get_region(locus_row[location_field(ref or REF)])
+    motif = locus_row["motif"]
+    names, t = tracts["contigs"], tracts["tracts"]
+    t = t[(t["period"] == len(motif)) & (t["code"] == canonical_code(motif))]
+    lo, hi = first - 1 - ALT_SPAN, last + ALT_SPAN
+    regions = []                                        # [contig index, start, end, longest tract]
+    for c, s, n in zip(t["contig"].tolist(), t["start"].tolist(), t["length"].tolist()):
+        if names[c] == contig and s < hi and s + n > lo:
+            continue
+        if regions and regions[-1][0] == c and s - regions[-1][2] < read_length:
+            regions[-1][2] = max(regions[-1][2], s + n)
+            regions[-1][3] = max(regions[-1][3], n)
+        else:
+            regions.append([c, s, s + n, n])
+    kept = sorted(regions, key=lambda r: (-r[3], r[0], r[1]))[:max_alts]
+    return "|".join("{}:{}-{}".format(names[c], s, e) for c, s, e, _ in sorted(kept))
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(prog="python -m tredparse_b200.strprofile",
                                  description="STR profiles of whole BAMs (in-repeat reads found on the GPU) and their "
@@ -318,6 +349,12 @@ def main(argv=None):
     pl.add_argument("--window", type=int, default=LOCUS_WINDOW, help="bases searched either side of a region")
     pl.add_argument("--min-ref-units", type=int, default=MIN_REF_UNITS)
     pl.add_argument("--out", default=os.path.join("sites", "discovered.json"))
+    pl.add_argument("--alts", action="store_true",
+                    help="give every locus the reference's other tracts of its motif as alt regions, where an aligner "
+                         "may have placed its in-repeat reads (one GPU scan of the FASTA)")
+    pl.add_argument("--max-alts", type=int, default=MAX_ALTS, help="alt regions kept per locus (longest tracts first)")
+    pl.add_argument("--min-alt-len", type=int, default=MIN_TRACT_LEN,
+                    help="bases an alt tract needs (default: BWA-MEM's minimum alignment score)")
     a = ap.parse_args(argv)
     if a.cmd == "loci":
         from .fasta import Fasta
@@ -339,6 +376,16 @@ def main(argv=None):
             where = r["contig"] if r["start"] is None else "{}:{}-{}".format(r["contig"], r["start"], r["end"])
             print("skipped {} {} (z {:.4f}): {}".format(where, r["motif"], r["z"], why), file=sys.stderr)
         print("{} rows below --min-z {}".format(below, a.min_z), file=sys.stderr)
+        if a.alts and sites:
+            from .meta import alts_field
+            try:
+                tracts = fasta.tracts({row["motif"] for row in sites.values()}, min_len=a.min_alt_len)
+            except _lib.TredswError as e:
+                ap.exit(1, "loci --alts: {}\n".format(e))
+            for name, row in sites.items():
+                row[alts_field(a.ref)] = alt_regions_for(row, tracts, read_length, a.max_alts, a.ref)
+                n = len(row[alts_field(a.ref)].split("|")) if row[alts_field(a.ref)] else 0
+                print("{}: {} alt regions".format(name, n), file=sys.stderr)
         if os.path.dirname(a.out):
             os.makedirs(os.path.dirname(a.out), exist_ok=True)
         with open(a.out, "w") as fp:

@@ -144,10 +144,10 @@ def runBam(inputParams):
 
 def alt_regions(tred, ref, alts, clip):
     """The mis-mapping regions whose reads are added to a locus (bam_parser.py:215-243): none without alts or with
-    clipped reads; contig names without the 'chr' prefix on a '_nochr' reference."""
+    clipped reads; on a '_nochr' reference a contig name loses its 'chr' prefix (a name without one is kept)."""
     if not alts or clip:
         return []
-    return [(c[3:] if "nochr" in ref else c, s, e) for (c, s, e) in tred.alt]
+    return [(c[3:] if "nochr" in ref and c.startswith("chr") else c, s, e) for (c, s, e) in tred.alt]
 
 
 def locus_evidence(ing, tred, readlen, alts, clip, ref):
