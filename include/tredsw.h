@@ -546,7 +546,7 @@ int tredsw_irr_classify_host(const int8_t *codes, int32_t len, const tredsw_irr_
 
 /* ------------------------------------------------------------------------------------------------
  * (E) Reference tract scan (csrc/ref_tracts_device.cuh, bgzf_gpu.cu; DESIGN §4.5): every tract of the requested
- * motifs in a plain-text FASTA, for the alt regions of discovered loci.  For a period k (2..20), a maximal stretch
+ * motifs in a FASTA, plain text or BGZF.  For a period k (2..20), a maximal stretch
  * [a, b) of bases in ACGTacgt (compared case-insensitively; N, IUPAC codes and anything else break it) with
  * s[j] == s[j + k] for every j in [a, b - k) gives the tract [a, a + c k), c = floor((b - a) / k), unit s[a, a + k) in
  * upper case.  It is kept when the unit's primitive root has period k, c >= min_units, c k >= min_len and the unit's
@@ -557,6 +557,14 @@ int tredsw_irr_classify_host(const int8_t *codes, int32_t len, const tredsw_irr_
  * step_bytes of text (0: 256 MiB; a larger contig is a step of its own), the read of step k + 1 on a host thread
  * while the device packs and scans step k.  A base position holding '\n', '\r' or '>' (the index does not fit the
  * file) or a file shorter than its index is TREDSW_ERR_IO; every error leaves no result.  No CPU fallback.
+ *
+ * The format comes from the file: one that starts with the gzip magic is read as BGZF (bgzip), anything else as text.
+ * For BGZF the .fai offsets are offsets into the inflated text (as samtools writes them), the call first walks the
+ * block headers (the .gzi is not read), and each step reads the compressed blocks from the one holding its first base
+ * to the one holding its last base and inflates them on the device with CRC-32 checks.  A block shared by two steps
+ * is read and inflated twice.  A block that is truncated, not BGZF (a plain gzip file), does not inflate or fails its
+ * CRC-32 / length check, and an index that reaches past the inflated end are TREDSW_ERR_IO; the message names the
+ * file and, where there is one, the block's file offset.
  * ---------------------------------------------------------------------------------------------- */
 typedef struct { int64_t length, offset; int32_t line_bases, line_width; } tredsw_fai_entry;   /* a .fai row */
 typedef struct { int32_t period, reserved_; uint64_t code; } tredsw_motif;     /* a canonical code of `period` bases */
@@ -566,10 +574,15 @@ typedef struct tredsw_tracts tredsw_tracts;
 typedef struct {                /* host arrays, valid until tredsw_ref_tracts_free */
     int64_t n_tracts;
     const tredsw_tract *tracts; /* by (contig, start, period); contig indexes the `contigs` of the call */
-    int64_t steps, bytes, bases, invalid_bases;   /* bytes: FASTA text read; invalid: bases not in ACGTacgt */
-    const double *step_read_ms, *step_device_ms;  /* per step: host read (overlaps the previous step's device work),
-                                                     device work (upload, kernels, copies back) */
+    int64_t steps, bytes, bases, invalid_bases;   /* bytes: FASTA text handed to the kernels (BGZF: the inflated
+                                                     bytes of every step's blocks, headers included); invalid: bases
+                                                     not in ACGTacgt */
+    const double *step_read_ms, *step_device_ms;  /* per step: host read (overlaps the previous step's device work;
+                                                     BGZF: read and framing), device work (upload, inflation, kernels,
+                                                     copies back) */
     double ms_total;
+    int64_t comp_bytes, blocks;                   /* BGZF: compressed bytes read and blocks inflated, a block shared
+                                                     by two steps counted twice; 0 for text */
 } tredsw_tracts_view;
 int tredsw_ref_tracts(tredsw_ctx *ctx, const char *fasta_path, const tredsw_fai_entry *contigs, int32_t ncontigs,
                       const tredsw_motif *motifs, int32_t nmotifs, const tredsw_tract_params *params,

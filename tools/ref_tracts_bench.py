@@ -10,10 +10,17 @@ of the later ones.  The card's name, power limit and max SM clock are read in th
 temporary directory, never into the repository, and is read from the page cache (the run writes it just before): a
 cold-cache read and a real reference genome are not measured.
 
-    python tools/ref_tracts_bench.py [--gbp 3.1] [--reps 3] [--step-mib 256] [--out profiles/r3_ref_tracts_bench.json]
+--bgzip adds a second arm: a BGZF copy of the same genome (64 KiB blocks at zlib level 6, as `bgzip` writes it; the
+blocks are compressed on every host core, since they are independent) with the same .fai, whose blocks the scan
+inflates on the GPU.  The two arms alternate call by call, and each reports its first call and the best of the later
+ones.  The synthetic genome (uniform random bases) compresses less well than hg38, whose repeats and soft-masking
+give DEFLATE more to work with: the compressed-to-text ratio here is not hg38's.
+
+    python tools/ref_tracts_bench.py [--gbp 3.1] [--reps 3] [--step-mib 256] [--bgzip] [--out profiles/r3_ref_tracts_bench.json]
 (without --out the result line is only printed)
 """
 import argparse
+import concurrent.futures
 import json
 import os
 import shutil
@@ -76,11 +83,29 @@ def write_genome(path, gbp, seed=0, width=60):
     return total
 
 
+def bgzip(src, dst, level=6, block=0xFF00, chunk_blocks=1024):
+    """a BGZF copy of src (the .fai copied too: its offsets are those of the inflated text), blocks compressed on a
+    thread pool (zlib releases the GIL)"""
+    from tredparse_b200.bamio import bgzf_block
+    with open(src, "rb") as fi, open(dst, "wb") as fo, \
+            concurrent.futures.ThreadPoolExecutor(os.cpu_count() or 1) as pool:
+        while True:
+            data = fi.read(block * chunk_blocks)
+            if not data:
+                break
+            parts = [data[i:i + block] for i in range(0, len(data), block)]
+            for b in pool.map(lambda x: bgzf_block(x, level), parts):
+                fo.write(b)
+        fo.write(bgzf_block(b"", level))
+    shutil.copyfile(src + ".fai", dst + ".fai")
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gbp", type=float, default=3.1)
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--step-mib", type=int, default=256)
+    ap.add_argument("--bgzip", action="store_true", help="also scan a BGZF copy of the genome, the arms alternating")
     ap.add_argument("--out", default=None)
     a = ap.parse_args()
     from tredparse_b200 import _lib
@@ -92,18 +117,23 @@ def main():
         t0 = time.time()
         bases = write_genome(path, a.gbp)
         t_write = time.time() - t0
-        fa = Fasta(path)
-        calls = []
-        for _ in range(a.reps + 1):
-            t0 = time.perf_counter()
-            r = fa.tracts(MOTIFS, step_bytes=a.step_mib << 20, ctx=ctx)
-            calls.append((time.perf_counter() - t0, r))
-        first, later = calls[0], calls[1:]
-        best = min(later, key=lambda c: c[0]) if later else first
-        if later:
-            for _, r in later:
-                assert np.array_equal(r["tracts"], first[1]["tracts"])
-        st = best[1]["stats"]
+        paths = {"text": path}
+        if a.bgzip:
+            t0 = time.time()
+            bgzip(path, path + ".gz")
+            t_bgzip = time.time() - t0
+            paths["bgzf"] = path + ".gz"
+        fas = {arm: Fasta(p) for arm, p in paths.items()}
+        calls = {arm: [] for arm in paths}
+        for _ in range(a.reps + 1):                     # the arms alternate call by call
+            for arm, fa in fas.items():
+                t0 = time.perf_counter()
+                r = fa.tracts(MOTIFS, step_bytes=a.step_mib << 20, ctx=ctx)
+                calls[arm].append((time.perf_counter() - t0, r))
+        ref = calls["text"][0][1]["tracts"]
+        for arm in calls:
+            for _, r in calls[arm]:
+                assert np.array_equal(r["tracts"], ref), arm
 
         def summary(wall, res):
             s = res["stats"]
@@ -111,14 +141,30 @@ def main():
                     "text_GB_per_s": round(s["bytes"] / wall / 1e9, 3),
                     "host_read_ms_sum": round(sum(s["step_read_ms"]), 2),
                     "device_ms_sum": round(sum(s["step_device_ms"]), 2)}
-        out = {"bench": "ref_tracts", "card": card(), "gbp": a.gbp, "bases": bases, "file_bytes": os.path.getsize(path),
-               "write_s": round(t_write, 1), "motifs": len(MOTIFS), "step_mib": a.step_mib,
-               "steps": st["steps"], "text_bytes": st["bytes"], "invalid_bases": st["invalid_bases"],
-               "tracts": st["tracts"], "first_call": summary(*first), "best_later_call": summary(*best),
-               "later_walls_s": [round(w, 4) for w, _ in later],
-               "per_step_best": [{"read_ms": round(x, 2), "device_ms": round(y, 2)}
-                                 for x, y in zip(st["step_read_ms"], st["step_device_ms"])],
-               "page_cache": "warm (file written in the same run); cold cache not measured"}
+
+        def arm_result(arm):
+            first, later = calls[arm][0], calls[arm][1:]
+            best = min(later, key=lambda c: c[0]) if later else first
+            st = best[1]["stats"]
+            return {"file_bytes": os.path.getsize(paths[arm]), "steps": st["steps"], "text_bytes": st["bytes"],
+                    "comp_bytes": st["comp_bytes"], "blocks": st["blocks"], "invalid_bases": st["invalid_bases"],
+                    "tracts": st["tracts"], "first_call": summary(*first), "best_later_call": summary(*best),
+                    "later_walls_s": [round(w, 4) for w, _ in later],
+                    "per_step_best": [{"read_ms": round(x, 2), "device_ms": round(y, 2)}
+                                      for x, y in zip(st["step_read_ms"], st["step_device_ms"])]}
+
+        head = {"card": card(), "gbp": a.gbp, "bases": bases, "write_s": round(t_write, 1), "motifs": len(MOTIFS),
+                "step_mib": a.step_mib}
+        cache = "warm (files written in the same run); cold cache not measured"
+        if not a.bgzip:
+            out = dict({"bench": "ref_tracts"}, **head, **arm_result("text"), page_cache=cache.replace("files", "file"))
+            del out["comp_bytes"], out["blocks"]
+        else:
+            arms = {arm: arm_result(arm) for arm in paths}
+            out = dict({"bench": "ref_tracts_bgzf"}, **head, bgzip_s=round(t_bgzip, 1), arms=arms,
+                       comp_ratio=round(arms["bgzf"]["file_bytes"] / arms["text"]["file_bytes"], 4),
+                       comp_ratio_note="uniform random bases with soft-masking and N runs: not hg38's ratio",
+                       tracts_equal_across_arms=True, page_cache=cache)
     finally:
         shutil.rmtree(d, ignore_errors=True)
     line = json.dumps(out)

@@ -105,7 +105,7 @@ class TractsView(ctypes.Structure):
     _fields_ = [("n_tracts", ctypes.c_int64), ("tracts", ctypes.c_void_p), ("steps", ctypes.c_int64),
                 ("bytes", ctypes.c_int64), ("bases", ctypes.c_int64), ("invalid_bases", ctypes.c_int64),
                 ("step_read_ms", ctypes.POINTER(ctypes.c_double)), ("step_device_ms", ctypes.POINTER(ctypes.c_double)),
-                ("ms_total", ctypes.c_double)]
+                ("ms_total", ctypes.c_double), ("comp_bytes", ctypes.c_int64), ("blocks", ctypes.c_int64)]
 
 
 assert GRID_PROBLEM_DTYPE.itemsize == ctypes.sizeof(GridProblem)
@@ -185,9 +185,9 @@ def check(rc, what):
 
 
 def ref_tracts(path, contigs, motifs, min_units, min_len, step_bytes=0, ctx=None, emulate=False):
-    """Every tract of `motifs` in the FASTA at `path` (tredsw_ref_tracts, DESIGN §4.5).  contigs: FAI_ENTRY_DTYPE rows
-    in FASTA order; motifs: (period, canonical code) pairs.  -> (TRACT_DTYPE array by (contig, start, period), stats
-    dict).  ``ctx``: a Context (default the process's); ``emulate`` runs the serial host emulation of the device code
+    """Every tract of `motifs` in the FASTA at `path`, plain text or BGZF (tredsw_ref_tracts, DESIGN §4.5).  contigs:
+    FAI_ENTRY_DTYPE rows in FASTA order; motifs: (period, canonical code) pairs.  -> (TRACT_DTYPE array by (contig,
+    start, period), stats dict; its comp_bytes and blocks are 0 for a text file).  ``ctx``: a Context (default the process's); ``emulate`` runs the serial host emulation of the device code
     instead — test infrastructure only.  Raises TredswError (no device, I/O, an index that does not fit the file)."""
     lib = load()
     cs = np.ascontiguousarray(contigs, dtype=FAI_ENTRY_DTYPE)
@@ -214,7 +214,8 @@ def ref_tracts(path, contigs, motifs, min_units, min_len, step_bytes=0, ctx=None
         stats = {"steps": int(v.steps), "bytes": int(v.bytes), "bases": int(v.bases),
                  "invalid_bases": int(v.invalid_bases), "tracts": n, "ms_total": float(v.ms_total),
                  "step_read_ms": [float(v.step_read_ms[i]) for i in range(v.steps)],
-                 "step_device_ms": [float(v.step_device_ms[i]) for i in range(v.steps)]}
+                 "step_device_ms": [float(v.step_device_ms[i]) for i in range(v.steps)],
+                 "comp_bytes": int(v.comp_bytes), "blocks": int(v.blocks)}
     finally:
         lib.tredsw_ref_tracts_free(res)
     return tracts, stats

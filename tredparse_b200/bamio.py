@@ -239,25 +239,70 @@ class BGZFReader:
         return b"".join(out)
 
 
+def bgzf_block(data: bytes, level: int = 6) -> bytes:
+    """one BGZF block holding `data` (at most 0xFF00 bytes); blocks are independent, so they can be made in parallel"""
+    comp = zlib.compressobj(level, zlib.DEFLATED, -15)
+    cdata = comp.compress(data) + comp.flush()
+    return (struct.pack("<BBBBIBBHBBHH", 31, 139, 8, 4, 0, 0, 255, 6, 66, 67, 2, len(cdata) + 25) + cdata +
+            struct.pack("<II", zlib.crc32(data) & 0xFFFFFFFF, len(data)))
+
+
+def bgzf_blocks(path: str) -> List[Tuple[int, int, int]]:
+    """(compressed offset, inflated offset, inflated size) of every block of a BGZF file, from one walk of the block
+    headers: BSIZE from each header, ISIZE from each block's last 4 bytes.  Nothing is inflated.  ValueError for a
+    file that is not BGZF, IOError for a truncated one."""
+    out = []
+    coff = uoff = 0
+    with open(path, "rb") as fh:
+        size = os.fstat(fh.fileno()).st_size
+        while coff < size:
+            fh.seek(coff)
+            head = fh.read(12)
+            if len(head) < 12:
+                raise IOError("{}: truncated BGZF block header at offset {}".format(path, coff))
+            id1, id2, _cm, flg, _mtime, _xfl, _os, xlen = struct.unpack("<BBBBIBBH", head)
+            if id1 != 31 or id2 != 139 or not (flg & 4):
+                raise ValueError("{}: not a BGZF block at offset {}".format(path, coff))
+            extra = fh.read(xlen)
+            bsize, off = None, 0
+            while off + 4 <= len(extra):
+                si1, si2, slen = struct.unpack_from("<BBH", extra, off)
+                if si1 == 66 and si2 == 67 and off + 6 <= len(extra):
+                    bsize = struct.unpack_from("<H", extra, off + 4)[0] + 1
+                off += 4 + slen
+            if len(extra) < xlen:
+                raise IOError("{}: truncated BGZF block header at offset {}".format(path, coff))
+            if bsize is None or bsize < xlen + 20:
+                raise ValueError("{}: BGZF block without a valid BC subfield at offset {}".format(path, coff))
+            if coff + bsize > size:
+                raise IOError("{}: truncated BGZF block at offset {}".format(path, coff))
+            fh.seek(coff + bsize - 4)
+            isize = struct.unpack("<I", fh.read(4))[0]
+            out.append((coff, uoff, isize))
+            coff += bsize
+            uoff += isize
+    return out
+
+
 class BGZFWriter:
-    def __init__(self, path: str, level: int = 6):
+    """`block_size` uncompressed bytes per block (at most 0xFF00, what htslib uses, so a stored block fits)"""
+    def __init__(self, path: str, level: int = 6, block_size: int = 0xFF00):
+        if not 0 < block_size <= 0xFF00:
+            raise ValueError("block_size must be in [1, 0xFF00]")
         self.fh = open(path, "wb")
         self.buf = bytearray()
         self.level = level
+        self.block_size = block_size
 
     def write(self, data: bytes):
         self.buf += data
-        while len(self.buf) >= 0xFF00:
-            self._flush_block(bytes(self.buf[:0xFF00]))
-            del self.buf[:0xFF00]
+        n = self.block_size
+        while len(self.buf) >= n:
+            self._flush_block(bytes(self.buf[:n]))
+            del self.buf[:n]
 
     def _flush_block(self, data: bytes):
-        comp = zlib.compressobj(self.level, zlib.DEFLATED, -15)
-        cdata = comp.compress(data) + comp.flush()
-        bsize = len(cdata) + 25
-        self.fh.write(struct.pack("<BBBBIBBHBBHH", 31, 139, 8, 4, 0, 0, 255, 6, 66, 67, 2, bsize))
-        self.fh.write(cdata)
-        self.fh.write(struct.pack("<II", zlib.crc32(data) & 0xFFFFFFFF, len(data)))
+        self.fh.write(bgzf_block(data, self.level))
 
     def tell(self) -> int:
         """Virtual offset of the next byte to be written."""

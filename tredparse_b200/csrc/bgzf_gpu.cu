@@ -391,7 +391,8 @@ double now_ms() { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv
 // The BGZF framing of the block at h, `avail` bytes of which are at hand: 1 parsed, 0 the block is not all there,
 // -1 not a valid block (*why says what is wrong or missing).
 struct BgzfFrame { int xlen, bsize /* bytes of the whole block */, clen; uint32_t crc, isize; };
-int parse_bgzf_block(const uint8_t *h, int64_t avail, BgzfFrame *f, const char **why) {
+// The header alone (xlen, bsize, clen): the same results, with the block's end not needed.
+int parse_bgzf_header(const uint8_t *h, int64_t avail, BgzfFrame *f, const char **why) {
     if (avail < 18) { *why = "truncated BGZF block header"; return 0; }
     if (h[0] != 31 || h[1] != 139 || !(h[3] & 4)) { *why = "not a BGZF block"; return -1; }
     f->xlen = h[10] | (h[11] << 8);
@@ -406,6 +407,11 @@ int parse_bgzf_block(const uint8_t *h, int64_t avail, BgzfFrame *f, const char *
     f->clen = bsize - f->xlen - 19;
     if (f->clen < 0) { *why = "bad BGZF block size"; return -1; }
     f->bsize = bsize + 1;
+    return 1;
+}
+int parse_bgzf_block(const uint8_t *h, int64_t avail, BgzfFrame *f, const char **why) {
+    const int rc = parse_bgzf_header(h, avail, f, why);
+    if (rc != 1) return rc;
     if (f->bsize > avail) { *why = "truncated BGZF block"; return 0; }
     memcpy(&f->crc, h + f->bsize - 8, 4); memcpy(&f->isize, h + f->bsize - 4, 4);
     if (f->isize > 65536) { *why = "BGZF block larger than 64 KiB"; return -1; }
@@ -1627,7 +1633,7 @@ int tredsw_inflate_raw_device_code(const uint8_t *in, int64_t in_len, uint8_t *o
 }  // extern "C"
 
 // ---------------------------------------------------------------------------------------------------------------
-// the reference tract scan: every tract of the requested motifs in a plain-text FASTA (ref_tracts_device.cuh)
+// the reference tract scan: every tract of the requested motifs in a FASTA, plain text or BGZF (ref_tracts_device.cuh)
 // ---------------------------------------------------------------------------------------------------------------
 struct tredsw_tracts {
     std::vector<TractOut> tracts;
@@ -1646,11 +1652,28 @@ int64_t fai_text_bytes(const tredsw_fai_entry &c) {     // bytes from a contig's
     return last / c.line_bases * c.line_width + last % c.line_bases + 1;
 }
 
-struct TractStep {                  // contigs [c0, c1) of the call, their text in one page-locked buffer
-    int32_t c0 = 0, c1 = 0;
-    int64_t bytes = 0;
-    uint8_t *text = nullptr;
-    const char *why = nullptr;      // I/O error
+int64_t pread_full(int fd, uint8_t *dst, int64_t n, int64_t off) {     // -> the bytes read (< n: end of file or error)
+    int64_t got = 0;
+    while (got < n) {
+        const ssize_t k = pread(fd, dst + got, (size_t)(n - got), (off_t)(off + got));
+        if (k <= 0) break;
+        got += k;
+    }
+    return got;
+}
+
+// One block of a BGZF FASTA, from the walk of its headers: compressed offset and size, inflated offset and size.  The
+// .fai of a bgzipped FASTA gives inflated offsets (samtools writes it so); the .gzi is not read.
+struct TractBlock { int64_t coff, uoff; int32_t bsize; uint32_t isize; };
+
+struct TractStep {                  // contigs [c0, c1) of the call; of a BGZF file, the blocks [b0, b1) that hold them
+    int32_t c0 = 0, c1 = 0, b0 = 0, b1 = 0;
+    int64_t bytes = 0;              // text handed to the kernels: the contigs' text, or the inflated blocks [b0, b1)
+    int64_t comp_bytes = 0;         // BGZF: the compressed blocks [b0, b1)
+    uint8_t *buf = nullptr;         // page-locked: the text, or the compressed blocks
+    std::vector<BlockDesc> blocks;  // BGZF: in_off into buf, out_off from block b0's first inflated byte
+    const char *why = nullptr;      // I/O or framing error
+    int64_t at = -1;                // the file offset of the block it concerns, where there is one
     double ms = 0;                  // host read time
 };
 
@@ -1660,16 +1683,109 @@ void read_tract_step(int fd, const tredsw_fai_entry *cs, TractStep *st) {
     int64_t at = 0;
     for (int32_t c = st->c0; c < st->c1 && !st->why; ++c) {
         const int64_t n = fai_text_bytes(cs[c]);
-        int64_t got = 0;
-        while (got < n) {
-            const ssize_t k = pread(fd, st->text + at + got, (size_t)(n - got), (off_t)(cs[c].offset + got));
-            if (k <= 0) break;
-            got += k;
-        }
-        if (got < n) st->why = "the file is shorter than its index says";
+        if (pread_full(fd, st->buf + at, n, cs[c].offset) < n) st->why = "the file is shorter than its index says";
         at += n;
     }
     st->ms = now_ms() - t0;
+}
+
+// A BGZF step: its compressed blocks in one read, each framed again and checked against the walk.
+void read_bgzf_step(int fd, const TractBlock *tb, TractStep *st) {
+    const double t0 = now_ms();
+    st->why = nullptr; st->at = -1;
+    st->blocks.clear();
+    const int64_t c0 = st->b1 > st->b0 ? tb[st->b0].coff : 0, n = st->comp_bytes;
+    const int64_t got = pread_full(fd, st->buf, n, c0);
+    if (got < n) { st->why = "the file is shorter than its BGZF blocks"; st->at = c0 + got; }
+    for (int32_t b = st->b0; b < st->b1 && !st->why; ++b) {
+        const int64_t o = tb[b].coff - c0;
+        BgzfFrame fr;
+        const char *why = nullptr;
+        if (parse_bgzf_block(st->buf + o, n - o, &fr, &why) != 1 || fr.bsize != tb[b].bsize || fr.isize != tb[b].isize) {
+            st->why = why ? why : "the BGZF framing differs from the block walk (the file changed)";
+            st->at = tb[b].coff;
+            break;
+        }
+        BlockDesc d;
+        d.in_off = o + 12 + fr.xlen; d.out_off = tb[b].uoff - tb[st->b0].uoff;
+        d.clen = (uint32_t)fr.clen; d.isize = fr.isize; d.crc = fr.crc; d.pad_ = 0;
+        st->blocks.push_back(d);
+    }
+    st->ms = now_ms() - t0;
+}
+
+// The block table of a BGZF file: one pass over the block headers, BSIZE from each header and ISIZE from each block's
+// last 4 bytes (one read per block: a block's ISIZE and the next block's header).  TREDSW_ERR_IO names the offset of a
+// block that is truncated or not BGZF (a plain gzip file fails here).
+int walk_bgzf(int fd, const char *path, std::vector<TractBlock> *tb) {
+    struct stat sb;
+    if (fstat(fd, &sb) != 0) { tredsw_set_error("%s: cannot stat: %s", path, strerror(errno)); return TREDSW_ERR_IO; }
+    const int64_t size = (int64_t)sb.st_size;
+    auto fail = [&](const char *why, int64_t at) {
+        tredsw_set_error("%s: %s at offset %lld", path, why, (long long)at);
+        return TREDSW_ERR_IO;
+    };
+    std::vector<uint8_t> h(4 + 64);                     // [ISIZE of the block before | the header of the block at o]
+    int64_t o = 0, u = 0, n = pread_full(fd, h.data() + 4, std::min<int64_t>(64, size), 0);
+    while (o < size) {
+        const int64_t need = n >= 12 ? 12 + (h[4 + 10] | (h[4 + 11] << 8)) : 18;     // extra subfields beyond BC
+        if (need > n && o + n < size) {
+            h.resize((size_t)(4 + need));
+            n = pread_full(fd, h.data() + 4, std::min(need, size - o), o);
+        }
+        BgzfFrame fr;
+        const char *why = nullptr;
+        if (parse_bgzf_header(h.data() + 4, n, &fr, &why) != 1) return fail(why, o);
+        const int64_t e = o + fr.bsize;
+        if (e > size) return fail("truncated BGZF block", o);
+        const int64_t want = 4 + std::min<int64_t>(64, size - e);
+        if (h.size() < 4 + 64) h.resize(4 + 64);
+        if (pread_full(fd, h.data(), want, e - 4) < want) return fail("short read", o);
+        uint32_t isize;
+        memcpy(&isize, h.data(), 4);
+        if (isize > 65536) return fail("BGZF block larger than 64 KiB", o);
+        tb->push_back(TractBlock{o, u, fr.bsize, isize});
+        u += isize;
+        o = e;
+        n = want - 4;
+    }
+    return TREDSW_OK;
+}
+
+// The blocks of every step of a BGZF file: from the block holding the step's first text byte to the one holding its
+// last (a block two steps share is read and inflated by both).  An index that reaches past the inflated end is
+// TREDSW_ERR_IO before anything is read.
+int plan_bgzf_steps(const char *path, const std::vector<TractBlock> &tb, const tredsw_fai_entry *cs,
+                    std::vector<TractStep> &steps) {
+    const int64_t total = tb.empty() ? 0 : tb.back().uoff + tb.back().isize;
+    auto block_of = [&](int64_t x) {                    // the last block starting at or before x (a non-empty one)
+        return (int32_t)(std::upper_bound(tb.begin(), tb.end(), x, [](int64_t v, const TractBlock &b) { return v < b.uoff; })
+                         - tb.begin()) - 1;
+    };
+    for (TractStep &st : steps) {
+        int64_t lo = -1, hi = -1;                       // the step's first and last text byte
+        for (int32_t c = st.c0; c < st.c1; ++c) {
+            const int64_t n = fai_text_bytes(cs[c]);
+            if (!n) continue;
+            if (cs[c].offset + n > total) {
+                tredsw_set_error("%s: contig %d ends at inflated byte %lld, past the end of the inflated text (%lld "
+                                 "bytes): the index does not fit the file", path, c, (long long)(cs[c].offset + n),
+                                 (long long)total);
+                return TREDSW_ERR_IO;
+            }
+            lo = lo < 0 ? cs[c].offset : std::min(lo, cs[c].offset);
+            hi = std::max(hi, cs[c].offset + n - 1);
+        }
+        st.bytes = st.comp_bytes = 0;
+        st.b0 = st.b1 = 0;
+        if (lo < 0) continue;                           // empty contigs only
+        st.b0 = block_of(lo);
+        st.b1 = block_of(hi) + 1;
+        const TractBlock &f = tb[st.b0], &l = tb[st.b1 - 1];
+        st.bytes = l.uoff + l.isize - f.uoff;
+        st.comp_bytes = l.coff + l.bsize - f.coff;
+    }
+    return TREDSW_OK;
 }
 
 template <class B>
@@ -1707,6 +1823,17 @@ int run_ref_tracts(B &be, tredsw_tracts *out, const char *path, const tredsw_fai
     const int fd = steps.empty() ? -1 : open(path, O_RDONLY);
     if (!steps.empty() && fd < 0) { tredsw_set_error("%s: cannot open: %s", path, strerror(errno)); return TREDSW_ERR_IO; }
     struct Close { int fd; ~Close() { if (fd >= 0) close(fd); } } close_fd{fd};
+    // the format, from the file: gzip magic -> BGZF (its blocks inflated on the device), anything else -> text
+    uint8_t magic[2] = {0, 0};
+    const bool bgzf = fd >= 0 && pread_full(fd, magic, 2, 0) == 2 && magic[0] == 31 && magic[1] == 139;
+    std::vector<TractBlock> tb;
+    if (bgzf) {
+        int rc = walk_bgzf(fd, path, &tb);
+        if (!rc) rc = plan_bgzf_steps(path, tb, cs, steps);
+        if (rc) return rc;
+        max_bytes = 0;
+        for (const TractStep &st : steps) max_bytes = std::max(max_bytes, st.comp_bytes);
+    }
     uint8_t *pinned[2] = {nullptr, nullptr};
     for (uint8_t *&p : pinned) if (!steps.empty()) p = static_cast<uint8_t *>(be.alloc_host((size_t)max_bytes + 64));
     int32_t *d_per = static_cast<int32_t *>(be.alloc(sizeof(int32_t) * (size_t)(2 * nper + 1)));
@@ -1718,18 +1845,21 @@ int run_ref_tracts(B &be, tredsw_tracts *out, const char *path, const tredsw_fai
     be.upload(d_codes, mcodes.data(), sizeof(uint64_t) * mcodes.size());
     const TractQuery q{d_per, d_per + nper, d_codes, nper, prm.min_units, (int64_t)prm.min_len};
     void *d_text = nullptr, *d_code = nullptr, *d_valid = nullptr, *d_cs = nullptr, *d_out = nullptr;
-    size_t c_text = 0, c_code = 0, c_valid = 0, c_cs = 0, c_out = 0;
+    void *d_comp = nullptr, *d_blocks = nullptr, *d_bstatus = nullptr;
+    size_t c_text = 0, c_code = 0, c_valid = 0, c_cs = 0, c_out = 0, c_comp = 0, c_blocks = 0, c_bstatus = 0;
     grow(be, d_out, c_out, sizeof(TractOut) * 65536);
-    int64_t invalid = 0, bytes = 0;
+    int64_t invalid = 0, bytes = 0, comp_bytes = 0, nblocks = 0;
+    auto read_step = [&](TractStep *st) { if (bgzf) read_bgzf_step(fd, tb.data(), st); else read_tract_step(fd, cs, st); };
     std::thread reader;
     struct Join { std::thread &t; ~Join() { if (t.joinable()) t.join(); } } join_reader{reader};
-    if (!steps.empty()) { steps[0].text = pinned[0]; read_tract_step(fd, cs, &steps[0]); }
+    if (!steps.empty()) { steps[0].buf = pinned[0]; read_step(&steps[0]); }
     for (size_t k = 0; k < steps.size(); ++k) {
         TractStep &st = steps[k];
+        if (st.why && st.at >= 0) { tredsw_set_error("%s: %s at offset %lld", path, st.why, (long long)st.at); return TREDSW_ERR_IO; }
         if (st.why) { tredsw_set_error("%s: %s", path, st.why); return TREDSW_ERR_IO; }
         if (k + 1 < steps.size()) {
-            steps[k + 1].text = pinned[(k + 1) & 1];
-            reader = std::thread(read_tract_step, fd, cs, &steps[k + 1]);
+            steps[k + 1].buf = pinned[(k + 1) & 1];
+            reader = std::thread(read_step, &steps[k + 1]);
         }
         const double t_dev = now_ms();
         // the step's contigs: text and word offsets
@@ -1738,6 +1868,7 @@ int run_ref_tracts(B &be, tredsw_tracts *out, const char *path, const tredsw_fai
         int64_t text_at = 0, words = 0;
         for (int i = 0; i < ncs; ++i) {
             const tredsw_fai_entry &f = cs[st.c0 + i];
+            if (bgzf) text_at = f.length > 0 ? f.offset - tb[st.b0].uoff : 0;      // (header lines are never addressed)
             tc[i] = TractContig{f.length, text_at, words, f.line_bases, f.line_width, st.c0 + i, 0};
             text_at += fai_text_bytes(f);
             words += tract_words(f.length);
@@ -1747,7 +1878,20 @@ int run_ref_tracts(B &be, tredsw_tracts *out, const char *path, const tredsw_fai
         uint32_t *valid = static_cast<uint32_t *>(grow(be, d_valid, c_valid, sizeof(uint32_t) * (size_t)std::max<int64_t>(1, words)));
         TractContig *dcs = static_cast<TractContig *>(grow(be, d_cs, c_cs, sizeof(TractContig) * (size_t)ncs));
         if (be.rc) return be.rc;
-        be.upload(text, st.text, (size_t)st.bytes);
+        const int nb = (int)st.blocks.size();
+        std::vector<uint8_t> h_bstatus(nb);
+        uint8_t *bstatus = nullptr;
+        if (bgzf) {                                     // the step's blocks, inflated into its text buffer
+            uint8_t *comp = static_cast<uint8_t *>(grow(be, d_comp, c_comp, (size_t)st.comp_bytes + 64));
+            BlockDesc *blocks = static_cast<BlockDesc *>(grow(be, d_blocks, c_blocks, sizeof(BlockDesc) * (size_t)std::max(1, nb)));
+            bstatus = static_cast<uint8_t *>(grow(be, d_bstatus, c_bstatus, (size_t)std::max(1, nb)));
+            if (be.rc) return be.rc;
+            be.upload(comp, st.buf, (size_t)st.comp_bytes);
+            be.upload(blocks, st.blocks.data(), sizeof(BlockDesc) * (size_t)nb);
+            be.inflate(comp, text, blocks, nb, bstatus, 1);
+        } else {
+            be.upload(text, st.buf, (size_t)st.bytes);
+        }
         be.upload(dcs, tc.data(), sizeof(TractContig) * (size_t)ncs);
         be.fill(d_small, 0, sizeof(unsigned long long) * 3);
         unsigned long long *cnt = d_small, *inval = d_small + 1, *err = d_small + 2;
@@ -1769,8 +1913,15 @@ int run_ref_tracts(B &be, tredsw_tracts *out, const char *path, const tredsw_fai
                 tract_runs(code, valid, c, w - c.word0, (int)(i - w * q.nper), q, tout, cnt, cap);
             });
             be.download(h_small, d_small, sizeof(h_small));
+            if (pass == 0) be.download(h_bstatus.data(), bstatus, (size_t)nb);
             be.sync();
             if (be.rc) return be.rc;
+            for (int b = 0; b < nb; ++b)
+                if (h_bstatus[b]) {
+                    tredsw_set_error("%s: the BGZF block at offset %lld %s", path, (long long)tb[st.b0 + b].coff,
+                                     h_bstatus[b] == 1 ? "does not inflate" : "fails its CRC-32 / length check");
+                    return TREDSW_ERR_IO;
+                }
             if (h_small[2]) { tredsw_set_error("%s: a base position holds a line break or a header: the index does not fit the file", path); return TREDSW_ERR_IO; }
             if (h_small[0] <= cap) break;
             if (pass) { tredsw_set_error("tract count changed between passes"); return TREDSW_ERR_CUDA; }
@@ -1786,6 +1937,8 @@ int run_ref_tracts(B &be, tredsw_tracts *out, const char *path, const tredsw_fai
         if (be.rc) return be.rc;
         invalid += (int64_t)h_small[1];
         bytes += st.bytes;
+        comp_bytes += st.comp_bytes;
+        nblocks += nb;
         out->read_ms.push_back(st.ms);
         out->device_ms.push_back(now_ms() - t_dev);
         if (reader.joinable()) reader.join();
@@ -1801,6 +1954,7 @@ int run_ref_tracts(B &be, tredsw_tracts *out, const char *path, const tredsw_fai
     v.steps = (int64_t)out->read_ms.size(); v.bytes = bytes; v.bases = bases; v.invalid_bases = invalid;
     v.step_read_ms = out->read_ms.data(); v.step_device_ms = out->device_ms.data();
     v.ms_total = now_ms() - t_begin;
+    v.comp_bytes = comp_bytes; v.blocks = nblocks;
     return TREDSW_OK;
 }
 

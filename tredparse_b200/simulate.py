@@ -16,6 +16,9 @@ Design follows SURVEY.md §8(d) (configs 3-5 of BASELINE.json):
 
 Everything is seeded: ``np.random.default_rng(0xB200 + 1000 * locus_idx + pair_idx)`` per problem.
 """
+import os
+import shutil
+
 import numpy as np
 
 from .ssw import encode
@@ -384,6 +387,19 @@ def write_fasta(path, contigs, width=60, fai=False):
         with open(path + ".fai", "w") as fp:
             fp.writelines(rows)
     return path
+
+
+def bgzip_fasta(src, dst, block_size=0xFF00, level=6):
+    """a BGZF copy of the FASTA at `src` (as `bgzip` writes it: `block_size` bytes a block, an empty last block) at
+    `dst`, with a copy of src.fai at dst.fai when there is one: its offsets are offsets into the inflated text"""
+    from .bamio import BGZFWriter
+    w = BGZFWriter(dst, level=level, block_size=block_size)
+    with open(src, "rb") as fp:
+        w.write(fp.read())
+    w.close()
+    if os.path.exists(src + ".fai"):
+        shutil.copyfile(src + ".fai", dst + ".fai")
+    return dst
 
 
 def reference_records(seq, tid, rep_start, rep_end, motif, alleles, readlen=150, cov_per_hap=15.0, flank=2000,

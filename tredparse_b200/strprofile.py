@@ -10,7 +10,7 @@ with more anchored IRRs in a region than the rest of the cohort — expansions o
     python -m tredparse_b200.strprofile profile x.bam [y.bam ... | -] --workdir w
     python -m tredparse_b200.tred samples.csv --workdir w --str-profile     # or: catalogue calls and profiles, one read
     python -m tredparse_b200.strprofile outliers w/*.str_profile.json --tsv out.tsv
-    python -m tredparse_b200.strprofile loci out.tsv --fasta ref.fa --profiles w/*.str_profile.json [--alts]
+    python -m tredparse_b200.strprofile loci out.tsv --fasta ref.fa[.gz] --profiles w/*.str_profile.json [--alts]
     python -m tredparse_b200.tred samples.csv --tred <name> ...          # from the directory that holds sites/
 
 Definitions (include/tredsw.h, tredsw_irr_params):
@@ -339,8 +339,8 @@ def main(argv=None):
                                     "tredparse_b200.tred - --str-profile` gives its catalogue calls and its profile "
                                     "from one read.")
     pl.add_argument("tsv", help="the table `outliers` wrote")
-    pl.add_argument("--fasta", required=True, help="the reference the BAMs are aligned to (plain text; its .fai is "
-                                                   "used when present)")
+    pl.add_argument("--fasta", required=True, help="the reference the BAMs are aligned to, plain text or bgzipped "
+                                                   "(bgzip, not plain gzip); its .fai is used when present")
     pl.add_argument("--profiles", nargs="+", required=True,
                     help="<sample>.str_profile.json files: the read length is the largest among them")
     pl.add_argument("--min-z", type=float, default=3.0)
