@@ -22,13 +22,18 @@
 // sample, slab by slab, that finds the record boundaries on the device and hands the records of every fetch to the
 // same selection / compaction / pairing steps (select_and_pair) — see the scan_* bodies of ingest_device.cuh.
 //
-// A third front end, run_ref_tracts (tredsw_ref_tracts), scans a plain-text FASTA for the tracts of requested motifs
-// with the same backend and the same staging (page-locked steps read by a host thread): ref_tracts_device.cuh.
+// A third front end, run_ref_tracts (tredsw_ref_tracts), scans a FASTA, plain text or BGZF, for the tracts of
+// requested motifs with the same backend and the same staging (page-locked steps read by a host thread; BGZF blocks
+// inflated by inflate_kernel): ref_tracts_device.cuh.
 //
 // The per-thread bodies live in ingest_device.cuh as __host__ __device__ functions; the pipeline below is written
 // once against a small backend (allocate / copy / for_each / scan) with a CUDA implementation and a serial host
 // implementation.  The host one is TEST INFRASTRUCTURE (tredsw_ingest_batch_emulate): it lets the CPU suite compare
 // the device logic with the host reader bit for bit; the package never calls it.
+//
+// The host side the three front ends share: typed allocation (alloc_n, alloc_host_n), device buffers reused from step
+// to step (Reused), a locus query's fetches (plan_fetches), a BGZF block's inflate job (block_desc), the thread that
+// reads the next step while the device works (ReadAhead), and the body of every C entry point (run_entry).
 #include <stdint.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -354,6 +359,53 @@ struct HostBackend {                                   // serial emulation of th
     void release() { for (void *p : mem) free(p); for (void *p : mem_keep) free(p); mem.clear(); mem_keep.clear(); }
 };
 
+// n elements of T, at least one (every buffer exists, so that an empty batch needs no special case)
+template <class T, class B> T *alloc_n(B &be, int64_t n, bool keep = false) {
+    void *p = be.alloc(sizeof(T) * (size_t)std::max<int64_t>(1, n), keep);
+    return static_cast<T *>(p);
+}
+template <class T, class B> T *alloc_host_n(B &be, int64_t n, bool keep = false) {
+    void *p = be.alloc_host(sizeof(T) * (size_t)std::max<int64_t>(1, n), keep);
+    return static_cast<T *>(p);
+}
+
+// A device buffer reused from step to step (slab, FASTA step) that grows geometrically.  An outgrown block is not
+// freed: it stays with the batch until release, because kernels in flight and the carry copy may still read it.
+template <class T> struct Reused {
+    T *p = nullptr;
+    int64_t cap = 0;                                    // elements
+    template <class B> T *get(B &be, int64_t n) {       // room for n elements (at least one)
+        n = std::max<int64_t>(1, n);
+        if (!p || n > cap) { cap = std::max(n, 2 * cap); p = alloc_n<T>(be, cap); }
+        return p;
+    }
+    // get() for a buffer whose first `used` elements must survive the growth: they are copied into the new block
+    template <class B> T *get_keeping(B &be, int64_t n, int64_t used) {
+        T *old = p;
+        get(be, n);
+        if (p != old) be.copy(p, old, sizeof(T) * (size_t)used);
+        return p;
+    }
+};
+
+// A host thread that reads step k + 1 while the device works on step k; joined at the end of the step and on every
+// return from the front end (an error return must not leave it writing into a released buffer).
+struct ReadAhead {
+    std::thread t;
+    template <class... A> void start(A &&...a) { t = std::thread(std::forward<A>(a)...); }
+    void join() { if (t.joinable()) t.join(); }
+    ~ReadAhead() { join(); }
+};
+
+// Per-problem status of a batch (tredsw_ingest_view.status); a scan gives all its problems the status of the scan.
+enum ProblemStatus : int32_t {
+    PROBLEM_OK = 0,
+    PROBLEM_STAGING = 1,        // the sample could not be staged: I/O, index, BGZF framing, contig out of range
+    PROBLEM_INFLATE = 2,        // a block failed to inflate or its CRC-32 / length differs
+    PROBLEM_CORRUPT = 3,        // corrupt or truncated records
+    PROBLEM_UNSORTED = 4,       // (scan only) the file is not sorted by coordinate
+};
+
 struct ProblemSummary {         // device -> host after the selection pass
     uint32_t read0, nreads, base0, nbases, name0, name_bytes, pe0, npe;
 };
@@ -364,13 +416,13 @@ struct ProblemSummary {         // device -> host after the selection pass
 // the batch object
 // ---------------------------------------------------------------------------------------------------------------
 struct tredsw_ingest_batch {
+    static constexpr bool keeps_backend = true;     // its device buffers are the view (run_entry)
     bool emulated = false;
     CudaBackend cuda;
     HostBackend host;
     int32_t nproblems = 0;
     std::vector<tredsw_locus_summary> summaries;
-    std::vector<int32_t> status;                    // per problem: 0 ok, 1 the sample could not be staged (I/O, index,
-                                                    // BGZF framing), 2 a block failed to inflate, 3 corrupt records
+    std::vector<int32_t> status;                    // per problem: a ProblemStatus
     std::vector<tredsw_problem_span> spans;
     tredsw_ingest_view view;
     double ms_host_stage = 0, ms_total = 0, ms_marks[4] = {0, 0, 0, 0};
@@ -381,6 +433,13 @@ struct tredsw_ingest_batch {
     std::vector<IrrEntry> irr_entries;
     std::vector<char> irr_names;
     tredsw_irr_view irr_view;
+    void reset(int32_t nq) {                        // nq problems, all ok, no evidence yet
+        nproblems = nq;
+        summaries.assign(nq, tredsw_locus_summary{});
+        status.assign(nq, PROBLEM_OK);
+        spans.assign(nq, tredsw_problem_span{});
+        memset(&view, 0, sizeof(view));
+    }
 };
 static_assert(sizeof(IrrEntry) == sizeof(tredsw_irr_entry), "IrrEntry mirrors tredsw_irr_entry");
 
@@ -417,6 +476,23 @@ int parse_bgzf_block(const uint8_t *h, int64_t avail, BgzfFrame *f, const char *
     if (f->isize > 65536) { *why = "BGZF block larger than 64 KiB"; return -1; }
     return 1;
 }
+// The inflate job of a parsed block that starts at in_off in the staging buffer and inflates to out_off.
+BlockDesc block_desc(const BgzfFrame &f, int64_t in_off, int64_t out_off) {
+    BlockDesc d;
+    d.in_off = in_off + 12 + f.xlen; d.out_off = out_off;
+    d.clen = (uint32_t)f.clen; d.isize = f.isize; d.crc = f.crc; d.pad_ = 0;
+    return d;
+}
+
+int64_t pread_full(int fd, uint8_t *dst, int64_t n, int64_t off) {     // -> the bytes read (< n: end of file or error)
+    int64_t got = 0;
+    while (got < n) {
+        const ssize_t k = pread(fd, dst + got, (size_t)(n - got), (off_t)(off + got));
+        if (k <= 0) break;
+        got += k;
+    }
+    return got;
+}
 
 // the windows of one locus (extract_locus_impl)
 ProblemParams problem_params(const tredsw_locus_query &q) {
@@ -428,6 +504,21 @@ ProblemParams problem_params(const tredsw_locus_query &q) {
     pp.pe_s = std::max<int64_t>(start - q.pe_window, 0); pp.pe_e = end + q.pe_window;
     pp.tstart = start - q.flankmatch; pp.tend = end + q.flankmatch;
     return pp;
+}
+
+// The fetches of one locus query, in output order: its window (kind 0), then its alt regions whose contig is in
+// [0, n_ref) (kind 1).  fetch(kind, tid, start, end), start clamped at 0.  False, and no fetch, when the locus's own
+// contig is out of range.
+template <class F> bool plan_fetches(const tredsw_locus_query &q, int32_t n_ref, ProblemParams *pp, F &&fetch) {
+    if (q.tid < 0 || q.tid >= n_ref) return false;
+    *pp = problem_params(q);
+    auto add = [&](int kind, int32_t tid, int64_t s, int64_t e) { fetch(kind, tid, s < 0 ? 0 : s, e); };
+    add(0, q.tid, std::min(pp->win_s, pp->pe_s), std::max(pp->win_e, pp->pe_e));
+    for (int a = 0; a < q.n_alts && q.alts; ++a) {
+        const int32_t atid = q.alts[3 * a], as = q.alts[3 * a + 1], ae = q.alts[3 * a + 2];
+        if (atid >= 0 && atid < n_ref) add(1, atid, as, ae);
+    }
+    return true;
 }
 
 // One sample: the fetches of its problems (the locus window, then the alt regions), their BAI chunks, and the merged
@@ -460,11 +551,7 @@ int run_pipeline(B &be, tredsw_ingest_batch *out, tredsw_bam *const *bams, const
     const double t_begin = now_ms();
     const bool want_names = (flags & TREDSW_INGEST_NO_NAMES) == 0;
     const int check_crc = (flags & TREDSW_INGEST_NO_CRC) == 0;
-    out->nproblems = nq;
-    out->summaries.assign(nq, tredsw_locus_summary{});
-    out->status.assign(nq, 0);
-    out->spans.assign(nq, tredsw_problem_span{});
-    memset(&out->view, 0, sizeof(out->view));
+    out->reset(nq);
     if (nq == 0) return TREDSW_OK;
 
     // ---- (1) plans per sample: fetches, chunks, merged block ranges --------------------------------------------
@@ -496,13 +583,10 @@ int run_pipeline(B &be, tredsw_ingest_batch *out, tredsw_bam *const *bams, const
         sp.file_size = fstat(fd, &st) == 0 ? (int64_t)st.st_size : 0;
         std::vector<std::pair<int64_t, int64_t>> raw;
         for (int p : sp.problems) {
-            const tredsw_locus_query &q = queries[p];
-            ProblemParams &pp = params[p];
-            if (q.tid < 0 || q.tid >= (int)sp.bam->names.size()) { out->status[p] = 1; continue; }
-            pp = problem_params(q);
-            auto add_fetch = [&](int kind, int tid, int64_t fs, int64_t fe) {
+            const bool planned = plan_fetches(queries[p], (int32_t)sp.bam->names.size(), &params[p],
+                                              [&](int kind, int32_t tid, int64_t fs, int64_t fe) {
                 SamplePlan::PFetch f;
-                f.problem = p; f.kind = kind; f.tid = tid; f.start = fs < 0 ? 0 : fs; f.end = fe;
+                f.problem = p; f.kind = kind; f.tid = tid; f.start = fs; f.end = fe;
                 f.chunks = sp.bam->chunks(tid, f.start, f.end);
                 for (auto &c : f.chunks) {
                     const int64_t cb = (int64_t)(c.first >> 16);
@@ -512,13 +596,8 @@ int run_pipeline(B &be, tredsw_ingest_batch *out, tredsw_bam *const *bams, const
                     raw.emplace_back(cb, ce);
                 }
                 sp.fetches.push_back(std::move(f));
-            };
-            add_fetch(0, q.tid, std::min(pp.win_s, pp.pe_s), std::max(pp.win_e, pp.pe_e));
-            for (int a = 0; a < q.n_alts && q.alts; ++a) {
-                const int32_t atid = q.alts[3 * a], as = q.alts[3 * a + 1], ae = q.alts[3 * a + 2];
-                if (atid < 0 || atid >= (int)sp.bam->names.size()) continue;
-                add_fetch(1, atid, as, ae);
-            }
+            });
+            if (!planned) out->status[p] = PROBLEM_STAGING;
         }
         std::sort(raw.begin(), raw.end());
         for (auto &r : raw) {
@@ -537,7 +616,7 @@ int run_pipeline(B &be, tredsw_ingest_batch *out, tredsw_bam *const *bams, const
             comp_total += (bytes + 15) & ~(int64_t)15;
         }
     }
-    uint8_t *h_comp = static_cast<uint8_t *>(be.alloc_host((size_t)comp_total + 16));
+    uint8_t *h_comp = alloc_host_n<uint8_t>(be, comp_total + 16);
     if (be.rc) return be.rc;
     std::vector<Chunk> chunks;
     std::vector<Fetch> fetches;
@@ -558,22 +637,14 @@ int run_pipeline(B &be, tredsw_ingest_batch *out, tredsw_bam *const *bams, const
         int64_t cursor = 0;
         for (size_t r = 0; r < sp.ranges.size() && ok; ++r) {
             uint8_t *dst = h_comp + sp.range_comp_off[r];
-            int64_t got = 0;
-            while (got < sp.range_bytes[r]) {
-                const ssize_t k = pread(fd, dst + got, (size_t)(sp.range_bytes[r] - got), (off_t)(sp.ranges[r].first + got));
-                if (k <= 0) break;
-                got += k;
-            }
+            const int64_t got = pread_full(fd, dst, sp.range_bytes[r], sp.ranges[r].first);
             const size_t first_block = lb.size();
             int64_t o = 0;
             while (sp.ranges[r].first + o <= sp.ranges[r].second) {
                 if (o == got) { if (got < sp.range_bytes[r]) { ok = false; why = "short read"; } break; }
                 BgzfFrame fr;
                 if (parse_bgzf_block(dst + o, got - o, &fr, &why) != 1) { ok = false; break; }
-                BlockDesc d;
-                d.in_off = sp.range_comp_off[r] + o + 12 + fr.xlen;
-                d.out_off = cursor; d.clen = (uint32_t)fr.clen; d.isize = fr.isize; d.crc = fr.crc; d.pad_ = 0;
-                sample_blocks[s].push_back(d);
+                sample_blocks[s].push_back(block_desc(fr, sp.range_comp_off[r] + o, cursor));
                 lb.push_back(LoadedBlock{sp.ranges[r].first + o, cursor, fr.isize, 0});
                 cursor += fr.isize;
                 o += fr.bsize;
@@ -590,7 +661,7 @@ int run_pipeline(B &be, tredsw_ingest_batch *out, tredsw_bam *const *bams, const
         for (LoadedBlock &b : loaded[s]) { b.out_off += ibuf_total; b.run_end += ibuf_total; }
         ibuf_total += sample_inflated[s];
         if (sample_error[s]) {
-            for (int p : plans[s].problems) if (!out->status[p]) out->status[p] = 1;
+            for (int p : plans[s].problems) if (!out->status[p]) out->status[p] = PROBLEM_STAGING;
             tredsw_set_error("%s: %s", plans[s].bam->path.c_str(), sample_error[s]);
         }
     }
@@ -612,7 +683,7 @@ int run_pipeline(B &be, tredsw_ingest_batch *out, tredsw_bam *const *bams, const
                 f.chunk_begin = (int32_t)chunks.size();
                 for (auto &c : pf->chunks) {
                     const LoadedBlock *b0 = find_block((int64_t)(c.first >> 16)), *b1 = find_block((int64_t)(c.second >> 16));
-                    if (!b0 || b0->coffset != (int64_t)(c.first >> 16) || !b1) { out->status[p] = 1; break; }
+                    if (!b0 || b0->coffset != (int64_t)(c.first >> 16) || !b1) { out->status[p] = PROBLEM_STAGING; break; }
                     Chunk ch;
                     ch.begin = b0->out_off + std::min<int64_t>((int64_t)(c.first & 0xffff), b0->isize);
                     ch.end = b1->coffset == (int64_t)(c.second >> 16) ? b1->out_off + std::min<int64_t>((int64_t)(c.second & 0xffff), b1->isize)
@@ -633,19 +704,19 @@ int run_pipeline(B &be, tredsw_ingest_batch *out, tredsw_bam *const *bams, const
     const int nblocks = (int)blocks.size(), nfetch = (int)fetches.size();
 
     // ---- (3) device: inflate ------------------------------------------------------------------------------------
-    uint8_t *d_comp = static_cast<uint8_t *>(be.alloc((size_t)comp_total + 16));
-    uint8_t *d_ibuf = static_cast<uint8_t *>(be.alloc((size_t)ibuf_total + 16));
-    BlockDesc *d_blocks = static_cast<BlockDesc *>(be.alloc(sizeof(BlockDesc) * (size_t)std::max(1, nblocks)));
-    uint8_t *d_bstatus = static_cast<uint8_t *>(be.alloc((size_t)std::max(1, nblocks)));
-    uint8_t *h_bstatus = static_cast<uint8_t *>(be.alloc_host((size_t)std::max(1, nblocks)));
-    Chunk *d_chunks = static_cast<Chunk *>(be.alloc(sizeof(Chunk) * std::max<size_t>(1, chunks.size())));
-    Fetch *d_fetches = static_cast<Fetch *>(be.alloc(sizeof(Fetch) * (size_t)std::max(1, nfetch)));
-    ProblemParams *d_params = static_cast<ProblemParams *>(be.alloc(sizeof(ProblemParams) * (size_t)nq));
-    ProblemCounts *d_counts = static_cast<ProblemCounts *>(be.alloc(sizeof(ProblemCounts) * (size_t)nq));
-    uint32_t *d_fcount = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)(nfetch + 1)));
-    uint32_t *d_fbase = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)(nfetch + 2)));
-    uint32_t *d_ferr = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)(nfetch + 1)));
-    uint32_t *h_fbase = static_cast<uint32_t *>(be.alloc_host(sizeof(uint32_t) * (size_t)(nfetch + 2)));
+    uint8_t *d_comp = alloc_n<uint8_t>(be, comp_total + 16);
+    uint8_t *d_ibuf = alloc_n<uint8_t>(be, ibuf_total + 16);
+    BlockDesc *d_blocks = alloc_n<BlockDesc>(be, nblocks);
+    uint8_t *d_bstatus = alloc_n<uint8_t>(be, nblocks);
+    uint8_t *h_bstatus = alloc_host_n<uint8_t>(be, nblocks);
+    Chunk *d_chunks = alloc_n<Chunk>(be, (int64_t)chunks.size());
+    Fetch *d_fetches = alloc_n<Fetch>(be, nfetch);
+    ProblemParams *d_params = alloc_n<ProblemParams>(be, nq);
+    ProblemCounts *d_counts = alloc_n<ProblemCounts>(be, nq);
+    uint32_t *d_fcount = alloc_n<uint32_t>(be, nfetch + 1);
+    uint32_t *d_fbase = alloc_n<uint32_t>(be, nfetch + 2);
+    uint32_t *d_ferr = alloc_n<uint32_t>(be, nfetch + 1);
+    uint32_t *h_fbase = alloc_host_n<uint32_t>(be, nfetch + 2);
     if (be.rc) return be.rc;
     be.upload(d_comp, h_comp, (size_t)comp_total);
     be.upload(d_blocks, blocks.data(), sizeof(BlockDesc) * (size_t)nblocks);
@@ -669,7 +740,7 @@ int run_pipeline(B &be, tredsw_ingest_batch *out, tredsw_bam *const *bams, const
     }
     be.scan(d_fcount, nfetch, d_fbase);
     be.download(h_fbase, d_fbase, sizeof(uint32_t) * (size_t)(nfetch + 1));
-    uint32_t *h_ferr = static_cast<uint32_t *>(be.alloc_host(sizeof(uint32_t) * (size_t)(nfetch + 1)));
+    uint32_t *h_ferr = alloc_host_n<uint32_t>(be, nfetch + 1);
     be.download(h_ferr, d_ferr, sizeof(uint32_t) * (size_t)nfetch);
     be.sync();                                                                                  // sync 1
     out->ms_marks[0] = now_ms() - t_begin;
@@ -684,15 +755,15 @@ int run_pipeline(B &be, tredsw_ingest_batch *out, tredsw_bam *const *bams, const
             for (int s = 0; s < nsamples; ++s) {
                 bool bad = false;
                 for (size_t k = 0; k < loaded[s].size(); ++k, ++b) bad = bad || h_bstatus[b] != 0;
-                if (bad) for (int p : plans[s].problems) if (!out->status[p]) out->status[p] = 2;
+                if (bad) for (int p : plans[s].problems) if (!out->status[p]) out->status[p] = PROBLEM_INFLATE;
             }
         }
-        for (int f = 0; f < nfetch; ++f) if (h_ferr[f] && !out->status[fetches[f].problem]) out->status[fetches[f].problem] = 3;
+        for (int f = 0; f < nfetch; ++f) if (h_ferr[f] && !out->status[fetches[f].problem]) out->status[fetches[f].problem] = PROBLEM_CORRUPT;
     }
     const int64_t nrec = h_fbase[nfetch];
     out->n_records = nrec;
-    int64_t *d_rpos = static_cast<int64_t *>(be.alloc(sizeof(int64_t) * (size_t)std::max<int64_t>(1, nrec)));
-    int32_t *d_rfetch = static_cast<int32_t *>(be.alloc(sizeof(int32_t) * (size_t)std::max<int64_t>(1, nrec)));
+    int64_t *d_rpos = alloc_n<int64_t>(be, nrec);
+    int32_t *d_rfetch = alloc_n<int32_t>(be, nrec);
     if (be.rc) return be.rc;
     {
         const uint8_t *ibuf = d_ibuf; const Fetch *fe = d_fetches; const Chunk *ch = d_chunks;
@@ -722,19 +793,19 @@ int select_and_pair(B &be, tredsw_ingest_batch *out, const uint8_t *d_rbytes, co
                     bool want_names, double t_begin) {
     const int32_t nq = out->nproblems;
     const uint8_t *d_ibuf = d_rbytes;
-    uint32_t *d_emit = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)(nrec + 1)));
-    uint32_t *d_bases = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)(nrec + 1)));
-    uint32_t *d_nameb = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)(nrec + 1)));
-    uint32_t *d_pe = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)(nrec + 1)));
-    uint32_t *d_semit = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)(nrec + 2)));
-    uint32_t *d_sbases = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)(nrec + 2)));
-    uint32_t *d_snameb = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)(nrec + 2)));
-    uint32_t *d_spe = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)(nrec + 2)));
-    Mate *d_mates = static_cast<Mate *>(be.alloc(sizeof(Mate) * (size_t)std::max<int64_t>(1, nrec)));
-    int32_t *d_ffirst = static_cast<int32_t *>(be.alloc(sizeof(int32_t) * (size_t)(nq + 1)));
-    ProblemSummary *d_psum = static_cast<ProblemSummary *>(be.alloc(sizeof(ProblemSummary) * (size_t)nq));
-    ProblemSummary *h_psum = static_cast<ProblemSummary *>(be.alloc_host(sizeof(ProblemSummary) * (size_t)nq));
-    ProblemCounts *h_counts = static_cast<ProblemCounts *>(be.alloc_host(sizeof(ProblemCounts) * (size_t)nq));
+    uint32_t *d_emit = alloc_n<uint32_t>(be, nrec + 1);
+    uint32_t *d_bases = alloc_n<uint32_t>(be, nrec + 1);
+    uint32_t *d_nameb = alloc_n<uint32_t>(be, nrec + 1);
+    uint32_t *d_pe = alloc_n<uint32_t>(be, nrec + 1);
+    uint32_t *d_semit = alloc_n<uint32_t>(be, nrec + 2);
+    uint32_t *d_sbases = alloc_n<uint32_t>(be, nrec + 2);
+    uint32_t *d_snameb = alloc_n<uint32_t>(be, nrec + 2);
+    uint32_t *d_spe = alloc_n<uint32_t>(be, nrec + 2);
+    Mate *d_mates = alloc_n<Mate>(be, nrec);
+    int32_t *d_ffirst = alloc_n<int32_t>(be, nq + 1);
+    ProblemSummary *d_psum = alloc_n<ProblemSummary>(be, nq);
+    ProblemSummary *h_psum = alloc_host_n<ProblemSummary>(be, nq);
+    ProblemCounts *h_counts = alloc_host_n<ProblemCounts>(be, nq);
     if (be.rc) return be.rc;
     be.upload(d_ffirst, fetch_first.data(), sizeof(int32_t) * (size_t)(nq + 1));
     {
@@ -794,26 +865,26 @@ int select_and_pair(B &be, tredsw_ingest_batch *out, const uint8_t *d_rbytes, co
         if (h_psum[p].npe == 0) sz = 0;
         tab_mask[p] = sz ? sz - 1 : 0;
         tab_off[p + 1] = tab_off[p] + sz;
-        if (h_counts[p].error && !out->status[p]) out->status[p] = 3;
+        if (h_counts[p].error && !out->status[p]) out->status[p] = PROBLEM_CORRUPT;
     }
     const int64_t nslots = tab_off[nq];
-    int8_t *d_rbuf = static_cast<int8_t *>(be.alloc((size_t)nbases + 16, true));
-    int64_t *d_roff = static_cast<int64_t *>(be.alloc(sizeof(int64_t) * (size_t)(nreads + 1), true));
-    int32_t *d_rprob = static_cast<int32_t *>(be.alloc(sizeof(int32_t) * (size_t)std::max<int64_t>(1, nreads), true));
-    char *d_names = want_names ? static_cast<char *>(be.alloc((size_t)name_bytes + 16)) : nullptr;
-    uint32_t *d_elist = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)std::max<int64_t>(1, nreads)));
-    uint32_t *d_plist = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)std::max<int64_t>(1, npe)));
-    uint32_t *d_tab = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * 3 * (size_t)std::max<int64_t>(1, nslots)));
-    uint32_t *d_taboff = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)(nq + 1)));
-    uint32_t *d_tabmask = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)nq));
-    uint32_t *d_slot = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)std::max<int64_t>(1, npe)));
-    uint32_t *d_isg = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)(npe + 1)));
-    uint32_t *d_ist = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)(npe + 1)));
-    int32_t *d_pval = static_cast<int32_t *>(be.alloc(sizeof(int32_t) * (size_t)std::max<int64_t>(1, npe)));
-    uint32_t *d_sg = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)(npe + 2)));
-    uint32_t *d_st = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * (size_t)(npe + 2)));
-    uint32_t *d_pcnt = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * 2 * (size_t)nq));
-    uint32_t *h_pcnt = static_cast<uint32_t *>(be.alloc_host(sizeof(uint32_t) * 2 * (size_t)nq));
+    int8_t *d_rbuf = alloc_n<int8_t>(be, nbases + 16, true);
+    int64_t *d_roff = alloc_n<int64_t>(be, nreads + 1, true);
+    int32_t *d_rprob = alloc_n<int32_t>(be, nreads, true);
+    char *d_names = want_names ? alloc_n<char>(be, name_bytes + 16) : nullptr;
+    uint32_t *d_elist = alloc_n<uint32_t>(be, nreads);
+    uint32_t *d_plist = alloc_n<uint32_t>(be, npe);
+    uint32_t *d_tab = alloc_n<uint32_t>(be, 3 * std::max<int64_t>(1, nslots));     // rep, first, second
+    uint32_t *d_taboff = alloc_n<uint32_t>(be, nq + 1);
+    uint32_t *d_tabmask = alloc_n<uint32_t>(be, nq);
+    uint32_t *d_slot = alloc_n<uint32_t>(be, npe);
+    uint32_t *d_isg = alloc_n<uint32_t>(be, npe + 1);
+    uint32_t *d_ist = alloc_n<uint32_t>(be, npe + 1);
+    int32_t *d_pval = alloc_n<int32_t>(be, npe);
+    uint32_t *d_sg = alloc_n<uint32_t>(be, npe + 2);
+    uint32_t *d_st = alloc_n<uint32_t>(be, npe + 2);
+    uint32_t *d_pcnt = alloc_n<uint32_t>(be, 2 * (int64_t)nq);
+    uint32_t *h_pcnt = alloc_host_n<uint32_t>(be, 2 * (int64_t)nq);
     if (be.rc) return be.rc;
     be.upload(d_taboff, tab_off.data(), sizeof(uint32_t) * (size_t)(nq + 1));
     be.upload(d_tabmask, tab_mask.data(), sizeof(uint32_t) * (size_t)nq);
@@ -881,12 +952,12 @@ int select_and_pair(B &be, tredsw_ingest_batch *out, const uint8_t *d_rbytes, co
         pe_off[2 * p] = n_pe_lens; n_pe_lens += h_pcnt[2 * p];
         pe_off[2 * p + 1] = n_pe_lens; n_pe_lens += h_pcnt[2 * p + 1];
     }
-    int32_t *d_pelens = static_cast<int32_t *>(be.alloc(sizeof(int32_t) * (size_t)std::max<int64_t>(1, n_pe_lens), true));
-    int64_t *d_peoff = static_cast<int64_t *>(be.alloc(sizeof(int64_t) * 2 * (size_t)nq));
-    int8_t *h_rbuf = static_cast<int8_t *>(be.alloc_host((size_t)nbases + 16, true));
-    int64_t *h_roff = static_cast<int64_t *>(be.alloc_host(sizeof(int64_t) * (size_t)(nreads + 1), true));
-    int32_t *h_pelens = static_cast<int32_t *>(be.alloc_host(sizeof(int32_t) * (size_t)std::max<int64_t>(1, n_pe_lens), true));
-    char *h_names = want_names ? static_cast<char *>(be.alloc_host((size_t)name_bytes + 16, true)) : nullptr;
+    int32_t *d_pelens = alloc_n<int32_t>(be, n_pe_lens, true);
+    int64_t *d_peoff = alloc_n<int64_t>(be, 2 * (int64_t)nq);
+    int8_t *h_rbuf = alloc_host_n<int8_t>(be, nbases + 16, true);
+    int64_t *h_roff = alloc_host_n<int64_t>(be, nreads + 1, true);
+    int32_t *h_pelens = alloc_host_n<int32_t>(be, n_pe_lens, true);
+    char *h_names = want_names ? alloc_host_n<char>(be, name_bytes + 16, true) : nullptr;
     if (be.rc) return be.rc;
     be.upload(d_peoff, pe_off.data(), sizeof(int64_t) * 2 * (size_t)nq);
     {
@@ -974,11 +1045,7 @@ void read_slab(ScanSource *src, int64_t off, int64_t want, const ScanSlab *prev,
     int64_t got = 0;
     if (!src->stream) {
         const int64_t n = std::max<int64_t>(0, std::min(want, src->file_size - off));
-        while (got < n) {
-            const ssize_t k = pread(src->fd, sl->comp + got, (size_t)(n - got), (off_t)(off + got));
-            if (k <= 0) break;
-            got += k;
-        }
+        got = pread_full(src->fd, sl->comp, n, off);
         if (got < n) sl->why = "short read";
     } else {
         const uint8_t *lead = prev ? prev->comp + (prev->next - prev->begin) : src->head;
@@ -1000,9 +1067,7 @@ void read_slab(ScanSource *src, int64_t off, int64_t want, const ScanSlab *prev,
         const int rc = parse_bgzf_block(sl->comp + o, got - o, &fr, &why);
         if (rc < 0 || (rc == 0 && at_end)) { sl->why = why; break; }
         if (rc == 0 || (sl->inflated + fr.isize > SCAN_MAX_INFLATED && !sl->blocks.empty())) break;
-        BlockDesc d;
-        d.in_off = o + 12 + fr.xlen; d.out_off = sl->inflated; d.clen = (uint32_t)fr.clen; d.isize = fr.isize; d.crc = fr.crc; d.pad_ = 0;
-        sl->blocks.push_back(d);
+        sl->blocks.push_back(block_desc(fr, o, sl->inflated));
         sl->inflated += fr.isize;
         o += fr.bsize;
     }
@@ -1010,15 +1075,55 @@ void read_slab(ScanSource *src, int64_t off, int64_t want, const ScanSlab *prev,
     sl->ms = now_ms() - t0;
 }
 
-// a device buffer that is reused from slab to slab and grows geometrically (the old one is released with the batch)
-template <class B> void *grow(B &be, void *&p, size_t &cap, size_t bytes) {
-    if (!p || bytes > cap) { cap = std::max(bytes, 2 * cap); p = be.alloc(cap); }
-    return p;
-}
+struct ScanBuffers {                // the device buffers of the slab loop, reused from slab to slab
+    Reused<uint8_t> ibuf[2];        // the carry + the slab's inflated blocks (alternating: the carry is copied across)
+    Reused<uint8_t> comp, bstatus;
+    Reused<BlockDesc> blocks;
+    Reused<ScanBlock> sblk;
+    Reused<int64_t> cand, land, first, recpos, epos;
+    Reused<uint32_t> rcnt, rbase, nm, kb, ebase, kbase;
+    Reused<int32_t> efetch;
+    Reused<uint32_t> iflag, inb, ibase, inbase;     // the STR profile
+    Reused<IrrEntry> ient;
+    Reused<char> iname;
+    Reused<uint8_t> kept;           // the kept-record stream of the whole scan (grows with its contents)
+};
 
 }  // namespace
 
 namespace { void irr_join(tredsw_ingest_batch *out, const unsigned long long *st); }
+
+// Verification and repair of a slab's record starts (DESIGN §4.4.1): h_first[b], the true first record of block b,
+// from the known start s0 of block 0.  Returns the next carry's start, or SCAN_BAD (corrupt records); *repaired counts
+// the blocks walked again.  The result means nothing after a backend error (be.rc).
+template <class B>
+int64_t verify_record_starts(B &be, uint8_t *s, int64_t len, ScanBlock *blk, int64_t *cand, int64_t *land, int64_t *stop,
+                             const std::vector<ScanBlock> &sblk, const std::vector<int64_t> &h_cand,
+                             std::vector<int64_t> &h_land, std::vector<int64_t> &h_first, int64_t s0, int64_t *repaired) {
+    const int nb = (int)sblk.size();
+    int64_t tf = s0;
+    for (int b = 0; b < nb && tf != SCAN_BAD;) {
+        h_first[b] = tf;
+        if (scan_agrees(sblk[b], h_cand[b], tf)) {
+            if (tf >= sblk[b].begin && tf < sblk[b].end) tf = h_land[b];
+            ++b;
+            continue;
+        }
+        const int b0 = b; const int64_t t0 = tf;
+        be.template for_each<ScanRepairTag>(1, [=] __host__ __device__(int64_t) { *stop = scan_repair_run(s, len, blk, cand, nb, b0, t0, land); });
+        int64_t h_stop = 0;
+        be.download(&h_stop, stop, sizeof(int64_t));
+        be.sync();
+        if (be.rc) return SCAN_BAD;
+        be.download(h_land.data() + b0, land + b0, sizeof(int64_t) * (size_t)(h_stop - b0));
+        be.sync();
+        for (int k = b0 + 1; k < (int)h_stop; ++k) h_first[k] = h_land[k - 1];
+        *repaired += h_stop - b0;
+        tf = h_land[h_stop - 1];
+        b = (int)h_stop;
+    }
+    return tf;
+}
 
 template <class B>
 int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locus_query *queries, int32_t nq,
@@ -1028,11 +1133,7 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
     const bool want_names = (flags & TREDSW_INGEST_NO_NAMES) == 0;
     const int check_crc = (flags & TREDSW_INGEST_NO_CRC) == 0;
     constexpr int NL = B::on_device ? 32 : 1;
-    out->nproblems = nq;
-    out->summaries.assign(nq, tredsw_locus_summary{});
-    out->status.assign(nq, 0);
-    out->spans.assign(nq, tredsw_problem_span{});
-    memset(&out->view, 0, sizeof(out->view));
+    out->reset(nq);
     const int32_t n_ref = (int32_t)bam->names.size();
 
     // ---- (1) the fetches (problem-major, like run_pipeline), then the depth regions; their elementary segments -----
@@ -1044,22 +1145,14 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
     auto add_id = [&](int32_t tid, int64_t s, int64_t e) { id_tid.push_back(tid); id_start.push_back(s < 0 ? 0 : s); id_end.push_back(e); };
     for (int p = 0; p < nq; ++p) {
         fetch_first[p] = (int32_t)fetches.size();
-        const tredsw_locus_query &q = queries[p];
-        if (q.tid < 0 || q.tid >= n_ref) { out->status[p] = 1; continue; }
-        const ProblemParams pp = params[p] = problem_params(q);
-        auto add_fetch = [&](int kind, int32_t tid, int64_t s, int64_t e) {
+        const bool planned = plan_fetches(queries[p], n_ref, &params[p], [&](int kind, int32_t tid, int64_t s, int64_t e) {
             Fetch f;
-            f.problem = p; f.kind = kind; f.tid = tid; f.start = s < 0 ? 0 : s; f.end = e;
+            f.problem = p; f.kind = kind; f.tid = tid; f.start = s; f.end = e;
             f.chunk_begin = f.chunk_end = 0; f.pad_ = 0;
             fetches.push_back(f);
             add_id(tid, s, e);
-        };
-        add_fetch(0, q.tid, std::min(pp.win_s, pp.pe_s), std::max(pp.win_e, pp.pe_e));
-        for (int a = 0; a < q.n_alts && q.alts; ++a) {
-            const int32_t atid = q.alts[3 * a], as = q.alts[3 * a + 1], ae = q.alts[3 * a + 2];
-            if (atid < 0 || atid >= n_ref) continue;
-            add_fetch(1, atid, as, ae);
-        }
+        });
+        if (!planned) out->status[p] = PROBLEM_STAGING;
     }
     fetch_first[nq] = (int32_t)fetches.size();
     const int32_t nfetch = (int32_t)fetches.size();
@@ -1095,19 +1188,19 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
         seg_f0.assign(xs.size() + 1, 0);
         for (size_t j = 0; j < xs.size(); ++j) { seg_f0[j + 1] = seg_f0[j] + (int32_t)lists[j].size(); seg_ids.insert(seg_ids.end(), lists[j].begin(), lists[j].end()); }
     }
-    int32_t *d_tid_x0 = static_cast<int32_t *>(be.alloc(sizeof(int32_t) * (size_t)(n_ref + 1)));
-    int64_t *d_xs = static_cast<int64_t *>(be.alloc(sizeof(int64_t) * std::max<size_t>(1, xs.size())));
-    int32_t *d_seg_f0 = static_cast<int32_t *>(be.alloc(sizeof(int32_t) * seg_f0.size()));
-    int32_t *d_seg_ids = static_cast<int32_t *>(be.alloc(sizeof(int32_t) * std::max<size_t>(1, seg_ids.size())));
-    int64_t *d_id_start = static_cast<int64_t *>(be.alloc(sizeof(int64_t) * 3 * (size_t)std::max(1, nids)));
-    unsigned long long *d_depth = static_cast<unsigned long long *>(be.alloc(sizeof(unsigned long long) * (size_t)std::max(1, n_depth)));
-    uint32_t *d_err = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * 2));
-    int64_t *d_small = static_cast<int64_t *>(be.alloc(sizeof(int64_t) * 2));     // last record's order key; repair stop
+    int32_t *d_tid_x0 = alloc_n<int32_t>(be, n_ref + 1);
+    int64_t *d_xs = alloc_n<int64_t>(be, (int64_t)xs.size());
+    int32_t *d_seg_f0 = alloc_n<int32_t>(be, (int64_t)seg_f0.size());
+    int32_t *d_seg_ids = alloc_n<int32_t>(be, (int64_t)seg_ids.size());
+    int64_t *d_id_start = alloc_n<int64_t>(be, 3 * (int64_t)std::max(1, nids));     // start, end, lo
+    unsigned long long *d_depth = alloc_n<unsigned long long>(be, n_depth);
+    uint32_t *d_err = alloc_n<uint32_t>(be, 2);
+    int64_t *d_small = alloc_n<int64_t>(be, 2);     // last record's order key; repair stop
     // the STR profile: counters over the whole scan; per slab the IRR flags / name bytes, their scans, the entries
     out->irr_on = irr != nullptr;
     const IrrParams ip = irr ? IrrParams{irr->min_period, irr->max_period, irr->purity_num, irr->purity_den, irr->min_read_len}
                              : IrrParams{0, 0, 0, 1, 0};
-    unsigned long long *d_irr_stats = irr ? static_cast<unsigned long long *>(be.alloc(sizeof(unsigned long long) * IRR_NSTATS)) : nullptr;
+    unsigned long long *d_irr_stats = irr ? alloc_n<unsigned long long>(be, IRR_NSTATS) : nullptr;
     if (be.rc) return be.rc;
     if (irr) be.fill(d_irr_stats, 0, sizeof(unsigned long long) * IRR_NSTATS);
     be.upload(d_tid_x0, tid_x0.data(), sizeof(int32_t) * tid_x0.size());
@@ -1137,41 +1230,33 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
         want = std::max({slab_bytes > 0 ? slab_bytes : SCAN_DEFAULT_SLAB, SCAN_MIN_SLAB, src.head_len});
     }
     ScanSlab slabs[2];
-    for (ScanSlab &sl : slabs) sl.comp = static_cast<uint8_t *>(be.alloc_host((size_t)want + 64));
+    for (ScanSlab &sl : slabs) sl.comp = alloc_host_n<uint8_t>(be, want + 64);
     if (be.rc) return be.rc;
-    void *ibuf[2] = {nullptr, nullptr}; size_t ibuf_cap[2] = {0, 0};
-    void *d_comp = nullptr, *d_blocks = nullptr, *d_bstatus = nullptr, *d_sblk = nullptr, *d_cand = nullptr, *d_land = nullptr;
-    void *d_first = nullptr, *d_rcnt = nullptr, *d_rbase = nullptr, *d_recpos = nullptr, *d_nm = nullptr, *d_kb = nullptr;
-    void *d_ebase = nullptr, *d_kbase = nullptr, *d_efetch = nullptr, *d_epos = nullptr, *d_kept = nullptr;
-    void *d_iflag = nullptr, *d_inb = nullptr, *d_ibase = nullptr, *d_inbase = nullptr, *d_ient = nullptr, *d_iname = nullptr;
-    size_t c_iflag = 0, c_inb = 0, c_ibase = 0, c_inbase = 0, c_ient = 0, c_iname = 0;
-    size_t c_comp = 0, c_blocks = 0, c_bstatus = 0, c_sblk = 0, c_cand = 0, c_land = 0, c_first = 0, c_rcnt = 0, c_rbase = 0;
-    size_t c_recpos = 0, c_nm = 0, c_kb = 0, c_ebase = 0, c_kbase = 0, c_efetch = 0, c_epos = 0, c_kept = 0;
+    ScanBuffers buf;
     std::vector<int32_t> ent_fetch;         // (record, fetch) entries of the whole file, in file order
     std::vector<int64_t> ent_pos;           // where the record is in the kept-record stream
     int64_t kept_total = 0, carry_len = 0, carry_at = 0, prev_key = INT64_MIN;
     int64_t s0 = (int64_t)(bam->first_record & 0xffff);
-    int32_t status = 0;
+    int32_t status = PROBLEM_OK;
     int64_t *stats = out->scan_stats;
-    std::thread reader;
-    struct Join { std::thread &t; ~Join() { if (t.joinable()) t.join(); } } join_reader{reader};
+    ReadAhead reader;
     bam->consumed = bam->is_stream();
     read_slab(&src, (int64_t)(bam->first_record >> 16), want, nullptr, &slabs[0]);
     if (src.stream) { bam->bgzf.sbuf = std::vector<unsigned char>(); src.head = nullptr; }
     for (int cur = 0;; cur ^= 1) {
         ScanSlab &sl = slabs[cur];
         stats[6] += (int64_t)(sl.ms * 1e3);
-        if (sl.why) { status = 1; tredsw_set_error("%s: %s", bam->path.c_str(), sl.why); break; }
+        if (sl.why) { status = PROBLEM_STAGING; tredsw_set_error("%s: %s", bam->path.c_str(), sl.why); break; }
         const int nb = (int)sl.blocks.size();
         if (nb == 0) break;                                                  // end of file
         const bool more = src.stream ? !(src.eof && sl.next == sl.begin + sl.got) : sl.next < src.file_size;
-        if (more) reader = std::thread(read_slab, &src, sl.next, want, &slabs[cur], &slabs[cur ^ 1]);
+        if (more) reader.start(read_slab, &src, sl.next, want, &slabs[cur], &slabs[cur ^ 1]);
         else { slabs[cur ^ 1].blocks.clear(); slabs[cur ^ 1].why = nullptr; slabs[cur ^ 1].ms = 0; }
         const double t_dev = now_ms();
         const int64_t len = carry_len + sl.inflated;
-        uint8_t *s = static_cast<uint8_t *>(grow(be, ibuf[cur], ibuf_cap[cur], (size_t)len + 64));
+        uint8_t *s = buf.ibuf[cur].get(be, len + 64);
         if (be.rc) return be.rc;
-        be.copy(s, static_cast<uint8_t *>(ibuf[cur ^ 1]) + carry_at, (size_t)carry_len);
+        be.copy(s, buf.ibuf[cur ^ 1].p + carry_at, (size_t)carry_len);
         std::vector<ScanBlock> sblk(nb);
         for (int b = 0; b < nb; ++b) {
             sl.blocks[b].out_off += carry_len;
@@ -1179,12 +1264,12 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
             sblk[b].end = sl.blocks[b].out_off + sl.blocks[b].isize;
         }
         // inflate; candidates and landings
-        uint8_t *comp = static_cast<uint8_t *>(grow(be, d_comp, c_comp, (size_t)(sl.next - sl.begin) + 64));
-        BlockDesc *blocks = static_cast<BlockDesc *>(grow(be, d_blocks, c_blocks, sizeof(BlockDesc) * nb));
-        uint8_t *bstatus = static_cast<uint8_t *>(grow(be, d_bstatus, c_bstatus, (size_t)nb));
-        ScanBlock *blk = static_cast<ScanBlock *>(grow(be, d_sblk, c_sblk, sizeof(ScanBlock) * nb));
-        int64_t *cand = static_cast<int64_t *>(grow(be, d_cand, c_cand, sizeof(int64_t) * nb));
-        int64_t *land = static_cast<int64_t *>(grow(be, d_land, c_land, sizeof(int64_t) * nb));
+        uint8_t *comp = buf.comp.get(be, sl.next - sl.begin + 64);
+        BlockDesc *blocks = buf.blocks.get(be, nb);
+        uint8_t *bstatus = buf.bstatus.get(be, nb);
+        ScanBlock *blk = buf.sblk.get(be, nb);
+        int64_t *cand = buf.cand.get(be, nb);
+        int64_t *land = buf.land.get(be, nb);
         if (be.rc) return be.rc;
         be.upload(comp, sl.comp, (size_t)(sl.next - sl.begin));
         be.upload(blocks, sl.blocks.data(), sizeof(BlockDesc) * nb);
@@ -1204,35 +1289,14 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
         be.download(h_land.data(), land, sizeof(int64_t) * nb);
         be.sync();
         if (be.rc) return be.rc;
-        if (std::any_of(h_bstatus.begin(), h_bstatus.end(), [](uint8_t v) { return v != 0; })) { status = 2; tredsw_set_error("%s: a BGZF block failed to inflate", bam->path.c_str()); break; }
-        // verification: the chain entering every block from the known start of block 0; repair where it disagrees
-        int64_t tf = s0;
-        for (int b = 0; b < nb && tf != SCAN_BAD;) {
-            h_first[b] = tf;
-            if (scan_agrees(sblk[b], h_cand[b], tf)) {
-                if (tf >= sblk[b].begin && tf < sblk[b].end) tf = h_land[b];
-                ++b;
-                continue;
-            }
-            int64_t *stop = d_small + 1;
-            const int b0 = b; const int64_t t0 = tf;
-            be.template for_each<ScanRepairTag>(1, [=] __host__ __device__(int64_t) { *stop = scan_repair_run(s, len, blk, cand, nb, b0, t0, land); });
-            int64_t h_stop = 0;
-            be.download(&h_stop, stop, sizeof(int64_t));
-            be.sync();
-            if (be.rc) return be.rc;
-            be.download(h_land.data() + b0, land + b0, sizeof(int64_t) * (size_t)(h_stop - b0));
-            be.sync();
-            for (int k = b0 + 1; k < (int)h_stop; ++k) h_first[k] = h_land[k - 1];
-            stats[3] += h_stop - b0;
-            tf = h_land[h_stop - 1];
-            b = (int)h_stop;
-        }
-        if (tf == SCAN_BAD) { status = 3; tredsw_set_error("%s: corrupt BAM records (implausible block_size)", bam->path.c_str()); break; }
+        if (std::any_of(h_bstatus.begin(), h_bstatus.end(), [](uint8_t v) { return v != 0; })) { status = PROBLEM_INFLATE; tredsw_set_error("%s: a BGZF block failed to inflate", bam->path.c_str()); break; }
+        const int64_t tf = verify_record_starts(be, s, len, blk, cand, land, d_small + 1, sblk, h_cand, h_land, h_first, s0, &stats[3]);
+        if (be.rc) return be.rc;
+        if (tf == SCAN_BAD) { status = PROBLEM_CORRUPT; tredsw_set_error("%s: corrupt BAM records (implausible block_size)", bam->path.c_str()); break; }
         // the records that start in every block, in file order
-        int64_t *first = static_cast<int64_t *>(grow(be, d_first, c_first, sizeof(int64_t) * nb));
-        uint32_t *rcnt = static_cast<uint32_t *>(grow(be, d_rcnt, c_rcnt, sizeof(uint32_t) * (nb + 1)));
-        uint32_t *rbase = static_cast<uint32_t *>(grow(be, d_rbase, c_rbase, sizeof(uint32_t) * (nb + 2)));
+        int64_t *first = buf.first.get(be, nb);
+        uint32_t *rcnt = buf.rcnt.get(be, nb + 1);
+        uint32_t *rbase = buf.rbase.get(be, nb + 2);
         if (be.rc) return be.rc;
         be.upload(first, h_first.data(), sizeof(int64_t) * nb);
         be.template for_each<ScanCountTag>(nb, [=] __host__ __device__(int64_t b) {
@@ -1246,11 +1310,11 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
         be.sync();
         if (be.rc) return be.rc;
         const int64_t nrec = h_nrec;
-        int64_t *recpos = static_cast<int64_t *>(grow(be, d_recpos, c_recpos, sizeof(int64_t) * (size_t)std::max<int64_t>(1, nrec)));
-        uint32_t *nm = static_cast<uint32_t *>(grow(be, d_nm, c_nm, sizeof(uint32_t) * (size_t)(nrec + 1)));
-        uint32_t *kb = static_cast<uint32_t *>(grow(be, d_kb, c_kb, sizeof(uint32_t) * (size_t)(nrec + 1)));
-        uint32_t *ebase = static_cast<uint32_t *>(grow(be, d_ebase, c_ebase, sizeof(uint32_t) * (size_t)(nrec + 2)));
-        uint32_t *kbase = static_cast<uint32_t *>(grow(be, d_kbase, c_kbase, sizeof(uint32_t) * (size_t)(nrec + 2)));
+        int64_t *recpos = buf.recpos.get(be, nrec);
+        uint32_t *nm = buf.nm.get(be, nrec + 1);
+        uint32_t *kb = buf.kb.get(be, nrec + 1);
+        uint32_t *ebase = buf.ebase.get(be, nrec + 2);
+        uint32_t *kbase = buf.kbase.get(be, nrec + 2);
         if (be.rc) return be.rc;
         {
             const int64_t pk = prev_key;
@@ -1274,10 +1338,10 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
         uint32_t *iflag = nullptr, *inb = nullptr, *ibase = nullptr, *inbase = nullptr;
         uint32_t h_itot[2] = {0, 0};
         if (irr) {
-            iflag = static_cast<uint32_t *>(grow(be, d_iflag, c_iflag, sizeof(uint32_t) * (size_t)(nrec + 1)));
-            inb = static_cast<uint32_t *>(grow(be, d_inb, c_inb, sizeof(uint32_t) * (size_t)(nrec + 1)));
-            ibase = static_cast<uint32_t *>(grow(be, d_ibase, c_ibase, sizeof(uint32_t) * (size_t)(nrec + 2)));
-            inbase = static_cast<uint32_t *>(grow(be, d_inbase, c_inbase, sizeof(uint32_t) * (size_t)(nrec + 2)));
+            iflag = buf.iflag.get(be, nrec + 1);
+            inb = buf.inb.get(be, nrec + 1);
+            ibase = buf.ibase.get(be, nrec + 2);
+            inbase = buf.inbase.get(be, nrec + 2);
             if (be.rc) return be.rc;
             unsigned long long *ist = d_irr_stats;
             be.template for_each<ScanIrrTag>(nrec, [=] __host__ __device__(int64_t i) {
@@ -1299,13 +1363,13 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
         if (nrec) be.download(&h_last, d_small, sizeof(int64_t));
         be.sync();
         if (be.rc) return be.rc;
-        if (h_err & SCAN_ERR_RECORD) { status = 3; tredsw_set_error("%s: corrupt BAM record", bam->path.c_str()); break; }
-        if (h_err & SCAN_ERR_ORDER) { status = 4; tredsw_set_error("%s is not sorted by coordinate", bam->path.c_str()); break; }
+        if (h_err & SCAN_ERR_RECORD) { status = PROBLEM_CORRUPT; tredsw_set_error("%s: corrupt BAM record", bam->path.c_str()); break; }
+        if (h_err & SCAN_ERR_ORDER) { status = PROBLEM_UNSORTED; tredsw_set_error("%s is not sorted by coordinate", bam->path.c_str()); break; }
         // the slab's IRR entries and names, appended to the host lists (IRRs are rare: the join by name is host work)
         if (h_itot[0]) {
             const int64_t nirr = h_itot[0], nnb = h_itot[1];
-            IrrEntry *ient = static_cast<IrrEntry *>(grow(be, d_ient, c_ient, sizeof(IrrEntry) * (size_t)nirr));
-            char *iname = static_cast<char *>(grow(be, d_iname, c_iname, (size_t)nnb + 1));
+            IrrEntry *ient = buf.ient.get(be, nirr);
+            char *iname = buf.iname.get(be, nnb + 1);
             if (be.rc) return be.rc;
             unsigned long long *ist = d_irr_stats;
             be.template for_each<ScanIrrFillTag>(nrec, [=] __host__ __device__(int64_t i) {
@@ -1335,17 +1399,10 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
         // copy the kept records once into the kept-record stream; one (fetch, position) entry per (record, fetch)
         const int64_t nent = h_tot[0], kbytes = h_tot[1];
         if (nent) {
-            if (kept_total + kbytes + 64 > (int64_t)c_kept) {
-                void *old = d_kept;
-                void *nw = be.alloc(std::max<size_t>((size_t)(kept_total + kbytes + 64), 2 * c_kept));
-                if (be.rc) return be.rc;
-                be.copy(nw, old, (size_t)kept_total);
-                d_kept = nw; c_kept = std::max<size_t>((size_t)(kept_total + kbytes + 64), 2 * c_kept);
-            }
-            int32_t *efetch = static_cast<int32_t *>(grow(be, d_efetch, c_efetch, sizeof(int32_t) * (size_t)nent));
-            int64_t *epos = static_cast<int64_t *>(grow(be, d_epos, c_epos, sizeof(int64_t) * (size_t)nent));
+            uint8_t *kept = buf.kept.get_keeping(be, kept_total + kbytes + 64, kept_total) + kept_total;
+            int32_t *efetch = buf.efetch.get(be, nent);
+            int64_t *epos = buf.epos.get(be, nent);
             if (be.rc) return be.rc;
-            uint8_t *kept = static_cast<uint8_t *>(d_kept) + kept_total;
             const int64_t k0 = kept_total;
             be.template for_each_warp<ScanKeepTag>(nrec, [=] __host__ __device__(int64_t i, int lane) {
                 if (!nm[i]) return;
@@ -1372,10 +1429,10 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
         stats[0] += 1; stats[1] += nb; stats[2] += nrec;
         stats[4] += sl.next - sl.begin; stats[5] += sl.inflated;
         stats[7] += (int64_t)((now_ms() - t_dev) * 1e3);
-        if (reader.joinable()) reader.join();
+        reader.join();
     }
-    if (reader.joinable()) reader.join();
-    if (!status && carry_len > 0) { status = 3; tredsw_set_error("%s ends inside a BAM record", bam->path.c_str()); }
+    reader.join();
+    if (!status && carry_len > 0) { status = PROBLEM_CORRUPT; tredsw_set_error("%s ends inside a BAM record", bam->path.c_str()); }
     stats[9] = status;
     if (irr) {
         unsigned long long h_ist[IRR_NSTATS];
@@ -1421,13 +1478,13 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
         v.ms_host_stage = out->ms_host_stage; v.ms_total = out->ms_total; v.ms_marks[0] = out->ms_marks[0];
         return TREDSW_OK;
     }
-    Fetch *d_fetches = static_cast<Fetch *>(be.alloc(sizeof(Fetch) * (size_t)std::max(1, nfetch)));
-    ProblemParams *d_params = static_cast<ProblemParams *>(be.alloc(sizeof(ProblemParams) * (size_t)nq));
-    ProblemCounts *d_counts = static_cast<ProblemCounts *>(be.alloc(sizeof(ProblemCounts) * (size_t)nq));
-    int64_t *d_rpos = static_cast<int64_t *>(be.alloc(sizeof(int64_t) * rpos.size()));
-    int32_t *d_rfetch = static_cast<int32_t *>(be.alloc(sizeof(int32_t) * rfetch.size()));
-    uint32_t *d_fbase = static_cast<uint32_t *>(be.alloc(sizeof(uint32_t) * fbase.size()));
-    if (!d_kept) d_kept = be.alloc(64);
+    Fetch *d_fetches = alloc_n<Fetch>(be, nfetch);
+    ProblemParams *d_params = alloc_n<ProblemParams>(be, nq);
+    ProblemCounts *d_counts = alloc_n<ProblemCounts>(be, nq);
+    int64_t *d_rpos = alloc_n<int64_t>(be, (int64_t)rpos.size());
+    int32_t *d_rfetch = alloc_n<int32_t>(be, (int64_t)rfetch.size());
+    uint32_t *d_fbase = alloc_n<uint32_t>(be, (int64_t)fbase.size());
+    const uint8_t *d_kept = buf.kept.get(be, 64);   // (a scan that kept nothing still hands over a buffer)
     if (be.rc) return be.rc;
     be.upload(d_fetches, fetches.data(), sizeof(Fetch) * (size_t)nfetch);
     be.upload(d_params, params.data(), sizeof(ProblemParams) * (size_t)nq);
@@ -1435,7 +1492,7 @@ int run_scan(B &be, tredsw_ingest_batch *out, tredsw_bam *bam, const tredsw_locu
     be.upload(d_rpos, rpos.data(), sizeof(int64_t) * (size_t)nrec);
     be.upload(d_rfetch, rfetch.data(), sizeof(int32_t) * (size_t)nrec);
     be.upload(d_fbase, fbase.data(), sizeof(uint32_t) * fbase.size());
-    const int rc = select_and_pair(be, out, static_cast<const uint8_t *>(d_kept), d_fetches, d_rpos, d_rfetch, d_fbase, nrec,
+    const int rc = select_and_pair(be, out, d_kept, d_fetches, d_rpos, d_rfetch, d_fbase, nrec,
                                    fetch_first, params, d_params, d_counts, want_names, t_begin);
     stats[8] = (int64_t)(out->ms_total * 1e3);
     return rc;
@@ -1494,6 +1551,37 @@ void keep_pool(int device) {
         pool_set[device] = true;
     }
 }
+
+// The body of every C entry point of this file: a new result R filled by run(backend, result).  With a context it runs
+// on the context's device and stream under its lock, and its kernel launches are added to ctx->launches; without one
+// (nullptr: the test emulations) it runs on the host backend.  An exception is TREDSW_ERR_IO named after `what`.  A
+// failed run releases its backend; a successful one too, unless R::keeps_backend (an ingest batch's device buffers
+// are its view).  On success *out owns the result.
+template <class R, class Run>
+int run_entry(tredsw_ctx *ctx, const char *what, R **out, Run &&run) {
+    *out = nullptr;
+    std::unique_lock<std::mutex> lock;
+    if (ctx) {
+        lock = std::unique_lock<std::mutex>(ctx->mu);
+        CUDA_TRY(cudaSetDevice(ctx->device));
+        keep_pool(ctx->device);
+    }
+    std::unique_ptr<R> r(new R());
+    r->emulated = !ctx;
+    r->cuda.stream = ctx ? ctx->stream : nullptr;
+    auto go = [&](auto &be) {
+        int rc;
+        try { rc = run(be, r.get()); }
+        catch (const std::exception &e) { tredsw_set_error("%s: %s", what, e.what()); rc = TREDSW_ERR_IO; }
+        if (ctx) ctx->launches += r->cuda.launches;
+        if (rc || !R::keeps_backend) be.release();
+        return rc;
+    };
+    const int rc = ctx ? go(r->cuda) : go(r->host);
+    if (rc) return rc;
+    *out = r.release();
+    return TREDSW_OK;
+}
 }  // namespace
 
 extern "C" {
@@ -1512,18 +1600,9 @@ int tredsw_ingest_scan_run_ex(tredsw_ctx *ctx, tredsw_bam *bam, const tredsw_loc
     if (!irr_params_ok(irr)) return TREDSW_ERR_ARG;
     *out = nullptr;
     if (bam->consumed) { tredsw_set_error("%s: stream already consumed", bam->path.c_str()); return TREDSW_ERR_ARG; }
-    std::lock_guard<std::mutex> lock(ctx->mu);
-    CUDA_TRY(cudaSetDevice(ctx->device));
-    keep_pool(ctx->device);
-    std::unique_ptr<tredsw_ingest_batch> b(new tredsw_ingest_batch());
-    b->cuda.stream = ctx->stream;
-    int rc;
-    try { rc = run_scan(b->cuda, b.get(), bam, queries, nqueries, depth_regions, n_depth, depth_out, slab_bytes, flags, irr); }
-    catch (const std::exception &e) { tredsw_set_error("tredsw_ingest_scan_run: %s", e.what()); rc = TREDSW_ERR_IO; }
-    ctx->launches += b->cuda.launches;
-    if (rc) { b->cuda.release(); return rc; }
-    *out = b.release();
-    return TREDSW_OK;
+    return run_entry(ctx, "tredsw_ingest_scan_run", out, [&](auto &be, tredsw_ingest_batch *b) {
+        return run_scan(be, b, bam, queries, nqueries, depth_regions, n_depth, depth_out, slab_bytes, flags, irr);
+    });
 }
 
 // TEST INFRASTRUCTURE: tredsw_ingest_scan_run with every kernel body run serially on the host.  Not used by the package.
@@ -1541,14 +1620,9 @@ int tredsw_ingest_scan_emulate_ex(tredsw_bam *bam, const tredsw_locus_query *que
     if (!irr_params_ok(irr)) return TREDSW_ERR_ARG;
     *out = nullptr;
     if (bam->consumed) { tredsw_set_error("%s: stream already consumed", bam->path.c_str()); return TREDSW_ERR_ARG; }
-    std::unique_ptr<tredsw_ingest_batch> b(new tredsw_ingest_batch());
-    b->emulated = true;
-    int rc;
-    try { rc = run_scan(b->host, b.get(), bam, queries, nqueries, depth_regions, n_depth, depth_out, slab_bytes, flags, irr); }
-    catch (const std::exception &e) { tredsw_set_error("tredsw_ingest_scan_emulate: %s", e.what()); rc = TREDSW_ERR_IO; }
-    if (rc) { b->host.release(); return rc; }
-    *out = b.release();
-    return TREDSW_OK;
+    return run_entry(nullptr, "tredsw_ingest_scan_emulate", out, [&](auto &be, tredsw_ingest_batch *b) {
+        return run_scan(be, b, bam, queries, nqueries, depth_regions, n_depth, depth_out, slab_bytes, flags, irr);
+    });
 }
 
 int tredsw_ingest_scan_irr(const tredsw_ingest_batch *b, tredsw_irr_view *v) {
@@ -1576,19 +1650,9 @@ int tredsw_ingest_scan_stats(const tredsw_ingest_batch *b, int64_t *stats) {
 int tredsw_ingest_batch_run(tredsw_ctx *ctx, tredsw_bam *const *bams, const int32_t *sample_of,
                             const tredsw_locus_query *queries, int32_t nqueries, uint32_t flags, tredsw_ingest_batch **out) {
     if (!ctx || !out || nqueries < 0 || (nqueries > 0 && (!bams || !sample_of || !queries))) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
-    *out = nullptr;
-    std::lock_guard<std::mutex> lock(ctx->mu);
-    CUDA_TRY(cudaSetDevice(ctx->device));
-    keep_pool(ctx->device);
-    std::unique_ptr<tredsw_ingest_batch> b(new tredsw_ingest_batch());
-    b->cuda.stream = ctx->stream;
-    int rc;
-    try { rc = run_pipeline(b->cuda, b.get(), bams, sample_of, queries, nqueries, flags); }
-    catch (const std::exception &e) { tredsw_set_error("tredsw_ingest_batch_run: %s", e.what()); rc = TREDSW_ERR_IO; }
-    ctx->launches += b->cuda.launches;
-    if (rc) { b->cuda.release(); return rc; }
-    *out = b.release();
-    return TREDSW_OK;
+    return run_entry(ctx, "tredsw_ingest_batch_run", out, [&](auto &be, tredsw_ingest_batch *b) {
+        return run_pipeline(be, b, bams, sample_of, queries, nqueries, flags);
+    });
 }
 
 // TEST INFRASTRUCTURE: the same pipeline with every kernel body run serially on the host (no CUDA calls).  The
@@ -1596,15 +1660,9 @@ int tredsw_ingest_batch_run(tredsw_ctx *ctx, tredsw_bam *const *bams, const int3
 int tredsw_ingest_batch_emulate(tredsw_bam *const *bams, const int32_t *sample_of, const tredsw_locus_query *queries,
                                 int32_t nqueries, uint32_t flags, tredsw_ingest_batch **out) {
     if (!out || nqueries < 0 || (nqueries > 0 && (!bams || !sample_of || !queries))) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
-    *out = nullptr;
-    std::unique_ptr<tredsw_ingest_batch> b(new tredsw_ingest_batch());
-    b->emulated = true;
-    int rc;
-    try { rc = run_pipeline(b->host, b.get(), bams, sample_of, queries, nqueries, flags); }
-    catch (const std::exception &e) { tredsw_set_error("tredsw_ingest_batch_emulate: %s", e.what()); rc = TREDSW_ERR_IO; }
-    if (rc) { b->host.release(); return rc; }
-    *out = b.release();
-    return TREDSW_OK;
+    return run_entry(nullptr, "tredsw_ingest_batch_emulate", out, [&](auto &be, tredsw_ingest_batch *b) {
+        return run_pipeline(be, b, bams, sample_of, queries, nqueries, flags);
+    });
 }
 
 int tredsw_ingest_batch_view(const tredsw_ingest_batch *b, tredsw_ingest_view *view) {
@@ -1636,6 +1694,10 @@ int tredsw_inflate_raw_device_code(const uint8_t *in, int64_t in_len, uint8_t *o
 // the reference tract scan: every tract of the requested motifs in a FASTA, plain text or BGZF (ref_tracts_device.cuh)
 // ---------------------------------------------------------------------------------------------------------------
 struct tredsw_tracts {
+    static constexpr bool keeps_backend = false;    // the results are host memory: the backend is released by run_entry
+    bool emulated = false;
+    CudaBackend cuda;
+    HostBackend host;
     std::vector<TractOut> tracts;
     std::vector<double> read_ms, device_ms;
     tredsw_tracts_view view;
@@ -1650,16 +1712,6 @@ int64_t fai_text_bytes(const tredsw_fai_entry &c) {     // bytes from a contig's
     if (c.length <= 0) return 0;
     const int64_t last = c.length - 1;
     return last / c.line_bases * c.line_width + last % c.line_bases + 1;
-}
-
-int64_t pread_full(int fd, uint8_t *dst, int64_t n, int64_t off) {     // -> the bytes read (< n: end of file or error)
-    int64_t got = 0;
-    while (got < n) {
-        const ssize_t k = pread(fd, dst + got, (size_t)(n - got), (off_t)(off + got));
-        if (k <= 0) break;
-        got += k;
-    }
-    return got;
 }
 
 // One block of a BGZF FASTA, from the walk of its headers: compressed offset and size, inflated offset and size.  The
@@ -1706,10 +1758,7 @@ void read_bgzf_step(int fd, const TractBlock *tb, TractStep *st) {
             st->at = tb[b].coff;
             break;
         }
-        BlockDesc d;
-        d.in_off = o + 12 + fr.xlen; d.out_off = tb[b].uoff - tb[st->b0].uoff;
-        d.clen = (uint32_t)fr.clen; d.isize = fr.isize; d.crc = fr.crc; d.pad_ = 0;
-        st->blocks.push_back(d);
+        st->blocks.push_back(block_desc(fr, o, tb[b].uoff - tb[st->b0].uoff));
     }
     st->ms = now_ms() - t0;
 }
@@ -1835,23 +1884,27 @@ int run_ref_tracts(B &be, tredsw_tracts *out, const char *path, const tredsw_fai
         for (const TractStep &st : steps) max_bytes = std::max(max_bytes, st.comp_bytes);
     }
     uint8_t *pinned[2] = {nullptr, nullptr};
-    for (uint8_t *&p : pinned) if (!steps.empty()) p = static_cast<uint8_t *>(be.alloc_host((size_t)max_bytes + 64));
-    int32_t *d_per = static_cast<int32_t *>(be.alloc(sizeof(int32_t) * (size_t)(2 * nper + 1)));
-    uint64_t *d_codes = static_cast<uint64_t *>(be.alloc(sizeof(uint64_t) * std::max<size_t>(1, mcodes.size())));
-    unsigned long long *d_small = static_cast<unsigned long long *>(be.alloc(sizeof(unsigned long long) * 3));
+    for (uint8_t *&p : pinned) if (!steps.empty()) p = alloc_host_n<uint8_t>(be, max_bytes + 64);
+    int32_t *d_per = alloc_n<int32_t>(be, 2 * nper + 1);
+    uint64_t *d_codes = alloc_n<uint64_t>(be, (int64_t)mcodes.size());
+    unsigned long long *d_small = alloc_n<unsigned long long>(be, 3);
     if (be.rc) return be.rc;
     be.upload(d_per, periods.data(), sizeof(int32_t) * (size_t)nper);
     be.upload(d_per + nper, mfirst.data(), sizeof(int32_t) * (size_t)(nper + 1));
     be.upload(d_codes, mcodes.data(), sizeof(uint64_t) * mcodes.size());
     const TractQuery q{d_per, d_per + nper, d_codes, nper, prm.min_units, (int64_t)prm.min_len};
-    void *d_text = nullptr, *d_code = nullptr, *d_valid = nullptr, *d_cs = nullptr, *d_out = nullptr;
-    void *d_comp = nullptr, *d_blocks = nullptr, *d_bstatus = nullptr;
-    size_t c_text = 0, c_code = 0, c_valid = 0, c_cs = 0, c_out = 0, c_comp = 0, c_blocks = 0, c_bstatus = 0;
-    grow(be, d_out, c_out, sizeof(TractOut) * 65536);
+    struct {                                            // device buffers reused from step to step
+        Reused<uint8_t> text, comp, bstatus;
+        Reused<uint64_t> code;
+        Reused<uint32_t> valid;
+        Reused<TractContig> cs;
+        Reused<BlockDesc> blocks;
+        Reused<TractOut> out;
+    } buf;
+    buf.out.get(be, 65536);
     int64_t invalid = 0, bytes = 0, comp_bytes = 0, nblocks = 0;
     auto read_step = [&](TractStep *st) { if (bgzf) read_bgzf_step(fd, tb.data(), st); else read_tract_step(fd, cs, st); };
-    std::thread reader;
-    struct Join { std::thread &t; ~Join() { if (t.joinable()) t.join(); } } join_reader{reader};
+    ReadAhead reader;
     if (!steps.empty()) { steps[0].buf = pinned[0]; read_step(&steps[0]); }
     for (size_t k = 0; k < steps.size(); ++k) {
         TractStep &st = steps[k];
@@ -1859,7 +1912,7 @@ int run_ref_tracts(B &be, tredsw_tracts *out, const char *path, const tredsw_fai
         if (st.why) { tredsw_set_error("%s: %s", path, st.why); return TREDSW_ERR_IO; }
         if (k + 1 < steps.size()) {
             steps[k + 1].buf = pinned[(k + 1) & 1];
-            reader = std::thread(read_step, &steps[k + 1]);
+            reader.start(read_step, &steps[k + 1]);
         }
         const double t_dev = now_ms();
         // the step's contigs: text and word offsets
@@ -1873,18 +1926,18 @@ int run_ref_tracts(B &be, tredsw_tracts *out, const char *path, const tredsw_fai
             text_at += fai_text_bytes(f);
             words += tract_words(f.length);
         }
-        uint8_t *text = static_cast<uint8_t *>(grow(be, d_text, c_text, (size_t)st.bytes + 64));
-        uint64_t *code = static_cast<uint64_t *>(grow(be, d_code, c_code, sizeof(uint64_t) * (size_t)std::max<int64_t>(1, words)));
-        uint32_t *valid = static_cast<uint32_t *>(grow(be, d_valid, c_valid, sizeof(uint32_t) * (size_t)std::max<int64_t>(1, words)));
-        TractContig *dcs = static_cast<TractContig *>(grow(be, d_cs, c_cs, sizeof(TractContig) * (size_t)ncs));
+        uint8_t *text = buf.text.get(be, st.bytes + 64);
+        uint64_t *code = buf.code.get(be, words);
+        uint32_t *valid = buf.valid.get(be, words);
+        TractContig *dcs = buf.cs.get(be, ncs);
         if (be.rc) return be.rc;
         const int nb = (int)st.blocks.size();
         std::vector<uint8_t> h_bstatus(nb);
         uint8_t *bstatus = nullptr;
         if (bgzf) {                                     // the step's blocks, inflated into its text buffer
-            uint8_t *comp = static_cast<uint8_t *>(grow(be, d_comp, c_comp, (size_t)st.comp_bytes + 64));
-            BlockDesc *blocks = static_cast<BlockDesc *>(grow(be, d_blocks, c_blocks, sizeof(BlockDesc) * (size_t)std::max(1, nb)));
-            bstatus = static_cast<uint8_t *>(grow(be, d_bstatus, c_bstatus, (size_t)std::max(1, nb)));
+            uint8_t *comp = buf.comp.get(be, st.comp_bytes + 64);
+            BlockDesc *blocks = buf.blocks.get(be, nb);
+            bstatus = buf.bstatus.get(be, nb);
             if (be.rc) return be.rc;
             be.upload(comp, st.buf, (size_t)st.comp_bytes);
             be.upload(blocks, st.blocks.data(), sizeof(BlockDesc) * (size_t)nb);
@@ -1905,8 +1958,8 @@ int run_ref_tracts(B &be, tredsw_tracts *out, const char *path, const tredsw_fai
         // the runs of every period, one thread per (word, period); more tracts than room: run again with room for all
         unsigned long long h_small[3] = {0, 0, 0};
         for (int pass = 0; pass < 2; ++pass) {
-            const unsigned long long cap = c_out / sizeof(TractOut);
-            TractOut *tout = static_cast<TractOut *>(d_out);
+            const unsigned long long cap = (unsigned long long)buf.out.cap;
+            TractOut *tout = buf.out.p;
             be.template for_each<TractRunsTag>(words * nper, [=] __host__ __device__(int64_t i) {
                 const int64_t w = i / q.nper;
                 const TractContig &c = dcs[tract_contig_of(dcs, ncs, w)];
@@ -1925,14 +1978,14 @@ int run_ref_tracts(B &be, tredsw_tracts *out, const char *path, const tredsw_fai
             if (h_small[2]) { tredsw_set_error("%s: a base position holds a line break or a header: the index does not fit the file", path); return TREDSW_ERR_IO; }
             if (h_small[0] <= cap) break;
             if (pass) { tredsw_set_error("tract count changed between passes"); return TREDSW_ERR_CUDA; }
-            c_out = sizeof(TractOut) * (size_t)(h_small[0] + h_small[0] / 4 + 1024);
-            d_out = be.alloc(c_out);
+            buf.out.cap = (int64_t)(h_small[0] + h_small[0] / 4 + 1024);      // room for all, not geometric
+            buf.out.p = alloc_n<TractOut>(be, buf.out.cap);
             be.fill(cnt, 0, sizeof(unsigned long long));
             if (be.rc) return be.rc;
         }
         const size_t t0 = out->tracts.size();
         out->tracts.resize(t0 + (size_t)h_small[0]);
-        be.download(out->tracts.data() + t0, d_out, sizeof(TractOut) * (size_t)h_small[0]);
+        be.download(out->tracts.data() + t0, buf.out.p, sizeof(TractOut) * (size_t)h_small[0]);
         be.sync();
         if (be.rc) return be.rc;
         invalid += (int64_t)h_small[1];
@@ -1941,7 +1994,7 @@ int run_ref_tracts(B &be, tredsw_tracts *out, const char *path, const tredsw_fai
         nblocks += nb;
         out->read_ms.push_back(st.ms);
         out->device_ms.push_back(now_ms() - t_dev);
-        if (reader.joinable()) reader.join();
+        reader.join();
     }
     std::sort(out->tracts.begin(), out->tracts.end(), [](const TractOut &x, const TractOut &y) {
         return x.contig != y.contig ? x.contig < y.contig : x.start != y.start ? x.start < y.start : x.period < y.period;
@@ -1989,21 +2042,9 @@ int tredsw_ref_tracts(tredsw_ctx *ctx, const char *fasta_path, const tredsw_fai_
                       tredsw_tracts **result) {
     if (!ctx) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
     if (!tract_args_ok(fasta_path, contigs, ncontigs, motifs, nmotifs, params, result)) return TREDSW_ERR_ARG;
-    *result = nullptr;
-    std::lock_guard<std::mutex> lock(ctx->mu);
-    CUDA_TRY(cudaSetDevice(ctx->device));
-    keep_pool(ctx->device);
-    std::unique_ptr<tredsw_tracts> r(new tredsw_tracts());
-    CudaBackend be;
-    be.stream = ctx->stream;
-    int rc;
-    try { rc = run_ref_tracts(be, r.get(), fasta_path, contigs, ncontigs, motifs, nmotifs, *params); }
-    catch (const std::exception &e) { tredsw_set_error("tredsw_ref_tracts: %s", e.what()); rc = TREDSW_ERR_IO; }
-    ctx->launches += be.launches;
-    be.release();
-    if (rc) return rc;
-    *result = r.release();
-    return TREDSW_OK;
+    return run_entry(ctx, "tredsw_ref_tracts", result, [&](auto &be, tredsw_tracts *r) {
+        return run_ref_tracts(be, r, fasta_path, contigs, ncontigs, motifs, nmotifs, *params);
+    });
 }
 
 // TEST INFRASTRUCTURE: tredsw_ref_tracts with every kernel body run serially on the host.  Not used by the package.
@@ -2011,16 +2052,9 @@ int tredsw_ref_tracts_emulate(tredsw_ctx *, const char *fasta_path, const tredsw
                               const tredsw_motif *motifs, int32_t nmotifs, const tredsw_tract_params *params,
                               tredsw_tracts **result) {
     if (!tract_args_ok(fasta_path, contigs, ncontigs, motifs, nmotifs, params, result)) return TREDSW_ERR_ARG;
-    *result = nullptr;
-    std::unique_ptr<tredsw_tracts> r(new tredsw_tracts());
-    HostBackend be;
-    int rc;
-    try { rc = run_ref_tracts(be, r.get(), fasta_path, contigs, ncontigs, motifs, nmotifs, *params); }
-    catch (const std::exception &e) { tredsw_set_error("tredsw_ref_tracts_emulate: %s", e.what()); rc = TREDSW_ERR_IO; }
-    be.release();
-    if (rc) return rc;
-    *result = r.release();
-    return TREDSW_OK;
+    return run_entry(nullptr, "tredsw_ref_tracts_emulate", result, [&](auto &be, tredsw_tracts *r) {
+        return run_ref_tracts(be, r, fasta_path, contigs, ncontigs, motifs, nmotifs, *params);
+    });
 }
 
 int tredsw_ref_tracts_view(const tredsw_tracts *r, tredsw_tracts_view *v) {

@@ -539,15 +539,11 @@ class ScanBatch(IngestBatch):
         out = ctypes.c_void_p()
         args = (handle.handle, qs, n, dr.ctypes.data if len(dr) else None, len(dr), depths.ctypes.data,
                 int(slab_bytes or 0), flags)
-        if irr is None:
-            if ctx is None:
-                rc = self.lib.tredsw_ingest_scan_emulate(*args, ctypes.byref(out))
-            else:
-                rc = self.lib.tredsw_ingest_scan_run(ctx.handle, *args, ctypes.byref(out))
-        elif ctx is None:
-            rc = self.lib.tredsw_ingest_scan_emulate_ex(*args, ctypes.byref(irr), ctypes.byref(out))
+        irr_arg = None if irr is None else ctypes.byref(irr)
+        if ctx is None:
+            rc = self.lib.tredsw_ingest_scan_emulate_ex(*args, irr_arg, ctypes.byref(out))
         else:
-            rc = self.lib.tredsw_ingest_scan_run_ex(ctx.handle, *args, ctypes.byref(irr), ctypes.byref(out))
+            rc = self.lib.tredsw_ingest_scan_run_ex(ctx.handle, *args, irr_arg, ctypes.byref(out))
         _lib.check(rc, "tredsw_ingest_scan_run")
         self._attach(out, n, want_names)
         self.irr = self._irr() if irr is not None else None
