@@ -37,15 +37,18 @@ def up_to_date():
     return all(os.path.getmtime(d) <= t for d in deps)
 
 
-def build(force=False, verbose=False):
-    if not force and up_to_date():
+def build(force=False, verbose=False, outdir=None, defines=()):
+    """Build the library in-tree, or with outdir: objects and library in that directory (always rebuilt), compiled
+    with the macros in defines (e.g. TREDSW_PHASE_CLOCKS for tools/phase_clock_bench.py)."""
+    lib = os.path.join(outdir, "libtredsw.so") if outdir else OUT
+    if not outdir and not force and up_to_date():
         return OUT
     objs = []
     procs = []
     for s in SOURCES:
-        o = os.path.join(CSRC, os.path.splitext(s)[0] + ".o")
-        cmd = [nvcc_path(), "-O3", "-std=c++17", *ARCH, "-lineinfo", "--extended-lambda", "-Xcompiler", "-fPIC", "-c",
-               os.path.join(CSRC, s), "-o", o]
+        o = os.path.join(outdir or CSRC, os.path.splitext(s)[0] + ".o")
+        cmd = [nvcc_path(), "-O3", "-std=c++17", *ARCH, "-lineinfo", "--extended-lambda", "-Xcompiler", "-fPIC",
+               *["-D" + d for d in defines], "-c", os.path.join(CSRC, s), "-o", o]
         if verbose:
             cmd += ["-Xptxas", "-v"]
         procs.append((s, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT)))
@@ -56,8 +59,8 @@ def build(force=False, verbose=False):
             sys.stderr.write(out.decode("utf-8", "replace"))
         if pr.returncode:
             raise RuntimeError("nvcc failed on {}".format(s))
-    subprocess.check_call([nvcc_path(), *ARCH, "-shared", "-o", OUT] + objs + ["-lz"])
-    return OUT
+    subprocess.check_call([nvcc_path(), *ARCH, "-shared", "-o", lib] + objs + ["-lz"])
+    return lib
 
 
 if __name__ == "__main__":

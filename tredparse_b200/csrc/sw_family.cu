@@ -83,6 +83,31 @@ struct ClassifyParams {
 
 __constant__ int8_t c_fmat25[25];
 
+// Phase clocks of the packed kernel (timing build only: -DTREDSW_PHASE_CLOCKS, tools/phase_clock_bench.py).  Lane 0
+// adds clock64() deltas per item to global counters [instance period][phase], so the build keeps the production
+// shared memory and occupancy.  All marks sit where the warp is converged; the per-lane begin sweep is counted as the
+// longest lane's sweep of the round.
+enum { PH_SETUP, PH_SUFFIX, PH_PREFIX, PH_MAIN, PH_LOC_MAIN, PH_LOC_SUFFIX, PH_BEGIN, PH_PICK, PH_ROUNDS, PH_ITEMS,
+       NPHASE };
+constexpr int PHASE_PERIODS = 13;  // instance periods 1..12 (index 0 unused)
+#ifdef TREDSW_PHASE_CLOCKS
+__device__ unsigned long long g_phase_clk[PHASE_PERIODS * NPHASE];
+__device__ __forceinline__ void phase_add(int pi, int ph, unsigned long long v) {
+    if (threadIdx.x == 0) atomicAdd(&g_phase_clk[pi * NPHASE + ph], v);
+}
+// adds the clocks since t to phase ph and restarts t
+__device__ __forceinline__ void phase_mark(int pi, int ph, long long &t) {
+    const long long t1 = clock64();
+    phase_add(pi, ph, (unsigned long long)(t1 - t));
+    t = t1;
+}
+#define PHASE_START(t) long long t = clock64()
+#define PHASE_MARK(pi, ph, t) phase_mark(pi, ph, t)
+#else
+#define PHASE_START(t)
+#define PHASE_MARK(pi, ph, t) ((void)0)
+#endif
+
 // Base codes of one read, one byte per base at an arbitrary byte address: the unaligned head byte by byte, the body
 // with 16-byte loads (LDG.128), then the tail — f(j, code) is called for j = 0..m-1 in order.
 template <class F>
@@ -468,6 +493,7 @@ __device__ __noinline__ void locate_packed(const FamilySmem &F, const SwLut *lut
 #endif
     const int sh = half ? 16 : 0;
     int found_col = -1, found_row = 0;
+    PHASE_START(t_clk);
     {
         // main strip tstar (the repeat table of phase 1 stays in shared memory).  Every lane restarts from its
         // own strip's stored boundary column: stage it into shared memory first — 2 x rows independent,
@@ -490,6 +516,7 @@ __device__ __noinline__ void locate_packed(const FamilySmem &F, const SwLut *lut
         }
     }
     __syncwarp();
+    PHASE_MARK(P, PH_LOC_MAIN, t_clk);
     cells += (unsigned long long)m * 2ull * (unsigned long long)NC;
     if (__any_sync(0xffffffffu, u_main <= 0 && cs < 0x7fff)) {
         // suffix block of every lane's own template, entered through the captured boundary
@@ -512,6 +539,7 @@ __device__ __noinline__ void locate_packed(const FamilySmem &F, const SwLut *lut
             }
         }
         __syncwarp();
+        PHASE_MARK(P, PH_LOC_SUFFIX, t_clk);
         cells += (unsigned long long)m * 2ull * (unsigned long long)FLANK;
     }
     *end_ref = found_col; *end_read = found_row;
@@ -533,6 +561,7 @@ __device__ __noinline__ int phase1_packed(const FamilySmem &F, const SwLut *lut,
     const uint32_t mge2 = (uint32_t)((-ge) & 0xffff) | ((uint32_t)((-ge) & 0xffff) << 16);
     const uint32_t go2 = (uint32_t)go * 0x00010001u;
     const int rows2 = (m_warp + 1) & ~1;
+    PHASE_START(t_clk);
     // ---- suffix potentials (table columns reversed: column c' = suffix base FLANK-1-c') ---------------
     if (lane < FLANK) colsel[lane] = sel2(suf_base(F, sa, FLANK - 1 - lane), suf_base(F, sb, FLANK - 1 - lane));
     __syncwarp();
@@ -541,6 +570,7 @@ __device__ __noinline__ int phase1_packed(const FamilySmem &F, const SwLut *lut,
     uint32_t fresh = 0;
     suffix_pass<FLANK>(stab, codes, lane, m, rows2, pot, fresh, mgo2, mge2);
     __syncwarp();
+    PHASE_MARK(P, PH_SUFFIX, t_clk);
     // ---- strip 0: the FLANK prefix columns -----------------------------------------------------------
     if (lane < FLANK) colsel[lane] = sel2(pre_base(F, sa, lane), pre_base(F, sb, lane));
     __syncwarp();
@@ -554,6 +584,7 @@ __device__ __noinline__ int phase1_packed(const FamilySmem &F, const SwLut *lut,
         run = seg0[0];
     }
     __syncwarp();
+    PHASE_MARK(P, PH_PREFIX, t_clk);
     // ---- main strips: K repeat units each; the suffix of every template is folded in by the potentials --
     for (int c = lane; c < NC; c += 32) colsel[c] = sel2(rep_base(F, sa, c % F.P), rep_base(F, sb, c % F.P));
     __syncwarp();
@@ -600,6 +631,7 @@ __device__ __noinline__ int phase1_packed(const FamilySmem &F, const SwLut *lut,
             break;
         }
     }
+    PHASE_MARK(P, PH_MAIN, t_clk);
     // (cells: the full plan, whether or not strips were skipped — the executed-cell statistic keeps its meaning;
     //  the skipped ones are counted apart)
     cells += (unsigned long long)m * 2ull * (unsigned long long)(2 * FLANK + nplan * NC);
@@ -615,8 +647,10 @@ __device__ __noinline__ int phase1_packed(const FamilySmem &F, const SwLut *lut,
 // Persistent: one warp per CTA, CTAs pull items (32 reads of one family, or 64 single-strand reads of one family
 // and strand, two per lane) from a counter; both kernels walk the same item list and skip the items of the other
 // kernel.
+// (One warp per CTA.  __maxnreg__ instead of __launch_bounds__(32): with the launch bound alone ptxas stops at 168
+//  registers and spills in phase 2; 8 resident single-warp CTAs per SM leave room for the full 255.)
 template <bool FAST>
-__global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
+__global__ void __maxnreg__(255) classify_kernel(ClassifyParams p) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ SwLut lut;
     __shared__ FamilySmem F;
@@ -643,8 +677,22 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
     uint32_t *pot = FAST ? bnd : p.pot_buf + (size_t)blockIdx.x * R * 32;
     uint32_t *gbnd = p.gbnd_buf + (size_t)blockIdx.x * (p.nslots + 1) * R * 32;    // [nslots + 1][R][32]
     const uint32_t one = p.one;
-    __shared__ unsigned long long skip_acc[TREDSW_STRIP_SKIP_STATS];   // this CTA's share, added up at the end
-    for (int i = lane; i < TREDSW_STRIP_SKIP_STATS; i += 32) skip_acc[i] = 0ull;
+    // Strip-skip counters of the instance period this CTA is working on (lane 0, registers): items come in period
+    // order (grp_perm), so they are flushed to the context's counters when the period changes and at the end.  (Not in
+    // shared memory: 85 x 8 B there cost the eighth resident CTA per SM at 150 bp, see DESIGN.md §4.1.)
+    int skip_pi = 0;
+    unsigned long long skip_acc[7] = {0ull, 0ull, 0ull, 0ull, 0ull, 0ull, 0ull};
+    auto flush_skip = [&]() {
+        if (lane == 0 && skip_pi > 0) {
+            unsigned long long *a = p.skip_stats + 1 + 4 * (skip_pi - 1), *b = p.skip_stats + 1 + 4 * 12 + 3 * (skip_pi - 1);
+#pragma unroll
+            for (int i = 0; i < 4; ++i) if (skip_acc[i]) atomicAdd(a + i, skip_acc[i]);
+#pragma unroll
+            for (int i = 0; i < 3; ++i) if (skip_acc[4 + i]) atomicAdd(b + i, skip_acc[4 + i]);
+        }
+#pragma unroll
+        for (int i = 0; i < 7; ++i) skip_acc[i] = 0ull;
+    };
     sw_build_lut(&lut, c_fmat25, lane, 32);
     const int nitems = p.chunk_start[p.ngroups];
     unsigned long long alg = 0, cells1 = 0, cells2 = 0, cells_skipped = 0;
@@ -652,6 +700,7 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
 
     for (;;) {
         __syncwarp();
+        PHASE_START(t_clk);
         int item = 0;
         if (lane == 0) item = atomicAdd(p.counter + (FAST ? 1 : 0), 1);
         item = __shfl_sync(0xffffffffu, item, 0);
@@ -700,31 +749,30 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
         __syncwarp();
 
         int last_slot = 0;              // last boundary slot phase 1 wrote (packed kernel)
+        const int pi = FAST ? instance_period(F.P) : 0;
         if constexpr (!FAST) {
             phase1_generic(F, &lut, codes, lane, m0, m_warp, bnd, scores, p.go, p.ge, cells1);
         } else {
-            const int pi = instance_period(F.P);
+            PHASE_MARK(pi, PH_SETUP, t_clk);
             int planned = 0, conv = 0;
             switch (pi) {
 #define PCASE(PP) case PP: last_slot = phase1_packed<PP>(F, &lut, stab, colsel, codes, lane, m_lane, m_warp, pot, gbnd, R, scores, runs, p.go, p.ge, one, F.P / PP, sa, sb, p.strip_skip != 0, &planned, &conv, cells1, cells_skipped); break;
                 PCASE(1) PCASE(2) PCASE(3) PCASE(4) PCASE(5) PCASE(7) PCASE(8) PCASE(9) PCASE(10) PCASE(11) PCASE(12)
 #undef PCASE
             }
-            if (lane == 0) {            // per instance period: planned / skipped main strips, items, items without a skip
-                unsigned long long *a = skip_acc + 1 + 4 * (pi - 1);
-                a[0] += (unsigned long long)planned; a[1] += (unsigned long long)(planned - last_slot);
-                a[2] += 1ull; a[3] += last_slot == planned ? 1ull : 0ull;
-            }
+#ifdef TREDSW_PHASE_CLOCKS
+            t_clk = clock64();          // (phase1_packed counted its own phases)
+#endif
+            if (pi != skip_pi) { flush_skip(); skip_pi = pi; }
+            // per instance period: planned / skipped main strips, items, items without a skip
+            skip_acc[0] += (unsigned long long)planned; skip_acc[1] += (unsigned long long)(planned - last_slot);
+            skip_acc[2] += 1ull; skip_acc[3] += last_slot == planned ? 1ull : 0ull;
             // per lane holding a read: the strips of the plan, those its warp skipped, and those it could skip on its
             // own (the bound that no grouping of reads into items can beat)
             const bool busy = m_lane > 0;
-            const unsigned lane_planned = __reduce_add_sync(0xffffffffu, busy ? (unsigned)planned : 0u);
-            const unsigned lane_skipped = __reduce_add_sync(0xffffffffu, busy ? (unsigned)(planned - last_slot) : 0u);
-            const unsigned lane_skippable = __reduce_add_sync(0xffffffffu, busy ? (unsigned)(planned - conv) : 0u);
-            if (lane == 0) {
-                unsigned long long *b = skip_acc + 1 + 4 * 12 + 3 * (pi - 1);
-                b[0] += lane_planned; b[1] += lane_skipped; b[2] += lane_skippable;
-            }
+            skip_acc[4] += __reduce_add_sync(0xffffffffu, busy ? (unsigned)planned : 0u);
+            skip_acc[5] += __reduce_add_sync(0xffffffffu, busy ? (unsigned)(planned - last_slot) : 0u);
+            skip_acc[6] += __reduce_add_sync(0xffffffffu, busy ? (unsigned)(planned - conv) : 0u);
         }
         __syncwarp();
 
@@ -760,6 +808,7 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
             const int max_units_eff = F.clip ? (m + F.P - 1) / F.P : F.U;
             auto own_code = [&](int j) { return FAST ? pair_half(codes[j * 32 + lane], h) : (int)codes[j * 32 + lane]; };
             while (__any_sync(0xffffffffu, cr >= 0)) {
+                if constexpr (FAST) PHASE_MARK(pi, PH_PICK, t_clk);
                 const bool pending = cr >= 0;
                 const int u = pending ? cr / 2 + 1 : 1, s = pending ? (cr & 1) : 0;
                 const int half = pair ? h : s;
@@ -775,7 +824,13 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
                         }
                         if (!pending) fast_end_ref = -1;
                     }
+#ifdef TREDSW_PHASE_CLOCKS
+                    t_clk = clock64();      // (locate_packed counted its own phases)
+#endif
                 }
+#ifdef TREDSW_PHASE_CLOCKS
+                long long t_begin = 0;      // this lane's begin sweep
+#endif
                 if (pending) {
                     const int n = F.Lp + F.Ls + F.P * u;
                     auto cc_f = [&](int i) { return fam_code(F, u, s, n, i); };
@@ -795,6 +850,9 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
                         // Reverse: only a path leaving the corner (end_ref, end_read) can reach cs (Appendix A); it
                         // lives in the (end_read+1) x (end_ref+1) rectangle, which bounds its aligned pairs and
                         // therefore how far it can drift from the corner's diagonal.
+#ifdef TREDSW_PHASE_CLOCKS
+                        t_begin = clock64();
+#endif
                         const int rdrift = sw_max_drift(cs, end_read + 1, end_ref + 1, p.match, p.go, p.ge);
                         int ci = -1, rj = 0;
                         if (rdrift == 0) {   // no gap affordable: walk the diagonal
@@ -814,6 +872,9 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
                             sw_sweep<FAM_W2, 1, false>(end_read + 1, end_read + 1, end_ref + 1, rc_r, cc_r, &lut, bnd + lane, 32,
                                                        p.go, p.ge, cs, &ci, &rj, nullptr, -rdrift, rdrift, &cells2);
                         }
+#ifdef TREDSW_PHASE_CLOCKS
+                        t_begin = clock64() - t_begin;
+#endif
                         const int c_rb = end_ref - ci, c_qb = end_read - rj;
                         const int t = sw_classify(cs, c_rb, end_ref, c_qb, end_read, m, n, u, F.P, max_units_eff);
                         if (t != TREDSW_TAG_NONE) {
@@ -826,6 +887,16 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
                     else { const int ls = cs, lr = cr; pick(ls, lr, cs, cr); }
                 }
                 __syncwarp();
+#ifdef TREDSW_PHASE_CLOCKS
+                if constexpr (FAST) {
+                    const unsigned begin = __reduce_max_sync(0xffffffffu, (unsigned)t_begin);
+                    const long long t1 = clock64();
+                    phase_add(pi, PH_BEGIN, begin);
+                    phase_add(pi, PH_PICK, (unsigned long long)(t1 - t_clk) - begin);
+                    phase_add(pi, PH_ROUNDS, 1ull);
+                    t_clk = t1;
+                }
+#endif
             }
             if (valid) {
                 int32_t *o = p.out + (int64_t)r * 8;
@@ -839,6 +910,13 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
                 nal += (unsigned)(2 * F.U);
             }
         }
+#ifdef TREDSW_PHASE_CLOCKS
+        if constexpr (FAST) {
+            __syncwarp();
+            PHASE_MARK(pi, PH_PICK, t_clk);
+            phase_add(pi, PH_ITEMS, 1ull);
+        }
+#endif
     }
     if (p.stats) {
         unsigned long long c1 = cells1, c2 = cells2, na = nal;
@@ -854,11 +932,9 @@ __global__ void __launch_bounds__(32) classify_kernel(ClassifyParams p) {
         }
     }
     if (FAST) {
+        flush_skip();
         for (int d = 16; d > 0; d >>= 1) cells_skipped += __shfl_down_sync(0xffffffffu, cells_skipped, d);
-        if (lane == 0) skip_acc[0] = cells_skipped;
-        __syncwarp();
-        for (int i = lane; i < TREDSW_STRIP_SKIP_STATS; i += 32)
-            if (skip_acc[i]) atomicAdd(&p.skip_stats[i], skip_acc[i]);
+        if (lane == 0 && cells_skipped) atomicAdd(&p.skip_stats[0], cells_skipped);
     }
 }
 
@@ -1043,6 +1119,10 @@ int classify_static_smem(size_t *out) {
     return TREDSW_OK;
 }
 
+#ifdef TREDSW_PHASE_CLOCKS
+int g_occupancy_fast = 0;         // the occupancy API's resident CTAs per SM for the packed kernel, last launch
+#endif
+
 // resident CTAs per SM of the persistent kernels (registers / shared memory), times the SM count
 int persistent_ctas(tredsw_ctx *ctx, size_t smem, size_t static_smem, bool need_fast, bool need_generic, int *out) {
     int a = 0, b = 0;
@@ -1052,6 +1132,9 @@ int persistent_ctas(tredsw_ctx *ctx, size_t smem, size_t static_smem, bool need_
     }
     if (need_fast) CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a, classify_kernel<true>, 32, smem));
     if (need_generic) CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, classify_kernel<false>, 32, smem));
+#ifdef TREDSW_PHASE_CLOCKS
+    if (need_fast) g_occupancy_fast = a;
+#endif
     int per_sm = need_fast ? a : b;          // the packed kernel is the one that matters when both run
     static const int env_cap = [] { const char *e = getenv("TREDSW_CTAS_PER_SM"); return e ? atoi(e) : 0; }();
     // measured on B200 (profiles/): beyond 8 resident warps per SM the strip loops of the concurrently running
@@ -1313,6 +1396,21 @@ int tredsw_internal_classify(tredsw_ctx *ctx, const int8_t *d_rbuf, const int64_
     ctx->mark(1);
     return TREDSW_OK;
 }
+
+#ifdef TREDSW_PHASE_CLOCKS
+// Timing build only (tools/phase_clock_bench.py): the phase clocks summed over every launch so far, out[13 * 10] as
+// [instance period][phase] in the order of the PH_ enum, and the occupancy API's resident CTAs per SM of the packed
+// kernel at its last launch.  Synchronises the context's stream.
+extern "C" int tredsw_phase_clocks(tredsw_ctx *ctx, int64_t *out, int32_t *ctas_per_sm) {
+    if (!ctx || !out || !ctas_per_sm) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    CUDA_TRY(cudaMemcpyFromSymbol(out, g_phase_clk, sizeof(g_phase_clk)));
+    *ctas_per_sm = g_occupancy_fast;
+    return TREDSW_OK;
+}
+#endif
 
 extern "C" int tredsw_classify_reads(tredsw_ctx *ctx, const int8_t *rbuf, const int64_t *roff, int32_t nreads,
                                      const int32_t *read_family, const tredsw_family *families,

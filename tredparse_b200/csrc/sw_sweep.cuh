@@ -68,6 +68,7 @@ __device__ __forceinline__ int sw_sweep(int m_real, int m_rows, int n, RowCode r
                                         int target, int *out_col, int *out_row, int32_t *colmax_out,
                                         int dlo = SW_NO_BAND_LO, int dhi = SW_NO_BAND_HI,
                                         unsigned long long *visited = nullptr) {
+    static_assert(W <= 32, "hit columns of a row are kept as a 32-bit mask");
     int mx = 0;
     int best_col = 0x7fffffff, best_row = 0;
     const int mge = -ge;
@@ -89,7 +90,65 @@ __device__ __forceinline__ int sw_sweep(int m_real, int m_rows, int n, RowCode r
         int hin_prev = 0;
         if (!first && jlo > 0 && jlo - 1 >= jlo_prev && jlo - 1 < jhi_prev)
             hin_prev = (int)(bnd[(size_t)(jlo - 1) * stride] & 0xffffu);
-        for (int j = jlo; j < jhi; ++j) {
+        // One DP cell of column c: hd = H diagonal in, H(above) read from / H written to Hrow[c], e = E along the row.
+        auto cell = [&](int &hd, int &e, int c, uint32_t w0, uint32_t w1) {
+            const int s = (int)sw_prmt(w0, w1, sel[c]);
+            const int t = max(e, F[c]);
+            const int h = __viaddmax_s32_relu(hd, s, t);
+            hd = Hrow[c];
+            Hrow[c] = h;
+            const int hgo = h - go;
+            e = __viaddmax_s32_relu(e, mge, hgo);
+            F[c] = __viaddmax_s32_relu(F[c], mge, hgo);
+            return h;
+        };
+        auto entering = [&](int j, int &hin, int &e) {
+            hin = 0; e = 0;
+            if (!first && j >= jlo_prev && j < jhi_prev) {
+                const uint32_t b = bnd[(size_t)j * stride];
+                hin = (int)(b & 0xffffu);
+                e = (int)(b >> 16);
+            }
+        };
+        // Rows in pairs, two dependency chains in flight: row j at column s while row j+1 is at column s-1 (row j+1's
+        // cell needs row j's cell of the same column, done one step earlier).  Same cells as one row at a time; the hit
+        // rule is kept: per row the smallest hit column, rows in order, a later row only wins with a smaller column.
+        int j = jlo;
+        for (; j + 1 < jhi; j += 2) {
+            int hinA, eA, hinB, eB;
+            entering(j, hinA, eA);
+            entering(j + 1, hinB, eB);
+            const int codeA = rowcode(j), codeB = rowcode(j + 1);
+            const uint32_t w0A = lut->w0[codeA], w1A = lut->w1[codeA], w0B = lut->w0[codeB], w1B = lut->w1[codeB];
+            int hdA = hin_prev, hdB = hinA;
+            hin_prev = hinB;
+            int hA = 0, hB = 0;
+            uint32_t hitA = 0u, hitB = 0u;           // hit columns of each row (bit c)
+#pragma unroll
+            for (int s = 0; s <= W; ++s) {
+                if (s < W) {
+                    hA = cell(hdA, eA, s, w0A, w1A);
+                    if (MODE == 1) hitA |= (hA == target) ? (1u << s) : 0u;
+                    else if (COLMAX) cm[s] = max(cm[s], hA);
+                    else mx = max(mx, hA);
+                }
+                if (s >= 1) {
+                    hB = cell(hdB, eB, s - 1, w0B, w1B);
+                    if (MODE == 1) hitB |= (hB == target) ? (1u << (s - 1)) : 0u;
+                    else if (COLMAX) cm[s - 1] = max(cm[s - 1], hB);
+                    else mx = max(mx, hB);
+                }
+            }
+            if (!last) {
+                bnd[(size_t)j * stride] = (uint32_t)hA | ((uint32_t)eA << 16);
+                bnd[(size_t)(j + 1) * stride] = (uint32_t)hB | ((uint32_t)eB << 16);
+            }
+            if (MODE == 1) {
+                if (hitA && j < m_real && c0 + __ffs(hitA) - 1 < best_col) { best_col = c0 + __ffs(hitA) - 1; best_row = j; }
+                if (hitB && j + 1 < m_real && c0 + __ffs(hitB) - 1 < best_col) { best_col = c0 + __ffs(hitB) - 1; best_row = j + 1; }
+            }
+        }
+        for (; j < jhi; ++j) {                       // the last row of an odd count
             int hin = 0, e = 0;
             if (!first && j >= jlo_prev && j < jhi_prev) {
                 uint32_t b = bnd[(size_t)j * stride];
