@@ -583,6 +583,8 @@ typedef struct {                /* host arrays, valid until tredsw_ref_tracts_fr
     double ms_total;
     int64_t comp_bytes, blocks;                   /* BGZF: compressed bytes read and blocks inflated, a block shared
                                                      by two steps counted twice; 0 for text */
+    const int32_t *segments;                      /* per tract: the segments of its chain (1: a pure tract, and
+                                                     every tract without chaining) */
 } tredsw_tracts_view;
 int tredsw_ref_tracts(tredsw_ctx *ctx, const char *fasta_path, const tredsw_fai_entry *contigs, int32_t ncontigs,
                       const tredsw_motif *motifs, int32_t nmotifs, const tredsw_tract_params *params,
@@ -592,6 +594,25 @@ int tredsw_ref_tracts(tredsw_ctx *ctx, const char *fasta_path, const tredsw_fai_
 int tredsw_ref_tracts_emulate(tredsw_ctx *ctx, const char *fasta_path, const tredsw_fai_entry *contigs,
                               int32_t ncontigs, const tredsw_motif *motifs, int32_t nmotifs,
                               const tredsw_tract_params *params, tredsw_tracts **result);
+/* Interrupted tracts (DESIGN §4.5.1).  A run is a maximal [a, e) with s[j] == s[j + k] (both bases in ACGTacgt) for
+ * every j in it, its bases [a, e + k); a segment is a run with e - a >= k.  A segment S = [a, e) links to the next
+ * segment T = [a', e') when both have root period k and one canonical code, a' - (e + k) <= max_interrupt (a deletion
+ * gives 0 or less) and every base of [e + k, a') is in ACGTacgt.  A maximal sequence of links S1 -> ... -> Sm is a
+ * chain; it gives the tract [a1, a1 + c k), c = floor((em + k - a1) / k), of S1's code, with `segments` = m, when
+ * A purity_den >= purity_num (em - a1), A the count of agreements in [a1, em) (the IRR classifier's purity test on the
+ * tract's own bases), and under the pure rule's filters.  A chain with m >= 2 that fails purity gives its segments,
+ * each judged alone by the pure rule; no sub-chain is searched.  max_interrupt 0 (or chain NULL) is exactly
+ * tredsw_ref_tracts, and so is purity 1 / 1.  0 <= max_interrupt <= 20, 0 < purity_num <= purity_den <= 1000, else
+ * TREDSW_ERR_ARG. */
+typedef struct { int32_t max_interrupt, purity_num, purity_den, reserved_; } tredsw_tract_chain;
+int tredsw_ref_tracts_ex(tredsw_ctx *ctx, const char *fasta_path, const tredsw_fai_entry *contigs, int32_t ncontigs,
+                         const tredsw_motif *motifs, int32_t nmotifs, const tredsw_tract_params *params,
+                         const tredsw_tract_chain *chain, tredsw_tracts **result);
+/* TEST INFRASTRUCTURE: tredsw_ref_tracts_ex run serially on the host, as tredsw_ref_tracts_emulate. */
+int tredsw_ref_tracts_emulate_ex(tredsw_ctx *ctx, const char *fasta_path, const tredsw_fai_entry *contigs,
+                                 int32_t ncontigs, const tredsw_motif *motifs, int32_t nmotifs,
+                                 const tredsw_tract_params *params, const tredsw_tract_chain *chain,
+                                 tredsw_tracts **result);
 int tredsw_ref_tracts_view(const tredsw_tracts *result, tredsw_tracts_view *view);
 void tredsw_ref_tracts_free(tredsw_tracts *result);
 

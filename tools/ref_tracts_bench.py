@@ -16,7 +16,14 @@ inflates on the GPU.  The two arms alternate call by call, and each reports its 
 ones.  The synthetic genome (uniform random bases) compresses less well than hg38, whose repeats and soft-masking
 give DEFLATE more to work with: the compressed-to-text ratio here is not hg38's.
 
-    python tools/ref_tracts_bench.py [--gbp 3.1] [--reps 3] [--step-mib 256] [--bgzip] [--out profiles/r3_ref_tracts_bench.json]
+--max-interruption N also plants interrupted tracts (one every 50 kb, from a second seeded stream, so the rest of the
+genome is unchanged: 6 to 40 copies of a motif with 1 to 3 substitutions, insertions or deletions) and splits every
+format into two arms that alternate call by call: the pure rule and the chain rule with interruptions of up to N bases
+at purity 9 / 10 (DESIGN §4.5.1).  Each arm reports its tracts and how many of them are chains.  Uniform random
+sequence rarely chains by chance, so those counts say nothing about hg38.
+
+    python tools/ref_tracts_bench.py [--gbp 3.1] [--reps 3] [--step-mib 256] [--bgzip] [--max-interruption N]
+                                     [--out profiles/r3_ref_tracts_bench.json]
 (without --out the result line is only printed)
 """
 import argparse
@@ -50,8 +57,27 @@ def card():
         return "unknown ({})".format(e)
 
 
-def write_genome(path, gbp, seed=0, width=60):
+def interrupted_tract(rng):
+    """a tract of 6 to 40 copies of a motif with 1 to 3 interruptions: a substitution, an insertion of 1 to 3 bases
+    or a deletion of one base"""
+    from tredparse_b200.simulate import interrupted_tract as planted
+    u = MOTIFS[int(rng.integers(len(MOTIFS)))]
+    n = int(rng.integers(6, 41))
+    edits = []
+    for c in sorted(set(int(x) for x in rng.integers(1, n, int(rng.integers(1, 4))))):
+        x = rng.random()
+        if x < 0.5:
+            edits.append((c, "sub", "ACGT"["ACGT".index(u[0]) ^ 1]))
+        elif x < 0.8:
+            edits.append((c, "ins", "".join("ACGT"[int(b)] for b in rng.integers(0, 4, int(rng.integers(1, 4))))))
+        else:
+            edits.append((c, "del", 1))
+    return planted(u, n, edits)
+
+
+def write_genome(path, gbp, seed=0, width=60, interrupted=False):
     rng = np.random.default_rng(seed)
+    irng = np.random.default_rng(seed + 1)
     lut = np.frombuffer(b"ACGT", np.uint8)
     scale = gbp * 1e3 / sum(HG38_MBP)
     total, fai = 0, []
@@ -63,6 +89,10 @@ def write_genome(path, gbp, seed=0, width=60):
                 u = MOTIFS[int(rng.integers(len(MOTIFS)))]
                 t = np.frombuffer((u * int(rng.integers(3, 41))).encode(), np.uint8)
                 a = int(rng.integers(0, L - len(t)))
+                s[a:a + len(t)] = t
+            for _ in range(L // 50000 if interrupted else 0):
+                t = np.frombuffer(interrupted_tract(irng).encode(), np.uint8)
+                a = int(irng.integers(0, L - len(t)))
                 s[a:a + len(t)] = t
             nb = L // 4096                                  # soft-masking: half of the 4 KiB blocks in lowercase
             blocks = s[:nb * 4096].reshape(nb, 4096)
@@ -106,8 +136,11 @@ def main():
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--step-mib", type=int, default=256)
     ap.add_argument("--bgzip", action="store_true", help="also scan a BGZF copy of the genome, the arms alternating")
+    ap.add_argument("--max-interruption", type=int, default=0,
+                    help="plant interrupted tracts and add a chain arm per format (1 to 20)")
     ap.add_argument("--out", default=None)
     a = ap.parse_args()
+    g = a.max_interruption
     from tredparse_b200 import _lib
     from tredparse_b200.fasta import Fasta
     ctx = _lib.default_context()
@@ -115,7 +148,7 @@ def main():
     try:
         path = os.path.join(d, "genome.fa")
         t0 = time.time()
-        bases = write_genome(path, a.gbp)
+        bases = write_genome(path, a.gbp, interrupted=g > 0)
         t_write = time.time() - t0
         paths = {"text": path}
         if a.bgzip:
@@ -123,17 +156,20 @@ def main():
             bgzip(path, path + ".gz")
             t_bgzip = time.time() - t0
             paths["bgzf"] = path + ".gz"
-        fas = {arm: Fasta(p) for arm, p in paths.items()}
-        calls = {arm: [] for arm in paths}
+        fas = {f: Fasta(p) for f, p in paths.items()}
+        # arm -> (format, max_interrupt)
+        arms_g = {f: (f, 0) for f in paths} if not g else \
+            {"{}_{}".format(f, r): (f, x) for f in paths for r, x in (("pure", 0), ("chain", g))}
+        calls = {arm: [] for arm in arms_g}
         for _ in range(a.reps + 1):                     # the arms alternate call by call
-            for arm, fa in fas.items():
+            for arm, (f, x) in arms_g.items():
                 t0 = time.perf_counter()
-                r = fa.tracts(MOTIFS, step_bytes=a.step_mib << 20, ctx=ctx)
+                r = fas[f].tracts(MOTIFS, step_bytes=a.step_mib << 20, ctx=ctx, max_interrupt=x)
                 calls[arm].append((time.perf_counter() - t0, r))
-        ref = calls["text"][0][1]["tracts"]
-        for arm in calls:
+        for arm, (_, x) in arms_g.items():              # every call of one rule gives the same tracts
+            ref = calls[next(b for b, (_, y) in arms_g.items() if y == x)][0][1]
             for _, r in calls[arm]:
-                assert np.array_equal(r["tracts"], ref), arm
+                assert np.array_equal(r["tracts"], ref["tracts"]) and np.array_equal(r["segments"], ref["segments"]), arm
 
         def summary(wall, res):
             s = res["stats"]
@@ -146,17 +182,27 @@ def main():
             first, later = calls[arm][0], calls[arm][1:]
             best = min(later, key=lambda c: c[0]) if later else first
             st = best[1]["stats"]
-            return {"file_bytes": os.path.getsize(paths[arm]), "steps": st["steps"], "text_bytes": st["bytes"],
-                    "comp_bytes": st["comp_bytes"], "blocks": st["blocks"], "invalid_bases": st["invalid_bases"],
-                    "tracts": st["tracts"], "first_call": summary(*first), "best_later_call": summary(*best),
+            out = {"file_bytes": os.path.getsize(paths[arms_g[arm][0]]), "steps": st["steps"], "text_bytes": st["bytes"],
+                   "comp_bytes": st["comp_bytes"], "blocks": st["blocks"], "invalid_bases": st["invalid_bases"],
+                   "tracts": st["tracts"]}
+            if g:                                       # counts only: the per-tract segments stay out of the card
+                out.update(max_interrupt=arms_g[arm][1], chains=int((best[1]["segments"] > 1).sum()))
+            return dict(out, **{"first_call": summary(*first), "best_later_call": summary(*best),
                     "later_walls_s": [round(w, 4) for w, _ in later],
                     "per_step_best": [{"read_ms": round(x, 2), "device_ms": round(y, 2)}
-                                      for x, y in zip(st["step_read_ms"], st["step_device_ms"])]}
+                                      for x, y in zip(st["step_read_ms"], st["step_device_ms"])]})
 
         head = {"card": card(), "gbp": a.gbp, "bases": bases, "write_s": round(t_write, 1), "motifs": len(MOTIFS),
                 "step_mib": a.step_mib}
         cache = "warm (files written in the same run); cold cache not measured"
-        if not a.bgzip:
+        if g:
+            arms = {arm: arm_result(arm) for arm in arms_g}
+            out = dict({"bench": "ref_tracts_chain"}, **head, max_interruption=g, purity=[9, 10], arms=arms,
+                       chain_note="uniform random sequence rarely chains by chance: the chain counts come from the "
+                                  "planted interrupted tracts and say nothing about hg38", page_cache=cache)
+            if a.bgzip:
+                out.update(bgzip_s=round(t_bgzip, 1))
+        elif not a.bgzip:
             out = dict({"bench": "ref_tracts"}, **head, **arm_result("text"), page_cache=cache.replace("files", "file"))
             del out["comp_bytes"], out["blocks"]
         else:

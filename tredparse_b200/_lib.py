@@ -42,6 +42,7 @@ EXPORTS = [
     "tredsw_ingest_scan_run_ex", "tredsw_ingest_scan_emulate_ex", "tredsw_ingest_scan_irr", "tredsw_irr_classify_host",
     # the reference tract scan (alt regions of discovered loci); *_emulate runs the device code on the host
     "tredsw_ref_tracts", "tredsw_ref_tracts_emulate", "tredsw_ref_tracts_view", "tredsw_ref_tracts_free",
+    "tredsw_ref_tracts_ex", "tredsw_ref_tracts_emulate_ex",
 ]
 
 
@@ -100,12 +101,19 @@ class TractParams(ctypes.Structure):
     _fields_ = [("min_units", ctypes.c_int32), ("min_len", ctypes.c_int32), ("step_bytes", ctypes.c_int64)]
 
 
+class TractChain(ctypes.Structure):
+    """tredsw_tract_chain (include/tredsw.h)"""
+    _fields_ = [("max_interrupt", ctypes.c_int32), ("purity_num", ctypes.c_int32), ("purity_den", ctypes.c_int32),
+                ("reserved_", ctypes.c_int32)]
+
+
 class TractsView(ctypes.Structure):
     """tredsw_tracts_view (include/tredsw.h)"""
     _fields_ = [("n_tracts", ctypes.c_int64), ("tracts", ctypes.c_void_p), ("steps", ctypes.c_int64),
                 ("bytes", ctypes.c_int64), ("bases", ctypes.c_int64), ("invalid_bases", ctypes.c_int64),
                 ("step_read_ms", ctypes.POINTER(ctypes.c_double)), ("step_device_ms", ctypes.POINTER(ctypes.c_double)),
-                ("ms_total", ctypes.c_double), ("comp_bytes", ctypes.c_int64), ("blocks", ctypes.c_int64)]
+                ("ms_total", ctypes.c_double), ("comp_bytes", ctypes.c_int64), ("blocks", ctypes.c_int64),
+                ("segments", ctypes.POINTER(ctypes.c_int32))]
 
 
 assert GRID_PROBLEM_DTYPE.itemsize == ctypes.sizeof(GridProblem)
@@ -167,6 +175,10 @@ def load():
             f.restype = ctypes.c_int
             f.argtypes = [_vp, ctypes.c_char_p, _vp, ctypes.c_int32, _vp, ctypes.c_int32,
                           ctypes.POINTER(TractParams), ctypes.POINTER(_vp)]
+        for f in (lib.tredsw_ref_tracts_ex, lib.tredsw_ref_tracts_emulate_ex):
+            f.restype = ctypes.c_int
+            f.argtypes = [_vp, ctypes.c_char_p, _vp, ctypes.c_int32, _vp, ctypes.c_int32,
+                          ctypes.POINTER(TractParams), ctypes.POINTER(TractChain), ctypes.POINTER(_vp)]
         lib.tredsw_ref_tracts_view.restype = ctypes.c_int
         lib.tredsw_ref_tracts_view.argtypes = [_vp, ctypes.POINTER(TractsView)]
         lib.tredsw_ref_tracts_free.restype = None
@@ -184,38 +196,46 @@ def check(rc, what):
         raise TredswError("{} failed (code {}): {}".format(what, rc, last_error()))
 
 
-def ref_tracts(path, contigs, motifs, min_units, min_len, step_bytes=0, ctx=None, emulate=False):
+def ref_tracts(path, contigs, motifs, min_units, min_len, step_bytes=0, ctx=None, emulate=False, max_interrupt=0,
+               purity_num=9, purity_den=10):
     """Every tract of `motifs` in the FASTA at `path`, plain text or BGZF (tredsw_ref_tracts, DESIGN §4.5).  contigs:
     FAI_ENTRY_DTYPE rows in FASTA order; motifs: (period, canonical code) pairs.  -> (TRACT_DTYPE array by (contig,
-    start, period), stats dict; its comp_bytes and blocks are 0 for a text file).  ``ctx``: a Context (default the process's); ``emulate`` runs the serial host emulation of the device code
-    instead — test infrastructure only.  Raises TredswError (no device, I/O, an index that does not fit the file)."""
+    start, period), stats dict; its comp_bytes and blocks are 0 for a text file, and its segments the int32 array of
+    each tract's chain segments).  ``max_interrupt`` >= 1 joins pure tracts across interruptions of up to that many
+    bases when the chain has purity purity_num / purity_den (tredsw_ref_tracts_ex, DESIGN §4.5.1); 0 is the pure rule.
+    ``ctx``: a Context (default the process's); ``emulate`` runs the serial host emulation of the device code
+    instead — test infrastructure only.  Raises TredswError (no device, I/O, an index that does not fit the file,
+    chain parameters out of range)."""
     lib = load()
     cs = np.ascontiguousarray(contigs, dtype=FAI_ENTRY_DTYPE)
     ms = np.zeros(len(motifs), dtype=MOTIF_DTYPE)
     for i, (k, code) in enumerate(motifs):
         ms[i]["period"], ms[i]["code"] = k, code
     prm = TractParams(int(min_units), int(min_len), int(step_bytes))
+    chain = TractChain(int(max_interrupt), int(purity_num), int(purity_den), 0)
     res = ctypes.c_void_p()
     if emulate:
-        rc = lib.tredsw_ref_tracts_emulate(None, path.encode(), ptr(cs), len(cs), ptr(ms), len(ms), ctypes.byref(prm),
-                                           ctypes.byref(res))
+        rc = lib.tredsw_ref_tracts_emulate_ex(None, path.encode(), ptr(cs), len(cs), ptr(ms), len(ms),
+                                              ctypes.byref(prm), ctypes.byref(chain), ctypes.byref(res))
     else:
         handle = (ctx or default_context()).handle
-        rc = lib.tredsw_ref_tracts(handle, path.encode(), ptr(cs), len(cs), ptr(ms), len(ms), ctypes.byref(prm),
-                                   ctypes.byref(res))
+        rc = lib.tredsw_ref_tracts_ex(handle, path.encode(), ptr(cs), len(cs), ptr(ms), len(ms), ctypes.byref(prm),
+                                      ctypes.byref(chain), ctypes.byref(res))
     check(rc, "tredsw_ref_tracts")
     try:
         v = TractsView()
         check(lib.tredsw_ref_tracts_view(res, ctypes.byref(v)), "tredsw_ref_tracts_view")
         n = int(v.n_tracts)
         tracts = np.zeros(n, dtype=TRACT_DTYPE)
+        segments = np.zeros(n, dtype=np.int32)
         if n:
             ctypes.memmove(tracts.ctypes.data, v.tracts, n * TRACT_DTYPE.itemsize)
+            ctypes.memmove(segments.ctypes.data, v.segments, n * 4)
         stats = {"steps": int(v.steps), "bytes": int(v.bytes), "bases": int(v.bases),
                  "invalid_bases": int(v.invalid_bases), "tracts": n, "ms_total": float(v.ms_total),
                  "step_read_ms": [float(v.step_read_ms[i]) for i in range(v.steps)],
                  "step_device_ms": [float(v.step_device_ms[i]) for i in range(v.steps)],
-                 "comp_bytes": int(v.comp_bytes), "blocks": int(v.blocks)}
+                 "comp_bytes": int(v.comp_bytes), "blocks": int(v.blocks), "segments": segments}
     finally:
         lib.tredsw_ref_tracts_free(res)
     return tracts, stats

@@ -63,7 +63,7 @@ struct ScanCandidateTag; struct ScanRepairTag; struct ScanCountTag; struct ScanF
 // its STR profile (in-repeat reads)
 struct ScanIrrTag; struct ScanIrrFillTag;
 // the reference tract scan
-struct TractPackTag; struct TractRunsTag;
+struct TractPackTag; struct TractRunsTag; struct TractChainsTag;
 }
 using namespace tredsw_gi;
 
@@ -1699,6 +1699,7 @@ struct tredsw_tracts {
     CudaBackend cuda;
     HostBackend host;
     std::vector<TractOut> tracts;
+    std::vector<int32_t> segments;                  // per tract: its chain's segments (1: a pure tract)
     std::vector<double> read_ms, device_ms;
     tredsw_tracts_view view;
 };
@@ -1839,7 +1840,7 @@ int plan_bgzf_steps(const char *path, const std::vector<TractBlock> &tb, const t
 
 template <class B>
 int run_ref_tracts(B &be, tredsw_tracts *out, const char *path, const tredsw_fai_entry *cs, int32_t nc,
-                   const tredsw_motif *ms, int32_t nm, const tredsw_tract_params &prm) {
+                   const tredsw_motif *ms, int32_t nm, const tredsw_tract_params &prm, const TractChain &ch) {
     const double t_begin = now_ms();
     // the requested codes by period, ascending
     std::vector<std::pair<int32_t, uint64_t>> mv;
@@ -1900,8 +1901,11 @@ int run_ref_tracts(B &be, tredsw_tracts *out, const char *path, const tredsw_fai
         Reused<TractContig> cs;
         Reused<BlockDesc> blocks;
         Reused<TractOut> out;
+        Reused<int32_t> segs;                           // with chains: per tract, its segments
     } buf;
+    const bool chained = ch.max_interrupt > 0;
     buf.out.get(be, 65536);
+    if (chained) buf.segs.get(be, 65536);
     int64_t invalid = 0, bytes = 0, comp_bytes = 0, nblocks = 0;
     auto read_step = [&](TractStep *st) { if (bgzf) read_bgzf_step(fd, tb.data(), st); else read_tract_step(fd, cs, st); };
     ReadAhead reader;
@@ -1960,11 +1964,20 @@ int run_ref_tracts(B &be, tredsw_tracts *out, const char *path, const tredsw_fai
         for (int pass = 0; pass < 2; ++pass) {
             const unsigned long long cap = (unsigned long long)buf.out.cap;
             TractOut *tout = buf.out.p;
-            be.template for_each<TractRunsTag>(words * nper, [=] __host__ __device__(int64_t i) {
-                const int64_t w = i / q.nper;
-                const TractContig &c = dcs[tract_contig_of(dcs, ncs, w)];
-                tract_runs(code, valid, c, w - c.word0, (int)(i - w * q.nper), q, tout, cnt, cap);
-            });
+            if (chained) {                              // interrupted tracts: replaces the pure runs
+                int32_t *tsegs = buf.segs.p;
+                be.template for_each<TractChainsTag>(words * nper, [=] __host__ __device__(int64_t i) {
+                    const int64_t w = i / q.nper;
+                    const TractContig &c = dcs[tract_contig_of(dcs, ncs, w)];
+                    tract_chains(code, valid, c, w - c.word0, (int)(i - w * q.nper), q, ch, tout, tsegs, cnt, cap);
+                });
+            } else {
+                be.template for_each<TractRunsTag>(words * nper, [=] __host__ __device__(int64_t i) {
+                    const int64_t w = i / q.nper;
+                    const TractContig &c = dcs[tract_contig_of(dcs, ncs, w)];
+                    tract_runs(code, valid, c, w - c.word0, (int)(i - w * q.nper), q, tout, cnt, cap);
+                });
+            }
             be.download(h_small, d_small, sizeof(h_small));
             if (pass == 0) be.download(h_bstatus.data(), bstatus, (size_t)nb);
             be.sync();
@@ -1980,12 +1993,15 @@ int run_ref_tracts(B &be, tredsw_tracts *out, const char *path, const tredsw_fai
             if (pass) { tredsw_set_error("tract count changed between passes"); return TREDSW_ERR_CUDA; }
             buf.out.cap = (int64_t)(h_small[0] + h_small[0] / 4 + 1024);      // room for all, not geometric
             buf.out.p = alloc_n<TractOut>(be, buf.out.cap);
+            if (chained) { buf.segs.cap = buf.out.cap; buf.segs.p = alloc_n<int32_t>(be, buf.segs.cap); }
             be.fill(cnt, 0, sizeof(unsigned long long));
             if (be.rc) return be.rc;
         }
         const size_t t0 = out->tracts.size();
         out->tracts.resize(t0 + (size_t)h_small[0]);
         be.download(out->tracts.data() + t0, buf.out.p, sizeof(TractOut) * (size_t)h_small[0]);
+        out->segments.resize(t0 + (size_t)h_small[0], 1);
+        if (chained) be.download(out->segments.data() + t0, buf.segs.p, sizeof(int32_t) * (size_t)h_small[0]);
         be.sync();
         if (be.rc) return be.rc;
         invalid += (int64_t)h_small[1];
@@ -1996,9 +2012,21 @@ int run_ref_tracts(B &be, tredsw_tracts *out, const char *path, const tredsw_fai
         out->device_ms.push_back(now_ms() - t_dev);
         reader.join();
     }
-    std::sort(out->tracts.begin(), out->tracts.end(), [](const TractOut &x, const TractOut &y) {
+    auto before = [](const TractOut &x, const TractOut &y) {
         return x.contig != y.contig ? x.contig < y.contig : x.start != y.start ? x.start < y.start : x.period < y.period;
-    });
+    };
+    if (!chained) {
+        std::sort(out->tracts.begin(), out->tracts.end(), before);
+    } else {                                            // the tracts and their segment counts, in one order
+        std::vector<size_t> ord(out->tracts.size());
+        for (size_t i = 0; i < ord.size(); ++i) ord[i] = i;
+        std::sort(ord.begin(), ord.end(), [&](size_t x, size_t y) { return before(out->tracts[x], out->tracts[y]); });
+        std::vector<TractOut> t(ord.size());
+        std::vector<int32_t> sg(ord.size());
+        for (size_t i = 0; i < ord.size(); ++i) { t[i] = out->tracts[ord[i]]; sg[i] = out->segments[ord[i]]; }
+        out->tracts.swap(t);
+        out->segments.swap(sg);
+    }
     be.release_intermediates();
     tredsw_tracts_view &v = out->view;
     memset(&v, 0, sizeof(v));
@@ -2008,6 +2036,7 @@ int run_ref_tracts(B &be, tredsw_tracts *out, const char *path, const tredsw_fai
     v.step_read_ms = out->read_ms.data(); v.step_device_ms = out->device_ms.data();
     v.ms_total = now_ms() - t_begin;
     v.comp_bytes = comp_bytes; v.blocks = nblocks;
+    v.segments = out->segments.data();
     return TREDSW_OK;
 }
 
@@ -2033,9 +2062,48 @@ bool tract_args_ok(const char *path, const tredsw_fai_entry *cs, int32_t nc, con
     return true;
 }
 
+// the chaining parameters of a call: NULL -> off; out of range -> false
+bool tract_chain_ok(const tredsw_tract_chain *c, TractChain *ch) {
+    *ch = TractChain{0, 1, 1};
+    if (!c) return true;
+    if (c->max_interrupt < 0 || c->max_interrupt > 20 || c->purity_num <= 0 || c->purity_num > c->purity_den ||
+        c->purity_den > 1000) {
+        tredsw_set_error("chain parameters out of range (0 <= max_interrupt <= 20, 0 < purity_num <= purity_den <= 1000): "
+                         "%d, %d / %d", c->max_interrupt, c->purity_num, c->purity_den);
+        return false;
+    }
+    *ch = TractChain{c->max_interrupt, c->purity_num, c->purity_den};
+    return true;
+}
+
 }  // namespace
 
 extern "C" {
+
+int tredsw_ref_tracts_ex(tredsw_ctx *ctx, const char *fasta_path, const tredsw_fai_entry *contigs, int32_t ncontigs,
+                         const tredsw_motif *motifs, int32_t nmotifs, const tredsw_tract_params *params,
+                         const tredsw_tract_chain *chain, tredsw_tracts **result) {
+    TractChain ch;
+    if (!ctx) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
+    if (!tract_args_ok(fasta_path, contigs, ncontigs, motifs, nmotifs, params, result) || !tract_chain_ok(chain, &ch))
+        return TREDSW_ERR_ARG;
+    return run_entry(ctx, "tredsw_ref_tracts", result, [&](auto &be, tredsw_tracts *r) {
+        return run_ref_tracts(be, r, fasta_path, contigs, ncontigs, motifs, nmotifs, *params, ch);
+    });
+}
+
+// TEST INFRASTRUCTURE: tredsw_ref_tracts_ex with every kernel body run serially on the host.  Not used by the package.
+int tredsw_ref_tracts_emulate_ex(tredsw_ctx *, const char *fasta_path, const tredsw_fai_entry *contigs,
+                                 int32_t ncontigs, const tredsw_motif *motifs, int32_t nmotifs,
+                                 const tredsw_tract_params *params, const tredsw_tract_chain *chain,
+                                 tredsw_tracts **result) {
+    TractChain ch;
+    if (!tract_args_ok(fasta_path, contigs, ncontigs, motifs, nmotifs, params, result) || !tract_chain_ok(chain, &ch))
+        return TREDSW_ERR_ARG;
+    return run_entry(nullptr, "tredsw_ref_tracts_emulate", result, [&](auto &be, tredsw_tracts *r) {
+        return run_ref_tracts(be, r, fasta_path, contigs, ncontigs, motifs, nmotifs, *params, ch);
+    });
+}
 
 int tredsw_ref_tracts(tredsw_ctx *ctx, const char *fasta_path, const tredsw_fai_entry *contigs, int32_t ncontigs,
                       const tredsw_motif *motifs, int32_t nmotifs, const tredsw_tract_params *params,
@@ -2043,7 +2111,7 @@ int tredsw_ref_tracts(tredsw_ctx *ctx, const char *fasta_path, const tredsw_fai_
     if (!ctx) { tredsw_set_error("bad arguments"); return TREDSW_ERR_ARG; }
     if (!tract_args_ok(fasta_path, contigs, ncontigs, motifs, nmotifs, params, result)) return TREDSW_ERR_ARG;
     return run_entry(ctx, "tredsw_ref_tracts", result, [&](auto &be, tredsw_tracts *r) {
-        return run_ref_tracts(be, r, fasta_path, contigs, ncontigs, motifs, nmotifs, *params);
+        return run_ref_tracts(be, r, fasta_path, contigs, ncontigs, motifs, nmotifs, *params, TractChain{0, 1, 1});
     });
 }
 
@@ -2053,7 +2121,7 @@ int tredsw_ref_tracts_emulate(tredsw_ctx *, const char *fasta_path, const tredsw
                               tredsw_tracts **result) {
     if (!tract_args_ok(fasta_path, contigs, ncontigs, motifs, nmotifs, params, result)) return TREDSW_ERR_ARG;
     return run_entry(nullptr, "tredsw_ref_tracts_emulate", result, [&](auto &be, tredsw_tracts *r) {
-        return run_ref_tracts(be, r, fasta_path, contigs, ncontigs, motifs, nmotifs, *params);
+        return run_ref_tracts(be, r, fasta_path, contigs, ncontigs, motifs, nmotifs, *params, TractChain{0, 1, 1});
     });
 }
 

@@ -101,9 +101,11 @@ TG_HD int ctz32(uint32_t x) {
 #endif
 }
 
-// appends t at a unique index below cap through a warp-aggregated counter; the count keeps going past cap, so the
-// caller sees an overflow and runs again with room for all
-TG_HD void tract_emit(TractOut *out, unsigned long long *count, unsigned long long cap, const TractOut &t) {
+// appends t (and, with segs, its segment count m at the same index) at a unique index below cap through a
+// warp-aggregated counter; the count keeps going past cap, so the caller sees an overflow and runs again with room
+// for all
+TG_HD void tract_emit(TractOut *out, unsigned long long *count, unsigned long long cap, const TractOut &t,
+                      int32_t *segs = nullptr, int32_t m = 1) {
 #if defined(__CUDA_ARCH__)
     namespace cg = cooperative_groups;
     const cg::coalesced_group g = cg::coalesced_threads();
@@ -113,7 +115,10 @@ TG_HD void tract_emit(TractOut *out, unsigned long long *count, unsigned long lo
 #else
     const unsigned long long at = (*count)++;
 #endif
-    if (at < cap) out[at] = t;
+    if (at < cap) {
+        out[at] = t;
+        if (segs) segs[at] = m;
+    }
 }
 
 struct TractQuery {             // what a step looks for
@@ -163,6 +168,148 @@ TG_HD void tract_runs(const uint64_t *code, const uint32_t *valid, const TractCo
         }
         if (lo == q.mfirst[p + 1] || q.mcodes[lo] != canon) continue;
         tract_emit(out, count, cap, TractOut{a, len, canon, c.id, k});
+    }
+}
+
+// ---- interrupted tracts (tredsw_tract_chain; DESIGN §4.5.1) ----------------------------------------------------
+// With ag(j) the agreement bit above, a run is a maximal [a, e) of agreements (its bases [a, e + k)) and a segment a
+// run with e - a >= k.  A segment S = [a, e) links to T = [a', e'), the next segment after it, when both have root
+// period k and one canonical code, a' - (e + k) <= g (a deletion gives 0 or less) and the bases [e + k, a') are all
+// in ACGTacgt.  A chain is a maximal sequence of links S1 -> ... -> Sm; it gives the tract [a1, a1 + c k),
+// c = floor((em + k - a1) / k), of S1's code and m segments when A den >= num C, C = em - a1 and A the agreements in
+// [a1, em); a chain with m >= 2 that fails this falls back to its segments, each judged alone.  Kept tracts pass the
+// pure rule's filters.  g <= 20 bounds every look-back and look-ahead to 2 k + g + 1 <= 61 positions.
+struct TractChain { int32_t max_interrupt, num, den; };
+
+TG_HD int clz64(uint64_t x) {
+#if defined(__CUDA_ARCH__)
+    return __clzll((long long)x);
+#else
+    return __builtin_clzll(x);
+#endif
+}
+
+// bit i: ag(pos + i), i < 64, for a contig of nw words (0 before its first base and past its end)
+TG_HD uint64_t tract_agree64(const uint64_t *code, const uint32_t *valid, int64_t word0, int64_t nw, int64_t pos, int k) {
+    const int64_t w = pos >= 0 ? pos >> 5 : -((31 - pos) >> 5);
+    const int off = (int)(pos - (w << 5));
+    uint32_t x[3];
+    for (int i = 0; i < 3; ++i) x[i] = w + i >= 0 ? tract_agree(code, valid, word0, nw, w + i, k) : 0u;
+    const uint64_t lo = (uint64_t)x[0] | ((uint64_t)x[1] << 32);
+    return off ? (lo >> off) | ((uint64_t)x[2] << (64 - off)) : lo;
+}
+
+// the first j >= a with ag(j) == 0
+TG_HD int64_t tract_run_end(const uint64_t *code, const uint32_t *valid, int64_t word0, int64_t nw, int64_t a, int k) {
+    int64_t v = a >> 5;
+    uint32_t z = ~tract_agree(code, valid, word0, nw, v, k) & (~0u << (a & 31));
+    while (!z) z = ~tract_agree(code, valid, word0, nw, ++v, k);
+    return (v << 5) + ctz32(z);
+}
+
+// whether every base of [x, y), y - x <= 32, of the contig is in ACGTacgt (true when y <= x)
+TG_HD bool tract_valid_span(const uint32_t *valid, int64_t word0, int64_t nw, int64_t x, int64_t y) {
+    if (y <= x) return true;
+    const int64_t w = x >> 5;
+    const int off = (int)(x & 31), n = (int)(y - x);
+    uint64_t v = valid[word0 + w];
+    if (w + 1 < nw) v |= (uint64_t)valid[word0 + w + 1] << 32;
+    const uint64_t m = (1ull << n) - 1ull;
+    return ((v >> off) & m) == m;
+}
+
+// the canonical code of the k bases from a when their primitive root has period k, else ~0
+TG_HD uint64_t tract_code_at(const uint64_t *code, int64_t word0, int64_t nw, int64_t a, int k) {
+    const int64_t w = a >> 5;
+    const int off = (int)(a & 31);
+    uint64_t unit = code[word0 + w] >> (2 * off);
+    if (off && w + 1 < nw) unit |= code[word0 + w + 1] << (64 - 2 * off);
+    unit &= (1ull << (2 * k)) - 1ull;
+    uint64_t canon;
+    return canonical_root(unit, k, &canon) == k ? canon : ~0ull;
+}
+
+// The segment S of the chain ending at e (code canon) links to the next segment T: -> T's start a' and, in *gap_agree,
+// the agreements in [e, a'); -1 when S ends its chain.
+TG_HD int64_t tract_link(const uint64_t *code, const uint32_t *valid, int64_t word0, int64_t nw, int64_t e, int k,
+                         int g, uint64_t canon, int *gap_agree) {
+    const int n = 2 * k + g;                            // positions [e, e + 2k + g): a' <= e + k + g, then k agreements
+    const uint64_t M = tract_agree64(code, valid, word0, nw, e, k) & ((1ull << n) - 1ull);
+    uint64_t F = M;                                     // bit i: ag at [i, i + k)
+    for (int t = 1; t < k; ++t) F &= M >> t;
+    const uint64_t cand = M & ~(M << 1) & F & ((2ull << (k + g)) - 1ull);      // run starts at e + i, i <= k + g
+    if (!cand) return -1;
+    const int i = (uint32_t)cand ? ctz32((uint32_t)cand) : 32 + ctz32((uint32_t)(cand >> 32));
+    const int64_t a2 = e + i;
+    if (!tract_valid_span(valid, word0, nw, e + k, a2) || tract_code_at(code, word0, nw, a2, k) != canon) return -1;
+    *gap_agree = popc64(M & ((1ull << i) - 1ull));
+    return a2;
+}
+
+// whether the segment at a (code canon) is linked to from the segment before it: the nearest earlier segment
+// [aP, eP) with eP >= a - k - g, when there is one
+TG_HD bool tract_linked_back(const uint64_t *code, const uint32_t *valid, int64_t word0, int64_t nw, int64_t a, int k,
+                             int g, uint64_t canon) {
+    const int n = 2 * k + g + 1;                        // positions [a - n, a): eP - 1 >= a - k - g - 1, then k agreements
+    const int64_t lo = a - n;
+    const uint64_t M = tract_agree64(code, valid, word0, nw, lo, k) & ((1ull << n) - 1ull);
+    uint64_t K = M;                                     // bit i: ag at [i - k + 1, i]
+    for (int t = 1; t < k; ++t) K &= M << t;
+    const uint64_t cand = M & ~(M >> 1) & K & (~0ull << k);     // run ends eP = lo + i + 1 >= a - k - g (bit n - 1,
+    if (!cand) return false;                                    // position a - 1, is 0: a starts a run)
+    const int64_t eP = lo + (63 - clz64(cand)) + 1;
+    return tract_valid_span(valid, word0, nw, eP + k, a) && tract_code_at(code, word0, nw, eP - k, k) == canon;
+}
+
+// The tracts of period q.periods[p] of the chains (tract_chains) whose first segment starts in word lw of contig c:
+// each run start that begins a segment of a requested code and is not linked to from the segment before it walks its
+// chain forward, hopping each interruption with tract_link, and emits the chain or, when it fails purity, its segments.
+TG_HD void tract_chains(const uint64_t *code, const uint32_t *valid, const TractContig &c, int64_t lw, int p,
+                        const TractQuery &q, const TractChain &ch, TractOut *out, int32_t *segs,
+                        unsigned long long *count, unsigned long long cap) {
+    const int k = q.periods[p], g = ch.max_interrupt;
+    const int64_t nw = tract_words(c.length);
+    const uint32_t A = tract_agree(code, valid, c.word0, nw, lw, k);
+    if (!A) return;
+    const uint32_t carry = lw > 0 ? tract_agree(code, valid, c.word0, nw, lw - 1, k) >> 31 : 0u;
+    uint32_t starts = A & ~((A << 1) | carry);
+    const uint64_t km = (1ull << k) - 1ull;
+    while (starts) {
+        const int j = ctz32(starts);
+        starts &= starts - 1;
+        const int64_t a = (lw << 5) + j;
+        // a segment (k agreements from a) of a requested code, first of its chain
+        const uint64_t f = j + k <= 32 ? (uint64_t)(A >> j) : tract_agree64(code, valid, c.word0, nw, a, k);
+        if ((f & km) != km) continue;
+        const uint64_t canon = tract_code_at(code, c.word0, nw, a, k);
+        if (canon == ~0ull) continue;
+        int lo = q.mfirst[p], hi = q.mfirst[p + 1];
+        while (lo < hi) {
+            const int mid = (lo + hi) >> 1;
+            if (q.mcodes[mid] < canon) lo = mid + 1; else hi = mid;
+        }
+        if (lo == q.mfirst[p + 1] || q.mcodes[lo] != canon) continue;
+        if (tract_linked_back(code, valid, c.word0, nw, a, k, g, canon)) continue;
+        // the chain: its last segment's end em, its segments m and its agreements
+        int64_t em = tract_run_end(code, valid, c.word0, nw, a, k), agree = em - a;
+        int32_t m = 1;
+        int gap;
+        for (int64_t a2; (a2 = tract_link(code, valid, c.word0, nw, em, k, g, canon, &gap)) >= 0; ++m) {
+            em = tract_run_end(code, valid, c.word0, nw, a2, k);
+            agree += gap + (em - a2);
+        }
+        auto emit = [&](int64_t s, int64_t e, int32_t nseg) {
+            const int64_t copies = (e + k - s) / k;
+            if (copies >= q.min_units && copies * k >= q.min_len)
+                tract_emit(out, count, cap, TractOut{s, copies * k, canon, c.id, k}, segs, nseg);
+        };
+        if (agree * ch.den >= (int64_t)ch.num * (em - a)) { emit(a, em, m); continue; }
+        // failed purity (m >= 2: a single segment agrees throughout): its segments, each alone
+        for (int64_t s = a;;) {
+            const int64_t e = tract_run_end(code, valid, c.word0, nw, s, k);
+            emit(s, e, 1);
+            if ((s = tract_link(code, valid, c.word0, nw, e, k, g, canon, &gap)) < 0) break;
+        }
     }
 }
 

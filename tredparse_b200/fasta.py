@@ -134,7 +134,8 @@ class Fasta:
     def lengths(self):
         return {name: e[0] for name, e in self.index.items()}
 
-    def tracts(self, motifs, min_units=MIN_REF_UNITS, min_len=MIN_TRACT_LEN, step_bytes=0, ctx=None, emulate=False):
+    def tracts(self, motifs, min_units=MIN_REF_UNITS, min_len=MIN_TRACT_LEN, step_bytes=0, ctx=None, emulate=False,
+               max_interrupt=0, purity=(9, 10)):
         """Every tract of the motifs (strings of 2 to 20 bases; a motif stands for all its rotations on both strands)
         in the whole file, from one scan on the GPU (``_lib.ref_tracts``, DESIGN §4.5; a BGZF file is inflated
         there block by block): a maximal stretch of exact
@@ -143,8 +144,11 @@ class Fasta:
         the contig names in FASTA order, tracts: a ``_lib.TRACT_DTYPE`` array by (contig, start, period) with contig
         an index into contigs, start 0-based, length a whole number of units, code the canonical code; stats: steps,
         bytes, bases, invalid_bases, tracts, per-step host read and device ms, and comp_bytes and blocks, the
-        compressed bytes read and blocks inflated, 0 for a text file).  ``ctx``: a ``_lib.Context``;
-        ``emulate``: the serial host emulation of the device code (test infrastructure only)."""
+        compressed bytes read and blocks inflated, 0 for a text file; segments: per tract, the segments of its chain,
+        an int32 array).  ``max_interrupt`` >= 1 (at most 20) also joins tracts of one motif across interruptions of
+        up to that many bases when the joined tract has `purity` (num, den) (DESIGN §4.5.1); 0 is the pure rule.
+        ``ctx``: a ``_lib.Context``; ``emulate``: the serial host emulation of the device code (test infrastructure
+        only)."""
         from . import _lib
         names = list(self.index)
         contigs = np.array([self.index[n] for n in names], dtype=np.int64).reshape(-1, 4)
@@ -152,8 +156,9 @@ class Fasta:
         for f, col in zip(("length", "offset", "line_bases", "line_width"), contigs.T):
             fai[f] = col
         motifs = sorted({(len(m), canonical_code(m)) for m in motifs})
-        tracts, stats = _lib.ref_tracts(self.path, fai, motifs, min_units, min_len, step_bytes, ctx=ctx, emulate=emulate)
-        return {"contigs": names, "tracts": tracts, "stats": stats}
+        tracts, stats = _lib.ref_tracts(self.path, fai, motifs, min_units, min_len, step_bytes, ctx=ctx, emulate=emulate,
+                                        max_interrupt=max_interrupt, purity_num=purity[0], purity_den=purity[1])
+        return {"contigs": names, "tracts": tracts, "stats": stats, "segments": stats["segments"]}
 
     def fetch(self, contig, start, end):
         """the bases [start, end) of `contig` (0-based), uppercase, clipped to the contig; KeyError for a contig the

@@ -354,16 +354,37 @@ def coordinate_sort(recs):
 # ---------------------------------------------------------------------------------------------------------
 # a reference and reads that agree with it: discovered loci (strprofile.locus_for) end to end
 # ---------------------------------------------------------------------------------------------------------
+def interrupted_tract(unit, copies, edits=()):
+    """`copies` back-to-back copies of `unit` with interruptions planted at given copies (0-based): an edit
+    (copy, "sub", base) replaces the copy's first base with `base`, (copy, "ins", bases) inserts `bases` before the
+    copy, (copy, "del", n) deletes the copy's first n bases.  Edits apply from the last copy to the first, so each
+    copy index is that of the uninterrupted tract."""
+    parts = [unit] * copies
+    for i, kind, arg in sorted(edits, key=lambda x: -x[0]):
+        if kind == "sub":
+            parts[i] = arg + parts[i][1:]
+        elif kind == "ins":
+            parts[i] = arg + parts[i]
+        elif kind == "del":
+            parts[i] = parts[i][arg:]
+        else:
+            raise ValueError("unknown edit `{}`".format(kind))
+    return "".join(parts)
+
+
 def planted_reference(lengths, sites, seed=0):
     """Random contigs {name: bases} of `lengths` [(name, length)] with repeat tracts planted: a site (contig, pos,
-    unit, copies) writes `copies` back-to-back copies of `unit` from 0-based `pos` on.  The base before a tract is
-    not the unit's last base and the base after it not its first, so no rotation of the unit runs longer: the tract is
+    unit, copies) writes `copies` back-to-back copies of `unit` from 0-based `pos` on; a site (contig, pos, unit,
+    copies, edits) writes ``interrupted_tract(unit, copies, edits)`` instead.  The base before a tract is not the
+    unit's last base and the base after it not its first, so no rotation of the unit runs longer: the tract is
     exactly the planted one."""
     rng = np.random.default_rng(seed)
     seqs = {n: rng.choice(list("ACGT"), L) for n, L in lengths}
-    for contig, pos, unit, copies in sites:
-        s, end = seqs[contig], pos + len(unit) * copies
-        s[pos:end] = list(unit * copies)
+    for site in sites:
+        contig, pos, unit, copies = site[:4]
+        text = interrupted_tract(unit, copies, site[4]) if len(site) > 4 else unit * copies
+        s, end = seqs[contig], pos + len(text)
+        s[pos:end] = list(text)
         if pos > 0 and s[pos - 1] == unit[-1]:
             s[pos - 1] = "ACGT"[("ACGT".index(unit[-1]) + 1) % 4]
         if end < len(s) and s[end] == unit[0]:

@@ -11,6 +11,7 @@ with more anchored IRRs in a region than the rest of the cohort — expansions o
     python -m tredparse_b200.tred samples.csv --workdir w --str-profile     # or: catalogue calls and profiles, one read
     python -m tredparse_b200.strprofile outliers w/*.str_profile.json --tsv out.tsv
     python -m tredparse_b200.strprofile loci out.tsv --fasta ref.fa[.gz] --profiles w/*.str_profile.json [--alts]
+        [--max-interruption N]
     python -m tredparse_b200.tred samples.csv --tred <name> ...          # from the directory that holds sites/
 
 Definitions (include/tredsw.h, tredsw_irr_params):
@@ -203,7 +204,45 @@ class Skip(ValueError):
     """an outlier row that gives no locus; str() is the reason"""
 
 
-def locus_for(row, fasta, read_length, window=LOCUS_WINDOW, min_ref_units=MIN_REF_UNITS, ref=None):
+def chain_tracts(seq, units, min_units, max_interrupt, purity):
+    """The kept tracts of the interrupted-tract rule (DESIGN §4.5.1, as ``Fasta.tracts(..., max_interrupt)`` computes
+    them on the GPU) in the text `seq` for one motif: `units` are the rotations of the motif and of its reverse
+    complement, all of one period k with root period k.  -> [(start, copies)] in seq coordinates, at least
+    `min_units` copies each."""
+    k = len(next(iter(units)))
+    num, den = purity
+    n = len(seq)
+    ag = [j + k < n and seq[j] in "ACGT" and seq[j] == seq[j + k] for j in range(n)]
+    chains, j = [], 0                                   # chains of segments [(a, e)]; None: a segment of another code
+    while j < n:
+        if not ag[j]:
+            j += 1
+            continue
+        a = j
+        while j < n and ag[j]:
+            j += 1
+        if j - a < k:
+            continue
+        last = chains[-1] if chains else None
+        if seq[a:a + k] not in units:
+            chains.append(None)
+        elif (last is not None and a - (last[-1][1] + k) <= max_interrupt
+              and all(b in "ACGT" for b in seq[last[-1][1] + k:a])):
+            last.append((a, j))
+        else:
+            chains.append([(a, j)])
+    out = []
+    for ch in chains:
+        if ch is None:
+            continue
+        a1, em = ch[0][0], ch[-1][1]
+        parts = [(a1, em)] if sum(ag[a1:em]) * den >= num * (em - a1) else ch
+        out += [(a, (e + k - a) // k) for a, e in parts if (e + k - a) // k >= min_units]
+    return out
+
+
+def locus_for(row, fasta, read_length, window=LOCUS_WINDOW, min_ref_units=MIN_REF_UNITS, ref=None, max_interrupt=0,
+              purity=(9, 10)):
     """The locus behind a region row of ``outliers`` -> (name, locus row for ``meta.TRED``); raises Skip(reason).
 
     Candidate units are the k rotations of the row's canonical motif (period k) and the k rotations of its reverse
@@ -213,6 +252,11 @@ def locus_for(row, fasta, read_length, window=LOCUS_WINDOW, min_ref_units=MIN_RE
     run.  Reasons to skip: ``no position`` (a motif-only row), ``contig not in FASTA``, ``no reference tract`` (fewer
     than `min_ref_units` copies), ``flank outside contig``, ``N in flank`` (any base but A, C, G, T in the 18 bases
     either side).
+
+    With ``max_interrupt`` >= 1 the tract is instead the longest tract (in copies) of the row's motif that the
+    interrupted-tract rule keeps in the window's text (``chain_tracts``: pure runs joined across interruptions of up
+    to max_interrupt bases at `purity` (num, den), DESIGN §4.5.1), with the same ties; a motif whose root period is
+    shorter than k has none.  Its prefix and suffix then lie outside the whole interrupted tract.
 
     The row: ``repeat`` = the unit as it reads on the reference at the tract's first base; the location
     ``contig:first-last`` (1-based, inclusive, the contig named as in the BAM header) under the field of `ref`
@@ -232,20 +276,25 @@ def locus_for(row, fasta, read_length, window=LOCUS_WINDOW, min_ref_units=MIN_RE
     seq = fasta.fetch(contig, lo, hi)
     rc = motif.translate(_RC)[::-1]
     units = {m[i:] + m[:i] for m in (motif, rc) for i in range(k)}
-    # copies[i]: back-to-back copies of the candidate unit seq[i:i+k] from i on (right to left: one pass)
-    copies = [0] * (len(seq) + k)
-    for i in range(len(seq) - k, -1, -1):
-        u = seq[i:i + k]
-        if u in units:
-            copies[i] = 1 + (copies[i + k] if seq[i + k:i + 2 * k] == u else 0)
     centre2 = row["start"] + row["end"] - 2 * lo         # twice the region's centre, in window coordinates
-    best = None
-    for i in range(len(seq) - k + 1):
-        c = copies[i]
-        if c and not (i >= k and seq[i - k:i] == seq[i:i + k]):          # the first copy of a run
-            key = (-c, abs(2 * i + c * k - centre2), i)
-            if best is None or key < best:
-                best = key
+    if max_interrupt:
+        primitive = all(motif != motif[d:] + motif[:d] for d in range(1, k))
+        found = chain_tracts(seq, units, min_ref_units, max_interrupt, purity) if primitive else []
+        best = min(((-c, abs(2 * i + c * k - centre2), i) for i, c in found), default=None)
+    else:
+        # copies[i]: back-to-back copies of the candidate unit seq[i:i+k] from i on (right to left: one pass)
+        copies = [0] * (len(seq) + k)
+        for i in range(len(seq) - k, -1, -1):
+            u = seq[i:i + k]
+            if u in units:
+                copies[i] = 1 + (copies[i + k] if seq[i + k:i + 2 * k] == u else 0)
+        best = None
+        for i in range(len(seq) - k + 1):
+            c = copies[i]
+            if c and not (i >= k and seq[i - k:i] == seq[i:i + k]):          # the first copy of a run
+                key = (-c, abs(2 * i + c * k - centre2), i)
+                if best is None or key < best:
+                    best = key
     if best is None or -best[0] < min_ref_units:
         raise Skip("no reference tract")
     first, n = lo + best[2], -best[0]
@@ -264,16 +313,17 @@ def locus_for(row, fasta, read_length, window=LOCUS_WINDOW, min_ref_units=MIN_RE
                   "cutoff_prerisk": cut, "cutoff_risk": cut}
 
 
-def discover_loci(rows, fasta, read_length, min_z=3.0, window=LOCUS_WINDOW, min_ref_units=MIN_REF_UNITS, ref=None):
+def discover_loci(rows, fasta, read_length, min_z=3.0, window=LOCUS_WINDOW, min_ref_units=MIN_REF_UNITS, ref=None,
+                  max_interrupt=0, purity=(9, 10)):
     """The loci of the outlier rows with z >= min_z, in row order -> ({name: locus row}, [(row, reason)] of the rows
     skipped).  Rows that resolve to one (contig, first base, repeat) — the left and right anchors of a long expansion
-    can make two regions — give one locus, the first row's."""
+    can make two regions — give one locus, the first row's.  ``max_interrupt`` and ``purity``: ``locus_for``."""
     sites, skipped = {}, []
     for row in rows:
         if row["z"] < min_z:
             continue
         try:
-            name, locus = locus_for(row, fasta, read_length, window, min_ref_units, ref)
+            name, locus = locus_for(row, fasta, read_length, window, min_ref_units, ref, max_interrupt, purity)
         except Skip as e:
             skipped.append((row, str(e)))
             continue
@@ -355,22 +405,38 @@ def main(argv=None):
     pl.add_argument("--max-alts", type=int, default=MAX_ALTS, help="alt regions kept per locus (longest tracts first)")
     pl.add_argument("--min-alt-len", type=int, default=MIN_TRACT_LEN,
                     help="bases an alt tract needs (default: BWA-MEM's minimum alignment score)")
+    pl.add_argument("--max-interruption", type=int, default=0,
+                    help="join tracts of one motif across interruptions of up to this many bases (0 to 20; 0: pure "
+                         "tracts only), for the locus tract and --alts, when the joined tract is as pure as an "
+                         "in-repeat read: the purity is the profiles' (DESIGN §4.5.1)")
     a = ap.parse_args(argv)
     if a.cmd == "loci":
         from .fasta import Fasta
         with open(a.tsv) as fp:
             rows = read_tsv(fp)
-        read_length = 0
+        read_length, purities = 0, set()
         for f in a.profiles:
             with open(f) as fp:
-                read_length = max(read_length, int(json.load(fp)["read_length"]))
+                prof = json.load(fp)
+            read_length = max(read_length, int(prof["read_length"]))
+            prm = prof.get("params", {})
+            purities.add((prm.get("purity_num"), prm.get("purity_den")))
         if read_length <= 0:
             ap.error("the profiles give no read length")
+        if not 0 <= a.max_interruption <= 20:
+            ap.error("--max-interruption must be 0 to 20 (got {})".format(a.max_interruption))
+        purity = (9, 10)
+        if a.max_interruption:                          # the in-repeat reads' purity, one for the cohort
+            if len(purities) != 1 or None in next(iter(purities)):
+                ap.error("--max-interruption needs one purity (params.purity_num / purity_den) in every profile; "
+                         "they give {}".format(sorted(purities, key=str)))
+            purity = next(iter(purities))
         try:
             fasta = Fasta(a.fasta)
         except (IOError, ValueError) as e:
             ap.error(str(e))
-        sites, skipped = discover_loci(rows, fasta, read_length, a.min_z, a.window, a.min_ref_units, a.ref)
+        sites, skipped = discover_loci(rows, fasta, read_length, a.min_z, a.window, a.min_ref_units, a.ref,
+                                       a.max_interruption, purity)
         below = sum(1 for r in rows if r["z"] < a.min_z)
         for r, why in skipped:
             where = r["contig"] if r["start"] is None else "{}:{}-{}".format(r["contig"], r["start"], r["end"])
@@ -379,7 +445,8 @@ def main(argv=None):
         if a.alts and sites:
             from .meta import alts_field
             try:
-                tracts = fasta.tracts({row["motif"] for row in sites.values()}, min_len=a.min_alt_len)
+                tracts = fasta.tracts({row["motif"] for row in sites.values()}, min_len=a.min_alt_len,
+                                      max_interrupt=a.max_interruption, purity=purity)
             except _lib.TredswError as e:
                 ap.exit(1, "loci --alts: {}\n".format(e))
             for name, row in sites.items():
