@@ -220,16 +220,18 @@ def test_json_and_vcf_writers(tmp_path, repo, capsys):
     assert T.counter_s({15: 4, 6: 1}) == "6|1;15|4"
 
 
-def test_run_chunks_keeps_order_prefetches_and_isolates_failures(monkeypatch):
+def test_run_chunks_keeps_order_prefetches_passes_str_profile_and_isolates_failures(monkeypatch):
     """tred.run_chunks: chunk k + 1 is prepared while chunk k is finished, results come back in input order, and with
-    isolate=True a chunk that raises yields error records for its samples instead of ending the run."""
+    isolate=True a chunk that raises yields error records for its samples instead of ending the run; every chunk gets
+    str_profile (one bool, or its slice of the per-sample list)."""
     import threading
     from tredparse_b200 import tred as T
-    log, lock = [], threading.Lock()
+    log, lock, profiles = [], threading.Lock(), {}
 
-    def fake_prepare(args, only=None, ctx=None):
+    def fake_prepare(args, only=None, ctx=None, str_profile=False):
         with lock:
             log.append(("prep", args[0][0]))
+            profiles[args[0][0]] = str_profile
         if args[0][0] == "s4":
             raise RuntimeError("boom")
         return list(args)
@@ -248,5 +250,12 @@ def test_run_chunks_keeps_order_prefetches_and_isolates_failures(monkeypatch):
     assert all("error" not in got[i] for i in (0, 1, 2, 3, 6))
     # chunk 1 (s2) is prepared before chunk 0 (s0) is finished: two stages deep
     assert log.index(("prep", "s2")) < log.index(("fin", "s2")) and ("fin", "s4") not in log
+    assert profiles == dict.fromkeys(("s0", "s2", "s4", "s6"), False)
     with pytest.raises(RuntimeError):
         list(T.run_chunks(args, chunk=2))
+    per_sample = [i % 3 == 0 for i in range(7)]
+    for flag, want in ((True, [True] * 4), (per_sample, [[True, False], [False, True], [False, False], [True]])):
+        profiles.clear()
+        got = list(T.run_chunks(args, chunk=2, isolate=True, str_profile=flag))
+        assert [r["samplekey"] for r in got] == [a[0] for a in args]
+        assert [profiles[k] for k in ("s0", "s2", "s4", "s6")] == want

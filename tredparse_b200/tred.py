@@ -32,6 +32,7 @@ import os.path as op
 import shutil
 import sys
 import time
+from collections import namedtuple
 from datetime import datetime as dt, timedelta
 
 import numpy as np
@@ -131,6 +132,10 @@ def counter_s(c):
     return ";".join("{}|{}".format(k, int(v)) for k, v in sorted(c.items()))
 
 
+# one sample's run arguments (``run``, ``run_chunk``, ``run_chunks`` take them as plain tuples in this order)
+Task = namedtuple("Task", "samplekey bam repo tredNames maxinsert fullsearch clip alts repeatpairs log")
+
+
 def runBam(inputParams):
     """Parse one BAM at one locus and run the caller on it.  :return: BamParserResults"""
     maxinsert = inputParams.kwargs["maxinsert"]
@@ -148,11 +153,6 @@ def alt_regions(tred, ref, alts, clip):
     if not alts or clip:
         return []
     return [(c[3:] if "nochr" in ref and c.startswith("chr") else c, s, e) for (c, s, e) in tred.alt]
-
-
-def locus_evidence(ing, tred, readlen, alts, clip, ref):
-    """One native pass over the BAM for one locus (reads + names + pair distances + depth)."""
-    return ing.extract_locus(tred, readlen, alts=alt_regions(tred, ref, alts, clip), want_names=True)
 
 
 TAGNAME = {1: "FULL", 2: "PREF", 3: "POST", 4: "REPT"}
@@ -232,7 +232,7 @@ def genotype_evidence(items, maxinsert=300, fullsearch=False, clip=False, repeat
 INGEST_THREADS = int(os.environ.get("TREDSW_INGEST_THREADS", "0")) or min(8, os.cpu_count() or 1)
 
 
-def ingest_loci(bam, repo, tredNames, READLEN, alts, clip, logger, threads=None, want_names=True):
+def ingest_loci(bam, repo, tredNames, READLEN, alts, clip, logger, threads=None):
     """Evidence of every requested locus of one BAM.
     Native ingest (csrc/ingest.cpp): one indexed pass per locus yields reads, pair distances AND depth; the loci
     are dealt to `threads` host threads, each with its own clone of the BAM handle (own file descriptor, shared
@@ -251,8 +251,9 @@ def ingest_loci(bam, repo, tredNames, READLEN, alts, clip, logger, threads=None,
     def one(handle, tred):
         xtred = repo[tred]
         try:
-            if handle is not None and handle.tid(xtred.chr) >= 0:
-                return tred, locus_evidence(handle, xtred, READLEN, alts, clip, repo.ref)
+            if handle is not None and handle.tid(xtred.chr) >= 0:      # one native pass: reads, names, pairs, depth
+                return tred, handle.extract_locus(xtred, READLEN, alts=alt_regions(xtred, repo.ref, alts, clip),
+                                                  want_names=True)
             return tred, extract_locus(bam, repo, tred, READLEN, alts, clip, logger)
         except Exception as e:
             logger.error("Exception on `{}` {} ({})".format(bam, tred, e))
@@ -287,31 +288,40 @@ GPU_INGEST = os.environ.get("TREDSW_GPU_INGEST", "1") != "0"
 DEVICE_HANDOFF = os.environ.get("TREDSW_DEVICE_HANDOFF", "1") != "0"     # genotype from the ingest's device buffers
 
 
+def locus_queries(s):
+    """(queries, keep-alive arrays, tredNames) of the wanted loci of a routed ``Sample`` on its handle
+    (``ingest.locus_query`` with the task's alt regions); a locus whose contig the header lacks is left out"""
+    from .ingest import locus_query
+    repo, qs, keep, names = s.task.repo, [], [], []
+    for t in s.wanted:
+        xtred = repo[t]
+        q = locus_query(s.handle, xtred, s.pre["readLen"], alts=alt_regions(xtred, repo.ref, s.task.alts, s.task.clip))
+        if q is not None:
+            qs.append(q[0]); keep.append(q[1]); names.append(t)
+    return qs, keep, names
+
+
 def ingest_chunk_gpu(samples, ctx=None, keep_batch=None):
     """Evidence of every (sample, locus) of a chunk through the GPU ingest (csrc/bgzf_gpu.cu): the host reads the
     compressed BGZF blocks behind the windows, the device inflates them, walks the records and applies the
     selection / pairing / depth rules — same evidence as ``ingest_loci`` locus by locus.
-    :param samples: [(key, run-argument tuple, wanted TRED names, READLEN, open ingest.BamIngest)]
+    :param samples: [(key, ``Sample`` on the "indexed" route)]
     :param keep_batch: a list; when every problem of the batch is good, (IngestBatch, [(key, tredName)]) is appended
                        and the batch stays open (the evidence objects are views into it): the caller genotypes from
                        its device buffers and closes it
     :return: {key: {tredName: LocusEvidence}} — loci the device path could not serve (contig missing, a block the
              decoder refused, corrupt records) are left out: the caller reads them with the host reader."""
     from . import _lib
-    from .ingest import IngestBatch, locus_query
+    from .ingest import IngestBatch
     handles, qs, so, keep, key = [], [], [], [], []
     try:
-        for k, arg, wanted, READLEN, h in samples:
-            samplekey, bam, repo, tredNames, maxinsert, fullsearch, clip, alts, repeatpairs, log = arg
-            if h is None:
-                continue
-            handles.append(h)
-            for t in wanted:
-                xtred = repo[t]
-                q = locus_query(h, xtred, READLEN, alts=alt_regions(xtred, repo.ref, alts, clip))
-                if q is None:
-                    continue
-                qs.append(q[0]); keep.append(q[1]); so.append(len(handles) - 1); key.append((k, t))
+        for k, s in samples:
+            handles.append(s.handle)
+            sq, sk, names = locus_queries(s)
+            qs += sq
+            keep += sk
+            so += [len(handles) - 1] * len(sq)
+            key += [(k, t) for t in names]
         got = {}
         if not qs:
             return got
@@ -337,86 +347,70 @@ def ingest_chunk_gpu(samples, ctx=None, keep_batch=None):
         return {}
 
 
-def ingest_sample_scan(arg, wanted, READLEN, h, with_gender, ctx=None, stream=False, str_profile=False):
-    """Evidence of every wanted locus of one sample whose BAM has no usable index (or whose STR profile is wanted),
-    and its chrY depth when ``with_gender``, in ONE streaming pass over the file on the GPU (``ingest.scan_sample``).
-    :param h: the sample's handle from ``ingest.BamIngest.unindexed`` or ``ingest.BamIngest.stream``
-    :param stream: `h` is a stream, which can be read only once: a scan that fails raises (no partial evidence, no
-                   second reader), and a header without the chrY regions gives gender ('Unknown', -1)
-    :param str_profile: the same pass also finds the in-repeat reads of the whole file (``IrrParams()``, the defaults
-                        of ``strprofile profile``) and the sample's STR profile is built from them
-                        (``strprofile.build_profile``; its sample is the sample key, its bam the path of the run)
-    :return: ({tredName: LocusEvidence}, (gender, depthY) or None, STR profile or None) — loci the scan could not
-             serve (contig missing, a corrupt or unsorted file) are left out, and so are the gender and the profile:
-             the caller reads the loci with the Python reader (not a stream's: a locus whose contig the header lacks
-             gets no call).  A file whose scan fails gets no profile, and the failure is logged as an error."""
+def ingest_sample_scan(s, ctx=None):
+    """Evidence of every wanted locus of a ``Sample`` on the "scan" or "stream" route, and its gender, in ONE streaming
+    pass over the file on the GPU (``ingest.scan_sample``).  The gender (from the chrY regions' depth, when an X-linked
+    locus is among the task's loci) goes into ``s.pre``; a file whose scan gives none (a failed scan, a header without
+    the chrY regions) gets it from ``infer_gender``.  A stream can be read only once: a scan that fails raises (no
+    partial evidence, no second reader), and a header without the chrY regions gives gender ('Unknown', -1).
+    With ``s.profile`` the same pass also finds the in-repeat reads of the whole file (``IrrParams()``, the defaults of
+    ``strprofile profile``) and the sample's STR profile is built from them (``strprofile.build_profile``; its sample
+    is the sample key, its bam the path of the run).
+    :return: ({tredName: LocusEvidence}, STR profile or None) — loci the scan could not serve (contig missing, a
+             corrupt or unsorted file) are left out, and so is the profile: the caller reads the loci with the Python
+             reader (not a stream's: a locus whose contig the header lacks gets no call).  A file whose scan fails
+             gets no profile, and the failure is logged as an error."""
     from . import _lib
-    from .ingest import IrrParams, locus_query, scan_sample
-    samplekey, bam, repo, tredNames, maxinsert, fullsearch, clip, alts, repeatpairs, log = arg
-    irr = IrrParams() if str_profile else None
-    qs, keep, names = [], [], []
-    for t in wanted:
-        xtred = repo[t]
-        q = locus_query(h, xtred, READLEN, alts=alt_regions(xtred, repo.ref, alts, clip))
-        if q is None:
-            continue
-        qs.append(q[0]); keep.append(q[1]); names.append(t)
+    from .ingest import IrrParams, scan_sample
+    task, h, stream = s.task, s.handle, s.route == "stream"
+    bam, key = task.bam, task.samplekey
+    irr = IrrParams() if s.profile else None
+    qs, keep, names = locus_queries(s)
+    with_gender = any(task.repo[t].is_xlinked for t in task.tredNames)
     yreg = []
     if with_gender:
-        rows = BamDepth.y_regions(repo.ref)
-        tids = [h.tid(c) for c, s, e in rows]
+        rows = BamDepth.y_regions(task.repo.ref)
+        tids = [h.tid(row[0]) for row in rows]
         if rows and min(tids) >= 0:
-            yreg = [(t, s, e) for t, (c, s, e) in zip(tids, rows)]
+            yreg = [(t, a, b) for t, (c, a, b) in zip(tids, rows)]
     got, gender, prof = {}, (("Unknown", -1) if stream and with_gender and not yreg else None), None
-    if not qs and not yreg and irr is None:
-        return got, gender, prof
-    try:
-        with scan_sample(ctx or _lib.default_context(), h, qs, keep, yreg, irr=irr) as b:
-            if stream and b.scan_status:
-                raise IOError("the GPU scan of `{}` failed (status {}): {}".format(bam, b.scan_status, _lib.last_error()))
-            for i, t in enumerate(names):
-                if b.status[i]:
-                    logger.debug("GPU scan handed {} / {} back (status {})".format(samplekey, t, int(b.status[i])))
-                    continue
-                got[t] = b.evidence(i)
-            if yreg and not b.scan_status:
-                ydepth = float(np.median(b.depths))
-                gender = ("Male" if ydepth > 1 else "Female", ydepth)
+    if qs or yreg or irr is not None:
+        try:
+            with scan_sample(ctx or _lib.default_context(), h, qs, keep, yreg, irr=irr) as b:
+                if stream and b.scan_status:
+                    raise IOError("the GPU scan of `{}` failed (status {}): {}".format(bam, b.scan_status,
+                                                                                      _lib.last_error()))
+                for i, t in enumerate(names):
+                    if b.status[i]:
+                        logger.debug("GPU scan handed {} / {} back (status {})".format(key, t, int(b.status[i])))
+                        continue
+                    got[t] = b.evidence(i)
+                if yreg and not b.scan_status:
+                    ydepth = float(np.median(b.depths))
+                    gender = ("Male" if ydepth > 1 else "Female", ydepth)
+                if irr is not None:
+                    if b.scan_status:
+                        logger.error("Sample `{}`: the GPU scan of `{}` failed (status {}): no STR profile".format(
+                            key, bam, b.scan_status))
+                    else:
+                        from .strprofile import build_profile
+                        prof = build_profile(b.irr, h.references(), irr, sample=key, bam=bam)
+        except Exception as e:
+            if stream:
+                raise
+            logger.error("GPU scan of `{}` failed ({}); reading with the Python reader".format(bam, e))
             if irr is not None:
-                if b.scan_status:
-                    logger.error("Sample `{}`: the GPU scan of `{}` failed (status {}): no STR profile".format(
-                        samplekey, bam, b.scan_status))
-                else:
-                    from .strprofile import build_profile
-                    prof = build_profile(b.irr, h.references(), irr, sample=samplekey, bam=bam)
-    except Exception as e:
-        if stream:
-            raise
-        logger.error("GPU scan of `{}` failed ({}); reading with the Python reader".format(bam, e))
-        if irr is not None:
-            logger.error("Sample `{}`: no STR profile (the GPU scan of `{}` raised: {})".format(samplekey, bam, e))
-        return {}, None, None
-    return got, gender, prof
+                logger.error("Sample `{}`: no STR profile (the GPU scan of `{}` raised: {})".format(key, bam, e))
+            got, gender, prof = {}, None, None
+    if gender is None and with_gender:          # (never a stream's: it has a gender or has raised)
+        gender = infer_gender(bam, task.repo, task.tredNames, logger)
+    if gender is not None:
+        logger.debug("Inferred gender: {} (depthY={})".format(*gender))
+        s.pre.update({"inferredGender": gender[0], "depthY": gender[1]})
+    return got, prof
 
 
 OPEN_STREAMS = {}       # stream path -> ingest.BamIngest whose header was read early (the sample key of `-`)
-
-
-def stream_presteps(bam):
-    """(handle, pre-steps) of a stream sample: its handle (``ingest.BamIngest.stream``) and the read length from the
-    records the handle reads ahead; gender comes later, from the chrY regions of the sample's one scan."""
-    from .ingest import BamIngest
-    from . import _lib
-    if not GPU_INGEST:
-        raise IOError("`{}` is a stream: only the GPU scan reads it (TREDSW_GPU_INGEST=0)".format(bam))
-    h = OPEN_STREAMS.pop(bam, None) or BamIngest.stream(bam)
-    READLEN = 150
-    try:
-        READLEN = h.read_length()[0]
-    except _lib.TredswError:
-        pass                    # no records (the scan finds none either) or a damaged stream (the scan reports it)
-    logger.debug("Read length: {}bp".format(READLEN))
-    return h, {"inferredGender": "Unknown", "depthY": -1, "readLen": READLEN}
 
 
 def infer_gender(bam, repo, tredNames, logger, ing=None):
@@ -447,6 +441,70 @@ def presteps(bam, repo, tredNames, logger, ing=None, with_gender=True):
     return {"inferredGender": gender, "depthY": ydepth, "readLen": READLEN}
 
 
+# How one sample of a chunk is read: decided once, by ``open_sample``, and followed by the rest of ``prepare_chunk``.
+#   route    "indexed": an indexed BAM, its loci from the chunk's one GPU ingest batch (``ingest_loci`` when the GPU
+#            ingest is off); "scan": one GPU scan of the whole file (a BAM without a usable index, or an indexed one
+#            whose STR profile is wanted); "stream": one GPU scan of a stream, which nothing else may read; "host":
+#            ``ingest_loci`` alone; None: the sample is not read (an error record when `error` is set)
+#   handle   the route's open ``ingest.BamIngest``, closed once the evidence is read; or None
+#   pre      the pre-step fields of tredCalls: inferredGender, depthY, readLen (a scan sets the gender later)
+#   wanted   the loci of the task this run reads
+#   profile  the sample's scan also makes its STR profile
+Sample = namedtuple("Sample", "task route handle pre wanted profile error",
+                    defaults=(None, None, None, (), False, None))
+
+
+def open_sample(task, wanted, profile):
+    """The ``Sample`` of one task: its route, its open handle and its pre-steps.  Gender looks at all of the task's
+    loci, not only the wanted ones, so that every rank of ``--gpus N`` reports the same."""
+    from . import _lib
+    from .ingest import BamIngest, is_stream
+    bam = task.bam
+    if is_stream(bam):
+        # a stream is read only by its one GPU scan, which also gives its gender; one that cannot be scanned makes its
+        # sample an error
+        try:
+            if not GPU_INGEST:
+                raise IOError("`{}` is a stream: only the GPU scan reads it (TREDSW_GPU_INGEST=0)".format(bam))
+            h = OPEN_STREAMS.pop(bam, None) or BamIngest.stream(bam)
+        except Exception as e:
+            return Sample(task, error=e)
+        READLEN = 150
+        try:
+            READLEN = h.read_length()[0]         # (from the records the handle reads ahead)
+        except _lib.TredswError:
+            pass                    # no records (the scan finds none either) or a damaged stream (the scan reports it)
+        logger.debug("Read length: {}bp".format(READLEN))
+        pre = {"inferredGender": "Unknown", "depthY": -1, "readLen": READLEN}
+        return Sample(task, "stream", h, pre, wanted, profile)
+    ing = None
+    try:
+        ing = BamIngest(bam_path(bam))
+    except Exception as e:
+        logger.debug("native BAM ingest unavailable for `{}` ({})".format(bam, e))
+        if check_bam(bam) is None:
+            return Sample(task, pre={"inferredGender": "Unknown", "depthY": -1})
+    # a BAM without a usable index is scanned once on the GPU (unless the GPU ingest is off), and so is an indexed BAM
+    # whose STR profile is wanted: the profile needs a pass over every record, and that pass serves the loci and gender
+    # as well, so the pre-steps here read only the read length
+    if GPU_INGEST and (ing is None or profile):
+        try:
+            uh = BamIngest.unindexed(bam_path(bam))
+        except Exception as e:
+            if ing is None:
+                logger.debug("GPU scan unavailable for `{}` ({})".format(bam, e))
+            else:
+                logger.error("Sample `{}`: GPU scan unavailable for `{}` ({}): no STR profile".format(
+                    task.samplekey, bam, e))
+        else:
+            if ing is not None:
+                ing.close()
+            pre = presteps(bam, task.repo, task.tredNames, logger, ing=uh, with_gender=False)
+            return Sample(task, "scan", uh, pre, wanted, profile)
+    pre = presteps(bam, task.repo, task.tredNames, logger, ing=ing)
+    return Sample(task, "host" if ing is None else "indexed", ing, pre, wanted)
+
+
 def run(arg):
     """Run the TRED caller on a list of TREDs for one sample.  :return: dict of calls"""
     return run_chunk([arg])[0]
@@ -455,133 +513,67 @@ def run(arg):
 STR_PROFILE = "_str_profile"       # key of a result's STR profile (not part of the JSON: ``main`` writes it apart)
 
 
-def _per_sample(flag, n):
-    """a ``str_profile`` argument (one bool for all the samples, or one per sample) as a list of n bools"""
-    return [bool(flag)] * n if isinstance(flag, bool) else [bool(x) for x in flag]
-
-
 def prepare_chunk(args, only=None, ctx=None, str_profile=False):
-    """First half of ``run_chunk``: per-sample pre-steps and the evidence of every (sample, locus) — the GPU ingest,
-    the host reader for what it hands back.  Touches no state of the genotyping context, so the next chunk can be
-    prepared (on ``ctx``, a context of its own) while the previous one is genotyped.
+    """First half of ``run_chunk``: per-sample pre-steps and the evidence of every (sample, locus), each sample on the
+    route ``open_sample`` gives it.  Touches no state of the genotyping context, so the next chunk can be prepared (on
+    ``ctx``, a context of its own) while the previous one is genotyped.
     :param str_profile: True, or one bool per sample: the sample's STR profile is made by its one GPU scan (an indexed
                         BAM is then scanned instead of read by the indexed ingest) and its result carries it under
                         ``STR_PROFILE``; a sample whose scan fails has none
     :return: an opaque state for ``finish_chunk``"""
-    profile_of = _per_sample(str_profile, len(args))
-    out, items, where, todo = [], [], [], []
-    for si, arg in enumerate(args):
-        samplekey, bam, repo, tredNames, maxinsert, fullsearch, clip, alts, repeatpairs, log = arg
-        tredCalls = {"inferredGender": "Unknown", "depthY": -1}
-        out.append({"samplekey": samplekey, "bam": bam, "tredCalls": tredCalls, "_fields": {}, "_names": list(tredNames)})
-    # per sample: one native handle (validity check, pre-steps, GPU ingest), the pre-steps (gender looks at every
-    # requested locus); the samples are dealt to host threads
-    # a BAM without a usable index is scanned once on the GPU (unless the GPU ingest is off): its gender comes from
-    # that scan, so its pre-steps here read only the read length.  So is a stream, which nothing else may read: a
-    # stream that cannot be scanned makes its sample an error.  So is an indexed BAM whose STR profile is wanted: the
-    # profile needs a pass over every record, and that pass serves the loci and gender as well
-    def pre(si):
-        samplekey, bam, repo, tredNames = args[si][:4]
-        from .ingest import BamIngest, is_stream
-        if is_stream(bam):
-            try:
-                return stream_presteps(bam) + ("stream",)
-            except Exception as e:
-                return e
-        ing = None
-        try:
-            ing = BamIngest(bam_path(bam))
-        except Exception as e:
-            logger.debug("native BAM ingest unavailable for `{}` ({})".format(bam, e))
-            if check_bam(bam) is None:
-                return None
-            if GPU_INGEST:
-                try:
-                    uh = BamIngest.unindexed(bam_path(bam))
-                    return uh, presteps(bam, repo, tredNames, logger, ing=uh, with_gender=False), True
-                except Exception as e2:
-                    logger.debug("GPU scan unavailable for `{}` ({})".format(bam, e2))
-        if ing is not None and profile_of[si] and GPU_INGEST:
-            try:
-                uh = BamIngest.unindexed(bam_path(bam))
-            except Exception as e2:
-                logger.error("Sample `{}`: GPU scan unavailable for `{}` ({}): no STR profile".format(samplekey, bam, e2))
-            else:
-                ing.close()
-                return uh, presteps(bam, repo, tredNames, logger, ing=uh, with_gender=False), True
-        return ing, presteps(bam, repo, tredNames, logger, ing=ing), False
-    if len(args) > 1 and INGEST_THREADS > 1:
-        from concurrent.futures import ThreadPoolExecutor
-        with ThreadPoolExecutor(max_workers=min(INGEST_THREADS, len(args))) as pool:
-            pres = list(pool.map(pre, range(len(args))))
-    else:
-        pres = [pre(si) for si in range(len(args))]
-    wanted_of, handle_of, unindexed, streams, failed = {}, {}, set(), set(), set()
+    tasks = [Task._make(a) for a in args]
+    profile_of = [str_profile] * len(tasks) if isinstance(str_profile, bool) else [bool(x) for x in str_profile]
 
-    def fail(si, e):
-        logger.error("Sample `{}`: {}".format(args[si][0], e))
-        failed.add(si)
-        out[si].update({"tredCalls": {}, "error": repr(e), "_names": []})
-    for si, ps in enumerate(pres):
-        if ps is None:
-            continue
-        if isinstance(ps, Exception):
-            fail(si, ps)
-            continue
-        todo.append(si)
-        handle_of[si] = ps[0]
-        if ps[2]:
-            unindexed.add(si)
-        if ps[2] == "stream":
-            streams.add(si)
-        out[si]["tredCalls"].update(ps[1])
-        tredNames = args[si][3]
-        wanted_of[si] = [t for t in tredNames if only is None or t in only[si]]
-        out[si]["_names"] = wanted_of[si]
-    # evidence: the GPU ingest for every (sample, locus) of the chunk in one pass, one GPU scan per sample without an
-    # index; the host reader for what they hand back (corrupt blocks, unsorted files, unknown contig) or when they are
-    # switched off (TREDSW_GPU_INGEST=0)
-    kept = []
+    def route(si):
+        wanted = [t for t in tasks[si].tredNames if only is None or t in only[si]]
+        return open_sample(tasks[si], wanted, profile_of[si])
+    # the samples' pre-steps are dealt to host threads
+    if len(tasks) > 1 and INGEST_THREADS > 1:
+        from concurrent.futures import ThreadPoolExecutor
+        with ThreadPoolExecutor(max_workers=min(INGEST_THREADS, len(tasks))) as pool:
+            samples = list(pool.map(route, range(len(tasks))))
+    else:
+        samples = [route(si) for si in range(len(tasks))]
+    # evidence: the GPU ingest for every (sample, locus) of the indexed samples in one pass, one GPU scan per sample on
+    # the scan and stream routes; the host reader for what they hand back (corrupt blocks, unsorted files, unknown
+    # contig) or when they are switched off (TREDSW_GPU_INGEST=0)
+    evidence, profiles, kept = {}, {}, []
     try:
-        got = ingest_chunk_gpu([(si, args[si], wanted_of[si], out[si]["tredCalls"]["readLen"],
-                                 None if si in unindexed else handle_of[si]) for si in todo],
-                               ctx=ctx, keep_batch=kept if DEVICE_HANDOFF else None) if GPU_INGEST else {}
-        for si in sorted(unindexed):
-            samplekey, bam, repo, tredNames = args[si][:4]
-            with_gender = any(repo[t].is_xlinked for t in tredNames)
-            try:
-                got[si], gender, prof = ingest_sample_scan(args[si], wanted_of[si], out[si]["tredCalls"]["readLen"],
-                                                           handle_of[si], with_gender, ctx=ctx, stream=si in streams,
-                                                           str_profile=profile_of[si])
-            except Exception as e:
-                if si not in streams:
-                    raise
-                fail(si, e)
-                continue
-            if prof is not None:
-                out[si][STR_PROFILE] = prof
-            if gender is None and with_gender:
-                gender = infer_gender(bam, repo, tredNames, logger)
-            if gender is not None:
-                logger.debug("Inferred gender: {} (depthY={})".format(*gender))
-                out[si]["tredCalls"].update({"inferredGender": gender[0], "depthY": gender[1]})
+        if GPU_INGEST:
+            evidence = ingest_chunk_gpu([(si, s) for si, s in enumerate(samples) if s.route == "indexed"], ctx=ctx,
+                                        keep_batch=kept if DEVICE_HANDOFF else None)
+        for si, s in enumerate(samples):
+            if s.route in ("scan", "stream"):
+                try:
+                    evidence[si], profiles[si] = ingest_sample_scan(s, ctx=ctx)
+                except Exception as e:
+                    if s.route != "stream":
+                        raise
+                    samples[si] = s._replace(error=e)
     finally:
-        for h in handle_of.values():
-            if h is not None:
-                h.close()
-    for si in todo:
-        if si in failed:
+        for s in samples:
+            if s.handle is not None:
+                s.handle.close()
+    out, items, where = [], [], []
+    for si, s in enumerate(samples):
+        task = s.task
+        out.append({"samplekey": task.samplekey, "bam": task.bam, "tredCalls": s.pre, "_fields": {},
+                    "_names": s.wanted})
+        if s.error is not None:
+            logger.error("Sample `{}`: {}".format(task.samplekey, s.error))
+            out[si].update({"tredCalls": {}, "error": repr(s.error)})
             continue
-        samplekey, bam, repo, tredNames, maxinsert, fullsearch, clip, alts, repeatpairs, log = args[si]
-        gender, READLEN = out[si]["tredCalls"]["inferredGender"], out[si]["tredCalls"]["readLen"]
-        wanted = wanted_of[si]
-        evidence = got.get(si, {})
-        rest = [t for t in wanted if t not in evidence]
-        if rest and si not in streams:              # (a stream's bytes are gone: its missing loci get no call)
-            evidence.update(ingest_loci(bam, repo, rest, READLEN, alts, clip, logger, want_names=True))
-        for t in wanted:
-            if t in evidence:
-                items.append((repo[t], READLEN, gender, evidence[t].depth, evidence[t]))
+        if profiles.get(si) is not None:
+            out[si][STR_PROFILE] = profiles[si]
+        if s.route is None:
+            continue
+        got = evidence.get(si, {})
+        rest = [t for t in s.wanted if t not in got]
+        if rest and s.route != "stream":            # (a stream's bytes are gone: its missing loci get no call)
+            got.update(ingest_loci(task.bam, task.repo, rest, s.pre["readLen"], task.alts, task.clip, logger))
+        for t in s.wanted:
+            if t in got:
+                items.append((task.repo[t], s.pre["readLen"], s.pre["inferredGender"], got[t].depth, got[t]))
                 where.append((si, t))
     # the fused call can run on the ingest's device buffers when the items are exactly the problems of the batch
     device_batch = None
@@ -592,7 +584,7 @@ def prepare_chunk(args, only=None, ctx=None, str_profile=False):
         else:                                   # (some locus came from the host reader: assemble the batch on the host)
             items = [(it[0], it[1], it[2], it[3], _own_evidence(it[4])) for it in items]
             b.close()
-    return args, out, items, where, device_batch
+    return tasks, out, items, where, device_batch
 
 
 def _own_evidence(ev):
@@ -606,15 +598,15 @@ def finish_chunk(state, ctx=None):
     """Second half of ``run_chunk``: ONE fused device call for the loci of all the samples of the chunk, then the
     reference's per-locus JSON fields.
     :return: list of {"samplekey", "bam", "tredCalls"}"""
-    args, out, items, where, device_batch = state
-    if not args:
+    tasks, out, items, where, device_batch = state
+    if not tasks:
         return []
-    _, _, _, _, maxinsert, fullsearch, clip, _, repeatpairs, _ = args[0]
+    t = tasks[0]
     # all the loci in one call: on the ingest's own device buffers when the whole chunk came from the GPU ingest,
     # else from a batch assembled on the host
     try:
-        res = genotype_evidence(items, maxinsert=maxinsert, fullsearch=fullsearch, clip=clip, repeatpairs=repeatpairs,
-                                ctx=ctx, device_batch=device_batch)
+        res = genotype_evidence(items, maxinsert=t.maxinsert, fullsearch=t.fullsearch, clip=t.clip,
+                                repeatpairs=t.repeatpairs, ctx=ctx, device_batch=device_batch)
     finally:
         if device_batch is not None:
             device_batch.close()
@@ -663,10 +655,8 @@ def run_chunks(args, only=None, chunk=None, isolate=False, str_profile=False):
 
     def prep(k):
         a, b = spans[k]
-        if not str_profile:
-            return prepare_chunk(args[a:b], None if only is None else only[a:b], ctx=ictx)
         return prepare_chunk(args[a:b], None if only is None else only[a:b], ctx=ictx,
-                             str_profile=_per_sample(str_profile, len(args))[a:b])
+                             str_profile=str_profile if isinstance(str_profile, bool) else str_profile[a:b])
     try:
         with ThreadPoolExecutor(max_workers=1) as pool:
             fut = pool.submit(prep, 0)
@@ -980,7 +970,7 @@ def main(args):
     ngpus = max(1, args.gpus)
     if ngpus == 1:
         # chunks of samples: one fused device call per chunk (all loci of all its samples)
-        for results in (run_chunks(task_args, str_profile=True) if args.str_profile else run_chunks(task_args)):
+        for results in run_chunks(task_args, str_profile=args.str_profile):
             emit(results)
     else:
         import multiprocessing as mp
